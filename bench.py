@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - pruned-attention throughput of the MXINT8 exponent-sign hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -20,6 +20,11 @@ Multi-GPU (one process per GPU, torchrun): independent (batch, head) units, no d
 NCCL is used for the barrier, the max-over-ranks time and that verification gather only.
 roofline: the dominant kernel of the default call (the fused launch where it applies: algorithmic bytes 16 N hd
 per head, SURVEY 8(d)) + full_path_frac of the whole step + the per-kernel view of the three-kernel path.
+--dump-outputs DIR: after the timed steps, DIR/out.npy holds what the last timed step returned (rank 0), so that two
+builds run with the same arguments can be compared output for output (see dump_outputs).  For that, the last timed
+step writes every layer into an output buffer of its own: one extra (B,N,H,hd) fp32 tensor per layer on rank 0.
+--steps sets the step count of every GPU timing (main loop, per-kernel view, e2e, other workloads); cpu_baseline runs
+on a time budget (cpu_port_heads_per_s).
 """
 import argparse
 import json
@@ -45,6 +50,7 @@ LONG_WORKLOADS = {
     "dit_long_c5": dict(B=16, H=16, N=4096, hd=72, top_k=1024, layers=1, bfloat=32, flush=False),   # BASELINE.json configs[4], N = 4096
 }
 CPU_SAMPLE_B = 8          # cpu_baseline / reference arm: a B=8 slice of one layer (BASELINE.md 4)
+DUMP_BYTES = 64 * 10 ** 6  # --dump-outputs writes at most this many bytes
 
 
 def mx_specs(bfloat, flush):
@@ -126,6 +132,28 @@ class ClockSampler:
                 "samples": len(sm), "reasons": sorted(reasons)}
 
 
+def dump_outputs(path, outs):
+    """Write the fp32 (B,H,N,hd) outputs ``outs`` of one step (one per layer) to path/out.npy, float32
+    (layers, rows, hd), a row being one (batch, head, query) entry in that order.  When every row of every layer would
+    exceed DUMP_BYTES, each layer contributes the same rows: the first `keep` of torch.randperm(B*H*N) under a CPU
+    generator seeded with 0, ascending - fixed for a workload, so the files of two builds line up.  Returns the bytes."""
+    import numpy as np
+    import torch
+    B, H, N, hd = outs[0].shape
+    rows = B * H * N
+    keep = min(rows, (DUMP_BYTES - 4096) // (4 * hd * len(outs)))      # 4096: room for the .npy header
+    sel = None
+    if keep < rows:
+        sel = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    arr = np.empty((len(outs), keep, hd), dtype=np.float32)
+    for i, o in enumerate(outs):
+        flat = o.reshape(rows, hd)
+        arr[i] = (flat if sel is None else flat[sel.to(flat.device)]).cpu().numpy()
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "out.npy"), arr)
+    return arr.nbytes
+
+
 def cpu_port_heads_per_s(w, budget_s=12.0, threads=None):
     """The oracle port of the reference's CPU path (torch.topk left in place, as the reference
     does), all host threads, on a B=CPU_SAMPLE_B slice of one layer."""
@@ -177,14 +205,16 @@ def run_reference(args, name, w):
     q, k, v = (torch.randn(B, w["H"], w["N"], w["hd"], generator=g) for _ in range(3))
 
     def step():
-        O.pruned_attention(q, k, v, w["top_k"], bfloat=w["bfloat"], flush=w["flush"], use_torch_topk=True)
+        return O.pruned_attention(q, k, v, w["top_k"], bfloat=w["bfloat"], flush=w["flush"], use_torch_topk=True)
 
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        res = step()
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [res["out"]])
     heads = B * w["H"]
     val = heads / dt
     sample = f"each step = B={B} slice of one layer ({heads} heads) of {name}"
@@ -213,12 +243,17 @@ def make_layers(torch, w, dev, seed, batch_slice=None):
     return layers
 
 
-def time_steps(torch, step, steps, barrier):
+def time_steps(torch, step, steps, barrier, last_outs=None):
+    """Mean ms per step over `steps` steps.  last_outs: output buffers the last step writes in place of the step's own
+    (the same work; what --dump-outputs saves)."""
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     ev0.record()
-    for _ in range(steps):
-        step()
+    for i in range(steps):
+        if last_outs is not None and i == steps - 1:
+            step(last_outs)
+        else:
+            step()
     ev1.record()
     barrier()
     return ev0.elapsed_time(ev1) / steps
@@ -248,7 +283,8 @@ def kernel_breakdown(torch, mxq, layers, specs, top_k, out_view, reps):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of every GPU timing (cpu_baseline runs on a time budget of its own)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="deit_base_c2", choices=sorted(WORKLOADS))
@@ -257,7 +293,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-others", action="store_true", help="skip the device-timed lines of the other workload shapes")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/out.npy (float32; a fixed sample when over 64 MB); "
+                         "holds one extra output buffer per layer on the GPU for the whole run (deit_base_c2: 1.9 GB, "
+                         "dit_xl2_c3 / pixart_c4: 8.5 GB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     name, w = args.workload, WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, name, w)
@@ -300,10 +342,14 @@ def main():
     heads_per_step_total = (B if strong else world * B) * H * L
     out = torch.empty(Bl, N, H, hd, device=dev)     # (B,N,H,hd): the module's transpose(1,2) is free
     out_view = out.permute(0, 2, 1, 3)
+    # --dump-outputs: the last timed step writes each layer's output into a buffer of its own, laid out like `out`
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = [torch.empty(Bl, N, H, hd, device=dev).permute(0, 2, 1, 3) for _ in range(L)]
 
-    def step():
-        for (q, k, v) in layers:
-            mxq.pruned_attention(q, k, v, specs, top_k, out=out_view)
+    def step(outs=None):
+        for li, (q, k, v) in enumerate(layers):
+            mxq.pruned_attention(q, k, v, specs, top_k, out=out_view if outs is None else outs[li])
 
     sampler = ClockSampler(local)
     if rank == 0:
@@ -312,8 +358,8 @@ def main():
     for _ in range(W):
         step()
     launches_per_call = mxq.last_launch_count()
-    ms_per_step = time_steps(torch, step, args.steps, barrier)
-    kb = kernel_breakdown(torch, mxq, layers, specs, top_k, out_view, max(1, min(args.steps, 3))) if rank == 0 or world > 1 else None
+    ms_per_step = time_steps(torch, step, args.steps, barrier, dump)
+    kb = kernel_breakdown(torch, mxq, layers, specs, top_k, out_view, args.steps) if rank == 0 or world > 1 else None
     if rank == 0:
         # the timed region (a few tens of ms) can be shorter than one nvidia-smi period: keep the SAME
         # step loop running, untimed, until a few samples have been taken under that load
@@ -330,6 +376,9 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms_per_step = float(t.item())
     value = heads_per_step_total / (ms_per_step * 1e-3)
+    if dump is not None:
+        dump_outputs(args.dump_outputs, dump)
+        del dump
 
     # ---- strong scaling: cross-rank verification, outside every timed region.  Each rank digests the masks and the
     # outputs of its slice of layer 0; the digests are all_gathered (NCCL over NVLink) and rank 0 compares them with
@@ -396,7 +445,7 @@ def main():
             s_cmp.wait_stream(s_out)
 
         e2e_step()
-        ems = time_steps(torch, e2e_step, max(1, min(args.steps, 3)), barrier)
+        ems = time_steps(torch, e2e_step, args.steps, barrier)
         if world > 1:
             t = torch.tensor([ems], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -428,7 +477,7 @@ def main():
 
             for _ in range(3):
                 ostep()
-            oms = time_steps(torch, ostep, 3, barrier)
+            oms = time_steps(torch, ostep, args.steps, barrier)
             oh = ow["B"] * ow["H"] * ow["layers"]
             ob = bytes_per_head(ow["N"], ow["hd"])
             peak, _ = hbm_peak()

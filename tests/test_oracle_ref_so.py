@@ -1,8 +1,8 @@
 """Second, independent oracle for the quantizer (stage A2): the reference's OWN C++ device
 functions (microxscaling/mx/cpp/{shared_exp,quantize}.cuh) compiled into oracle/_ref/libmxref.so
 by oracle/ref_build/Makefile.  Checks the Python-path restatement (oracle/mxint8_oracle.py)
-against it; skipped when the .so was not built (it is built in the authoring container and
-travels with the repo snapshot)."""
+against it; skipped when the .so was not built.  The .so is not part of the repository: it can only be
+built where the reference's sources are at hand (oracle/ref_build/Makefile, REF = their mx/cpp directory)."""
 import ctypes
 import os
 
