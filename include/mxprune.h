@@ -289,8 +289,9 @@ int mxp_set_predict_path(int path);
  *                faster than the three kernels; the cost-follows-k attention kernel alone for smaller problems;
  *                everything else on the three-kernel path
  *   2            the fused launch wherever the shape is in its domain, dense epilogue included (tests, A/B)
- *   0            always the three-kernel path with the dense-epilogue attention kernels (A/B aid); for Nk > 256 also the
- *                round-1 attention kernel and the long-sequence selection with its radix levels alone (no sampled window)
+ *   0            always the three-kernel path with the dense-epilogue attention kernels (A/B aid); for Nk > 256, where
+ *                the attention kernel is the same in every mode, the long-sequence selection with its radix levels
+ *                alone (no sampled window)
  * Process-wide; returns MXP_E_BADARG for any other value.
  */
 int mxp_set_fused_path(int path);

@@ -49,12 +49,10 @@ inline int row_splits(int heads, int Nq) {
 }
 
 // ------------------------------------------------------------------------------------
-// K0a: standalone quantizer (codes / exps / sign words), one warp per row
+// K0a: standalone exponent-sign approximation (+-2^e per element, mxp_exp_sign_approx), one warp per row
 // ------------------------------------------------------------------------------------
-template <bool APPROX>
 __global__ void __launch_bounds__(THREADS)
 k_quantize(View x, int rows_per_bh, int H, int64_t total_rows, int hd, int bf16, int flush,
-           int8_t* __restrict__ codes, int8_t* __restrict__ exps, uint32_t* __restrict__ signs,
            float* __restrict__ approx) {
     const int lane = threadIdx.x & 31;
     const int nb = (hd + 31) >> 5;
@@ -68,16 +66,7 @@ k_quantize(View x, int rows_per_bh, int H, int64_t total_rows, int hd, int bf16,
             const float v = d < hd ? __ldg(xr + d) : 0.f;
             int e, ep;
             const int c = quantize_block_warp(v, bf16, flush, e, ep);
-            const uint32_t sw = __ballot_sync(FULL, c < 0);
-            if (APPROX) {
-                if (d < hd) approx[row * hd + d] = c < 0 ? -exp2i(ep) : exp2i(ep);
-            } else {
-                if (d < hd) codes[row * hd + d] = (int8_t)c;
-                if (lane == 0) {
-                    exps[row * nb + b] = (int8_t)e;
-                    if (signs) signs[row * nb + b] = sw;
-                }
-            }
+            if (d < hd) approx[row * hd + d] = c < 0 ? -exp2i(ep) : exp2i(ep);
         }
     }
 }
@@ -138,7 +127,7 @@ k_quantize_blocks(View x, int rows_per_bh, int H, int64_t total_rows, int hd, in
 // All warps of the CTA cooperate, one row per warp per step.
 template <int NB>
 __device__ __forceinline__ void stage_keys(const PredParams& p, int head, int nkp,
-                                           uint32_t* s_ksign, float* s_kw, bool write_k) {
+                                           uint32_t* s_ksign, float* s_kw) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int bb = head / p.H, hh = head % p.H;
     const float* kb = p.k.p + bb * p.k.sB + hh * p.k.sH;
@@ -154,11 +143,6 @@ __device__ __forceinline__ void stage_keys(const PredParams& p, int head, int nk
                 s_ksign[b * nkp + j] = sw;
                 s_kw[b * nkp + j] = j < p.Nk ? exp2i(ep) : 0.f;
             }
-            if (write_k && j < p.Nk) {
-                const int64_t row = (int64_t)head * p.Nk + j;
-                if (d < p.hd) p.k_codes[row * p.hd + d] = (int8_t)c;
-                if (lane == 0) p.k_exps[row * NB + b] = (int8_t)e;
-            }
         }
     }
 }
@@ -166,7 +150,6 @@ __device__ __forceinline__ void stage_keys(const PredParams& p, int head, int nk
 // Quantize one query row held by a warp: warp-uniform sign words and 2^e weights.
 template <int NB>
 __device__ __forceinline__ void quantize_query_row(const PredParams& p, const float* qrow,
-                                                   int64_t row, bool write_q,
                                                    uint32_t (&sq)[NB], float (&wq)[NB]) {
     const int lane = threadIdx.x & 31;
 #pragma unroll
@@ -177,10 +160,6 @@ __device__ __forceinline__ void quantize_query_row(const PredParams& p, const fl
         const int c = quantize_block_warp(x, p.bf16, p.flush, e, ep);
         sq[b] = __ballot_sync(FULL, c < 0);
         wq[b] = exp2i(ep);
-        if (write_q) {
-            if (d < p.hd) p.q_codes[row * p.hd + d] = (int8_t)c;
-            if (lane == 0) p.q_exps[row * NB + b] = (int8_t)e;
-        }
     }
 }
 
@@ -218,7 +197,7 @@ k_predict_scores(const PredParams p, int nkp) {
     float* s_kw = reinterpret_cast<float*>(s_ksign + NB * nkp);
     const int head = blockIdx.x;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    stage_keys<NB>(p, head, nkp, s_ksign, s_kw, false);
+    stage_keys<NB>(p, head, nkp, s_ksign, s_kw);
     __syncthreads();
     float c24[NB];
 #pragma unroll
@@ -229,7 +208,7 @@ k_predict_scores(const PredParams p, int nkp) {
         const int64_t row = (int64_t)head * p.Nq + i;
         uint32_t sq[NB];
         float wq[NB];
-        quantize_query_row<NB>(p, qb + (int64_t)i * p.q.sN, row, false, sq, wq);
+        quantize_query_row<NB>(p, qb + (int64_t)i * p.q.sN, sq, wq);
         for (int j = lane; j < p.Nk; j += 32) {
             uint32_t sk[NB];
             float wk[NB];
@@ -529,51 +508,39 @@ inline void prof_mark(int i, cudaStream_t st) {
     cudaEventRecord(g_ev[i], st);
 }
 
-int launch_attend_umma(const AttnParams& p, cudaStream_t st) {
+// Exact attention over the MMA-ready operands: Nk > 256 streams key blocks of 128 (k_attend_long_pair,
+// mxprune_attend_long.cuh), one key block runs k_attend_pair (two lanes per query row, 256 threads).
+int launch_attend(const AttnParams& p, cudaStream_t st) {
     const OpsLayout O = ops_layout(p.Nq, p.Nk, p.hd);
+    if (p.key_bias && !O.single)
+        return fail(MXP_E_UNSUPPORTED, "key_bias: the additive key bias is implemented for Nk <= 256 (cross-attention)");
+    if (!O.single) return launch_attend_long_pair(p, st);
     const K2Smem L = k2_smem_layout(O);
-    if (!O.single) {                // Nk > 256: two lanes per row, pipelined key-block stream (mxprune_attend_long.cuh)
-        int rc = MXP_OK;
-        if (attend_long_pair_try(p, st, &rc) == 0) return rc;
-    }
     MXP_ENSURE_DYN_SMEM((k_attend_pair<true, false>), 160 * 1024);
     MXP_ENSURE_DYN_SMEM((k_attend_pair<false, false>), 160 * 1024);
     MXP_ENSURE_DYN_SMEM((k_attend_pair<true, true>), 160 * 1024);
     MXP_ENSURE_DYN_SMEM((k_attend_pair<false, true>), 160 * 1024);
-    MXP_ENSURE_DYN_SMEM((k_attend_umma<false, true>), 160 * 1024);
-    MXP_ENSURE_DYN_SMEM((k_attend_umma<false, false>), 160 * 1024);
     if (L.total > 160 * 1024) return fail(MXP_E_UNSUPPORTED, "attention operands need %zu bytes of shared memory", L.total);
     const int heads = p.B * p.H;
     int splits = (148 * 2 + heads - 1) / heads;
-    // key blocks streamed per query tile (Nk > 256): a CTA holds nothing across tiles, so one CTA per tile costs
-    // nothing and fills the last wave (256 heads x 2 splits = 1.73 waves of 296 CTAs -> 27.7 waves)
-    if (!O.single) splits = O.q_tiles;
     if (splits > O.q_tiles) splits = O.q_tiles;
     if (splits < 1) splits = 1;
     dim3 grid((unsigned)heads, (unsigned)splits);
     // Never let more CTAs become resident on an SM than its 512 TMEM columns can serve: a CTA
     // whose tcgen05.alloc cannot be satisfied would sit blocked inside the allocator.  Residency is
     // bounded through the dynamic shared-memory request (227 KiB per SM).
-    const int tcols = O.single ? k2p_tmem_cols(O) : L.tmem_cols;
-    const int max_ctas = 512 / tcols;
+    const int max_ctas = 512 / k2p_tmem_cols(O);
     size_t dyn = L.total;
     const size_t floor_bytes = (size_t)232448 / (size_t)(max_ctas + 1) + 1024;
     if (dyn < floor_bytes) dyn = floor_bytes;
-    if (p.key_bias && !O.single)
-        return fail(MXP_E_UNSUPPORTED, "key_bias: the additive key bias is implemented for Nk <= 256 (cross-attention)");
-    if (O.single) {                 // one key block: two lanes per query row, 256 threads
-        if (p.key_bias) {
-            if (p.bf16) k_attend_pair<true, true><<<grid, K2P_T, dyn, st>>>(p);
-            else k_attend_pair<false, true><<<grid, K2P_T, dyn, st>>>(p);
-        } else {
-            if (p.bf16) k_attend_pair<true, false><<<grid, K2P_T, dyn, st>>>(p);
-            else k_attend_pair<false, false><<<grid, K2P_T, dyn, st>>>(p);
-        }
-    } else {                        // key blocks of 128 with online softmax, one thread per row
-        if (p.bf16) k_attend_umma<false, true><<<grid, K2T, dyn, st>>>(p);
-        else k_attend_umma<false, false><<<grid, K2T, dyn, st>>>(p);
+    if (p.key_bias) {
+        if (p.bf16) k_attend_pair<true, true><<<grid, K2P_T, dyn, st>>>(p);
+        else k_attend_pair<false, true><<<grid, K2P_T, dyn, st>>>(p);
+    } else {
+        if (p.bf16) k_attend_pair<true, false><<<grid, K2P_T, dyn, st>>>(p);
+        else k_attend_pair<false, false><<<grid, K2P_T, dyn, st>>>(p);
     }
-    return check_launch("k_attend_umma");
+    return check_launch("k_attend_pair");
 }
 
 int launch_prep_v(const View& v, int B, int H, int Nq, int Nk, int hd, int bf16, int flush, unsigned char* v_op,
@@ -641,7 +608,7 @@ static int try_predict_topk_tc(const PredParams& p, cudaStream_t st, int* rc_out
     if (splits > tiles) splits = tiles;
     if (splits < 1) splits = 1;
     dim3 grid((unsigned)heads, (unsigned)splits);
-    // residency bounded by the 512 TMEM columns of an SM (see launch_attend_umma)
+    // residency bounded by the 512 TMEM columns of an SM (see launch_attend)
     const int max_ctas = 512 / L.tmem_cols;
     size_t dyn = L.total;
     const size_t floor_bytes = (size_t)232448 / (size_t)(max_ctas + 1) + 1024;
@@ -888,7 +855,7 @@ static int quantize_common(const float* x, int64_t sB, int64_t sH, int64_t sN, i
     View v{x, sB, sH, sN};
     cudaStream_t st = (cudaStream_t)stream;
     if (approx) {
-        k_quantize<true><<<(unsigned)blocks, THREADS, 0, st>>>(v, N, H, rows, hd, bfloat_bits == 16, flush != 0, nullptr, nullptr, nullptr, approx);
+        k_quantize<<<(unsigned)blocks, THREADS, 0, st>>>(v, N, H, rows, hd, bfloat_bits == 16, flush != 0, approx);
         return check_launch("k_quantize");
     }
     const int nb = (hd + 31) / 32;
@@ -1058,7 +1025,7 @@ int mxp_sparse_attention(const int8_t* q_codes, const int8_t* q_exps, const int8
     p.B = B; p.H = H; p.Nq = Nq; p.Nk = Nk; p.hd = hd;
     p.scale = scale; p.bf16 = bfloat_bits == 16; p.flush = flush != 0;
     p.out = out; p.o_sB = o_sB; p.o_sH = o_sH; p.o_sN = o_sN;
-    return launch_attend_umma(p, st);
+    return launch_attend(p, st);
 }
 
 size_t mxp_pruned_attention_workspace_bytes(int B, int H, int Nq, int Nk, int hd) {
@@ -1149,7 +1116,7 @@ static int pruned_attention_impl(const float* q, int64_t q_sB, int64_t q_sH, int
         ap.key_bias = key_bias; ap.kb_sB = kb_sB;
         int rc2 = MXP_OK;
         if (attend_sparse_try(ap, top_k, st, &rc2) == 0) rc = rc2;      // cost follows top_k (small top_k / Nk)
-        else rc = launch_attend_umma(ap, st);
+        else rc = launch_attend(ap, st);
         prof_mark(3, st);
         return rc;
     }

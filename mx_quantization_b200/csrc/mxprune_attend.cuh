@@ -1,4 +1,5 @@
-// K2: exact MXINT8 attention over the kept keys on the Blackwell tensor cores (any Nk).
+// K2: exact MXINT8 attention over the kept keys on the Blackwell tensor cores - the MMA-ready operand layout every
+// exact-attention kernel reads, and the one-key-block kernel k_attend_pair (Nk <= 256).
 //
 // Key fact: every MXINT8 value c * 2^(e-6) (|c| <= 127) is EXACTLY representable in bf16 (8
 // significant bits, fp32 exponent range).  So both contractions of the reference,
@@ -15,15 +16,12 @@
 // (matmul.py:76-83).  K2 therefore stages with TMA bulk copies (cp.async.bulk + mbarrier
 // complete_tx) and spends its instructions on the softmax / P-quantisation epilogue only.
 //
-// One CTA (128 threads) per (head, row split); thread t owns query row t of the tile == TMEM
-// lane t, so the epilogue needs no cross-thread communication.
-//   Nk <= 256  one key block: S = Q.K^T (hd/16 MMAs, N = Nk) -> TMEM; pass A max over kept keys;
-//              pass B E = exp(s - max) (0 where pruned) written back over S, row sum; pass C
-//              P = E/sum -> A1 -> MXINT8 per 32-key window -> bf16 A operand, O += P_w.V_w
-//              (O reuses the TMEM columns of windows already consumed).
-//   Nk  > 256  key blocks of 128: pass 1 streams the blocks with an online max/sum, pass 2
-//              streams them again (S recomputed by the tensor core) to form P and accumulate O
-//              in its own TMEM columns.
+// Nk <= 256 (k_attend_pair): one key block, the head's K and V operands resident in shared memory.  Per query tile
+// S = Q.K^T (hd/16 MMAs, N = Nk) -> TMEM; pass A max over the kept keys; pass B E = exp(t - max) (0 where pruned)
+// written back over S, row sum; pass C P = E/sum -> A1 -> MXINT8 per 32-key window -> bf16 A operand, O += P_w.V_w
+// (O reuses the TMEM columns of windows already consumed).  k_attend_sparse (mxprune_attend_sparse.cuh) runs the same
+// stages on compacted row lists when top_k is small; Nk > 256 streams key blocks of 128 through k_attend_long_pair
+// (mxprune_attend_long.cuh).
 #pragma once
 #include "mxprune_device.cuh"
 #include "mxprune_umma.cuh"
@@ -31,8 +29,7 @@
 namespace mxp {
 
 constexpr int K2T = 128;
-constexpr int K2_PW = 4;                           // P windows buffered per MMA group (4 x 32 keys)
-constexpr int K2_P_BYTES = K2_PW * 4 * K2T * 16;   // 32 KiB
+constexpr int K2_P_BYTES = 4 * 4 * K2T * 16;       // P operand of one MMA group of four 32-key windows: 32 KiB
 constexpr int K2_SINGLE_MAX = 256;                 // largest Nk handled as one key block
 
 struct AttnParams {
@@ -85,16 +82,12 @@ __host__ __device__ inline size_t v_op_offset(const OpsLayout& L, int tc, int d)
     return (size_t)blk * L.v_blk_bytes + ((size_t)tl * L.hdp + d) * 16;
 }
 
+// shared memory of the one-key-block kernels: the head's K and V operands, then the P window group
 struct K2Smem {
-    int tmem_cols;
     size_t off_v, off_p, total;
 };
 __host__ __device__ inline K2Smem k2_smem_layout(const OpsLayout& O) {
     K2Smem L;
-    int need = O.single ? (O.kb_rows > O.hdp ? O.kb_rows : O.hdp) : 256;
-    int c = 32;
-    while (c < need) c <<= 1;
-    L.tmem_cols = c;
     size_t o = O.k_blk_bytes;
     L.off_v = o; o += O.v_blk_bytes;
     L.off_p = o; o += K2_P_BYTES;                    // P window group; also the Q tile (<= 32 KiB)
@@ -111,305 +104,6 @@ __device__ __forceinline__ void tma_bulk_g2s(void* dst_smem, const void* src_gme
                      smem_u32(dst_smem)),
                  "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
-}
-
-// r[w] for a runtime w without dynamic register indexing (a 3-level select tree)
-__device__ __forceinline__ uint32_t pick8(const uint32_t (&r)[8], int w) {
-    const uint32_t a = (w & 1) ? r[1] : r[0], b = (w & 1) ? r[3] : r[2];
-    const uint32_t c = (w & 1) ? r[5] : r[4], d = (w & 1) ? r[7] : r[6];
-    const uint32_t ab = (w & 2) ? b : a, cd = (w & 2) ? d : c;
-    return (w & 4) ? cd : ab;
-}
-
-template <bool SINGLE, bool BF16>   // SINGLE: Nk <= 256, one key block (else blocks of 128, online softmax); BF16: A1 rounding on
-__global__ void __launch_bounds__(K2T)
-k_attend_umma(const AttnParams p) {
-    extern __shared__ __align__(128) unsigned char smem[];
-    __shared__ uint64_t bar_ld, bar_s, bar_o;
-    __shared__ uint32_t tmem_base_s;
-    const int Nk = p.Nk, Nq = p.Nq, hd = p.hd;
-    const OpsLayout O = ops_layout(Nq, Nk, hd);
-    const K2Smem L = k2_smem_layout(O);
-    const int hdp = O.hdp, NW = O.nw, kbr = O.kb_rows;
-    constexpr bool single = SINGLE;
-    unsigned char* sK = smem;
-    unsigned char* sV = smem + L.off_v;
-    unsigned char* sP = smem + L.off_p;
-    const int head = blockIdx.x, bb = head / p.H, hh = head % p.H;
-    const int tid = threadIdx.x, warp = tid >> 5;
-    constexpr bool bf16 = BF16;
-    const bool flush = p.flush;
-    const unsigned char* q_op = p.q_op + (size_t)head * O.q_head_bytes;
-    const unsigned char* k_op = p.k_op + (size_t)head * O.k_head_bytes;
-    const unsigned char* v_op = p.v_op + (size_t)head * O.v_head_bytes;
-
-    if (tid == 0) { mbar_init(&bar_ld, 1); mbar_init(&bar_s, 1); mbar_init(&bar_o, 1); }
-    if (warp == 0) tmem_alloc(&tmem_base_s, (uint32_t)L.tmem_cols);
-    tcgen05_fence_before_sync();
-    __syncthreads();
-    tcgen05_fence_after_sync();
-    const uint32_t tmem = tmem_base_s;
-    const uint32_t my_tmem = tmem + ((uint32_t)(warp * 32) << 16);      // this warp's 32 lanes
-    const uint32_t o_col = single ? 0u : 128u;
-    const uint32_t idesc_s = umma_idesc_bf16_f32(128, kbr);
-    const uint32_t idesc_o = umma_idesc_bf16_f32(128, hdp);
-    uint32_t ph_ld = 0, ph_s = 0, ph_o = 0;
-
-    if (single) {                                  // the head's K and V operands stay resident
-        if (tid == 0) {
-            mbar_expect_tx(&bar_ld, (uint32_t)(O.k_blk_bytes + O.v_blk_bytes));
-            tma_bulk_g2s(sK, k_op, (uint32_t)O.k_blk_bytes, &bar_ld);
-            tma_bulk_g2s(sV, v_op, (uint32_t)O.v_blk_bytes, &bar_ld);
-        }
-        mbar_wait(&bar_ld, ph_ld);
-        ph_ld ^= 1u;
-    }
-
-    for (int tile = blockIdx.y; tile < O.q_tiles; tile += gridDim.y) {
-        const int i = tile * K2T + tid;
-        const bool valid = i < Nq;
-        const int64_t row = (int64_t)head * Nq + (valid ? i : 0);
-        const uint32_t* mrow = p.mask + row * NW;
-
-        // ---- Q tile (A operand) -> the P buffer region, by TMA
-        if (tid == 0) {
-            mbar_expect_tx(&bar_ld, (uint32_t)O.q_tile_bytes);
-            tma_bulk_g2s(sP, q_op + (size_t)tile * O.q_tile_bytes, (uint32_t)O.q_tile_bytes, &bar_ld);
-        }
-        mbar_wait(&bar_ld, ph_ld);
-        ph_ld ^= 1u;
-
-        float m = -INFINITY, l = 0.f;
-        // =============== pass 1: row max and sum of exp over the kept keys
-        for (int blk = 0; blk < O.nblk; ++blk) {
-            const int wbase = blk * O.wpb, nwb = min(O.wpb, NW - wbase);
-            if (!single) {
-                if (tid == 0) {
-                    mbar_expect_tx(&bar_ld, (uint32_t)O.k_blk_bytes);
-                    tma_bulk_g2s(sK, k_op + (size_t)blk * O.k_blk_bytes, (uint32_t)O.k_blk_bytes, &bar_ld);
-                }
-                mbar_wait(&bar_ld, ph_ld);
-                ph_ld ^= 1u;
-            }
-            if (tid == 0) {
-                tcgen05_fence_after_sync();
-                for (int ks = 0; ks < (hdp >> 4); ++ks) {
-                    const uint64_t da = umma_smem_desc(smem_u32(sP + (size_t)(2 * ks) * K2T * 16), K2T * 16, 128);
-                    const uint64_t db = umma_smem_desc(smem_u32(sK + (size_t)(2 * ks) * kbr * 16), kbr * 16, 128);
-                    umma_bf16_ss(tmem, da, db, idesc_s, ks > 0);
-                }
-                umma_commit(&bar_s);
-            }
-            uint32_t mreg[8];
-#pragma unroll
-            for (int w = 0; w < 8; ++w) mreg[w] = (valid && w < nwb) ? __ldg(mrow + wbase + w) : 0u;
-            mbar_wait(&bar_s, ph_s);
-            ph_s ^= 1u;
-            tcgen05_fence_after_sync();
-
-            // pass A (A7: bf16 rounding of the matmul output, * scale)
-            float mb4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};   // 4 chains: no serial dependency
-            for (int w = 0; w < nwb; ++w) {
-                const uint32_t mw = pick8(mreg, w);
-                uint32_t r[32];
-                tmem_ld_32x32b_x32(my_tmem + w * 32, r);
-                tmem_ld_wait();
-#pragma unroll
-                for (int c = 0; c < 32; ++c) {
-                    float s = __uint_as_float(r[c]);
-                    if (bf16) s = bf16_half_away(s);
-                    const float tv = __fmul_rn(s, p.scale);
-                    mb4[c & 3] = fmaxf(mb4[c & 3], ((mw >> c) & 1u) ? tv : -INFINITY);
-                }
-            }
-            const float mb = fmaxf(fmaxf(mb4[0], mb4[1]), fmaxf(mb4[2], mb4[3]));
-            const float m_new = fmaxf(m, mb);
-            const float m_use = (m_new == -INFINITY) ? 0.f : m_new;     // no kept key so far
-            if (m != -INFINITY) l *= exp_nonpos(m - m_use);
-            // pass B: exp(t - m) on kept keys; single block: written back over S for pass 2
-            float sum4[4] = {0.f, 0.f, 0.f, 0.f};
-            for (int w = 0; w < nwb; ++w) {
-                const uint32_t mw = pick8(mreg, w);
-                uint32_t r[32];
-                tmem_ld_32x32b_x32(my_tmem + w * 32, r);
-                tmem_ld_wait();
-#pragma unroll
-                for (int c = 0; c < 32; ++c) {
-                    float s = __uint_as_float(r[c]);
-                    if (bf16) s = bf16_half_away(s);
-                    // evaluated for every position (branch-free), zeroed where the key is pruned
-                    const float ex = exp_nonpos(__fsub_rn(__fmul_rn(s, p.scale), m_use));
-                    const float ev = ((mw >> c) & 1u) ? ex : 0.f;
-                    sum4[c & 3] += ev;
-                    r[c] = __float_as_uint(ev);
-                }
-                if (single) tmem_st_32x32b_x32(my_tmem + w * 32, r);
-            }
-            if (single) tmem_st_wait();
-            l += (sum4[0] + sum4[1]) + (sum4[2] + sum4[3]);
-            m = m_new;
-            if (!single) {                          // S columns and sK are reused by the next block
-                tcgen05_fence_before_sync();
-                __syncthreads();
-                tcgen05_fence_after_sync();
-            }
-        }
-        const float m_fin = (m == -INFINITY) ? 0.f : m;
-        const float inv = l > 0.f ? 1.0f / l : 0.f;
-
-        // =============== pass 2: P = E/sum -> A1 -> MXINT8 per window -> bf16; O += P_w . V_w
-        bool first_mma = true;
-        for (int blk = 0; blk < O.nblk; ++blk) {
-            const int wbase = blk * O.wpb, nwb = min(O.wpb, NW - wbase);
-            uint32_t mreg[8];
-#pragma unroll
-            for (int w = 0; w < 8; ++w) mreg[w] = 0u;
-            if (!single) {
-                if (blk > 0) {                      // previous block's P.V MMAs are done with sP / sV
-                    mbar_wait(&bar_o, ph_o);
-                    ph_o ^= 1u;
-                }
-                if (tid == 0) {
-                    const bool need_q = true;       // sP was overwritten by P: re-fetch the Q tile
-                    mbar_expect_tx(&bar_ld, (uint32_t)(O.k_blk_bytes + O.v_blk_bytes + (need_q ? O.q_tile_bytes : 0)));
-                    tma_bulk_g2s(sK, k_op + (size_t)blk * O.k_blk_bytes, (uint32_t)O.k_blk_bytes, &bar_ld);
-                    tma_bulk_g2s(sV, v_op + (size_t)blk * O.v_blk_bytes, (uint32_t)O.v_blk_bytes, &bar_ld);
-                    tma_bulk_g2s(sP, q_op + (size_t)tile * O.q_tile_bytes, (uint32_t)O.q_tile_bytes, &bar_ld);
-                }
-#pragma unroll
-                for (int w = 0; w < 8; ++w) mreg[w] = (valid && w < nwb) ? __ldg(mrow + wbase + w) : 0u;
-                mbar_wait(&bar_ld, ph_ld);
-                ph_ld ^= 1u;
-                if (tid == 0) {
-                    tcgen05_fence_after_sync();
-                    for (int ks = 0; ks < (hdp >> 4); ++ks) {
-                        const uint64_t da = umma_smem_desc(smem_u32(sP + (size_t)(2 * ks) * K2T * 16), K2T * 16, 128);
-                        const uint64_t db = umma_smem_desc(smem_u32(sK + (size_t)(2 * ks) * kbr * 16), kbr * 16, 128);
-                        umma_bf16_ss(tmem, da, db, idesc_s, ks > 0);
-                    }
-                    umma_commit(&bar_s);
-                }
-                mbar_wait(&bar_s, ph_s);            // S ready AND the Q tile in sP has been consumed
-                ph_s ^= 1u;
-                tcgen05_fence_after_sync();
-            }
-            for (int g0 = 0; g0 < nwb; g0 += K2_PW) {
-                if (g0 > 0) {                       // previous group's MMAs have finished reading sP
-                    mbar_wait(&bar_o, ph_o);
-                    ph_o ^= 1u;
-                }
-                const int g1 = min(g0 + K2_PW, nwb);
-                for (int w = g0; w < g1; ++w) {
-                    const uint32_t mw = pick8(mreg, w);
-                    uint32_t r[32];
-                    tmem_ld_32x32b_x32(my_tmem + w * 32, r);
-                    tmem_ld_wait();
-                    uint32_t mx4[4] = {0u, 0u, 0u, 0u};
-#pragma unroll
-                    for (int c = 0; c < 32; ++c) {
-                        float ev = __uint_as_float(r[c]);
-                        if (!single) {
-                            if (bf16) ev = bf16_half_away(ev);
-                            const float ex = exp_nonpos(__fsub_rn(__fmul_rn(ev, p.scale), m_fin));
-                            ev = ((mw >> c) & 1u) ? ex : 0.f;
-                        }
-                        uint32_t pb = __float_as_uint(ev * inv);
-                        if (bf16) pb = bf16_half_away(pb);
-                        r[c] = pb;
-                        mx4[c & 3] = max(mx4[c & 3], pb);      // p >= 0: bit patterns order like the values
-                    }
-                    const uint32_t mx = max(max(mx4[0], mx4[1]), max(mx4[2], mx4[3]));
-                    const int e = mx_shared_exp(mx);
-                    const bool dead = (flush && e <= -127) || mx == 0u;
-                    unsigned char* pdst = sP + ((size_t)((w - g0) * 4) * K2T + tid) * 16;
-                    if (single && (dead || e >= -120)) {
-                        // p >= 0.  code = min(127, floor(p * 2^(6-e) + 0.5)) without F2I / I2F: the
-                        // add rounded toward -inf against 2^23 + 0x4300 leaves the bf16 pattern of
-                        // 128 + code in the low 16 bits; (128 + code) * w - 128 * w = code * w exactly.
-                        // A dead window (no kept key / flushed) runs the same code with scale 0: code 0.
-                        const int ec = max(e, -120);
-                        const float s1 = dead ? 0.f : exp2i(6 - ec);
-                        const __nv_bfloat162 w2 = u32_as_bf2(bf16_pow2_bits(ec - 6) * 0x00010001u);
-                        const __nv_bfloat162 nw2 = u32_as_bf2((bf16_pow2_bits(ec + 1) | 0x8000u) * 0x00010001u);
-#pragma unroll
-                        for (int q = 0; q < 4; ++q) {
-                            uint32_t ow[4];
-#pragma unroll
-                            for (int h = 0; h < 4; ++h) {
-                                const float v0 = fminf(fmaf(__uint_as_float(r[q * 8 + 2 * h]), s1, 0.5f), 127.0f);
-                                const float v1 = fminf(fmaf(__uint_as_float(r[q * 8 + 2 * h + 1]), s1, 0.5f), 127.0f);
-                                const uint32_t v2 = __byte_perm(__float_as_uint(__fadd_rd(v0, 8405760.0f)),
-                                                                __float_as_uint(__fadd_rd(v1, 8405760.0f)), 0x5410);
-                                ow[h] = bf2_as_u32(__hfma2(u32_as_bf2(v2), w2, nw2));
-                            }
-                            *reinterpret_cast<uint4*>(pdst + (size_t)q * K2T * 16) = make_uint4(ow[0], ow[1], ow[2], ow[3]);
-                        }
-                    } else {
-                        const float s1 = exp2i(-e), wgt = exp2i(e - 6);
-#pragma unroll
-                        for (int q = 0; q < 4; ++q) {
-                            float f[8];
-#pragma unroll
-                            for (int t = 0; t < 8; ++t) {
-                                const float rr = __uint_as_float(r[q * 8 + t]) * s1 * 64.0f + 0.5f;
-                                const int c = dead ? 0 : min(__float2int_rz(rr), 127);
-                                f[t] = (float)c * wgt;
-                            }
-                            *reinterpret_cast<uint4*>(pdst + (size_t)q * K2T * 16) =
-                                make_uint4(pack_bf16_trunc(f[0], f[1]), pack_bf16_trunc(f[2], f[3]),
-                                           pack_bf16_trunc(f[4], f[5]), pack_bf16_trunc(f[6], f[7]));
-                        }
-                    }
-                }
-                fence_proxy_async_smem();
-                tcgen05_fence_before_sync();
-                __syncthreads();
-                if (tid == 0) {
-                    tcgen05_fence_after_sync();
-                    for (int w = g0; w < g1; ++w)
-#pragma unroll
-                        for (int h = 0; h < 2; ++h) {
-                            const uint64_t da = umma_smem_desc(
-                                smem_u32(sP + (size_t)((w - g0) * 4 + 2 * h) * K2T * 16), K2T * 16, 128);
-                            const uint64_t db = umma_smem_desc(
-                                smem_u32(sV + (size_t)(w * 4 + 2 * h) * hdp * 16), hdp * 16, 128);
-                            umma_bf16_ss(tmem + o_col, da, db, idesc_o, !first_mma);
-                            first_mma = false;
-                        }
-                    umma_commit(&bar_o);
-                }
-            }
-        }
-        mbar_wait(&bar_o, ph_o);
-        ph_o ^= 1u;
-        tcgen05_fence_after_sync();
-
-        // ---- O -> A1 -> global (thread t writes row t)
-        float* orow = p.out + bb * p.o_sB + hh * p.o_sH + (int64_t)(valid ? i : 0) * p.o_sN;
-        for (int c0 = 0; c0 < hdp; c0 += 16) {
-            uint32_t r[16];
-            tmem_ld_32x32b_x16(my_tmem + o_col + c0, r);
-            tmem_ld_wait();
-            if (valid) {
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    if (c0 + q * 4 < hd) {
-                        float4 o = make_float4(__uint_as_float(r[q * 4]), __uint_as_float(r[q * 4 + 1]),
-                                               __uint_as_float(r[q * 4 + 2]), __uint_as_float(r[q * 4 + 3]));
-                        if (bf16) {
-                            o.x = bf16_half_away(o.x); o.y = bf16_half_away(o.y);
-                            o.z = bf16_half_away(o.z); o.w = bf16_half_away(o.w);
-                        }
-                        *reinterpret_cast<float4*>(orow + c0 + q * 4) = o;
-                    }
-                }
-            }
-        }
-        tcgen05_fence_before_sync();
-        __syncthreads();                        // every lane has read O before TMEM / sP are reused
-        tcgen05_fence_after_sync();
-    }
-    if (warp == 0) tmem_dealloc(tmem, (uint32_t)L.tmem_cols);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -1,10 +1,7 @@
 // K2-long-pair: exact MXINT8 attention over the kept keys for Nk > 256 (config C5, the sequence-length sweep) with TWO
-// LANES PER QUERY ROW and a pipelined key-block stream.
-//
-// k_attend_umma<SINGLE = false> (mxprune_attend.cuh) walks the key blocks with one thread per query row, 128 threads
-// per CTA and everything in series (TMA of a block -> wait -> MMA -> wait -> epilogue): 8 warps per SM - the TMEM
-// budget allows two CTAs - and every latency exposed (ncu at N = 4096: 11 % warps active, issue slots 53 % busy).
-// Same arithmetic here, 256 threads per CTA:
+// LANES PER QUERY ROW and a pipelined key-block stream.  The key blocks of 128 (OpsLayout) are streamed twice per query
+// tile: pass 1 forms the row maximum and sum with an online softmax, pass 2 recomputes S on the tensor core to form P
+// and accumulate O in its own TMEM columns.  256 threads per CTA, two CTAs per SM (256 TMEM columns each):
 //   * a warp owns 16 query rows (TMEM lanes), lanes l and l + 16 share row l; of a block's four 32-key windows lane
 //     half h takes windows 2h and 2h + 1 (tcgen05.ld.16x32bx2, column split 64).  Each lane keeps its own running
 //     maximum / sum over its columns; the row's two halves are combined once, after the last block.
@@ -15,7 +12,7 @@
 //     keeps its own region (no re-fetch per block), V blocks are double-buffered, K(blk + 1) is fetched as soon as
 //     S(blk) is complete and S(blk + 1) is issued right behind the P.V MMAs of block blk.
 // Reference semantics: workloads/DiT/models.py:168-225 at N > 256 (gather -> softmax over the kept keys -> scatter ->
-// mx.matmul(attn, v)), as k_attend_umma.
+// mx.matmul(attn, v)), as k_attend_pair for Nk <= 256.
 #pragma once
 #include "mxprune_attend.cuh"
 
@@ -317,8 +314,8 @@ k_attend_long_pair(const AttnParams p) {
     if (warp == 0) tmem_dealloc(tmem, 256u);
 }
 
-// defined in mxprune_long.cu: returns 1 when the shape is outside this kernel's domain (the caller falls back to
-// k_attend_umma), else 0 with the launch status in *rc_out
-int attend_long_pair_try(const AttnParams& p, cudaStream_t st, int* rc_out);
+// defined in mxprune_long.cu: launches k_attend_long_pair, returns the status (MXP_E_UNSUPPORTED when the layout does
+// not fit the kernel's shared memory)
+int launch_attend_long_pair(const AttnParams& p, cudaStream_t st);
 
 }  // namespace mxp

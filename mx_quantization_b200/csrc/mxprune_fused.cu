@@ -28,7 +28,7 @@ int attend_sparse_try(const AttnParams& p, int top_k, cudaStream_t st, int* rc_o
         if (splits > O.q_tiles) splits = O.q_tiles;
         if (splits < 1) splits = 1;
         dim3 grid((unsigned)heads, (unsigned)splits);
-        // residency bounded by the 512 TMEM columns of an SM (see launch_attend_umma)
+        // residency bounded by the 512 TMEM columns of an SM (see launch_attend)
         const int max_ctas = 512 / k2p_tmem_cols(O);
         size_t dyn = L.total;
         const size_t floor_bytes = SMEM_PER_SM / (size_t)(max_ctas + 1) + 1024;

@@ -11,27 +11,25 @@
 
 namespace mxp {
 
-int attend_long_pair_try(const AttnParams& p, cudaStream_t st, int* rc_out) {
+int launch_attend_long_pair(const AttnParams& p, cudaStream_t st) {
     const OpsLayout O = ops_layout(p.Nq, p.Nk, p.hd);
-    // domain: streamed key blocks, no additive bias; path switch 0 (mxp_set_fused_path) keeps the round-1 kernel for A/B
-    if (g_fused_path.load() == 0 || O.single || p.key_bias) return 1;
     const KLPSmem L = klp_smem_layout(O);
-    if (O.k_blk_bytes != O.v_blk_bytes || L.total > SMEM_PER_SM - 2048) return 1;
-    auto run = [&]() -> int {
-        MXP_ENSURE_DYN_SMEM((k_attend_long_pair<true>), (int)(SMEM_PER_SM - 2048));
-        MXP_ENSURE_DYN_SMEM((k_attend_long_pair<false>), (int)(SMEM_PER_SM - 2048));
-        // one CTA per query tile (a CTA holds nothing across tiles); 256 TMEM columns per CTA: at most two CTAs per SM,
-        // which the dynamic shared-memory request enforces (see launch_attend_umma)
-        dim3 grid((unsigned)((size_t)p.B * p.H * O.q_tiles));
-        size_t dyn = L.total;
-        const size_t floor_bytes = SMEM_PER_SM / 3 + 1024;
-        if (dyn < floor_bytes) dyn = floor_bytes;
-        if (p.bf16) k_attend_long_pair<true><<<grid, K2P_T, dyn, st>>>(p);
-        else k_attend_long_pair<false><<<grid, K2P_T, dyn, st>>>(p);
-        return check_launch("k_attend_long_pair");
-    };
-    *rc_out = run();
-    return 0;
+    // pass 1 uses V buffer 0 as its second K buffer; with key blocks of 128 rows both blocks are 256 hdp bytes and the
+    // layout is at most 160 KiB (hd = 128), so these hold for every supported head_dim
+    if (O.k_blk_bytes != O.v_blk_bytes || L.total > SMEM_PER_SM - 2048)
+        return fail(MXP_E_UNSUPPORTED, "head_dim %d: the long-sequence attention kernel needs K / V blocks of equal size "
+                    "(%zu / %zu bytes) and %zu bytes of shared memory", p.hd, O.k_blk_bytes, O.v_blk_bytes, L.total);
+    MXP_ENSURE_DYN_SMEM((k_attend_long_pair<true>), (int)(SMEM_PER_SM - 2048));
+    MXP_ENSURE_DYN_SMEM((k_attend_long_pair<false>), (int)(SMEM_PER_SM - 2048));
+    // one CTA per query tile (a CTA holds nothing across tiles); 256 TMEM columns per CTA: at most two CTAs per SM,
+    // which the dynamic shared-memory request enforces (see launch_attend)
+    dim3 grid((unsigned)((size_t)p.B * p.H * O.q_tiles));
+    size_t dyn = L.total;
+    const size_t floor_bytes = SMEM_PER_SM / 3 + 1024;
+    if (dyn < floor_bytes) dyn = floor_bytes;
+    if (p.bf16) k_attend_long_pair<true><<<grid, K2P_T, dyn, st>>>(p);
+    else k_attend_long_pair<false><<<grid, K2P_T, dyn, st>>>(p);
+    return check_launch("k_attend_long_pair");
 }
 
 }  // namespace mxp

@@ -74,9 +74,9 @@ def set_predict_path(path: str) -> None:
 def set_fused_path(mode) -> None:
     """True / 1 (default): the round-2 launch plans where they are measured faster - the fused one-launch kernel (DeiT-shaped
     calls: 129-256 keys staged in 128-row steps, top_k / Nk <= 0.35), the cost-follows-k attention kernel (Nk <= 256, same
-    bound), the two-lanes-per-row kernel for Nk > 256 and the sampled fine window of the long-sequence selection; 2: the fused launch
-    wherever the shape is in its domain; False / 0: always the three kernels of round 1 with the dense epilogue, the long-sequence
-    selection on its radix levels alone.  Results agree (A/B aid)."""
+    bound) and the sampled fine window of the long-sequence selection; 2: the fused launch wherever the shape is in its domain;
+    False / 0: always the three kernels with the dense epilogue, and for Nk > 256 the long-sequence selection on its radix
+    levels alone (the attention kernel for Nk > 256 is the same in every mode).  Results agree (A/B aid)."""
     _lib.check(_lib.load().mxp_set_fused_path(int(mode)), "mxp_set_fused_path")
 
 

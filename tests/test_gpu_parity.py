@@ -424,6 +424,8 @@ LONG_SHAPES = [  # B, H, N, hd, bfloat  -- key counts beyond one key block (Nk >
     (1, 1, 1000, 64, 32),
     (1, 2, 300, 72, 16),
     (1, 1, 2048, 72, 32),
+    (1, 1, 600, 128, 32),      # head_dim 128: the largest shared-memory layout of the long-sequence kernel
+    (1, 2, 400, 40, 16),       # head_dim 40: operands padded to 48
 ]
 
 
@@ -440,6 +442,27 @@ def test_exact_attention_long_sequences(mxq, B, H, N, hd, bfloat):
                                ref["k_exps"].cuda(), v.cuda(), mask_i32.cuda(), specs,
                                scale=O.default_scale(hd)).cpu()
     assert_out_close(out, ref, v, N, bfloat, OUT_TOL)
+
+
+@pytest.mark.parametrize("kfrac", [0.1, 0.5])
+@pytest.mark.parametrize("bfloat", [16, 32])
+@pytest.mark.parametrize("hd", [64, 72, 128])
+@pytest.mark.parametrize("N", [300, 1000])
+def test_long_attention_same_in_every_fused_mode(mxq, N, hd, bfloat, kfrac):
+    """Nk > 256: fused path 0 changes only how the selection finds a row's threshold (same masks), not the attention
+    kernel - masks and outputs are bit-identical to the default's."""
+    top_k = max(1, int(kfrac * N))
+    q, k, v = (t.cuda() for t in make_qkv(1, 2, N, hd, seed=9))
+    specs = mx_specs(bfloat, False)
+    res = {}
+    try:
+        for mode in (0, 1):
+            mxq.set_fused_path(mode)
+            res[mode] = mxq.pruned_attention(q, k, v, specs, top_k, return_mask=True)
+    finally:
+        mxq.set_fused_path(True)
+    assert torch.equal(res[0][1], res[1][1])
+    assert torch.equal(res[0][0], res[1][0])
 
 
 @pytest.mark.parametrize("B,H,N,hd,kind,bfloat,kfrac", [
