@@ -16,6 +16,16 @@
  *   - plain contiguous (B,H,N,hd)       benchmarks / tests
  * Requirements: hd % 4 == 0, 4 <= hd <= 128, base pointers and row strides 16-byte aligned.
  *
+ * 16-bit activations (the *_dt entry points, MXP_DT_BF16 / MXP_DT_F16): q, k and v share one element type, and the
+ * result is the result of the same call on the exactly widened fp32 values - identical masks, indices, codes and
+ * exponents, and the same fp32 output before its final store.  A1 (bfloat 16) and the subnormal flush act on the
+ * widened values.  out is fp32 or the input type; a 16-bit out is the fp32 result rounded to nearest even.  There is
+ * no conversion pass: a 16-bit call enqueues the launches of the fp32 call of the same shape and needs the same
+ * workspace.  Views: strides in elements, base pointers and the three strides 16-byte aligned (strides % 8 == 0).
+ * Scope: the exponent-sign predictor with the default path switches (the tensor-core predictor and attention; any
+ * fused-path mode), head_dim a multiple of 8 in [32, 128], every Nk the fp32 path accepts, with or without key_bias;
+ * anything else returns MXP_E_UNSUPPORTED.  key_bias stays fp32.
+ *
  * Compact MXINT8 format shared by all entry points (SURVEY.md section 8a):
  *   code  int8  in [-127,127]   (sign-magnitude semantics; -128 never produced)
  *   exp   int8  in [-127,127]   one per 32 elements of head_dim; -126 marks an all-zero block
@@ -37,7 +47,15 @@
 extern "C" {
 #endif
 
-#define MXP_ABI_VERSION 3
+#define MXP_ABI_VERSION 4
+
+/*
+ * Element types of q/k/v/x and out for the *_dt entry points.  The fp32 entry points are the *_dt ones with
+ * MXP_DT_F32 everywhere.
+ */
+#define MXP_DT_F32  0
+#define MXP_DT_BF16 1
+#define MXP_DT_F16  2
 
 #define MXP_OK             0
 #define MXP_E_BADARG      -1   /* null pointer, bad shape/stride/alignment, k out of range */
@@ -63,6 +81,10 @@ void mxp_limits(int* max_keys, int* max_head_dim);
 int mxp_quantize_mxint8(const float* x, int64_t sB, int64_t sH, int64_t sN,
                         int B, int H, int N, int hd, int bfloat_bits, int flush,
                         int8_t* codes, int8_t* exps, uint32_t* signs, void* stream);
+/* x of element type x_dtype (MXP_DT_*); 16-bit x: head_dim a multiple of 8 (any such head_dim of the fp32 call) */
+int mxp_quantize_mxint8_dt(const void* x, int x_dtype, int64_t sB, int64_t sH, int64_t sN,
+                           int B, int H, int N, int hd, int bfloat_bits, int flush,
+                           int8_t* codes, int8_t* exps, uint32_t* signs, void* stream);
 
 /*
  * Dense exponent-sign approximation, (code<0 ? -1 : +1) * 2^exp per element, fp32 contiguous
@@ -107,6 +129,14 @@ int mxp_predict_topk(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
                      uint32_t* mask, int32_t* idx,
                      int8_t* q_codes, int8_t* q_exps, int8_t* k_codes, int8_t* k_exps,
                      void* workspace, size_t workspace_bytes, void* stream);
+/* q and k of element type in_dtype (MXP_DT_*) */
+int mxp_predict_topk_dt(const void* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
+                        const void* k, int64_t k_sB, int64_t k_sH, int64_t k_sN, int in_dtype,
+                        int B, int H, int Nq, int Nk, int hd, int top_k,
+                        int bfloat_bits, int flush,
+                        uint32_t* mask, int32_t* idx,
+                        int8_t* q_codes, int8_t* q_exps, int8_t* k_codes, int8_t* k_exps,
+                        void* workspace, size_t workspace_bytes, void* stream);
 
 /*
  * Exact MXINT8 attention over the kept keys.  Replaces
@@ -126,6 +156,15 @@ int mxp_sparse_attention(const int8_t* q_codes, const int8_t* q_exps,
                          float scale, int bfloat_bits, int flush,
                          float* out, int64_t o_sB, int64_t o_sH, int64_t o_sN,
                          void* workspace, size_t workspace_bytes, void* stream);
+/* v of element type v_dtype, out of element type out_dtype (MXP_DT_*; fp32 or v_dtype) */
+int mxp_sparse_attention_dt(const int8_t* q_codes, const int8_t* q_exps,
+                            const int8_t* k_codes, const int8_t* k_exps,
+                            const void* v, int64_t v_sB, int64_t v_sH, int64_t v_sN, int v_dtype,
+                            const uint32_t* mask,
+                            int B, int H, int Nq, int Nk, int hd,
+                            float scale, int bfloat_bits, int flush,
+                            void* out, int64_t o_sB, int64_t o_sH, int64_t o_sN, int out_dtype,
+                            void* workspace, size_t workspace_bytes, void* stream);
 
 /*
  * The whole path in one call: q,k,v -> out.  Replaces lines 101-152 of
@@ -162,6 +201,17 @@ int mxp_pruned_attention_biased(const float* q, int64_t q_sB, int64_t q_sH, int6
                                 const float* key_bias, int64_t kb_sB,
                                 uint32_t* mask_out,
                                 void* workspace, size_t workspace_bytes, void* stream);
+/* mxp_pruned_attention / mxp_pruned_attention_biased with q, k, v of element type in_dtype and out of element type
+ * out_dtype (MXP_DT_*; fp32 or in_dtype); key_bias may be NULL */
+int mxp_pruned_attention_dt(const void* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
+                            const void* k, int64_t k_sB, int64_t k_sH, int64_t k_sN,
+                            const void* v, int64_t v_sB, int64_t v_sH, int64_t v_sN, int in_dtype,
+                            int B, int H, int Nq, int Nk, int hd, int top_k,
+                            float scale, int bfloat_bits, int flush,
+                            void* out, int64_t o_sB, int64_t o_sH, int64_t o_sN, int out_dtype,
+                            const float* key_bias, int64_t kb_sB,
+                            uint32_t* mask_out,
+                            void* workspace, size_t workspace_bytes, void* stream);
 
 /*
  * The reference's other sources of the top-k ranking (SURVEY 8 f3), behind the same call:

@@ -9,9 +9,10 @@ from ctypes import c_float, c_int, c_int64, c_size_t, c_void_p
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # MXPRUNE_LIB: developer override (e.g. the phase-accounting build csrc/libmxprune_timing.so, `make timing`)
 LIB_PATH = os.environ.get("MXPRUNE_LIB") or os.path.join(_HERE, "csrc", "libmxprune.so")
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 MXP_OK, MXP_E_BADARG, MXP_E_UNSUPPORTED, MXP_E_CUDA = 0, -1, -2, -3
+MXP_DT_F32, MXP_DT_BF16, MXP_DT_F16 = 0, 1, 2
 
 _VIEW = [c_void_p, c_int64, c_int64, c_int64]          # ptr, sB, sH, sN
 
@@ -26,18 +27,24 @@ _SIGNATURES = {
     "mxp_debug_fused_pingpong": (c_int, [c_int]),
     "mxp_limits": (None, [ctypes.POINTER(c_int), ctypes.POINTER(c_int)]),
     "mxp_quantize_mxint8": (c_int, _VIEW + [c_int] * 6 + [c_void_p] * 4),
+    "mxp_quantize_mxint8_dt": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64] + [c_int] * 6 + [c_void_p] * 4),
     "mxp_exp_sign_approx": (c_int, _VIEW + [c_int] * 6 + [c_void_p] * 2),
     "mxp_predict_scores": (c_int, _VIEW + _VIEW + [c_int] * 7 + [c_void_p] * 2),
     "mxp_predict_topk_workspace_bytes": (c_size_t, [c_int] * 5),
     "mxp_predict_topk": (c_int, _VIEW + _VIEW + [c_int] * 8 + [c_void_p] * 7 + [c_size_t, c_void_p]),
+    "mxp_predict_topk_dt": (c_int, _VIEW + _VIEW + [c_int] * 9 + [c_void_p] * 7 + [c_size_t, c_void_p]),
     "mxp_sparse_attention_workspace_bytes": (c_size_t, [c_int] * 5),
     "mxp_sparse_attention": (c_int, [c_void_p] * 4 + _VIEW + [c_void_p] + [c_int] * 5 + [c_float, c_int, c_int]
                              + _VIEW + [c_void_p, c_size_t, c_void_p]),
+    "mxp_sparse_attention_dt": (c_int, [c_void_p] * 4 + _VIEW + [c_int, c_void_p] + [c_int] * 5 + [c_float, c_int, c_int]
+                                + _VIEW + [c_int, c_void_p, c_size_t, c_void_p]),
     "mxp_pruned_attention_workspace_bytes": (c_size_t, [c_int] * 5),
     "mxp_pruned_attention": (c_int, _VIEW * 3 + [c_int] * 6 + [c_float, c_int, c_int] + _VIEW
                              + [c_void_p, c_void_p, c_size_t, c_void_p]),
     "mxp_pruned_attention_biased": (c_int, _VIEW * 3 + [c_int] * 6 + [c_float, c_int, c_int] + _VIEW
                                     + [c_void_p, ctypes.c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "mxp_pruned_attention_dt": (c_int, _VIEW * 3 + [c_int] * 7 + [c_float, c_int, c_int] + _VIEW
+                                + [c_int, c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
     "mxp_pruned_attention_mode": (c_int, _VIEW * 3 + [c_int] * 7 + [c_float, c_int, c_int] + _VIEW
                                   + [c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
     "mxp_predict_topk_mode": (c_int, _VIEW * 2 + [c_int] * 7 + [c_float, c_int, c_int]

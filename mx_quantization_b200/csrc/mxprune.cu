@@ -23,10 +23,12 @@ namespace {
 constexpr int MAX_HD = 128;
 constexpr int MAX_KEYS_FUSED = 256;   // keys held in registers, 8 per lane
 
-int check_view(const char* name, const float* p, int64_t sB, int64_t sH, int64_t sN, int hd) {
+int check_view(const char* name, const void* p, int64_t sB, int64_t sH, int64_t sN, int hd, int dt = DT_F32) {
     if (!p) return fail(MXP_E_BADARG, "%s: null pointer", name);
-    if (((uintptr_t)p & 15) || (sB & 3) || (sH & 3) || (sN & 3))
-        return fail(MXP_E_BADARG, "%s: base pointer and strides must be 16-byte aligned", name);
+    const int64_t m = dt == DT_F32 ? 3 : 7;                 // 16 bytes of elements - 1
+    if (((uintptr_t)p & 15) || (sB & m) || (sH & m) || (sN & m))
+        return fail(MXP_E_BADARG, "%s: base pointer and strides must be 16-byte aligned (strides multiples of %d elements)",
+                    name, (int)m + 1);
     if (sN < hd) return fail(MXP_E_BADARG, "%s: row stride %lld < head_dim %d", name, (long long)sN, hd);
     return MXP_OK;
 }
@@ -36,6 +38,22 @@ int check_shape(int B, int H, int Nq, int Nk, int hd, int bfloat_bits) {
     if (hd < 4 || hd > MAX_HD || (hd & 3)) return fail(MXP_E_UNSUPPORTED, "head_dim %d: need a multiple of 4 in [4,%d]", hd, MAX_HD);
     if (bfloat_bits != 16 && bfloat_bits != 32) return fail(MXP_E_UNSUPPORTED, "bfloat=%d: only 16 or 32 are on the path", bfloat_bits);
     if ((int64_t)B * H > 0x7fffffffLL) return fail(MXP_E_UNSUPPORTED, "B*H too large");
+    return MXP_OK;
+}
+
+int check_dtype(const char* name, int dt) {
+    if (dt != DT_F32 && dt != DT_BF16 && dt != DT_F16)
+        return fail(MXP_E_BADARG, "%s: element type %d is not MXP_DT_F32, MXP_DT_BF16 or MXP_DT_F16", name, dt);
+    return MXP_OK;
+}
+
+// the scope of 16-bit activations (include/mxprune.h): the tensor-core kernels, head_dim a multiple of 8 in [32, 128]
+int check_half_scope(int dt, int hd) {
+    if (dt == DT_F32) return MXP_OK;
+    if (g_attn_path != 0 || g_predict_path != 0)
+        return fail(MXP_E_UNSUPPORTED, "16-bit inputs need the tensor-core predictor and attention paths (the default)");
+    if (hd < 32 || (hd & 7))
+        return fail(MXP_E_UNSUPPORTED, "head_dim %d: 16-bit inputs need a multiple of 8 in [32, 128]", hd);
     return MXP_OK;
 }
 
@@ -78,7 +96,7 @@ k_quantize(View x, int rows_per_bh, int H, int64_t total_rows, int hd, int bf16,
 // thread and writes 1 KB of contiguous codes.  Replaces the reference's quantize_mx_innermost / _by_tile CUDA
 // kernels (microxscaling/mx/cpp/mx.cuh:57-158) on this path: tools/bench_quant.py times them side by side.
 // ------------------------------------------------------------------------------------
-template <bool SIGNS>
+template <bool SIGNS, int DT = DT_F32>
 __global__ void __launch_bounds__(256)
 k_quantize_blocks(View x, int rows_per_bh, int H, int64_t total_rows, int hd, int nb, int bf16, int flush,
                   int8_t* __restrict__ codes, int8_t* __restrict__ exps, uint32_t* __restrict__ signs) {
@@ -88,15 +106,10 @@ k_quantize_blocks(View x, int rows_per_bh, int H, int64_t total_rows, int hd, in
         const int b = (int)(t - row * nb);
         const int64_t bh = row / rows_per_bh;
         const int n = (int)(row - bh * rows_per_bh);
-        const float* src = x.p + (bh / H) * x.sB + (bh % H) * x.sH + (int64_t)n * x.sN + 32 * b;
+        const float* src = view_elem<DT>(x.p, (bh / H) * x.sB + (bh % H) * x.sH + (int64_t)n * x.sN + 32 * b);
         const int nd = min(32, hd - 32 * b);
         uint32_t xv[32];
-#pragma unroll
-        for (int s = 0; s < 8; ++s) {
-            uint4 v = make_uint4(0u, 0u, 0u, 0u);
-            if (4 * s < nd) v = __ldg(reinterpret_cast<const uint4*>(src) + s);
-            xv[4 * s] = v.x; xv[4 * s + 1] = v.y; xv[4 * s + 2] = v.z; xv[4 * s + 3] = v.w;
-        }
+        load_block_bits<DT>(src, nd, true, xv);
         BlockQ r;
         quantize_block_thread<true, false>(xv, nd, bf16 != 0, flush != 0, r);
         exps[row * nb + b] = (int8_t)r.e;
@@ -444,12 +457,14 @@ inline int pick_kpl(int Nk) {
     return 8;
 }
 
-template <int NB>
+template <int NB, int DT = DT_F32>
 int launch_predict_topk_long(const PredParams& p, cudaStream_t st) {
+    if (DT == DT_F32 && p.dt == DT_BF16) return launch_predict_topk_long<NB, DT_BF16>(p, st);
+    if (DT == DT_F32 && p.dt == DT_F16) return launch_predict_topk_long<NB, DT_F16>(p, st);
     const K1LSmem L = k1l_smem_layout(NB, p.Nk);
     if (L.total > 200 * 1024)
         return fail(MXP_E_UNSUPPORTED, "Nk=%d: key records need %zu bytes of shared memory (limit 200 KiB)", p.Nk, L.total);
-    cudaError_t e = cudaFuncSetAttribute(k_predict_topk_long<NB>,
+    cudaError_t e = cudaFuncSetAttribute(k_predict_topk_long<NB, DT>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
     if (e != cudaSuccess) return fail(MXP_E_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     const int heads = p.B * p.H;
@@ -458,13 +473,15 @@ int launch_predict_topk_long(const PredParams& p, cudaStream_t st) {
     if (splits > tiles) splits = tiles;
     if (splits < 1) splits = 1;
     dim3 grid((unsigned)heads, (unsigned)splits);
-    k_predict_topk_long<NB><<<grid, K1T, L.total, st>>>(p);
+    k_predict_topk_long<NB, DT><<<grid, K1T, L.total, st>>>(p);
     return check_launch("k_predict_topk_long");
 }
 
 template <int NB>
 int launch_predict_topk_nb(const PredParams& p, cudaStream_t st) {
     if (p.Nk > K1_MAX_KEYS) return launch_predict_topk_long<NB>(p, st);
+    if (p.dt != DT_F32)                     // only reached outside the tensor-core kernel's domain
+        return fail(MXP_E_UNSUPPORTED, "16-bit q/k: Nk=%d hd=%d is outside the tensor-core predictor's domain", p.Nk, p.hd);
     const K1Smem L = k1_smem_layout(NB, p.Nk);
     cudaError_t e = cudaFuncSetAttribute(k_predict_topk_rows<NB>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
@@ -508,6 +525,22 @@ inline void prof_mark(int i, cudaStream_t st) {
     cudaEventRecord(g_ev[i], st);
 }
 
+// k_attend_pair with output element type OT (== p.out_dt); grid and dyn from launch_attend
+template <int OT>
+int launch_attend_pair_ot(const AttnParams& p, dim3 grid, size_t dyn, cudaStream_t st) {
+    MXP_ENSURE_DYN_SMEM((k_attend_pair<true, false, OT>), 160 * 1024);
+    MXP_ENSURE_DYN_SMEM((k_attend_pair<false, false, OT>), 160 * 1024);
+    MXP_ENSURE_DYN_SMEM((k_attend_pair<true, true, OT>), 160 * 1024);
+    MXP_ENSURE_DYN_SMEM((k_attend_pair<false, true, OT>), 160 * 1024);
+    if (p.key_bias) {
+        if (p.bf16) k_attend_pair<true, true, OT><<<grid, K2P_T, dyn, st>>>(p);
+        else k_attend_pair<false, true, OT><<<grid, K2P_T, dyn, st>>>(p);
+    } else {
+        if (p.bf16) k_attend_pair<true, false, OT><<<grid, K2P_T, dyn, st>>>(p);
+        else k_attend_pair<false, false, OT><<<grid, K2P_T, dyn, st>>>(p);
+    }
+    return check_launch("k_attend_pair");
+}
 // Exact attention over the MMA-ready operands: Nk > 256 streams key blocks of 128 (k_attend_long_pair,
 // mxprune_attend_long.cuh), one key block runs k_attend_pair (two lanes per query row, 256 threads).
 int launch_attend(const AttnParams& p, cudaStream_t st) {
@@ -516,10 +549,6 @@ int launch_attend(const AttnParams& p, cudaStream_t st) {
         return fail(MXP_E_UNSUPPORTED, "key_bias: the additive key bias is implemented for Nk <= 256 (cross-attention)");
     if (!O.single) return launch_attend_long_pair(p, st);
     const K2Smem L = k2_smem_layout(O);
-    MXP_ENSURE_DYN_SMEM((k_attend_pair<true, false>), 160 * 1024);
-    MXP_ENSURE_DYN_SMEM((k_attend_pair<false, false>), 160 * 1024);
-    MXP_ENSURE_DYN_SMEM((k_attend_pair<true, true>), 160 * 1024);
-    MXP_ENSURE_DYN_SMEM((k_attend_pair<false, true>), 160 * 1024);
     if (L.total > 160 * 1024) return fail(MXP_E_UNSUPPORTED, "attention operands need %zu bytes of shared memory", L.total);
     const int heads = p.B * p.H;
     int splits = (148 * 2 + heads - 1) / heads;
@@ -533,22 +562,20 @@ int launch_attend(const AttnParams& p, cudaStream_t st) {
     size_t dyn = L.total;
     const size_t floor_bytes = (size_t)232448 / (size_t)(max_ctas + 1) + 1024;
     if (dyn < floor_bytes) dyn = floor_bytes;
-    if (p.key_bias) {
-        if (p.bf16) k_attend_pair<true, true><<<grid, K2P_T, dyn, st>>>(p);
-        else k_attend_pair<false, true><<<grid, K2P_T, dyn, st>>>(p);
-    } else {
-        if (p.bf16) k_attend_pair<true, false><<<grid, K2P_T, dyn, st>>>(p);
-        else k_attend_pair<false, false><<<grid, K2P_T, dyn, st>>>(p);
-    }
-    return check_launch("k_attend_pair");
+    if (p.out_dt == DT_BF16) return launch_attend_pair_ot<DT_BF16>(p, grid, dyn, st);
+    if (p.out_dt == DT_F16) return launch_attend_pair_ot<DT_F16>(p, grid, dyn, st);
+    return launch_attend_pair_ot<DT_F32>(p, grid, dyn, st);
 }
 
+// dt: element type of the V view (DT_*)
 int launch_prep_v(const View& v, int B, int H, int Nq, int Nk, int hd, int bf16, int flush, unsigned char* v_op,
-                  cudaStream_t st) {
+                  cudaStream_t st, int dt = DT_F32) {
     const OpsLayout O = ops_layout(Nq, Nk, hd);
     VPrepParams vp{v, H, Nq, Nk, hd, bf16, flush, v_op};
     dim3 grid((unsigned)(B * H), (unsigned)((O.nblk * O.wpb + 3) / 4));
-    k_prep_v<<<grid, K2T, 0, st>>>(vp);
+    if (dt == DT_BF16) k_prep_v<DT_BF16><<<grid, K2T, 0, st>>>(vp);
+    else if (dt == DT_F16) k_prep_v<DT_F16><<<grid, K2T, 0, st>>>(vp);
+    else k_prep_v<<<grid, K2T, 0, st>>>(vp);
     return check_launch("k_prep_v");
 }
 
@@ -571,29 +598,16 @@ inline OpsBytes ops_bytes(int B, int H, int Nq, int Nk, int hd) {
 
 inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// ---- K1-TC launch (tensor maps: make_view_maps, mxprune_predict_tc.cuh) ----------------------
-template <int NC, bool CODES, bool BIASED, int HG = 0, int HD = 0, int BF = -1>
-static int launch_predict_topk_tc_one(const PredParams& p, const K1cMaps& maps, const K1cSmem& L, size_t dyn,
-                                      dim3 grid, cudaStream_t st) {
-    MXP_ENSURE_DYN_SMEM((k_predict_topk_tc<NC, CODES, BIASED, HG, HD, BF>), 227 * 1024);
-    k_predict_topk_tc<NC, CODES, BIASED, HG, HD, BF><<<grid, K1C_T, dyn, st>>>(p, maps, L.ring, L.G);
-    return check_launch("k_predict_topk_tc");
-}
-// the workload head shapes get instantiations with head_dim and the A1 switch folded at compile time
-template <int NC, int HG, int HD>
-static int launch_predict_topk_tc_hd(const PredParams& p, const K1cMaps& maps, const K1cSmem& L, size_t dyn,
-                                     dim3 grid, cudaStream_t st) {
-    return p.bf16 ? launch_predict_topk_tc_one<NC, false, false, HG, HD, 1>(p, maps, L, dyn, grid, st)
-                  : launch_predict_topk_tc_one<NC, false, false, HG, HD, 0>(p, maps, L, dyn, grid, st);
-}
-
-
 // returns 1 if the shape is outside the tensor-core kernel's domain (caller uses the CUDA-core kernel)
 static int try_predict_topk_tc(const PredParams& p, cudaStream_t st, int* rc_out) {
     if (g_predict_path != 0 || p.Nk > 256 || p.hd < 32 || (p.hd & 7)) return 1;
     K1cMaps maps;
-    if (!make_view_maps(p.q, p.B, p.H, p.Nq, p.hd, &maps.q_main, &maps.q_tail)) return 1;
-    if (!make_view_maps(p.k, p.B, p.H, p.Nk, p.hd, &maps.k_main, &maps.k_tail)) return 1;
+    if (!make_view_maps(p.q, p.B, p.H, p.Nq, p.hd, &maps.q_main, &maps.q_tail, p.dt) ||
+        !make_view_maps(p.k, p.B, p.H, p.Nk, p.hd, &maps.k_main, &maps.k_tail, p.dt)) {
+        if (p.dt == DT_F32) return 1;
+        *rc_out = fail(MXP_E_UNSUPPORTED, "16-bit q/k: the views cannot be described by a TMA tensor map");
+        return 0;
+    }
     // step = 64 G rows (G = 2 when a 64-row box gives fewer than 256 block tasks); ring depth: as many
     // slots as fit with two CTAs per SM
     const size_t per_cta1 = K1C_PER_CTA1;
@@ -615,31 +629,10 @@ static int try_predict_topk_tc(const PredParams& p, cudaStream_t st, int* rc_out
     if (dyn < floor_bytes) dyn = floor_bytes;
     const bool codes = p.q_codes != nullptr || p.k_codes != nullptr;
     if (biased && codes) return 1;          // codes + bias: the CUDA-core kernel handles it
-#define MXP_TC(NC_)                                                                                     \
-    *rc_out = biased ? launch_predict_topk_tc_one<NC_, false, true>(p, maps, L, dyn, grid, st)          \
-            : codes  ? launch_predict_topk_tc_one<NC_, true, false>(p, maps, L, dyn, grid, st)          \
-                     : launch_predict_topk_tc_one<NC_, false, false>(p, maps, L, dyn, grid, st)
-    switch (nc) {
-        case 1: MXP_TC(1); break;
-        case 2: MXP_TC(2); break;
-        case 4: MXP_TC(4); break;
-        case 7:
-            // 193 .. 224 keys: the two lanes of a row split the columns at 104 / 112 instead of 128 (no dummy chunk)
-            if (!biased && !codes && p.Nk > 192 && p.Nk <= 208 && p.hd == 64)       // DeiT / ViT-224 heads
-                *rc_out = launch_predict_topk_tc_hd<7, 13, 64>(p, maps, L, dyn, grid, st);
-            else if (!biased && !codes && p.Nk > 192 && p.Nk <= 208)
-                *rc_out = launch_predict_topk_tc_one<7, false, false, 13>(p, maps, L, dyn, grid, st);
-            else if (!biased && !codes && p.Nk > 208)
-                *rc_out = launch_predict_topk_tc_one<7, false, false, 14>(p, maps, L, dyn, grid, st);
-            else
-                MXP_TC(7);
-            break;
-        default:
-            if (!biased && !codes && p.hd == 72) *rc_out = launch_predict_topk_tc_hd<8, 0, 72>(p, maps, L, dyn, grid, st);   // DiT / PixArt heads
-            else MXP_TC(8);
-            break;
-    }
-#undef MXP_TC
+    // one instantiation policy for every element type (launch_predict_topk_tc_dt, mxprune_predict_tc.cuh); the 16-bit
+    // instantiations are compiled in mxprune_predict16.cu
+    *rc_out = p.dt == DT_F32 ? launch_predict_topk_tc_dt<DT_F32>(p, maps, L, dyn, grid, nc, st)
+                             : launch_predict_topk_tc_16(p, maps, L, dyn, grid, nc, st);
     return 0;
 }
 
@@ -760,8 +753,17 @@ static int try_predict_topk_long_tc(const PredParams& p, cudaStream_t st, int* r
         const int want = (148 * 8 + heads - 1) / heads;
         if (gy > want) gy = want;
         dim3 grid((unsigned)heads, (unsigned)gy);
-        if (codes) k_quantize_ops<true><<<grid, 256, 0, st>>>(qp);
-        else k_quantize_ops<false><<<grid, 256, 0, st>>>(qp);
+        if (p.dt == DT_BF16) {
+            if (codes) k_quantize_ops<true, DT_BF16><<<grid, 256, 0, st>>>(qp);
+            else k_quantize_ops<false, DT_BF16><<<grid, 256, 0, st>>>(qp);
+        } else if (p.dt == DT_F16) {
+            if (codes) k_quantize_ops<true, DT_F16><<<grid, 256, 0, st>>>(qp);
+            else k_quantize_ops<false, DT_F16><<<grid, 256, 0, st>>>(qp);
+        } else if (codes) {
+            k_quantize_ops<true><<<grid, 256, 0, st>>>(qp);
+        } else {
+            k_quantize_ops<false><<<grid, 256, 0, st>>>(qp);
+        }
         if ((*rc_out = check_launch("k_quantize_ops"))) return 0;
     }
     {
@@ -841,14 +843,18 @@ void mxp_limits(int* max_keys, int* max_head_dim) {
     if (max_head_dim) *max_head_dim = MAX_HD;
 }
 
-static int quantize_common(const float* x, int64_t sB, int64_t sH, int64_t sN, int B, int H, int N,
+static int quantize_common(const void* xp, int dt, int64_t sB, int64_t sH, int64_t sN, int B, int H, int N,
                            int hd, int bfloat_bits, int flush, int8_t* codes, int8_t* exps,
                            uint32_t* signs, float* approx, void* stream) {
     g_launches = 0;
     int rc = check_shape(B, H, N, N, hd, bfloat_bits);
     if (rc) return rc;
-    rc = check_view("x", x, sB, sH, sN, hd);
+    if ((rc = check_dtype("x", dt))) return rc;
+    if (dt != DT_F32 && (hd & 7))          // 16-byte loads of 8 elements: a row holds whole chunks
+        return fail(MXP_E_UNSUPPORTED, "head_dim %d: 16-bit x needs a multiple of 8", hd);
+    rc = check_view("x", xp, sB, sH, sN, hd, dt);
     if (rc) return rc;
+    const float* x = (const float*)xp;
     const int64_t rows = (int64_t)B * H * N;
     int64_t blocks = (rows + WARPS - 1) / WARPS;
     if (blocks > 148 * 16) blocks = 148 * 16;
@@ -862,24 +868,33 @@ static int quantize_common(const float* x, int64_t sB, int64_t sH, int64_t sN, i
     int64_t qblocks = (rows * nb + 255) / 256;
     const int64_t cap = (int64_t)sm_count() * 32;
     if (qblocks > cap) qblocks = cap;
-    if (signs)
-        k_quantize_blocks<true><<<(unsigned)qblocks, 256, 0, st>>>(v, N, H, rows, hd, nb, bfloat_bits == 16, flush != 0, codes, exps, signs);
-    else
-        k_quantize_blocks<false><<<(unsigned)qblocks, 256, 0, st>>>(v, N, H, rows, hd, nb, bfloat_bits == 16, flush != 0, codes, exps, signs);
+#define MXP_QB(S_, DT_) k_quantize_blocks<S_, DT_><<<(unsigned)qblocks, 256, 0, st>>>(v, N, H, rows, hd, nb, bfloat_bits == 16, \
+                                                                               flush != 0, codes, exps, signs)
+    if (dt == DT_BF16) { if (signs) MXP_QB(true, DT_BF16); else MXP_QB(false, DT_BF16); }
+    else if (dt == DT_F16) { if (signs) MXP_QB(true, DT_F16); else MXP_QB(false, DT_F16); }
+    else if (signs) MXP_QB(true, DT_F32);
+    else MXP_QB(false, DT_F32);
+#undef MXP_QB
     return check_launch("k_quantize_blocks");
+}
+
+int mxp_quantize_mxint8_dt(const void* x, int x_dtype, int64_t sB, int64_t sH, int64_t sN, int B, int H, int N,
+                           int hd, int bfloat_bits, int flush, int8_t* codes, int8_t* exps,
+                           uint32_t* signs, void* stream) {
+    if (!codes || !exps) return fail(MXP_E_BADARG, "codes/exps: null pointer");
+    return quantize_common(x, x_dtype, sB, sH, sN, B, H, N, hd, bfloat_bits, flush, codes, exps, signs, nullptr, stream);
 }
 
 int mxp_quantize_mxint8(const float* x, int64_t sB, int64_t sH, int64_t sN, int B, int H, int N,
                         int hd, int bfloat_bits, int flush, int8_t* codes, int8_t* exps,
                         uint32_t* signs, void* stream) {
-    if (!codes || !exps) return fail(MXP_E_BADARG, "codes/exps: null pointer");
-    return quantize_common(x, sB, sH, sN, B, H, N, hd, bfloat_bits, flush, codes, exps, signs, nullptr, stream);
+    return mxp_quantize_mxint8_dt(x, MXP_DT_F32, sB, sH, sN, B, H, N, hd, bfloat_bits, flush, codes, exps, signs, stream);
 }
 
 int mxp_exp_sign_approx(const float* x, int64_t sB, int64_t sH, int64_t sN, int B, int H, int N,
                         int hd, int bfloat_bits, int flush, float* approx, void* stream) {
     if (!approx) return fail(MXP_E_BADARG, "approx: null pointer");
-    return quantize_common(x, sB, sH, sN, B, H, N, hd, bfloat_bits, flush, nullptr, nullptr, nullptr, approx, stream);
+    return quantize_common(x, DT_F32, sB, sH, sN, B, H, N, hd, bfloat_bits, flush, nullptr, nullptr, nullptr, approx, stream);
 }
 
 int mxp_predict_scores(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
@@ -941,29 +956,40 @@ static int predict_topk_impl(const PredParams& p, cudaStream_t st) {
     }
 }
 
-int mxp_predict_topk(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
-                     const float* k, int64_t k_sB, int64_t k_sH, int64_t k_sN,
-                     int B, int H, int Nq, int Nk, int hd, int top_k, int bfloat_bits, int flush,
-                     uint32_t* mask, int32_t* idx, int8_t* q_codes, int8_t* q_exps,
-                     int8_t* k_codes, int8_t* k_exps, void* workspace, size_t workspace_bytes, void* stream) {
+int mxp_predict_topk_dt(const void* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
+                        const void* k, int64_t k_sB, int64_t k_sH, int64_t k_sN, int in_dtype,
+                        int B, int H, int Nq, int Nk, int hd, int top_k, int bfloat_bits, int flush,
+                        uint32_t* mask, int32_t* idx, int8_t* q_codes, int8_t* q_exps,
+                        int8_t* k_codes, int8_t* k_exps, void* workspace, size_t workspace_bytes, void* stream) {
     g_launches = 0;
     int rc = check_shape(B, H, Nq, Nk, hd, bfloat_bits);
     if (rc) return rc;
-    if ((rc = check_view("q", q, q_sB, q_sH, q_sN, hd))) return rc;
-    if ((rc = check_view("k", k, k_sB, k_sH, k_sN, hd))) return rc;
+    if ((rc = check_dtype("q/k", in_dtype)) || (rc = check_half_scope(in_dtype, hd))) return rc;
+    if ((rc = check_view("q", q, q_sB, q_sH, q_sN, hd, in_dtype))) return rc;
+    if ((rc = check_view("k", k, k_sB, k_sH, k_sN, hd, in_dtype))) return rc;
     if (!mask) return fail(MXP_E_BADARG, "mask: null pointer");
     if (top_k < 1 || top_k > Nk) return fail(MXP_E_BADARG, "top_k=%d outside [1, Nk=%d]", top_k, Nk);
     if ((q_codes == nullptr) != (q_exps == nullptr) || (k_codes == nullptr) != (k_exps == nullptr))
         return fail(MXP_E_BADARG, "codes and exps outputs must be given together");
     PredParams p{};
-    p.q = View{q, q_sB, q_sH, q_sN};
-    p.k = View{k, k_sB, k_sH, k_sN};
+    p.q = View{(const float*)q, q_sB, q_sH, q_sN};
+    p.k = View{(const float*)k, k_sB, k_sH, k_sN};
+    p.dt = in_dtype;
     p.B = B; p.H = H; p.Nq = Nq; p.Nk = Nk; p.hd = hd; p.top_k = top_k;
     p.bf16 = bfloat_bits == 16; p.flush = flush != 0;
     p.mask = mask; p.idx = idx;
     p.q_codes = q_codes; p.q_exps = q_exps; p.k_codes = k_codes; p.k_exps = k_exps;
     p.long_ws = workspace; p.long_ws_bytes = workspace_bytes;
     return predict_topk_impl(p, (cudaStream_t)stream);
+}
+
+int mxp_predict_topk(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
+                     const float* k, int64_t k_sB, int64_t k_sH, int64_t k_sN,
+                     int B, int H, int Nq, int Nk, int hd, int top_k, int bfloat_bits, int flush,
+                     uint32_t* mask, int32_t* idx, int8_t* q_codes, int8_t* q_exps,
+                     int8_t* k_codes, int8_t* k_exps, void* workspace, size_t workspace_bytes, void* stream) {
+    return mxp_predict_topk_dt(q, q_sB, q_sH, q_sN, k, k_sB, k_sH, k_sN, MXP_DT_F32, B, H, Nq, Nk, hd, top_k, bfloat_bits,
+                               flush, mask, idx, q_codes, q_exps, k_codes, k_exps, workspace, workspace_bytes, stream);
 }
 
 size_t mxp_sparse_attention_workspace_bytes(int B, int H, int Nq, int Nk, int hd) {
@@ -983,16 +1009,23 @@ static int attend_core_impl(const AttnCoreParams& p, cudaStream_t st) {
     }
 }
 
-int mxp_sparse_attention(const int8_t* q_codes, const int8_t* q_exps, const int8_t* k_codes,
-                         const int8_t* k_exps, const float* v, int64_t v_sB, int64_t v_sH,
-                         int64_t v_sN, const uint32_t* mask, int B, int H, int Nq, int Nk, int hd,
-                         float scale, int bfloat_bits, int flush, float* out, int64_t o_sB,
-                         int64_t o_sH, int64_t o_sN, void* workspace, size_t workspace_bytes, void* stream) {
+int mxp_sparse_attention_dt(const int8_t* q_codes, const int8_t* q_exps, const int8_t* k_codes,
+                            const int8_t* k_exps, const void* vp, int64_t v_sB, int64_t v_sH,
+                            int64_t v_sN, int v_dtype, const uint32_t* mask, int B, int H, int Nq, int Nk, int hd,
+                            float scale, int bfloat_bits, int flush, void* outp, int64_t o_sB,
+                            int64_t o_sH, int64_t o_sN, int out_dtype, void* workspace, size_t workspace_bytes,
+                            void* stream) {
     g_launches = 0;
     int rc = check_shape(B, H, Nq, Nk, hd, bfloat_bits);
     if (rc) return rc;
-    if ((rc = check_view("v", v, v_sB, v_sH, v_sN, hd))) return rc;
-    if ((rc = check_view("out", out, o_sB, o_sH, o_sN, hd))) return rc;
+    if ((rc = check_dtype("v", v_dtype)) || (rc = check_dtype("out", out_dtype))) return rc;
+    if (out_dtype != DT_F32 && out_dtype != v_dtype)
+        return fail(MXP_E_BADARG, "out: element type %d must be fp32 or v's (%d)", out_dtype, v_dtype);
+    if ((rc = check_half_scope(v_dtype, hd))) return rc;
+    if ((rc = check_view("v", vp, v_sB, v_sH, v_sN, hd, v_dtype))) return rc;
+    if ((rc = check_view("out", outp, o_sB, o_sH, o_sN, hd, out_dtype))) return rc;
+    const float* v = (const float*)vp;
+    float* out = (float*)outp;
     if (!q_codes || !q_exps || !k_codes || !k_exps || !mask)
         return fail(MXP_E_BADARG, "codes/exps/mask: null pointer");
     if (((uintptr_t)q_codes & 7) || ((uintptr_t)k_codes & 7) || ((uintptr_t)mask & 3))
@@ -1019,13 +1052,24 @@ int mxp_sparse_attention(const int8_t* q_codes, const int8_t* q_exps, const int8
     unsigned char* v_op = w;
     if ((rc = launch_codes_to_ops(q_codes, q_exps, q_op, B * H, Nq, Nk, hd, 0, st))) return rc;
     if ((rc = launch_codes_to_ops(k_codes, k_exps, k_op, B * H, Nq, Nk, hd, 1, st))) return rc;
-    if ((rc = launch_prep_v(View{v, v_sB, v_sH, v_sN}, B, H, Nq, Nk, hd, bfloat_bits == 16, flush != 0, v_op, st))) return rc;
+    if ((rc = launch_prep_v(View{v, v_sB, v_sH, v_sN}, B, H, Nq, Nk, hd, bfloat_bits == 16, flush != 0, v_op, st,
+                            v_dtype))) return rc;
     AttnParams p{};
     p.q_op = q_op; p.k_op = k_op; p.v_op = v_op; p.mask = mask;
     p.B = B; p.H = H; p.Nq = Nq; p.Nk = Nk; p.hd = hd;
     p.scale = scale; p.bf16 = bfloat_bits == 16; p.flush = flush != 0;
-    p.out = out; p.o_sB = o_sB; p.o_sH = o_sH; p.o_sN = o_sN;
+    p.out = out; p.o_sB = o_sB; p.o_sH = o_sH; p.o_sN = o_sN; p.out_dt = out_dtype;
     return launch_attend(p, st);
+}
+
+int mxp_sparse_attention(const int8_t* q_codes, const int8_t* q_exps, const int8_t* k_codes,
+                         const int8_t* k_exps, const float* v, int64_t v_sB, int64_t v_sH,
+                         int64_t v_sN, const uint32_t* mask, int B, int H, int Nq, int Nk, int hd,
+                         float scale, int bfloat_bits, int flush, float* out, int64_t o_sB,
+                         int64_t o_sH, int64_t o_sN, void* workspace, size_t workspace_bytes, void* stream) {
+    return mxp_sparse_attention_dt(q_codes, q_exps, k_codes, k_exps, v, v_sB, v_sH, v_sN, MXP_DT_F32, mask, B, H, Nq, Nk,
+                                   hd, scale, bfloat_bits, flush, out, o_sB, o_sH, o_sN, MXP_DT_F32, workspace,
+                                   workspace_bytes, stream);
 }
 
 size_t mxp_pruned_attention_workspace_bytes(int B, int H, int Nq, int Nk, int hd) {
@@ -1046,18 +1090,26 @@ static int pruned_attention_impl(const float* q, int64_t q_sB, int64_t q_sH, int
                                  int bfloat_bits, int flush, float* out, int64_t o_sB, int64_t o_sH,
                                  int64_t o_sN, const float* key_bias, int64_t kb_sB, uint32_t* mask_out,
                                  void* workspace, size_t workspace_bytes, void* stream, int pred_mode = 0,
-                                 const float* elsa_proj = nullptr, float elsa_cap = 0.f) {
+                                 const float* elsa_proj = nullptr, float elsa_cap = 0.f, int dt = DT_F32,
+                                 int out_dt = DT_F32) {
     g_launches = 0;
+    if (check_dtype("q/k/v", dt) || check_dtype("out", out_dt)) return MXP_E_BADARG;
+    if (out_dt != DT_F32 && out_dt != dt)
+        return fail(MXP_E_BADARG, "out: element type %d must be fp32 or the inputs' (%d)", out_dt, dt);
+    if (dt != DT_F32 && pred_mode != 0)
+        return fail(MXP_E_UNSUPPORTED, "pred_mode %d: 16-bit inputs are implemented for the exponent-sign predictor only",
+                    pred_mode);
     if (pred_mode != 0 && g_attn_path != 0)
         return fail(MXP_E_UNSUPPORTED, "pred_mode %d needs the tcgen05 attention path", pred_mode);
     if (key_bias && (g_attn_path != 0 || ((uintptr_t)key_bias & 3)))
         return fail(MXP_E_UNSUPPORTED, "key_bias needs the tcgen05 attention path and a 4-byte aligned pointer");
     int rc = check_shape(B, H, Nq, Nk, hd, bfloat_bits);
     if (rc) return rc;
-    if ((rc = check_view("q", q, q_sB, q_sH, q_sN, hd))) return rc;
-    if ((rc = check_view("k", k, k_sB, k_sH, k_sN, hd))) return rc;
-    if ((rc = check_view("v", v, v_sB, v_sH, v_sN, hd))) return rc;
-    if ((rc = check_view("out", out, o_sB, o_sH, o_sN, hd))) return rc;
+    if ((rc = check_half_scope(dt, hd))) return rc;
+    if ((rc = check_view("q", q, q_sB, q_sH, q_sN, hd, dt))) return rc;
+    if ((rc = check_view("k", k, k_sB, k_sH, k_sN, hd, dt))) return rc;
+    if ((rc = check_view("v", v, v_sB, v_sH, v_sN, hd, dt))) return rc;
+    if ((rc = check_view("out", out, o_sB, o_sH, o_sN, hd, out_dt))) return rc;
     if (top_k < 1 || top_k > Nk) return fail(MXP_E_BADARG, "top_k=%d outside [1, Nk=%d]", top_k, Nk);
     const size_t need = mxp_pruned_attention_workspace_bytes(B, H, Nq, Nk, hd);
     if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255))
@@ -1074,6 +1126,7 @@ static int pruned_attention_impl(const float* q, int64_t q_sB, int64_t q_sH, int
     PredParams pp{};
     pp.q = View{q, q_sB, q_sH, q_sN};
     pp.k = View{k, k_sB, k_sH, k_sN};
+    pp.dt = dt;
     pp.B = B; pp.H = H; pp.Nq = Nq; pp.Nk = Nk; pp.hd = hd; pp.top_k = top_k;
     pp.bf16 = bfloat_bits == 16; pp.flush = flush != 0;
     pp.mask = mask; pp.idx = nullptr;
@@ -1086,6 +1139,7 @@ static int pruned_attention_impl(const float* q, int64_t q_sB, int64_t q_sH, int
         // one persistent launch for the whole path (mxprune_fused.cuh) where it applies
         FusedArgs fa{};
         fa.q = pp.q; fa.k = pp.k; fa.v = View{v, v_sB, v_sH, v_sN};
+        fa.dt = dt; fa.out_dt = out_dt;
         fa.B = B; fa.H = H; fa.Nq = Nq; fa.Nk = Nk; fa.hd = hd; fa.top_k = top_k;
         fa.bf16 = bfloat_bits == 16; fa.flush = flush != 0; fa.scale = scale;
         fa.out = out; fa.o_sB = o_sB; fa.o_sH = o_sH; fa.o_sN = o_sN;
@@ -1106,13 +1160,14 @@ static int pruned_attention_impl(const float* q, int64_t q_sB, int64_t q_sH, int
         prof_mark(0, st);
         if ((rc = predict_topk_impl(pp, st))) return rc;
         prof_mark(1, st);
-        if ((rc = launch_prep_v(View{v, v_sB, v_sH, v_sN}, B, H, Nq, Nk, hd, bfloat_bits == 16, flush != 0, v_op, st))) return rc;
+        if ((rc = launch_prep_v(View{v, v_sB, v_sH, v_sN}, B, H, Nq, Nk, hd, bfloat_bits == 16, flush != 0, v_op, st, dt)))
+            return rc;
         prof_mark(2, st);
         AttnParams ap{};
         ap.q_op = q_op; ap.k_op = k_op; ap.v_op = v_op; ap.mask = mask;
         ap.B = B; ap.H = H; ap.Nq = Nq; ap.Nk = Nk; ap.hd = hd;
         ap.scale = scale; ap.bf16 = bfloat_bits == 16; ap.flush = flush != 0;
-        ap.out = out; ap.o_sB = o_sB; ap.o_sH = o_sH; ap.o_sN = o_sN;
+        ap.out = out; ap.o_sB = o_sB; ap.o_sH = o_sH; ap.o_sN = o_sN; ap.out_dt = out_dt;
         ap.key_bias = key_bias; ap.kb_sB = kb_sB;
         int rc2 = MXP_OK;
         if (attend_sparse_try(ap, top_k, st, &rc2) == 0) rc = rc2;      // cost follows top_k (small top_k / Nk)
@@ -1136,6 +1191,19 @@ static int pruned_attention_impl(const float* q, int64_t q_sB, int64_t q_sH, int
     return attend_core_impl(ap, st);
 }
 
+int mxp_pruned_attention_dt(const void* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
+                            const void* k, int64_t k_sB, int64_t k_sH, int64_t k_sN,
+                            const void* v, int64_t v_sB, int64_t v_sH, int64_t v_sN, int in_dtype,
+                            int B, int H, int Nq, int Nk, int hd, int top_k, float scale,
+                            int bfloat_bits, int flush, void* out, int64_t o_sB, int64_t o_sH,
+                            int64_t o_sN, int out_dtype, const float* key_bias, int64_t kb_sB, uint32_t* mask_out,
+                            void* workspace, size_t workspace_bytes, void* stream) {
+    return pruned_attention_impl((const float*)q, q_sB, q_sH, q_sN, (const float*)k, k_sB, k_sH, k_sN,
+                                 (const float*)v, v_sB, v_sH, v_sN, B, H, Nq, Nk, hd, top_k, scale, bfloat_bits, flush,
+                                 (float*)out, o_sB, o_sH, o_sN, key_bias, kb_sB, mask_out, workspace, workspace_bytes,
+                                 stream, 0, nullptr, 0.f, in_dtype, out_dtype);
+}
+
 int mxp_pruned_attention(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
                          const float* k, int64_t k_sB, int64_t k_sH, int64_t k_sN,
                          const float* v, int64_t v_sB, int64_t v_sH, int64_t v_sN,
@@ -1143,9 +1211,9 @@ int mxp_pruned_attention(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_s
                          int bfloat_bits, int flush, float* out, int64_t o_sB, int64_t o_sH,
                          int64_t o_sN, uint32_t* mask_out, void* workspace, size_t workspace_bytes,
                          void* stream) {
-    return pruned_attention_impl(q, q_sB, q_sH, q_sN, k, k_sB, k_sH, k_sN, v, v_sB, v_sH, v_sN, B, H, Nq, Nk, hd,
-                                 top_k, scale, bfloat_bits, flush, out, o_sB, o_sH, o_sN, nullptr, 0, mask_out,
-                                 workspace, workspace_bytes, stream);
+    return mxp_pruned_attention_dt(q, q_sB, q_sH, q_sN, k, k_sB, k_sH, k_sN, v, v_sB, v_sH, v_sN, MXP_DT_F32, B, H, Nq,
+                                   Nk, hd, top_k, scale, bfloat_bits, flush, out, o_sB, o_sH, o_sN, MXP_DT_F32, nullptr, 0,
+                                   mask_out, workspace, workspace_bytes, stream);
 }
 
 int mxp_pruned_attention_biased(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
@@ -1156,9 +1224,9 @@ int mxp_pruned_attention_biased(const float* q, int64_t q_sB, int64_t q_sH, int6
                                 int64_t o_sN, const float* key_bias, int64_t kb_sB, uint32_t* mask_out,
                                 void* workspace, size_t workspace_bytes, void* stream) {
     if (!key_bias) return fail(MXP_E_BADARG, "key_bias: null pointer (use mxp_pruned_attention)");
-    return pruned_attention_impl(q, q_sB, q_sH, q_sN, k, k_sB, k_sH, k_sN, v, v_sB, v_sH, v_sN, B, H, Nq, Nk, hd,
-                                 top_k, scale, bfloat_bits, flush, out, o_sB, o_sH, o_sN, key_bias, kb_sB, mask_out,
-                                 workspace, workspace_bytes, stream);
+    return mxp_pruned_attention_dt(q, q_sB, q_sH, q_sN, k, k_sB, k_sH, k_sN, v, v_sB, v_sH, v_sN, MXP_DT_F32, B, H, Nq,
+                                   Nk, hd, top_k, scale, bfloat_bits, flush, out, o_sB, o_sH, o_sN, MXP_DT_F32, key_bias,
+                                   kb_sB, mask_out, workspace, workspace_bytes, stream);
 }
 
 int mxp_pruned_attention_mode(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,

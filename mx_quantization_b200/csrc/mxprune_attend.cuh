@@ -38,8 +38,9 @@ struct AttnParams {
     int B, H, Nq, Nk, hd;
     float scale;
     int bf16, flush;
-    float* out;
+    float* out;                 // element type out_dt
     int64_t o_sB, o_sH, o_sN;
+    int out_dt;                 // DT_* (host side: selects the kernel instantiation)
     const float* key_bias;      // optional additive bias per (batch, key), added to score * scale (fp32)
     int64_t kb_sB;
 };
@@ -188,9 +189,11 @@ __device__ __forceinline__ void group_sync(const GroupCtx& g) {
 // quarter w & 3 and the column half w >> 2; 32 x 32 blocks are transposed through the warp's private 4 KiB of shared
 // memory (stage_base + 4096 w; conflict-free 16-byte chunks, chunk q of row l at position q ^ (l & 7)) so that 8 lanes
 // store 128 contiguous bytes of one output row: 4 full lines per store instruction instead of 32 partial ones.
-template <bool BF16>
+// OT (DT_*): a 16-bit output type the tile may be stored in - when out16, the fp32 values are rounded to nearest even at
+// the store (64 contiguous bytes per 8 lanes); OT = DT_F32 stores fp32 only.
+template <bool BF16, int OT = DT_F32>
 __device__ __forceinline__ void store_o_tile(uint32_t tmem, unsigned char* stage_base, int warp, int lane, int tile,
-                                             int Nq, int hd, int hdp, float* out_head, int64_t o_sN) {
+                                             int Nq, int hd, int hdp, float* out_head, int64_t o_sN, bool out16 = false) {
     const int half_cols = hdp >> 1;                                 // multiple of 8
     const uint32_t ot = tmem + ((uint32_t)(32 * (warp & 3)) << 16);
     unsigned char* const stg = stage_base + warp * 4096;
@@ -220,7 +223,10 @@ __device__ __forceinline__ void store_o_tile(uint32_t tmem, unsigned char* stage
             for (int it = 0; it < 8; ++it) {
                 const int rl = (lane >> 3) + 4 * it;
                 const uint4 v = *reinterpret_cast<const uint4*>(stg + rl * 128 + ((ch ^ (rl & 7)) << 4));
-                if (row0 + rl < Nq) *reinterpret_cast<uint4*>(out_head + (int64_t)(row0 + rl) * o_sN + col) = v;
+                if (row0 + rl < Nq) {
+                    if (OT != DT_F32 && out16) store_out4<OT>(out_head, (int64_t)(row0 + rl) * o_sN + col, v);
+                    else store_out4<DT_F32>(out_head, (int64_t)(row0 + rl) * o_sN + col, v);
+                }
             }
         }
         __syncwarp();
@@ -230,12 +236,13 @@ __device__ __forceinline__ void store_o_tile(uint32_t tmem, unsigned char* stage
 // One head (query tiles tile_begin, tile_begin + tile_step, ...) through the dense-epilogue exact attention.
 // q_op / k_op / v_op: this head's MMA-ready operands; mask_head: its [Nq][NW] mask words; out_head: its output rows;
 // bias_b: the batch's additive key bias (BIAS only); s_bias: 256 floats of shared memory (BIAS only).
-template <bool BF16, bool BIAS>
+// OT / out16: output type (store_o_tile)
+template <bool BF16, bool BIAS, int OT = DT_F32>
 __device__ __forceinline__ void attend_pair_head(GroupCtx& gc, const OpsLayout& O, int Nq, int Nk, int hd, float scale,
                                                  bool flush, const unsigned char* q_op, const unsigned char* k_op,
                                                  const unsigned char* v_op, const uint32_t* mask_head, float* out_head,
                                                  int64_t o_sN, const float* bias_b, float* s_bias, int tile_begin,
-                                                 int tile_step) {
+                                                 int tile_step, bool out16 = false) {
     constexpr bool bf16 = BF16;
     const K2Smem L = k2_smem_layout(O);
     const int hdp = O.hdp, NW = O.nw, kbr = O.kb_rows;
@@ -463,7 +470,7 @@ __device__ __forceinline__ void attend_pair_head(GroupCtx& gc, const OpsLayout& 
         tcgen05_fence_after_sync();
 
         // ---- O -> A1 -> global (coalesced through the P region, which the finished MMAs no longer read)
-        store_o_tile<BF16>(tmem, sP, warp, lane, tile, Nq, hd, hdp, out_head, o_sN);
+        store_o_tile<BF16, OT>(tmem, sP, warp, lane, tile, Nq, hd, hdp, out_head, o_sN, out16);
         fence_proxy_async_smem();               // P writes (generic proxy) before the next TMA into the region
         tcgen05_fence_before_sync();
         group_sync(gc);                          // every lane has read O before TMEM / sP are reused
@@ -471,7 +478,8 @@ __device__ __forceinline__ void attend_pair_head(GroupCtx& gc, const OpsLayout& 
     }
 }
 
-template <bool BF16, bool BIAS>
+// OT: output element type (DT_*)
+template <bool BF16, bool BIAS, int OT = DT_F32>
 __global__ void __launch_bounds__(K2P_T, 2)
 k_attend_pair(const AttnParams p) {
     extern __shared__ __align__(128) unsigned char smem[];
@@ -488,10 +496,11 @@ k_attend_pair(const AttnParams p) {
     __syncthreads();
     tcgen05_fence_after_sync();
     GroupCtx g{tid, 0, smem, &bars[0], &bars[1], &bars[2], tmem_base_s, 0u, 0u, 0u, nullptr, 0};
-    attend_pair_head<BF16, BIAS>(g, O, p.Nq, p.Nk, p.hd, p.scale, p.flush != 0, p.q_op + (size_t)head * O.q_head_bytes,
-                                 p.k_op + (size_t)head * O.k_head_bytes, p.v_op + (size_t)head * O.v_head_bytes,
-                                 p.mask + (size_t)head * p.Nq * O.nw, p.out + bb * p.o_sB + hh * p.o_sH, p.o_sN,
-                                 BIAS ? p.key_bias + bb * p.kb_sB : nullptr, s_bias, (int)blockIdx.y, (int)gridDim.y);
+    attend_pair_head<BF16, BIAS, OT>(g, O, p.Nq, p.Nk, p.hd, p.scale, p.flush != 0, p.q_op + (size_t)head * O.q_head_bytes,
+                                     p.k_op + (size_t)head * O.k_head_bytes, p.v_op + (size_t)head * O.v_head_bytes,
+                                     p.mask + (size_t)head * p.Nq * O.nw, out_elem(p.out, bb * p.o_sB + hh * p.o_sH, OT != DT_F32), p.o_sN,
+                                     BIAS ? p.key_bias + bb * p.kb_sB : nullptr, s_bias, (int)blockIdx.y, (int)gridDim.y,
+                                     OT != DT_F32);
     if ((tid >> 5) == 0) tmem_dealloc(g.tmem, tcols);
 }
 
@@ -507,26 +516,28 @@ struct VPrepParams {
     unsigned char* v_op;
 };
 
+// DT: element type of the V view (DT_*)
+template <int DT = DT_F32>
 static __global__ void __launch_bounds__(K2T)
 k_prep_v(const VPrepParams p) {
     const OpsLayout O = ops_layout(p.Nq, p.Nk, p.hd);
     const int head = blockIdx.x, bb = head / p.H, hh = head % p.H;
     const int hdp = O.hdp, Nk = p.Nk, hd = p.hd;
     const int nw_pad = O.nblk * O.wpb;                         // windows incl. block padding
-    const float* vb = p.v.p + bb * p.v.sB + hh * p.v.sH;
+    const float* vb = view_elem<DT>(p.v.p, bb * p.v.sB + hh * p.v.sH);
     unsigned char* dst = p.v_op + (size_t)head * O.v_head_bytes;
     const int w0 = blockIdx.y * 4, w1 = min(w0 + 4, nw_pad);
     for (int t = threadIdx.x; t < (w1 - w0) * hdp; t += K2T) {
         const int w = w0 + t / hdp, d = t % hdp;
         uint32_t xb[32];
         uint32_t mx = 0u;
-        const float* vp = vb + (int64_t)(w * 32) * p.v.sN + d;
+        const float* vp = view_elem<DT>(vb, (int64_t)(w * 32) * p.v.sN + d);
         const int nvalid = (d < hd) ? max(0, min(32, Nk - w * 32)) : 0;
 #pragma unroll
         for (int tt = 0; tt < 32; ++tt) {
             uint32_t b = 0u;
-            if (tt < nvalid) b = __float_as_uint(__ldg(vp));
-            vp += p.v.sN;
+            if (tt < nvalid) b = load_elem_bits<DT>(vp, 0);
+            vp = view_elem<DT>(vp, p.v.sN);
             if (p.bf16) b = bf16_half_away(b);
             xb[tt] = b;
             mx = max(mx, b & 0x7fffffffu);
@@ -619,6 +630,7 @@ int attend_sparse_try(const AttnParams& p, int top_k, cudaStream_t st, int* rc_o
 // call is outside its domain (the caller then runs the three-kernel path), else 0 with the launch status in *rc_out.
 struct FusedArgs {
     View q, k, v;
+    int dt, out_dt;                  // element types (DT_*) of q / k / v and of out
     int B, H, Nq, Nk, hd, top_k, bf16, flush;
     float scale;
     float* out;

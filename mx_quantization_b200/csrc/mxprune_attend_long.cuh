@@ -32,7 +32,8 @@ __host__ __device__ inline KLPSmem klp_smem_layout(const OpsLayout& O) {
     return L;
 }
 
-template <bool BF16>
+// OT: output element type (DT_*)
+template <bool BF16, int OT = DT_F32>
 __global__ void __launch_bounds__(K2P_T, 2)
 k_attend_long_pair(const AttnParams p) {
     extern __shared__ __align__(128) unsigned char smem_klp[];
@@ -62,7 +63,7 @@ k_attend_long_pair(const AttnParams p) {
     const unsigned char* q_op = p.q_op + (size_t)head * O.q_head_bytes;
     const unsigned char* k_op = p.k_op + (size_t)head * O.k_head_bytes;
     const unsigned char* v_op = p.v_op + (size_t)head * O.v_head_bytes;
-    float* out_head = p.out + bb * p.o_sB + hh * p.o_sH;
+    float* out_head = out_elem(p.out, bb * p.o_sB + hh * p.o_sH, OT != DT_F32);
     const uint32_t kbytes = (uint32_t)O.k_blk_bytes, vbytes = (uint32_t)O.v_blk_bytes;
 
     if (tid == 0) {
@@ -305,7 +306,7 @@ k_attend_long_pair(const AttnParams p) {
         tcgen05_fence_after_sync();
 
         // ---- O -> A1 -> global (coalesced through the P region, which the finished MMAs no longer read)
-        store_o_tile<BF16>(tmem + o_col, sP, warp, lane, tile, Nq, hd, hdp, out_head, p.o_sN);
+        store_o_tile<BF16, OT>(tmem + o_col, sP, warp, lane, tile, Nq, hd, hdp, out_head, p.o_sN, OT != DT_F32);
         fence_proxy_async_smem();
         tcgen05_fence_before_sync();
         __syncthreads();                                            // O read; smem / TMEM reusable by the next tile

@@ -53,13 +53,13 @@ __device__ __forceinline__ float exp_sub(float x, float m) { return exp_nonpos(_
 
 // One head (all its query tiles) through the sparse exact-attention epilogue.  q_op / k_op / v_op: this head's
 // MMA-ready operands (global memory); mask_head: this head's [Nq][NW] mask words (global or shared memory);
-// out_head: the head's output rows (row stride o_sN).
-template <bool BF16>
+// out_head: the head's output rows (row stride o_sN); OT / out16: output type (store_o_tile).
+template <bool BF16, int OT = DT_F32>
 __device__ __forceinline__ void attend_sparse_head(GroupCtx& g, const OpsLayout& O, const K2sSmem& L, int Nq, int Nk,
                                                    int hd, float scale, bool flush, const unsigned char* q_op,
                                                    const unsigned char* k_op, const unsigned char* v_op,
                                                    const uint32_t* mask_head, float* out_head, int64_t o_sN,
-                                                   int tile_begin, int tile_step) {
+                                                   int tile_begin, int tile_step, bool out16 = false) {
     constexpr bool bf16 = BF16;
     const int hdp = O.hdp, NW = O.nw, kbr = O.kb_rows;
     const int NG = (NW + 3) >> 2;
@@ -342,7 +342,7 @@ __device__ __forceinline__ void attend_sparse_head(GroupCtx& g, const OpsLayout&
         MXP_PROF(g, 18);
 
         // ---- O -> A1 -> global (coalesced through the P region, which the finished MMAs no longer read)
-        store_o_tile<BF16>(tmem, sP, warp, lane, tile, Nq, hd, hdp, out_head, o_sN);
+        store_o_tile<BF16, OT>(tmem, sP, warp, lane, tile, Nq, hd, hdp, out_head, o_sN, out16);
         MXP_PROF(g, 19);
         fence_proxy_async_smem();               // list / P writes (generic proxy) before the next tile's TMA overwrites them
         tcgen05_fence_before_sync();
@@ -352,7 +352,7 @@ __device__ __forceinline__ void attend_sparse_head(GroupCtx& g, const OpsLayout&
     }
 }
 
-template <bool BF16>
+template <bool BF16, int OT = DT_F32>
 __global__ void __launch_bounds__(K2P_T, 2)
 k_attend_sparse(const AttnParams p, const int top_k) {
     extern __shared__ __align__(128) unsigned char smem_k2s[];
@@ -369,10 +369,11 @@ k_attend_sparse(const AttnParams p, const int top_k) {
     __syncthreads();
     tcgen05_fence_after_sync();
     GroupCtx g{tid, 0, smem_k2s, &bars[0], &bars[1], &bars[2], tmem_base_s, 0u, 0u, 0u, nullptr, 0};
-    attend_sparse_head<BF16>(g, O, L, p.Nq, p.Nk, p.hd, p.scale, p.flush != 0,
-                             p.q_op + (size_t)head * O.q_head_bytes, p.k_op + (size_t)head * O.k_head_bytes,
-                             p.v_op + (size_t)head * O.v_head_bytes, p.mask + (size_t)head * p.Nq * O.nw,
-                             p.out + bb * p.o_sB + hh * p.o_sH, p.o_sN, (int)blockIdx.y, (int)gridDim.y);
+    attend_sparse_head<BF16, OT>(g, O, L, p.Nq, p.Nk, p.hd, p.scale, p.flush != 0,
+                                 p.q_op + (size_t)head * O.q_head_bytes, p.k_op + (size_t)head * O.k_head_bytes,
+                                 p.v_op + (size_t)head * O.v_head_bytes, p.mask + (size_t)head * p.Nq * O.nw,
+                                 out_elem(p.out, bb * p.o_sB + hh * p.o_sH, OT != DT_F32), p.o_sN, (int)blockIdx.y,
+                                 (int)gridDim.y, OT != DT_F32);
     if ((tid >> 5) == 0) tmem_dealloc(g.tmem, tcols);
 }
 

@@ -18,10 +18,98 @@ constexpr int WARPS = 8;
 constexpr int THREADS = WARPS * 32;
 constexpr int ZERO_BLOCK_EXP = -126;   // floor(log2(2^-126)), mx_ops.py:83-87
 
-struct View {   // fp32 (B,H,N,hd) view, element strides, innermost stride 1
-    const float* p;
+struct View {   // (B,H,N,hd) view, element strides, innermost stride 1
+    const float* p;  // fp32 elements, or the 16-bit elements of a kernel instantiated for DT_BF16 / DT_F16
     int64_t sB, sH, sN;
 };
+
+// Element types of the activation views and of the attention output (MXP_DT_* of include/mxprune.h).  A kernel that
+// touches activations takes its element type as a template parameter; loads widen 16-bit values to their fp32 bit
+// pattern (exact), so everything after the load is the fp32 arithmetic, and only the final output store narrows.
+constexpr int DT_F32 = 0, DT_BF16 = 1, DT_F16 = 2;
+
+// eight 16-bit elements (one 16-byte chunk) -> their exact fp32 bit patterns
+template <int DT>
+__device__ __forceinline__ void widen8(const uint4 v, uint32_t* x) {
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        if (DT == DT_BF16) {
+            x[2 * i] = w[i] << 16;
+            x[2 * i + 1] = w[i] & 0xffff0000u;
+        } else {
+            float lo, hi;
+            asm("{\n\t.reg .b16 l, h;\n\tmov.b32 {l, h}, %2;\n\tcvt.f32.f16 %0, l;\n\tcvt.f32.f16 %1, h;\n\t}"
+                : "=f"(lo), "=f"(hi) : "r"(w[i]));
+            x[2 * i] = __float_as_uint(lo);
+            x[2 * i + 1] = __float_as_uint(hi);
+        }
+    }
+}
+template <int DT>
+__device__ __forceinline__ uint32_t widen1(uint16_t h) {
+    if (DT == DT_BF16) return (uint32_t)h << 16;
+    float f;
+    asm("cvt.f32.f16 %0, %1;" : "=f"(f) : "h"(h));
+    return __float_as_uint(f);
+}
+
+// One 32-element block of a row from global memory as fp32 bit patterns (elements >= nd are 0): eight 16-byte loads of
+// fp32, four of 16-bit values.  src is 16-byte aligned.
+template <int DT>
+__device__ __forceinline__ void load_block_bits(const float* src, int nd, bool ok, uint32_t (&xv)[32]) {
+    if constexpr (DT == DT_F32) {
+#pragma unroll
+        for (int s = 0; s < 8; ++s) {
+            uint4 v = make_uint4(0u, 0u, 0u, 0u);
+            if (ok && 4 * s < nd) v = __ldg(reinterpret_cast<const uint4*>(src) + s);
+            xv[4 * s] = v.x; xv[4 * s + 1] = v.y; xv[4 * s + 2] = v.z; xv[4 * s + 3] = v.w;
+        }
+    } else {
+#pragma unroll
+        for (int s = 0; s < 4; ++s) {
+            uint4 v = make_uint4(0u, 0u, 0u, 0u);
+            if (ok && 8 * s < nd) v = __ldg(reinterpret_cast<const uint4*>(src) + s);
+            widen8<DT>(v, &xv[8 * s]);
+        }
+    }
+}
+// element pointer of a view row (element offsets, in the view's element type)
+template <int DT>
+__device__ __forceinline__ const float* view_elem(const float* p, int64_t off) {
+    if constexpr (DT == DT_F32) return p + off;
+    else return reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(p) + off);
+}
+// fp32 bit pattern of one element at element offset off
+template <int DT>
+__device__ __forceinline__ uint32_t load_elem_bits(const float* p, int64_t off) {
+    if constexpr (DT == DT_F32) return __float_as_uint(__ldg(p + off));
+    else return widen1<DT>(__ldg(reinterpret_cast<const unsigned short*>(p) + off));
+}
+// output element at element offset off of an fp32 (out16 false) or 16-bit output
+__device__ __forceinline__ float* out_elem(float* p, int64_t off, bool out16) {
+    return out16 ? reinterpret_cast<float*>(reinterpret_cast<uint16_t*>(p) + off) : p + off;
+}
+// four fp32 output values (bit patterns) -> the output type, round to nearest even; dst 16- (fp32) or 8-byte aligned
+template <int DT>
+__device__ __forceinline__ void store_out4(float* dst, int64_t off, const uint4 v) {
+    if constexpr (DT == DT_F32) {
+        *reinterpret_cast<uint4*>(dst + off) = v;
+    } else {
+        const uint32_t in[4] = {v.x, v.y, v.z, v.w};
+        uint32_t o[2];
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+            uint32_t r;
+            if (DT == DT_BF16)
+                asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(__uint_as_float(in[2 * i + 1])), "f"(__uint_as_float(in[2 * i])));
+            else
+                asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(__uint_as_float(in[2 * i + 1])), "f"(__uint_as_float(in[2 * i])));
+            o[i] = r;
+        }
+        *reinterpret_cast<uint2*>(reinterpret_cast<uint16_t*>(dst) + off) = make_uint2(o[0], o[1]);
+    }
+}
 
 struct PredParams {
     View q, k;
@@ -40,6 +128,7 @@ struct PredParams {
     float score_scale;           // pred_mode 3: the attention scale the true scores are ranked with
     const float* elsa_proj;      // pred_mode 7 (ELSA): the hd x hd projection matrix, fp32 row-major (hash j = sign(x . P[j]))
     float elsa_cap;              // pred_mode 7: hash dot products above this value tie (the reference's angle clamp)
+    int dt;                      // element type of q / k (DT_*; host side: selects the kernel instantiation)
 };
 
 // 2^e as fp32 for e in [-149, 127] (subnormal below -126).

@@ -13,6 +13,16 @@
 
 namespace mxp {
 
+// k_attend_sparse with output element type OT (== p.out_dt); grid and dyn from attend_sparse_try
+template <int OT>
+static int launch_attend_sparse_ot(const AttnParams& p, int top_k, dim3 grid, size_t dyn, cudaStream_t st) {
+    MXP_ENSURE_DYN_SMEM((k_attend_sparse<true, OT>), 160 * 1024);
+    MXP_ENSURE_DYN_SMEM((k_attend_sparse<false, OT>), 160 * 1024);
+    if (p.bf16) k_attend_sparse<true, OT><<<grid, K2P_T, dyn, st>>>(p, top_k);
+    else k_attend_sparse<false, OT><<<grid, K2P_T, dyn, st>>>(p, top_k);
+    return check_launch("k_attend_sparse");
+}
+
 int attend_sparse_try(const AttnParams& p, int top_k, cudaStream_t st, int* rc_out) {
     const OpsLayout O = ops_layout(p.Nq, p.Nk, p.hd);
     // domain: one key block, no additive bias, a uniform row population of at most 35 % of the keys, and the row
@@ -21,8 +31,6 @@ int attend_sparse_try(const AttnParams& p, int top_k, cudaStream_t st, int* rc_o
     const K2sSmem L = k2s_smem_layout(O, top_k);
     if (L.total > SMEM_2CTA) return 1;
     auto run = [&]() -> int {
-        MXP_ENSURE_DYN_SMEM((k_attend_sparse<true>), 160 * 1024);
-        MXP_ENSURE_DYN_SMEM((k_attend_sparse<false>), 160 * 1024);
         const int heads = p.B * p.H;
         int splits = (148 * 2 + heads - 1) / heads;
         if (splits > O.q_tiles) splits = O.q_tiles;
@@ -33,9 +41,9 @@ int attend_sparse_try(const AttnParams& p, int top_k, cudaStream_t st, int* rc_o
         size_t dyn = L.total;
         const size_t floor_bytes = SMEM_PER_SM / (size_t)(max_ctas + 1) + 1024;
         if (dyn < floor_bytes) dyn = floor_bytes;
-        if (p.bf16) k_attend_sparse<true><<<grid, K2P_T, dyn, st>>>(p, top_k);
-        else k_attend_sparse<false><<<grid, K2P_T, dyn, st>>>(p, top_k);
-        return check_launch("k_attend_sparse");
+        if (p.out_dt == DT_BF16) return launch_attend_sparse_ot<DT_BF16>(p, top_k, grid, dyn, st);
+        if (p.out_dt == DT_F16) return launch_attend_sparse_ot<DT_F16>(p, top_k, grid, dyn, st);
+        return launch_attend_sparse_ot<DT_F32>(p, top_k, grid, dyn, st);
     };
     *rc_out = run();
     return 0;
@@ -79,6 +87,8 @@ static int launch_fused_one(const FusedParams& p, const FusedMaps& maps, int gri
     return launch_fused_hd<NC, HG, 0>(p, maps, grid, st);
 }
 
+int launch_fused_16(int dt, int nc, int hg, const FusedParams& p, const FusedMaps& maps, int grid, cudaStream_t st);
+
 int fused_try(const FusedArgs& a, cudaStream_t st, int* rc_out) {
     // domain: the exponent-sign predictor on the tensor-core paths, one key block of 129..256 keys, a real selection
     // (top_k < Nk), no key bias, enough heads to give every group of half the chip one
@@ -114,19 +124,25 @@ int fused_try(const FusedArgs& a, cudaStream_t st, int* rc_out) {
     if (grid > heads) grid = heads;
     if (!a.slots || a.slots_bytes < (size_t)2 * grid * S.bytes) return 1;
     FusedMaps maps;
-    if (!make_view_maps(a.q, a.B, a.H, a.Nq, a.hd, &maps.q_main, &maps.q_tail)) return 1;
-    if (!make_view_maps(a.k, a.B, a.H, a.Nk, a.hd, &maps.k_main, &maps.k_tail)) return 1;
-    if (!make_view_maps(a.v, a.B, a.H, a.Nk, a.hd, &maps.v_main, &maps.v_tail)) return 1;
+    if (!make_view_maps(a.q, a.B, a.H, a.Nq, a.hd, &maps.q_main, &maps.q_tail, a.dt) ||
+        !make_view_maps(a.k, a.B, a.H, a.Nk, a.hd, &maps.k_main, &maps.k_tail, a.dt) ||
+        !make_view_maps(a.v, a.B, a.H, a.Nk, a.hd, &maps.v_main, &maps.v_tail, a.dt)) {
+        if (a.dt == DT_F32) return 1;
+        *rc_out = fail(MXP_E_UNSUPPORTED, "16-bit q/k/v: the views cannot be described by a TMA tensor map");
+        return 0;
+    }
     FusedParams p{};
     p.B = a.B; p.H = a.H; p.Nq = a.Nq; p.Nk = a.Nk; p.hd = a.hd; p.top_k = a.top_k; p.bf16 = a.bf16; p.flush = a.flush;
     p.scale = a.scale;
-    p.out = a.out; p.o_sB = a.o_sB; p.o_sH = a.o_sH; p.o_sN = a.o_sN;
+    p.out = a.out; p.o_sB = a.o_sB; p.o_sH = a.o_sH; p.o_sN = a.o_sN; p.out16 = a.out_dt != DT_F32;
     p.mask_out = a.mask_out;
     p.slots = a.slots; p.slot_bytes = S.bytes; p.slot_k = S.k; p.slot_v = S.v; p.slot_mask = S.mask;
     p.ring = ring; p.G = G; p.sparse = sparse ? 1 : 0;
     p.timing = g_fused_timing.load();
     p.pingpong = (g_fused_pingpong.load() && sparse) ? 1 : 0;   // the phase-1 token pays when phase 2 is the latency-bound one
-    if (nc == 8) *rc_out = launch_fused_one<8, 0>(p, maps, grid, st);
+    const int hg = nc == 8 ? 0 : (a.Nk > 192 && a.Nk <= 208) ? 13 : a.Nk > 208 ? 14 : 0;
+    if (a.dt != DT_F32) *rc_out = launch_fused_16(a.dt, nc, hg, p, maps, grid, st);      // mxprune_fused16.cu
+    else if (nc == 8) *rc_out = launch_fused_one<8, 0>(p, maps, grid, st);
     else if (a.Nk > 192 && a.Nk <= 208) *rc_out = launch_fused_one<7, 13>(p, maps, grid, st);
     else if (a.Nk > 208) *rc_out = launch_fused_one<7, 14>(p, maps, grid, st);
     else *rc_out = launch_fused_one<7, 0>(p, maps, grid, st);

@@ -47,7 +47,7 @@ struct FusedMaps {
 struct FusedParams {
     int B, H, Nq, Nk, hd, top_k, bf16, flush;
     float scale;
-    float* out;
+    float* out;                  // fp32, or the kernel's 16-bit input type when out16
     int64_t o_sB, o_sH, o_sN;
     uint32_t* mask_out;          // optional [B*H][Nq][NW]: when given, the masks are written there instead of the slot
     unsigned char* slots;        // workspace: one slot per group
@@ -56,6 +56,7 @@ struct FusedParams {
     int sparse;                  // phase 2: 1 = cost-follows-k epilogue, 0 = dense epilogue
     int pingpong;                // 1: at most one group of a CTA inside phase 1 at a time (drives the groups into anti-phase)
     unsigned long long* timing;  // debug: [2 * gridDim][32] per-phase cycle sums of each group's thread 0 (null = off)
+    int out16;                   // 16-bit input kernels: out holds the input type instead of fp32
 };
 
 struct K1State {                 // phase-1 pipeline state carried from head to head
@@ -67,7 +68,7 @@ struct K1State {                 // phase-1 pipeline state carried from head to 
 // HD: head_dim as a compile-time constant (0 = run time): with it every staging / operand offset of the quantize steps folds
 // (The token count folded as well - 197 - gave no smaller code and 116 bytes of spills at the 128-register cap:
 // 5.40 -> 5.92 ms per DeiT-base step.  Not a template parameter.)
-template <int NC, int HG, bool BF16, int HD>
+template <int NC, int HG, bool BF16, int HD, int DT>
 __device__ __forceinline__ void predict_topk_head(GroupCtx& gc, K1State& st, uint64_t* bar_full, uint64_t* bar_mma,
                                                   const FusedParams& p, const FusedMaps& maps, const K1cSmem& L,
                                                   const OpsLayout& OL, int head, unsigned char* q_op, unsigned char* k_op,
@@ -114,7 +115,7 @@ __device__ __forceinline__ void predict_topk_head(GroupCtx& gc, K1State& st, uin
     const int tiles = tiles_all > tile_begin ? (tiles_all - tile_begin + tile_step - 1) / tile_step : 0;   // this group's query tiles
     const int nsteps = nks + nvs + qsteps * tiles;
     const uint32_t box_main = (uint32_t)L.box_main, box_tail = (uint32_t)L.box_tail;
-    const uint32_t slot_tx = (uint32_t)G * (box_main + box_tail);
+    const uint32_t slot_tx = (uint32_t)G * (box_main + box_tail) / (DT == DT_F32 ? 1 : 2);
     const uint32_t slot_bytes = (uint32_t)L.slot_bytes;
     const uint32_t tail_base = (uint32_t)G * box_main;
 
@@ -181,7 +182,18 @@ __device__ __forceinline__ void predict_topk_head(GroupCtx& gc, K1State& st, uin
                 const int w = (row0 >> 5) + wl;
                 if (w >= NWk) continue;
                 uint32_t xv[32];
-                if (d < 32 * nfull) {
+                if (DT != DT_F32 && d < 32 * nfull) {             // 64-byte rows, SWIZZLE_64B (staged_block_bits)
+                    const int b = d >> 5, dd = d & 31;
+                    const unsigned char* src = slot + ((wl >> 1) * box_main) + (size_t)(b * 64 + (wl & 1) * 32) * 64 + ((dd & 7) << 1);
+                    const int ch = dd >> 3;
+#pragma unroll
+                    for (int tt = 0; tt < 32; ++tt)
+                        xv[tt] = widen1<DT>(*reinterpret_cast<const uint16_t*>(src + tt * 64 + ((ch ^ ((tt >> 1) & 3)) << 4)));
+                } else if (DT != DT_F32 && d < hd) {
+                    const unsigned char* src = slot + tail_base + (wl >> 1) * box_tail + (size_t)((wl & 1) * 32) * tail * 2 + (d - 32 * nfull) * 2;
+#pragma unroll
+                    for (int tt = 0; tt < 32; ++tt) xv[tt] = widen1<DT>(*reinterpret_cast<const uint16_t*>(src + tt * tail * 2));
+                } else if (d < 32 * nfull) {
                     const int b = d >> 5, dd = d & 31;
                     const unsigned char* src = slot + ((wl >> 1) * box_main) + (size_t)(b * 64 + (wl & 1) * 32) * 128 + ((dd & 3) << 2);
                     const int ch = dd >> 2;
@@ -212,7 +224,9 @@ __device__ __forceinline__ void predict_topk_head(GroupCtx& gc, K1State& st, uin
                 const bool in_range = row < nrows;
                 const bool full = b < nfull;
                 uint32_t xv[32];
-                if (full) {
+                if constexpr (DT != DT_F32) {
+                    staged_block_bits_16<DT>(slot, g, box_main, tail_base, box_tail, b, rl6, full, tail, xv);
+                } else if (full) {
                     const unsigned char* src = slot + g * box_main + (b * 64 + rl6) * 128;
                     const int sw7 = (rl6 & 7) << 4;
 #pragma unroll
@@ -465,36 +479,37 @@ __device__ __forceinline__ void predict_topk_head(GroupCtx& gc, K1State& st, uin
 // The two phases of a head.  (Inlined: as separate functions the call ABI's callee-saved registers cost 0.5 - 1.2 KB
 // of spills per thread; inlined the kernel stays at the 128-register cap with a handful of spilled loop invariants.
 // Keep an eye on `-Xptxas -v`: spills next to in-flight tcgen05.ld results are not something to live with.)
-template <int NC, int HG, bool BF16, int HD>
+template <int NC, int HG, bool BF16, int HD, int DT>
 __device__ __forceinline__ void fused_phase1(GroupCtx& gc, K1State& st, uint64_t* bars, const FusedParams& p, const FusedMaps& maps,
                                           int head, unsigned char* slot, uint32_t* mask_head, int tile_begin, int tile_step) {
     const K1cSmem L1 = HD ? k1c_smem_layout(HD, NC, fused_ring(HD, NC), fused_G(HD, NC)) : k1c_smem_layout(p.hd, NC, p.ring, p.G);
     const OpsLayout O = ops_layout(p.Nq, p.Nk, HD ? HD : p.hd);
-    predict_topk_head<NC, HG, BF16, HD>(gc, st, &bars[0], &bars[K1C_MAXR], p, maps, L1, O, head, slot, slot + p.slot_k, slot + p.slot_v,
+    predict_topk_head<NC, HG, BF16, HD, DT>(gc, st, &bars[0], &bars[K1C_MAXR], p, maps, L1, O, head, slot, slot + p.slot_k, slot + p.slot_v,
                               mask_head, tile_begin, tile_step);
 }
 // HD != 0: head_dim at compile time; such instantiations carry the cost-follows-k epilogue only (the launcher sends
 // dense-epilogue calls to the HD = 0 kernels)
-template <bool BF16, int HD>
+template <bool BF16, int HD, int DT>
 __device__ __forceinline__ void fused_phase2(GroupCtx& gc, const FusedParams& p, int head, const unsigned char* slot,
                                           const uint32_t* mask_head, int tile_begin, int tile_step) {
     const int hd = HD ? HD : p.hd, Nq = p.Nq, Nk = p.Nk;
     const OpsLayout O = ops_layout(Nq, Nk, hd);
     const int bb = head / p.H, hh = head - bb * p.H;
-    float* out_head = p.out + bb * p.o_sB + hh * p.o_sH;
+    const bool out16 = DT != DT_F32 && p.out16 != 0;
+    float* out_head = out16 ? out_elem(p.out, bb * p.o_sB + hh * p.o_sH, true) : p.out + bb * p.o_sB + hh * p.o_sH;
     if (HD != 0 || p.sparse) {
         const K2sSmem L2 = k2s_smem_layout(O, p.top_k);
-        attend_sparse_head<BF16>(gc, O, L2, Nq, Nk, hd, p.scale, p.flush != 0, slot, slot + p.slot_k, slot + p.slot_v,
-                                 mask_head, out_head, p.o_sN, tile_begin, tile_step);
+        attend_sparse_head<BF16, DT>(gc, O, L2, Nq, Nk, hd, p.scale, p.flush != 0, slot, slot + p.slot_k, slot + p.slot_v,
+                                     mask_head, out_head, p.o_sN, tile_begin, tile_step, out16);
     } else {
-        attend_pair_head<BF16, false>(gc, O, Nq, Nk, hd, p.scale, p.flush != 0, slot, slot + p.slot_k, slot + p.slot_v,
-                                      mask_head, out_head, p.o_sN, nullptr, nullptr, tile_begin, tile_step);
+        attend_pair_head<BF16, false, DT>(gc, O, Nq, Nk, hd, p.scale, p.flush != 0, slot, slot + p.slot_k, slot + p.slot_v,
+                                          mask_head, out_head, p.o_sN, nullptr, nullptr, tile_begin, tile_step, out16);
     }
 }
 
 // NC, HG: key-column geometry of phase 1 (see k_predict_topk_tc); BF16: A1 rounding on (bfloat 16); HD: head_dim at
-// compile time (0 = any)
-template <int NC, int HG, bool BF16, int HD>
+// compile time (0 = any); DT: element type of q / k / v (DT_*) - the output is fp32 or, with p.out16, that type
+template <int NC, int HG, bool BF16, int HD, int DT = DT_F32>
 __global__ void __launch_bounds__(FUSED_T, 1)
 k_fused_pruned_attention(const __grid_constant__ FusedParams p, const __grid_constant__ FusedMaps maps) {
     extern __shared__ __align__(1024) unsigned char smem_fused[];
@@ -562,7 +577,7 @@ k_fused_pruned_attention(const __grid_constant__ FusedParams p, const __grid_con
             }
             group_sync(gc);
         }
-        fused_phase1<NC, HG, BF16, HD>(gc, st, bars, p, maps, head, slot, mask_head, tile_begin, tile_step);
+        fused_phase1<NC, HG, BF16, HD, DT>(gc, st, bars, p, maps, head, slot, mask_head, tile_begin, tile_step);
         // phase 1 -> phase 2: the slot's operands (generic-proxy global stores) are read back by TMA bulk copies
         // (async proxy), the masks by ordinary loads of other threads of the group; phase 2 also re-purposes the
         // shared memory that phase 1 wrote with generic stores as TMA destinations
@@ -573,7 +588,7 @@ k_fused_pruned_attention(const __grid_constant__ FusedParams p, const __grid_con
         tcgen05_fence_after_sync();
         if (lock && tid == 0) atomicExch(&s_lock, 0);               // every thread of the group has left phase 1
         MXP_PROF(gc, 21);
-        fused_phase2<BF16, HD>(gc, p, head, slot, mask_head, tile_begin, tile_step);
+        fused_phase2<BF16, HD, DT>(gc, p, head, slot, mask_head, tile_begin, tile_step);
         // phase 2 ends with fence.proxy.async + group barrier: its shared memory and TMEM may be reused, and its TMA
         // reads of the slot have completed (every copy was waited for), so the next head may overwrite the slot
     }

@@ -6,15 +6,16 @@
 
 namespace mxp {
 
-template <int NC, int HG, int HD>
+// DT: element type of q / k / v (DT_*)
+template <int NC, int HG, int HD, int DT = DT_F32>
 int launch_fused_hd(const FusedParams& p, const FusedMaps& maps, int grid, cudaStream_t st) {
     const size_t dyn = 2 * FUSED_GROUP_SMEM;
     if (p.bf16) {
-        MXP_ENSURE_DYN_SMEM((k_fused_pruned_attention<NC, HG, true, HD>), (int)dyn);
-        k_fused_pruned_attention<NC, HG, true, HD><<<grid, FUSED_T, dyn, st>>>(p, maps);
+        MXP_ENSURE_DYN_SMEM((k_fused_pruned_attention<NC, HG, true, HD, DT>), (int)dyn);
+        k_fused_pruned_attention<NC, HG, true, HD, DT><<<grid, FUSED_T, dyn, st>>>(p, maps);
     } else {
-        MXP_ENSURE_DYN_SMEM((k_fused_pruned_attention<NC, HG, false, HD>), (int)dyn);
-        k_fused_pruned_attention<NC, HG, false, HD><<<grid, FUSED_T, dyn, st>>>(p, maps);
+        MXP_ENSURE_DYN_SMEM((k_fused_pruned_attention<NC, HG, false, HD, DT>), (int)dyn);
+        k_fused_pruned_attention<NC, HG, false, HD, DT><<<grid, FUSED_T, dyn, st>>>(p, maps);
     }
     return check_launch("k_fused_pruned_attention");
 }

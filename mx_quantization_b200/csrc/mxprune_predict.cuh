@@ -64,7 +64,8 @@ struct RowQ {
 // One thread quantizes one row of hd fp32 values (16-byte aligned).  Optionally writes the int8
 // codes (4-byte aligned destination).
 // op_row (optional): address of this row's first 16-byte bf16 operand chunk, chunks op_stride apart.
-template <int NB>
+// DT: element type of the row (DT_*; 16-bit rows are widened to their exact fp32 bit patterns as they are loaded).
+template <int NB, int DT = DT_F32>
 __device__ __forceinline__ void quantize_row_thread(const float* __restrict__ row, int hd, bool bf16,
                                                     bool flush, RowQ<NB>& rq, int8_t* codes_out,
                                                     unsigned char* op_row = nullptr, int op_stride = 0) {
@@ -73,14 +74,18 @@ __device__ __forceinline__ void quantize_row_thread(const float* __restrict__ ro
 #pragma unroll
     for (int b = 0; b < NB; ++b) {
         const int nd = min(32, hd - 32 * b);
+        if constexpr (DT == DT_F32) {
 #pragma unroll
-        for (int v = 0; v < 8; ++v) {
-            float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (4 * v < nd) f = __ldg(reinterpret_cast<const float4*>(row + 32 * b) + v);
-            xall[b][4 * v + 0] = __float_as_uint(f.x);
-            xall[b][4 * v + 1] = __float_as_uint(f.y);
-            xall[b][4 * v + 2] = __float_as_uint(f.z);
-            xall[b][4 * v + 3] = __float_as_uint(f.w);
+            for (int v = 0; v < 8; ++v) {
+                float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (4 * v < nd) f = __ldg(reinterpret_cast<const float4*>(row + 32 * b) + v);
+                xall[b][4 * v + 0] = __float_as_uint(f.x);
+                xall[b][4 * v + 1] = __float_as_uint(f.y);
+                xall[b][4 * v + 2] = __float_as_uint(f.z);
+                xall[b][4 * v + 3] = __float_as_uint(f.w);
+            }
+        } else {
+            load_block_bits<DT>(view_elem<DT>(row, 32 * b), nd, true, xall[b]);
         }
     }
 #pragma unroll
@@ -544,7 +549,8 @@ __device__ __forceinline__ uint32_t long_key(const LongRow<NB>& R, const uint32_
     return ordered_key(s);
 }
 
-template <int NB>
+// DT: element type of the q / k views (DT_*)
+template <int NB, int DT = DT_F32>
 __global__ void __launch_bounds__(K1T)
 k_predict_topk_long(const PredParams p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -572,11 +578,11 @@ k_predict_topk_long(const PredParams p) {
     if (tid < 4) { s_kmin[tid] = 0x7fffffff; s_kmax[tid] = -0x7fffffff; }
     __syncthreads();
     {
-        const float* kb = p.k.p + bb * p.k.sB + hh * p.k.sH;
+        const float* kb = view_elem<DT>(p.k.p, bb * p.k.sB + hh * p.k.sH);
         for (int j = tid; j < Nk; j += K1T) {
             RowQ<NB> kq;
             const int64_t krow = (int64_t)head * Nk + j;
-            quantize_row_thread<NB>(kb + (int64_t)j * p.k.sN, hd, bf16, flush, kq,
+            quantize_row_thread<NB, DT>(view_elem<DT>(kb, (int64_t)j * p.k.sN), hd, bf16, flush, kq,
                                     write_k ? p.k_codes + krow * hd : nullptr,
                                     write_kop ? k_op + k_op_offset(OL, j, 0) : nullptr, OL.kb_rows * 16);
             uint32_t epw = 0u;
@@ -617,7 +623,7 @@ k_predict_topk_long(const PredParams p) {
     }
     __syncthreads();
 
-    const float* qb = p.q.p + bb * p.q.sB + hh * p.q.sH;
+    const float* qb = view_elem<DT>(p.q.p, bb * p.q.sB + hh * p.q.sH);
     const int NW = (Nk + 31) >> 5;
     uint32_t* my_hist = s_hist + tid;               // bin b at my_hist[b * K1T]
 
@@ -632,9 +638,9 @@ k_predict_topk_long(const PredParams p) {
                     *reinterpret_cast<uint4*>(q_op + q_op_offset(OL, i, kc)) = make_uint4(0u, 0u, 0u, 0u);
         }
         if (valid) {
-            quantize_row_thread<NB>(qb + (int64_t)i * p.q.sN, hd, bf16, flush, rq,
-                                    p.q_codes ? p.q_codes + row * hd : nullptr,
-                                    q_op ? q_op + q_op_offset(OL, i, 0) : nullptr, K2T * 16);
+            quantize_row_thread<NB, DT>(view_elem<DT>(qb, (int64_t)i * p.q.sN), hd, bf16, flush, rq,
+                                        p.q_codes ? p.q_codes + row * hd : nullptr,
+                                        q_op ? q_op + q_op_offset(OL, i, 0) : nullptr, K2T * 16);
             if (p.q_exps) {
 #pragma unroll
                 for (int b = 0; b < NB; ++b) p.q_exps[row * NB + b] = (int8_t)rq.e[b];

@@ -47,14 +47,15 @@ struct QuantOpsParams {
     int8_t *codes, *exps;
 };
 
-template <bool CODES>
+// DT: element type of the view (DT_*)
+template <bool CODES, int DT = DT_F32>
 __global__ void __launch_bounds__(256)
 k_quantize_ops(const QuantOpsParams p) {
     const OpsLayout OL = ops_layout(p.Nq, p.Nk, p.hd);
     const int head = blockIdx.x, bb = head / p.H, hh = head - bb * p.H;
     const int hd = p.hd, nb = (hd + 31) >> 5, nfull = hd >> 5, tail = hd & 31;
     const int kch = OL.hdp >> 3, tail_chunks = kch - 4 * nfull;
-    const float* xb = p.x.p + bb * p.x.sB + hh * p.x.sH;
+    const float* xb = DT == DT_F32 ? p.x.p + bb * p.x.sB + hh * p.x.sH : view_elem<DT>(p.x.p, bb * p.x.sB + hh * p.x.sH);
     const size_t head_bytes = p.which == 0 ? OL.q_head_bytes : OL.k_head_bytes;
     unsigned char* op = p.op ? p.op + (size_t)head * head_bytes : nullptr;
     unsigned char* pp = p.pp + (size_t)head * head_bytes;
@@ -65,12 +66,16 @@ k_quantize_ops(const QuantOpsParams p) {
         const bool full = b < nfull;
         const int nd = full ? 32 : tail;
         uint32_t xv[32];
+        if constexpr (DT == DT_F32) {
 #pragma unroll
-        for (int s = 0; s < 8; ++s) {
-            float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (in_range && 4 * s < nd) f = __ldg(reinterpret_cast<const float4*>(xb + (int64_t)row * p.x.sN + 32 * b) + s);
-            xv[4 * s] = __float_as_uint(f.x); xv[4 * s + 1] = __float_as_uint(f.y);
-            xv[4 * s + 2] = __float_as_uint(f.z); xv[4 * s + 3] = __float_as_uint(f.w);
+            for (int s = 0; s < 8; ++s) {
+                float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (in_range && 4 * s < nd) f = __ldg(reinterpret_cast<const float4*>(xb + (int64_t)row * p.x.sN + 32 * b) + s);
+                xv[4 * s] = __float_as_uint(f.x); xv[4 * s + 1] = __float_as_uint(f.y);
+                xv[4 * s + 2] = __float_as_uint(f.z); xv[4 * s + 3] = __float_as_uint(f.w);
+            }
+        } else {
+            load_block_bits<DT>(view_elem<DT>(xb, (int64_t)row * p.x.sN + 32 * b), nd, in_range, xv);
         }
         BlockQ r;
         quantize_block_thread<CODES>(xv, nd, p.bf16, p.flush, r);

@@ -39,6 +39,7 @@
 
 #include <cuda_runtime.h>
 
+#include "mxprune_host.cuh"
 #include "mxprune_predict.cuh"
 
 namespace mxp {
@@ -126,27 +127,33 @@ inline EncodeTiledFn encode_tiled_fn() {
 
 // main map: dims {32 floats, N, hd/32, H, B}, box {32, 64, hd/32, 1, 1}, SWIZZLE_128B;
 // tail map (hd % 32 floats at column 32*(hd/32)): dims {tail, N, H, B}, box {tail, 64, 1, 1}.
-inline bool make_view_maps(const View& v, int B, int H, int N, int hd, CUtensorMap* m_main, CUtensorMap* m_tail) {
+// dt (DT_*): element type of the view.  16-bit views: the same boxes in elements, 64-byte rows, SWIZZLE_64B (a box fills
+// half of the space an fp32 box takes; slot geometry is the fp32 one).
+inline bool make_view_maps(const View& v, int B, int H, int N, int hd, CUtensorMap* m_main, CUtensorMap* m_tail,
+                           int dt = DT_F32) {
     EncodeTiledFn enc = encode_tiled_fn();
     if (!enc) return false;
     const int nfull = hd >> 5, tail = hd & 31;
-    const cuuint64_t sN = (cuuint64_t)v.sN * 4, sH = (cuuint64_t)(H > 1 ? v.sH : hd) * 4,
-                     sB = (cuuint64_t)(B > 1 ? v.sB : (int64_t)N * v.sN) * 4;
+    const int es_b = dt == DT_F32 ? 4 : 2;
+    const CUtensorMapDataType tdt = dt == DT_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
+                                  : dt == DT_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+    const cuuint64_t sN = (cuuint64_t)v.sN * es_b, sH = (cuuint64_t)(H > 1 ? v.sH : hd) * es_b,
+                     sB = (cuuint64_t)(B > 1 ? v.sB : (int64_t)N * v.sN) * es_b;
     if (!sN || !sH || !sB || (sN >> 40) || (sH >> 40) || (sB >> 40)) return false;
     if (nfull) {
         cuuint64_t dims[5] = {32, (cuuint64_t)N, (cuuint64_t)nfull, (cuuint64_t)H, (cuuint64_t)B};
-        cuuint64_t strides[4] = {sN, 128, sH, sB};
+        cuuint64_t strides[4] = {sN, (cuuint64_t)(32 * es_b), sH, sB};
         cuuint32_t box[5] = {32, (cuuint32_t)K1C_ROWS, (cuuint32_t)nfull, 1, 1}, es[5] = {1, 1, 1, 1, 1};
-        if (enc(m_main, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, (void*)v.p, dims, strides, box, es,
-                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+        if (enc(m_main, tdt, 5, (void*)v.p, dims, strides, box, es,
+                CU_TENSOR_MAP_INTERLEAVE_NONE, dt == DT_F32 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
             return false;
     }
     if (tail) {
         cuuint64_t dims[4] = {(cuuint64_t)tail, (cuuint64_t)N, (cuuint64_t)H, (cuuint64_t)B};
         cuuint64_t strides[3] = {sN, sH, sB};
         cuuint32_t box[4] = {(cuuint32_t)tail, (cuuint32_t)K1C_ROWS, 1, 1}, es[4] = {1, 1, 1, 1};
-        if (enc(m_tail, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, (void*)(v.p + 32 * nfull), dims, strides, box, es,
+        if (enc(m_tail, tdt, 4, (void*)((const char*)v.p + (size_t)32 * nfull * es_b), dims, strides, box, es,
                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
             return false;
@@ -172,6 +179,30 @@ __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* tm, in
 }
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* tm) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(tm)) : "memory");
+}
+
+// One MX block of a staged 16-bit row as fp32 bit patterns (the fp32 kernels read their 128-byte SWIZZLE_128B rows
+// inline).  Box g of the ring slot: main box at slot + g box_main - rows of 32 elements, block-major, 64 bytes per row,
+// SWIZZLE_64B (16-byte chunk s of row r at s ^ ((r >> 1) & 3): conflict-free for consecutive rows on consecutive lanes);
+// tail box at slot + tail_base + g box_tail - tail elements per row, unswizzled; rl6: row within the box.
+template <int DT>
+__device__ __forceinline__ void staged_block_bits_16(const unsigned char* slot, int g, uint32_t box_main,
+                                                     uint32_t tail_base, uint32_t box_tail, int b, int rl6, bool full,
+                                                     int tail, uint32_t (&xv)[32]) {
+    if (full) {
+        const unsigned char* src = slot + g * box_main + (b * 64 + rl6) * 64;
+        const int sw = ((rl6 >> 1) & 3) << 4;
+#pragma unroll
+        for (int s = 0; s < 4; ++s) widen8<DT>(*reinterpret_cast<const uint4*>(src + ((s << 4) ^ sw)), &xv[8 * s]);
+    } else {
+        const unsigned char* src = slot + tail_base + g * box_tail + rl6 * tail * 2;
+#pragma unroll
+        for (int s = 0; s < 4; ++s) {
+            uint4 v = make_uint4(0u, 0u, 0u, 0u);
+            if (8 * s < tail) v = *reinterpret_cast<const uint4*>(src + (s << 4));
+            widen8<DT>(v, &xv[8 * s]);
+        }
+    }
 }
 
 // Results of quantizing one MX block (<= 32 elements) held by one thread.
@@ -462,8 +493,8 @@ __device__ __forceinline__ void tmem_ld_16x32bx2_x8(uint32_t taddr, uint32_t (&r
 // does not cost a whole extra 32-key chunk of selection work per lane; the row mask is then written byte-wise
 // (8 HG is a byte boundary of the bitmask).  HG = 0: halves of NCH 32-key chunks, mask written in words.
 // HD: head_dim at compile time (0 = run time) - staging geometry and operand offsets fold; BF: A1 rounding at compile
-// time (-1 = run time, 0 = bfloat 32, 1 = bfloat 16)
-template <int NC, bool CODES, bool BIASED, int HG = 0, int HD = 0, int BF = -1>
+// time (-1 = run time, 0 = bfloat 32, 1 = bfloat 16); DT: element type of the q / k views (DT_*)
+template <int NC, bool CODES, bool BIASED, int HG = 0, int HD = 0, int BF = -1, int DT = DT_F32>
 __global__ void __launch_bounds__(K1C_T, 2)
 k_predict_topk_tc(const PredParams p, const __grid_constant__ K1cMaps maps, const int ring_arg, const int G_arg) {
     extern __shared__ __align__(1024) unsigned char smem_k1c[];     // 1024-byte aligned: SWIZZLE_128B boxes
@@ -524,7 +555,7 @@ k_predict_topk_tc(const PredParams p, const __grid_constant__ K1cMaps maps, cons
     const int my_tiles = (tiles - (int)blockIdx.y + (int)gridDim.y - 1) / (int)gridDim.y;
     const int nsteps = nks + qsteps * my_tiles;
     const uint32_t box_main = (uint32_t)L.box_main, box_tail = (uint32_t)L.box_tail;
-    const uint32_t slot_tx = (uint32_t)G * (box_main + box_tail);
+    const uint32_t slot_tx = (uint32_t)G * (box_main + box_tail) / (DT == DT_F32 ? 1 : 2);   // 16-bit: half-filled slots
     const uint32_t slot_bytes = (uint32_t)L.slot_bytes;
     const uint32_t tail_base = (uint32_t)G * box_main;
 
@@ -595,7 +626,9 @@ k_predict_topk_tc(const PredParams p, const __grid_constant__ K1cMaps maps, cons
             const bool in_range = row < nrows;
             const bool full = b < nfull;
             uint32_t xv[32];
-            if (full) {
+            if constexpr (DT != DT_F32) {
+                staged_block_bits_16<DT>(slot, g, box_main, tail_base, box_tail, b, rl6, full, tail, xv);
+            } else if (full) {
                 const unsigned char* src = slot + g * box_main + (b * 64 + rl6) * 128;
                 const int sw7 = (rl6 & 7) << 4;
 #pragma unroll
@@ -935,5 +968,54 @@ k_predict_topk_tc(const PredParams p, const __grid_constant__ K1cMaps maps, cons
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem, (uint32_t)L.tmem_cols);
 }
+
+// ---- K1-TC launch: which instantiation serves a call (host side; maps, layout L, dyn and grid set by the caller) ----
+template <int NC, bool CODES, bool BIASED, int HG = 0, int HD = 0, int BF = -1, int DT = DT_F32>
+static int launch_predict_topk_tc_one(const PredParams& p, const K1cMaps& maps, const K1cSmem& L, size_t dyn,
+                                      dim3 grid, cudaStream_t st) {
+    MXP_ENSURE_DYN_SMEM((k_predict_topk_tc<NC, CODES, BIASED, HG, HD, BF, DT>), 227 * 1024);
+    k_predict_topk_tc<NC, CODES, BIASED, HG, HD, BF, DT><<<grid, K1C_T, dyn, st>>>(p, maps, L.ring, L.G);
+    return check_launch("k_predict_topk_tc");
+}
+// the workload head shapes get instantiations with head_dim and the A1 switch folded at compile time
+template <int NC, int HG, int HD, int DT>
+static int launch_predict_topk_tc_hd(const PredParams& p, const K1cMaps& maps, const K1cSmem& L, size_t dyn,
+                                     dim3 grid, cudaStream_t st) {
+    return p.bf16 ? launch_predict_topk_tc_one<NC, false, false, HG, HD, 1, DT>(p, maps, L, dyn, grid, st)
+                  : launch_predict_topk_tc_one<NC, false, false, HG, HD, 0, DT>(p, maps, L, dyn, grid, st);
+}
+// nc = key chunks; q / k of element type DT (== p.dt).  Key bias and code outputs are never requested together.
+template <int DT>
+static int launch_predict_topk_tc_dt(const PredParams& p, const K1cMaps& maps, const K1cSmem& L, size_t dyn, dim3 grid,
+                                     int nc, cudaStream_t st) {
+    const bool biased = p.key_bias != nullptr, codes = p.q_codes != nullptr || p.k_codes != nullptr;
+#define MXP_TC(NC_)                                                                                        \
+    return biased ? launch_predict_topk_tc_one<NC_, false, true, 0, 0, -1, DT>(p, maps, L, dyn, grid, st)     \
+         : codes  ? launch_predict_topk_tc_one<NC_, true, false, 0, 0, -1, DT>(p, maps, L, dyn, grid, st)     \
+                  : launch_predict_topk_tc_one<NC_, false, false, 0, 0, -1, DT>(p, maps, L, dyn, grid, st)
+    switch (nc) {
+        case 1: MXP_TC(1);
+        case 2: MXP_TC(2);
+        case 4: MXP_TC(4);
+        case 7:
+            // 193 .. 224 keys: the two lanes of a row split the columns at 104 / 112 instead of 128 (no dummy chunk)
+            if (!biased && !codes && p.Nk > 192 && p.Nk <= 208 && p.hd == 64)       // DeiT / ViT-224 heads
+                return launch_predict_topk_tc_hd<7, 13, 64, DT>(p, maps, L, dyn, grid, st);
+            if (!biased && !codes && p.Nk > 192 && p.Nk <= 208)
+                return launch_predict_topk_tc_one<7, false, false, 13, 0, -1, DT>(p, maps, L, dyn, grid, st);
+            if (!biased && !codes && p.Nk > 208)
+                return launch_predict_topk_tc_one<7, false, false, 14, 0, -1, DT>(p, maps, L, dyn, grid, st);
+            MXP_TC(7);
+        default:
+            if (!biased && !codes && p.hd == 72)                                      // DiT / PixArt heads
+                return launch_predict_topk_tc_hd<8, 0, 72, DT>(p, maps, L, dyn, grid, st);
+            MXP_TC(8);
+    }
+#undef MXP_TC
+}
+
+// launch_predict_topk_tc_dt for 16-bit q / k (p.dt), compiled in mxprune_predict16.cu
+int launch_predict_topk_tc_16(const PredParams& p, const K1cMaps& maps, const K1cSmem& L, size_t dyn, dim3 grid, int nc,
+                              cudaStream_t st);
 
 }  // namespace mxp

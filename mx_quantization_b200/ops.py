@@ -20,19 +20,63 @@ def _ptr(t: Optional[torch.Tensor]) -> c_void_p:
     return c_void_p(0 if t is None else t.data_ptr())
 
 
-def _view4(t: torch.Tensor, name: str) -> torch.Tensor:
-    """Accept the strided (B,H,N,hd) views the attention modules produce; copy only when the
-    layout is outside what the kernels address (innermost stride 1, 16-byte aligned rows)."""
+# Element types of the activations (MXP_DT_* of include/mxprune.h).  fp32 is the reference's fake-quant dtype; bf16 and
+# fp16 are what autocast / 16-bit pipelines hand over, read natively by the exponent-sign path (widening is exact).
+DTYPE_CODES = {torch.float32: _lib.MXP_DT_F32, torch.bfloat16: _lib.MXP_DT_BF16, torch.float16: _lib.MXP_DT_F16}
+
+
+def _dtype_code(dtype: torch.dtype, name: str) -> int:
+    if dtype not in DTYPE_CODES:
+        raise ValueError(f"{name}: expected float32, bfloat16 or float16, got {dtype}")
+    return DTYPE_CODES[dtype]
+
+
+def _same_dtype(*named) -> torch.dtype:
+    """The one element type shared by the (name, tensor) pairs; mixed dtypes raise."""
+    for name, t in named:
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"{name}: expected a torch.Tensor")
+    dt = named[0][1].dtype
+    for name, t in named[1:]:
+        if t.dtype != dt:
+            raise ValueError(f"{named[0][0]} is {dt} but {name} is {t.dtype}: q, k and v must share one dtype")
+    return dt
+
+
+def _view4(t: torch.Tensor, name: str, half_ok: bool = False) -> torch.Tensor:
+    """Accept the strided (B,H,N,hd) views the attention modules produce.  fp32: copy only when the
+    layout is outside what the kernels address (innermost stride 1, 16-byte aligned rows).  bf16 / fp16
+    (``half_ok``: the entry point reads them natively): the same 16-byte rules (strides multiples of 8
+    elements), and a view that breaks them raises - a copy would be the conversion pass the native path avoids."""
     if not isinstance(t, torch.Tensor):
         raise TypeError(f"{name}: expected a torch.Tensor")
     if t.device.type != "cuda":
         raise ValueError(f"{name}: expected a CUDA tensor (device={t.device}); there is no CPU fallback")
     if t.dim() != 4:
         raise ValueError(f"{name}: expected a 4-D (B,H,N,head_dim) tensor, got shape {tuple(t.shape)}")
+    if t.dtype in (torch.bfloat16, torch.float16) and half_ok:
+        if not (t.stride(-1) == 1 and t.data_ptr() % 16 == 0 and all(s % 8 == 0 for s in t.stride()[:3])):
+            raise ValueError(f"{name}: a {t.dtype} view needs innermost stride 1, a 16-byte aligned base and strides "
+                             f"that are multiples of 8 elements, got strides {tuple(t.stride())}")
+        return t
     if t.dtype != torch.float32:
-        raise ValueError(f"{name}: expected float32 (the reference's fake-quant dtype), got {t.dtype}")
+        raise ValueError(f"{name}: expected float32 (the reference's fake-quant dtype)"
+                         f"{', bfloat16 or float16' if half_ok else ''}, got {t.dtype}")
     ok = t.stride(-1) == 1 and t.data_ptr() % 16 == 0 and all(s % 4 == 0 for s in t.stride()[:3])
     return t if ok else t.contiguous()
+
+
+def _out_tensor(out, shape, in_dtype, dev):
+    """The output buffer and its MXP_DT_* code: a new (B,H,Nq,hd) tensor of the inputs' dtype (as
+    torch.nn.functional.scaled_dot_product_attention), or the caller's fp32 / input-dtype view with innermost
+    stride 1."""
+    if out is None:
+        out = torch.empty(shape, dtype=in_dtype, device=dev)
+    elif (tuple(out.shape) != tuple(shape) or out.dtype not in (torch.float32, in_dtype) or out.stride(-1) != 1
+          or out.device != dev):
+        raise ValueError(f"out must be a (B,H,Nq,head_dim) view of dtype float32 or {in_dtype} with innermost stride 1 "
+                         "on the inputs' device")
+    return out, _dtype_code(out.dtype, "out")
 
 
 def _strides(t: torch.Tensor) -> Tuple[int, int, int]:
@@ -87,18 +131,20 @@ def last_launch_count() -> int:
 def quantize_mxint8(x: torch.Tensor, mx_specs, with_signs: bool = False):
     """MXINT8 codes/exponents of ``x`` along head_dim (replaces quantize_mx_op on this path).
 
+    ``x``: float32, bfloat16 or float16 (head_dim a multiple of 8); a 16-bit x gives exactly the result of
+    ``x.float()``.
     Returns (codes int8 (B,H,N,hd), exps int8 (B,H,N,nb)[, signs int32 (B,H,N,nb)])."""
     sp = resolve_specs(mx_specs)
     lib = _lib.load()
-    x = _view4(x, "x")
+    x = _view4(x, "x", half_ok=True)
     B, H, N, hd = x.shape
     nb = (hd + 31) // 32
     with torch.cuda.device(x.device):
         codes = torch.empty((B, H, N, hd), dtype=torch.int8, device=x.device)
         exps = torch.empty((B, H, N, nb), dtype=torch.int8, device=x.device)
         signs = torch.empty((B, H, N, nb), dtype=torch.int32, device=x.device) if with_signs else None
-        rc = lib.mxp_quantize_mxint8(_ptr(x), *_strides(x), B, H, N, hd, sp.bfloat_bits, int(sp.flush),
-                                     _ptr(codes), _ptr(exps), _ptr(signs), _stream())
+        rc = lib.mxp_quantize_mxint8_dt(_ptr(x), _dtype_code(x.dtype, "x"), *_strides(x), B, H, N, hd, sp.bfloat_bits,
+                                        int(sp.flush), _ptr(codes), _ptr(exps), _ptr(signs), _stream())
     _lib.check(rc, "mxp_quantize_mxint8")
     return (codes, exps, signs) if with_signs else (codes, exps)
 
@@ -182,7 +228,9 @@ def predict_topk(q: torch.Tensor, k: torch.Tensor, mx_specs, top_k: int, return_
     Returns a dict: mask int32 (B,H,Nq,ceil(Nk/32)) [bit j%32 of word j//32 = key j kept],
     optionally idx int32 (B,H,Nq,top_k) ascending key order, and q/k codes+exps.
     pred_mode: "ex_pred" (exponent-sign, default), "partial_Q", "partial_K", "MXINT4" or "exact" (top-k of the
-    true scores * scale) - see PRED_MODES."""
+    true scores * scale) - see PRED_MODES.
+    q, k: float32, or (pred_mode "ex_pred", head_dim a multiple of 8 in [32, 128]) both bfloat16 or both float16 -
+    the result of the same call on q.float(), k.float()."""
     if pred_mode == "ELSA":
         return _predict_topk_elsa(q, k, mx_specs, top_k, return_idx, return_codes, key_bias, orthogonal_matrix)
     mode = _pred_mode_code(pred_mode)
@@ -192,7 +240,8 @@ def predict_topk(q: torch.Tensor, k: torch.Tensor, mx_specs, top_k: int, return_
         raise ValueError("predict_topk with pred_mode='ex_pred' takes no key_bias (use pruned_attention)")
     sp = resolve_specs(mx_specs)
     lib = _lib.load()
-    q, k = _view4(q, "q"), _view4(k, "k")
+    dt = _dtype_code(_same_dtype(("q", q), ("k", k)), "q")
+    q, k = _view4(q, "q", half_ok=True), _view4(k, "k", half_ok=True)
     dev = _same_device(q, k)
     B, H, Nq, Nk, hd = _qk_shapes(q, k)
     nb, nw = (hd + 31) // 32, (Nk + 31) // 32
@@ -208,11 +257,11 @@ def predict_topk(q: torch.Tensor, k: torch.Tensor, mx_specs, top_k: int, return_
             res["k_exps"] = torch.empty((B, H, Nk, nb), dtype=torch.int8, device=dev)
         ws_bytes = lib.mxp_predict_topk_workspace_bytes(B, H, Nq, Nk, hd)
         ws = torch.empty((max(ws_bytes, 1),), dtype=torch.uint8, device=dev) if ws_bytes else None
-        rc = lib.mxp_predict_topk(_ptr(q), *_strides(q), _ptr(k), *_strides(k), B, H, Nq, Nk, hd, int(top_k),
-                                  sp.bfloat_bits, int(sp.flush), _ptr(res["mask"]), _ptr(res.get("idx")),
-                                  _ptr(res.get("q_codes")), _ptr(res.get("q_exps")),
-                                  _ptr(res.get("k_codes")), _ptr(res.get("k_exps")),
-                                  _ptr(ws), ws_bytes, _stream())
+        rc = lib.mxp_predict_topk_dt(_ptr(q), *_strides(q), _ptr(k), *_strides(k), dt, B, H, Nq, Nk, hd, int(top_k),
+                                     sp.bfloat_bits, int(sp.flush), _ptr(res["mask"]), _ptr(res.get("idx")),
+                                     _ptr(res.get("q_codes")), _ptr(res.get("q_exps")),
+                                     _ptr(res.get("k_codes")), _ptr(res.get("k_exps")),
+                                     _ptr(ws), ws_bytes, _stream())
     _lib.check(rc, "mxp_predict_topk")
     return res
 
@@ -270,10 +319,13 @@ def _predict_topk_elsa(q, k, mx_specs, top_k, return_idx, return_codes, key_bias
 
 def sparse_attention(q_codes, q_exps, k_codes, k_exps, v: torch.Tensor, mask: torch.Tensor, mx_specs,
                      scale: Optional[float] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Exact MXINT8 softmax(QK^T*scale)V over the keys selected by ``mask``."""
+    """Exact MXINT8 softmax(QK^T*scale)V over the keys selected by ``mask``.
+
+    ``v``: float32, bfloat16 or float16 (head_dim a multiple of 8 in [32, 128] for 16-bit); the output is of v's
+    dtype unless an fp32 ``out`` is given."""
     sp = resolve_specs(mx_specs)
     lib = _lib.load()
-    v = _view4(v, "v")
+    v = _view4(v, "v", half_ok=True)
     B, H, Nk, hd = v.shape
     if q_codes.dim() != 4:
         raise ValueError(f"q_codes: expected a 4-D (B,H,Nq,head_dim) tensor, got shape {tuple(q_codes.shape)}")
@@ -289,17 +341,13 @@ def sparse_attention(q_codes, q_exps, k_codes, k_exps, v: torch.Tensor, mask: to
             raise ValueError(f"{name}: expected shape {shape} (from v {tuple(v.shape)}), got {tuple(t.shape)}")
     scale = float(hd) ** -0.5 if scale is None else float(scale)
     with torch.cuda.device(dev):
-        if out is None:
-            out = torch.empty((B, H, Nq, hd), dtype=torch.float32, device=dev)
-        elif (tuple(out.shape) != (B, H, Nq, hd) or out.dtype != torch.float32 or out.stride(-1) != 1
-              or out.device != dev):
-            raise ValueError("out must be an fp32 (B,H,Nq,head_dim) view with innermost stride 1 on the inputs' device")
+        out, out_dt = _out_tensor(out, (B, H, Nq, hd), v.dtype, dev)
         ws_bytes = lib.mxp_sparse_attention_workspace_bytes(B, H, Nq, Nk, hd)
         ws = torch.empty((max(ws_bytes, 1),), dtype=torch.uint8, device=dev)
-        rc = lib.mxp_sparse_attention(_ptr(q_codes), _ptr(q_exps), _ptr(k_codes), _ptr(k_exps),
-                                      _ptr(v), *_strides(v), _ptr(mask), B, H, Nq, Nk, hd,
-                                      scale, sp.bfloat_bits, int(sp.flush),
-                                      _ptr(out), *_strides(out), _ptr(ws), ws_bytes, _stream())
+        rc = lib.mxp_sparse_attention_dt(_ptr(q_codes), _ptr(q_exps), _ptr(k_codes), _ptr(k_exps),
+                                         _ptr(v), *_strides(v), _dtype_code(v.dtype, "v"), _ptr(mask), B, H, Nq, Nk, hd,
+                                         scale, sp.bfloat_bits, int(sp.flush),
+                                         _ptr(out), *_strides(out), out_dt, _ptr(ws), ws_bytes, _stream())
     _lib.check(rc, "mxp_sparse_attention")
     return out
 
@@ -309,7 +357,12 @@ def pruned_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, mx_specs
                      out: Optional[torch.Tensor] = None, _kernel_ms: Optional[list] = None,
                      key_bias: Optional[torch.Tensor] = None, pred_mode: str = "ex_pred",
                      orthogonal_matrix: Optional[torch.Tensor] = None):
-    """MXINT8 exponent-sign predicted top-k attention: q,k,v (B,H,N,hd) fp32 -> out (B,H,Nq,hd).
+    """MXINT8 exponent-sign predicted top-k attention: q,k,v (B,H,N,hd) -> out (B,H,Nq,hd).
+
+    q, k, v: float32, or all bfloat16 or all float16 (pred_mode "ex_pred", head_dim a multiple of 8 in [32, 128],
+    the default path switches): a 16-bit call gives the masks of the same call on q.float(), k.float(), v.float()
+    and the same fp32 output before its final store.  The output dtype is ``out``'s, else q's (a 16-bit output is
+    the fp32 result rounded to nearest even).  No conversion pass runs: the same launches as the fp32 call.
 
     ``pred_mode``: what ranks the keys - "ex_pred" (default), "partial_Q", "partial_K", "MXINT4" (the reference's
     pred_mode values, workloads/deit/scripts/main.py:109-118) or "exact" (its approx_flag=False branch:
@@ -318,17 +371,22 @@ def pruned_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, mx_specs
 
     Drop-in for lines 101-152 of workloads/deit/scripts/main.py (DiT models.py:168-225, PixArt
     MX_transformer_block.py:647-710) when mx_quant, top_k, approx_flag and pred_mode=="ex_pred".
-    ``out`` may be any fp32 (B,H,Nq,hd) *view* with innermost stride 1, e.g. a permuted
+    ``out`` may be any fp32 or q-dtype (B,H,Nq,hd) *view* with innermost stride 1, e.g. a permuted
     (B,Nq,H,hd) buffer so that the module's transpose(1,2).reshape(B,N,C) is free.
 
     ``key_bias``: PixArt cross-attention's additive text mask (MX_transformer_block.py:794-803,
-    821-822), any fp32 tensor with B * Nk elements laid out (B, ..., Nk) - e.g. the reference's
+    821-822), any fp32 tensor (also with 16-bit q, k, v) with B * Nk elements laid out (B, ..., Nk) - e.g. the reference's
     (B,1,1,S) attention_mask; it is added to the true AND the predicted scores.  Nq may differ
     from Nk (Nk <= 256 with a bias).
     """
     sp = resolve_specs(mx_specs)
     lib = _lib.load()
-    q, k, v = _view4(q, "q"), _view4(k, "k"), _view4(v, "v")
+    in_dtype = _same_dtype(("q", q), ("k", k), ("v", v))
+    dt = _dtype_code(in_dtype, "q")
+    if dt != _lib.MXP_DT_F32 and (pred_mode != "ex_pred" or _kernel_ms is not None):
+        raise ValueError(f"{in_dtype} q/k/v: pred_mode='ex_pred' without the per-kernel profile entry only "
+                         f"(got pred_mode={pred_mode!r}); pass float32 tensors for the other modes")
+    q, k, v = _view4(q, "q", half_ok=True), _view4(k, "k", half_ok=True), _view4(v, "v", half_ok=True)
     dev = _same_device(q, k, v, out)
     B, H, Nq, Nk, hd = _qk_shapes(q, k)
     if tuple(v.shape) != (B, H, Nk, hd):
@@ -342,10 +400,7 @@ def pruned_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, mx_specs
     if mode != 0 and _kernel_ms is not None:
         raise ValueError("the per-kernel profile entry is available with pred_mode='ex_pred' only")
     with torch.cuda.device(dev):
-        if out is None:
-            out = torch.empty((B, H, Nq, hd), dtype=torch.float32, device=dev)
-        elif tuple(out.shape) != (B, H, Nq, hd) or out.dtype != torch.float32 or out.stride(-1) != 1:
-            raise ValueError("out must be an fp32 (B,H,Nq,head_dim) view with innermost stride 1")
+        out, out_dt = _out_tensor(out, (B, H, Nq, hd), in_dtype, dev)
         mask = torch.empty((B, H, Nq, (Nk + 31) // 32), dtype=torch.int32, device=dev) if return_mask else None
         ws_bytes = lib.mxp_pruned_attention_workspace_bytes(B, H, Nq, Nk, hd)
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
@@ -358,6 +413,9 @@ def pruned_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, mx_specs
                                                *args[18:])
         elif mode != 0:
             rc = lib.mxp_pruned_attention_mode(*args[:18], mode, *args[18:-4], _ptr(kb), Nk, *args[-4:])
+        elif dt != _lib.MXP_DT_F32 or out_dt != _lib.MXP_DT_F32:
+            rc = lib.mxp_pruned_attention_dt(*args[:12], dt, *args[12:25], out_dt, _ptr(kb), Nk if kb is not None else 0,
+                                             *args[-4:])
         elif key_bias is not None:
             if _kernel_ms is not None:
                 raise ValueError("the per-kernel profile entry takes no key_bias")
