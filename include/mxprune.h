@@ -47,7 +47,7 @@
 extern "C" {
 #endif
 
-#define MXP_ABI_VERSION 4
+#define MXP_ABI_VERSION 5
 
 /*
  * Element types of q/k/v/x and out for the *_dt entry points.  The fp32 entry points are the *_dt ones with
@@ -297,6 +297,20 @@ int mxp_mx_linear_prepare_weight(const float* w, int64_t ldw, int N, int K, int 
 int mxp_mx_linear(const float* x, int64_t ldx, int M, int K, const void* w_op, int N, const float* bias,
                   int bfloat_bits, int flush, float* out, int64_t ldo,
                   void* workspace, size_t workspace_bytes, void* stream);
+/*
+ * 16-bit MX Linear: W (w_dtype), x (x_dtype) and bias (bias_dtype) are each MXP_DT_F32, MXP_DT_BF16 or MXP_DT_F16,
+ * independently; out has x_dtype.  The result is the fp32 call on the exactly widened W, x and bias, rounded to
+ * nearest even when out is 16-bit (with bfloat 16 the fp32 result is already a bf16 value, so a bf16 out is
+ * lossless).  A w_op prepared from a 16-bit W is byte-equal to the one of the widened W.  No conversion pass: a
+ * 16-bit call enqueues the launches of the fp32 call and needs the same workspace.  A 16-bit x or W needs a 16-byte
+ * aligned base and a row stride that is a multiple of 8 elements; a 16-bit out needs an 8-byte aligned base and a
+ * row stride that is a multiple of 4 elements.  The fp32 entry points are these with MXP_DT_F32 everywhere.
+ */
+int mxp_mx_linear_prepare_weight_dt(const void* w, int w_dtype, int64_t ldw, int N, int K, int bfloat_bits,
+                                    int flush, void* w_op, void* stream);
+int mxp_mx_linear_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N,
+                     const void* bias, int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo,
+                     void* workspace, size_t workspace_bytes, void* stream);
 
 /*
  * Measurement aid: same as mxp_pruned_attention (tcgen05 path), but brackets the three kernels

@@ -9,7 +9,7 @@ from ctypes import c_float, c_int, c_int64, c_size_t, c_void_p
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # MXPRUNE_LIB: developer override (e.g. the phase-accounting build csrc/libmxprune_timing.so, `make timing`)
 LIB_PATH = os.environ.get("MXPRUNE_LIB") or os.path.join(_HERE, "csrc", "libmxprune.so")
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 MXP_OK, MXP_E_BADARG, MXP_E_UNSUPPORTED, MXP_E_CUDA = 0, -1, -2, -3
 MXP_DT_F32, MXP_DT_BF16, MXP_DT_F16 = 0, 1, 2
@@ -58,6 +58,10 @@ _SIGNATURES = {
     "mxp_mx_linear_prepare_weight": (c_int, [c_void_p, c_int64, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "mxp_mx_linear": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p,
                               c_int64, c_void_p, c_size_t, c_void_p]),
+    "mxp_mx_linear_prepare_weight_dt": (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_int, c_int, c_void_p,
+                                                c_void_p]),
+    "mxp_mx_linear_dt": (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int,
+                                 c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
     "mxp_pruned_attention_profile": (c_int, _VIEW * 3 + [c_int] * 6 + [c_float, c_int, c_int] + _VIEW
                                      + [c_void_p, c_void_p, c_size_t, c_void_p, ctypes.POINTER(c_float)]),
 }

@@ -1310,14 +1310,29 @@ static int check_linear(int M, int N, int K, int bfloat_bits) {
     if (bfloat_bits != 16 && bfloat_bits != 32) return fail(MXP_E_UNSUPPORTED, "bfloat=%d: only 16 or 32 are on the path", bfloat_bits);
     return MXP_OK;
 }
-static int launch_quantize_gemm_operand(const float* x, int64_t ld, int rows, int K, int rows_tile, int bf16, int flush,
-                                        void* op, cudaStream_t st) {
+static int launch_quantize_gemm_operand(const void* x, int dt, int64_t ld, int rows, int K, int rows_tile, int bf16,
+                                        int flush, void* op, cudaStream_t st) {
     const int rows_pad = (rows + rows_tile - 1) / rows_tile * rows_tile;
     const int64_t ntask = (int64_t)rows_pad * (K / 32);
     int64_t blocks = (ntask + 255) / 256;
     if (blocks > 148 * 32) blocks = 148 * 32;
-    k_quantize_gemm_operand<<<(unsigned)blocks, 256, 0, st>>>(x, ld, rows, rows_pad, K, rows_tile, bf16, flush, (unsigned char*)op);
+#define MXP_QG(DT_) k_quantize_gemm_operand<DT_><<<(unsigned)blocks, 256, 0, st>>>((const float*)x, ld, rows, rows_pad, K, \
+                                                                                rows_tile, bf16, flush, (unsigned char*)op)
+    if (dt == DT_BF16) MXP_QG(DT_BF16);
+    else if (dt == DT_F16) MXP_QG(DT_F16);
+    else MXP_QG(DT_F32);
+#undef MXP_QG
     return check_launch("k_quantize_gemm_operand");
+}
+
+// rows of a GEMM input (x or W): a 16-byte aligned base, a row stride >= K whose rows stay 16-byte aligned
+// (a multiple of 4 fp32 or 8 16-bit elements)
+static int check_linear_rows(const char* name, const void* p, int dt, int64_t ld, int K) {
+    const int64_t m = dt == DT_F32 ? 3 : 7;
+    if (!p || ((uintptr_t)p & 15) || (ld & m) || ld < K)
+        return fail(MXP_E_BADARG, "%s: null or misaligned pointer, or row stride %lld not >= %d and a multiple of %d elements",
+                    name, (long long)ld, K, (int)m + 1);
+    return MXP_OK;
 }
 
 size_t mxp_mx_linear_weight_bytes(int N, int K) {
@@ -1327,42 +1342,58 @@ size_t mxp_mx_linear_workspace_bytes(int M, int N, int K) {
     return align256((size_t)((M + GL_BM - 1) / GL_BM) * GL_BM * (size_t)K * 2) + align256((size_t)N * 4);
 }
 
-int mxp_mx_linear_prepare_weight(const float* w, int64_t ldw, int N, int K, int bfloat_bits, int flush, void* w_op,
-                                 void* stream) {
+int mxp_mx_linear_prepare_weight_dt(const void* w, int w_dtype, int64_t ldw, int N, int K, int bfloat_bits, int flush,
+                                    void* w_op, void* stream) {
     g_launches = 0;
     int rc = check_linear(1, N, K, bfloat_bits);
     if (rc) return rc;
-    if (!w || !w_op || ((uintptr_t)w & 15) || ((uintptr_t)w_op & 15) || (ldw & 3) || ldw < K)
-        return fail(MXP_E_BADARG, "weight: null / misaligned pointer or row stride");
-    return launch_quantize_gemm_operand(w, ldw, N, K, GL_BN, bfloat_bits == 16, flush != 0, w_op, (cudaStream_t)stream);
+    if ((rc = check_dtype("weight", w_dtype))) return rc;
+    if ((rc = check_linear_rows("weight", w, w_dtype, ldw, K))) return rc;
+    if (!w_op || ((uintptr_t)w_op & 15)) return fail(MXP_E_BADARG, "w_op: null or misaligned pointer");
+    return launch_quantize_gemm_operand(w, w_dtype, ldw, N, K, GL_BN, bfloat_bits == 16, flush != 0, w_op,
+                                        (cudaStream_t)stream);
 }
 
-int mxp_mx_linear(const float* x, int64_t ldx, int M, int K, const void* w_op, int N, const float* bias,
-                  int bfloat_bits, int flush, float* out, int64_t ldo, void* workspace, size_t workspace_bytes,
-                  void* stream) {
+int mxp_mx_linear_prepare_weight(const float* w, int64_t ldw, int N, int K, int bfloat_bits, int flush, void* w_op,
+                                 void* stream) {
+    return mxp_mx_linear_prepare_weight_dt(w, MXP_DT_F32, ldw, N, K, bfloat_bits, flush, w_op, stream);
+}
+
+int mxp_mx_linear_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N, const void* bias,
+                     int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo, void* workspace,
+                     size_t workspace_bytes, void* stream) {
     g_launches = 0;
     int rc = check_linear(M, N, K, bfloat_bits);
     if (rc) return rc;
-    if (!x || !w_op || !out || ((uintptr_t)x & 15) || ((uintptr_t)w_op & 15) || ((uintptr_t)out & 15) || (ldx & 3) ||
-        (ldo & 3) || ldx < K || ldo < N)
-        return fail(MXP_E_BADARG, "x / w_op / out: null or misaligned pointer, or bad row stride");
+    if ((rc = check_dtype("x", x_dtype)) || (rc = check_dtype("bias", bias_dtype))) return rc;
+    if ((rc = check_linear_rows("x", x, x_dtype, ldx, K))) return rc;
+    // out has x's element type; its rows take 16-byte (fp32) or 8-byte (16-bit) stores of four elements
+    const uintptr_t out_align = x_dtype == DT_F32 ? 15 : 7;
+    if (!w_op || !out || ((uintptr_t)w_op & 15) || ((uintptr_t)out & out_align) || (ldo & 3) || ldo < N)
+        return fail(MXP_E_BADARG, "w_op / out: null or misaligned pointer, or out row stride %lld not >= %d and a multiple "
+                    "of 4", (long long)ldo, N);
     const size_t need = mxp_mx_linear_workspace_bytes(M, N, K);
     if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255))
         return fail(MXP_E_BADARG, "workspace: need %zu bytes, 256-byte aligned", need);
     cudaStream_t st = (cudaStream_t)stream;
     unsigned char* a_op = (unsigned char*)workspace;
     float* rbias = (float*)(a_op + align256((size_t)((M + GL_BM - 1) / GL_BM) * GL_BM * (size_t)K * 2));
-    if ((rc = launch_quantize_gemm_operand(x, ldx, M, K, GL_BM, bfloat_bits == 16, flush != 0, a_op, st))) return rc;
+    if ((rc = launch_quantize_gemm_operand(x, x_dtype, ldx, M, K, GL_BM, bfloat_bits == 16, flush != 0, a_op, st)))
+        return rc;
     if (bias) {
-        k_round_bias<<<(N + 255) / 256, 256, 0, st>>>(bias, rbias, N, bfloat_bits == 16);
+        const float* b = (const float*)bias;
+        const unsigned nblk = (unsigned)((N + 255) / 256);
+        if (bias_dtype == DT_BF16) k_round_bias<DT_BF16><<<nblk, 256, 0, st>>>(b, rbias, N, bfloat_bits == 16);
+        else if (bias_dtype == DT_F16) k_round_bias<DT_F16><<<nblk, 256, 0, st>>>(b, rbias, N, bfloat_bits == 16);
+        else k_round_bias<DT_F32><<<nblk, 256, 0, st>>>(b, rbias, N, bfloat_bits == 16);
         if ((rc = check_launch("k_round_bias"))) return rc;
     }
-    MXP_ENSURE_DYN_SMEM(k_mx_linear_umma, 227 * 1024);
     LinearParams lp{};
     lp.a_op = a_op; lp.w_op = (const unsigned char*)w_op; lp.bias = bias ? rbias : nullptr;
-    lp.out = out; lp.ldo = ldo; lp.M = M; lp.N = N; lp.K = K; lp.bf16 = bfloat_bits == 16; lp.stages = 4;
+    lp.out = (float*)out; lp.ldo = ldo; lp.M = M; lp.N = N; lp.K = K; lp.bf16 = bfloat_bits == 16; lp.stages = 4;
     const GemmOpLayout L = gemm_op_layout(K);
-    // persistent: one CTA per SM (4 stages of 48 KiB, 512 TMEM columns for the double-buffered accumulator)
+    // persistent: one CTA per SM (4 stages of 48 KiB, 512 TMEM columns for the double-buffered accumulator); the
+    // same grid and shared memory for every output type
     const size_t dyn = lp.stages * (L.a_stage + L.b_stage) + 2048 + 4 * 32 * 36 * 4 + 1024;
     const int ntiles = ((M + GL_BM - 1) / GL_BM) * ((N + GL_BN - 1) / GL_BN);
     int sms = 148;
@@ -1372,8 +1403,25 @@ int mxp_mx_linear(const float* x, int64_t ldx, int M, int K, const void* w_op, i
             cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0)
             sms = n;
     }
-    k_mx_linear_umma<<<(unsigned)(ntiles < sms ? ntiles : sms), GL_T, dyn, st>>>(lp);
+    const unsigned grid = (unsigned)(ntiles < sms ? ntiles : sms);
+    if (x_dtype == DT_BF16) {
+        MXP_ENSURE_DYN_SMEM(k_mx_linear_umma<DT_BF16>, 227 * 1024);
+        k_mx_linear_umma<DT_BF16><<<grid, GL_T, dyn, st>>>(lp);
+    } else if (x_dtype == DT_F16) {
+        MXP_ENSURE_DYN_SMEM(k_mx_linear_umma<DT_F16>, 227 * 1024);
+        k_mx_linear_umma<DT_F16><<<grid, GL_T, dyn, st>>>(lp);
+    } else {
+        MXP_ENSURE_DYN_SMEM(k_mx_linear_umma<DT_F32>, 227 * 1024);
+        k_mx_linear_umma<DT_F32><<<grid, GL_T, dyn, st>>>(lp);
+    }
     return check_launch("k_mx_linear_umma");
+}
+
+int mxp_mx_linear(const float* x, int64_t ldx, int M, int K, const void* w_op, int N, const float* bias,
+                  int bfloat_bits, int flush, float* out, int64_t ldo, void* workspace, size_t workspace_bytes,
+                  void* stream) {
+    return mxp_mx_linear_dt(x, MXP_DT_F32, ldx, M, K, w_op, N, bias, MXP_DT_F32, bfloat_bits, flush, out, ldo, workspace,
+                            workspace_bytes, stream);
 }
 
 int mxp_pruned_attention_profile(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,

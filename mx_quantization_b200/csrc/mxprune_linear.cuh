@@ -5,14 +5,16 @@
 // is exact in bf16, so the contraction is a bf16 x bf16 -> fp32 GEMM on the tcgen05 tensor cores with
 // no product altered (only the fp32 summation order differs from the reference's BLAS).
 //
-//   k_quantize_gemm_operand  fp32 (rows, K) -> bf16 operand in the MMA-ready order the GEMM streams:
+//   k_quantize_gemm_operand  fp32 / bf16 / fp16 (rows, K) -> bf16 operand in the MMA-ready order the GEMM streams:
 //                            [row tile][k step of 64][8 chunks][tile rows][16 B]  (K-major, no swizzle:
 //                            one stage of one tile is ONE contiguous block -> one TMA bulk copy).
-//                            One thread per 32-wide MX block, same F2I-free arithmetic as the predictor.
+//                            One thread per 32-wide MX block, same F2I-free arithmetic as the predictor; a
+//                            16-bit row is widened to its exact fp32 values as it loads.
 //   k_mx_linear_umma         128 x 256 output tile per CTA, 192 threads, warp-specialised:
 //                              warp 0   TMA producer   (cp.async.bulk, ring of stages, full/empty mbarriers)
 //                              warp 1   MMA issuer     (4 tcgen05.mma of K = 16 per stage, commit -> empty)
-//                              warps 2-5 epilogue      (TMEM lane = output row: A1, + bias, A1, 128-bit stores)
+//                              warps 2-5 epilogue      (TMEM lane = output row: A1, + bias, A1, then the store in
+//                                                       the output type: 128-bit fp32 or 64-bit bf16 / fp16, RNE)
 //                            Two CTAs per SM (2 x 256 TMEM columns): one CTA's epilogue overlaps the
 //                            other's main loop.
 #pragma once
@@ -37,7 +39,9 @@ __host__ __device__ inline GemmOpLayout gemm_op_layout(int K) {
     return L;
 }
 
-// rows_tile = 128 (activations) or 256 (weights); rows_pad = multiple of rows_tile (zero rows past `rows`)
+// rows_tile = 128 (activations) or 256 (weights); rows_pad = multiple of rows_tile (zero rows past `rows`).
+// x holds elements of type DT (DT_*); ld in elements.
+template <int DT>
 __global__ void __launch_bounds__(256)
 k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int rows_pad, int K, int rows_tile,
                         int bf16, int flush, unsigned char* __restrict__ op) {
@@ -47,13 +51,7 @@ k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int r
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < ntask; t += (int64_t)gridDim.x * blockDim.x) {
         const int b = (int)(t / rows_pad), row = (int)(t - (int64_t)b * rows_pad);      // block-major: coalesced stores
         uint32_t xv[32];
-#pragma unroll
-        for (int s = 0; s < 8; ++s) {
-            float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (row < rows) f = __ldg(reinterpret_cast<const float4*>(x + (int64_t)row * ld + 32 * b) + s);
-            xv[4 * s] = __float_as_uint(f.x); xv[4 * s + 1] = __float_as_uint(f.y);
-            xv[4 * s + 2] = __float_as_uint(f.z); xv[4 * s + 3] = __float_as_uint(f.w);
-        }
+        load_block_bits<DT>(view_elem<DT>(x, (int64_t)row * ld + 32 * b), 32, row < rows, xv);
         BlockQ r;
         quantize_block_thread<false, false>(xv, 32, bf16, flush, r);
         const int tile = row / rows_tile, rt = row - tile * rows_tile;
@@ -67,15 +65,19 @@ k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int r
 struct LinearParams {
     const unsigned char *a_op, *w_op;
     const float* bias;                // already A1-rounded by the host wrapper kernel, or null
-    float* out;
+    float* out;                       // elements of the kernel's OUT_DT
     int64_t ldo;
     int M, N, K, bf16, stages;
 };
 
-// bias -> A1(bias), N floats (tiny)
+// bias of element type DT -> A1(bias), N floats (tiny)
+template <int DT>
 __global__ void k_round_bias(const float* __restrict__ b, float* __restrict__ o, int N, int bf16) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < N) o[i] = bf16 ? bf16_half_away(b[i]) : b[i];
+    if (i < N) {
+        const float v = __uint_as_float(load_elem_bits<DT>(b, i));
+        o[i] = bf16 ? bf16_half_away(v) : v;
+    }
 }
 
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
@@ -88,6 +90,8 @@ __device__ __forceinline__ void epilogue_barrier() {               // the 128 ep
 // Persistent: one CTA per SM walks the output tiles (feature tile fastest, so the CTAs that share an
 // activation tile run together and the weight operand stays L2-resident).  The accumulator is
 // double-buffered in TMEM (2 x 256 columns): the epilogue of tile i overlaps the main loop of tile i+1.
+// OUT_DT (DT_*) is the element type of p.out; only the final store depends on it.
+template <int OUT_DT>
 __global__ void __launch_bounds__(GL_T, 1)
 k_mx_linear_umma(const LinearParams p) {
     extern __shared__ __align__(1024) unsigned char smem_gl[];
@@ -178,7 +182,8 @@ k_mx_linear_umma(const LinearParams p) {
             const uint32_t t0 = tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * GL_BN);
             // Coalesced stores: each warp transposes its 32 rows x 32 columns through shared memory
             // (row pitch 36 words: conflict-free 128-bit writes and reads), so that 8 lanes write 128
-            // contiguous bytes of one output row instead of 32 lanes writing 16 bytes of 32 rows.
+            // contiguous bytes of one fp32 output row (64 bytes of a 16-bit one) instead of 32 lanes
+            // writing 16 bytes of 32 rows.
             float* tr = s_tr + (warp - 2) * (32 * 36);
             const int lr = lane >> 3, lc = (lane & 7) * 4;          // this lane's row (mod 4) and column group
             const int row_base = tile_m * GL_BM + q * 32;
@@ -202,7 +207,9 @@ k_mx_linear_umma(const LinearParams p) {
                         y.x = __fadd_rn(y.x, b4.x); y.y = __fadd_rn(y.y, b4.y); y.z = __fadd_rn(y.z, b4.z); y.w = __fadd_rn(y.w, b4.w);
                         if (bf16) { y.x = bf16_half_away(y.x); y.y = bf16_half_away(y.y); y.z = bf16_half_away(y.z); y.w = bf16_half_away(y.w); }   // :89-93
                     }
-                    if (row < p.M && col_ok) *reinterpret_cast<float4*>(p.out + (int64_t)row * p.ldo + n0 + c0 + lc) = y;
+                    if (row < p.M && col_ok)
+                        store_out4<OUT_DT>(p.out, (int64_t)row * p.ldo + n0 + c0 + lc,
+                                           make_uint4(__float_as_uint(y.x), __float_as_uint(y.y), __float_as_uint(y.z), __float_as_uint(y.w)));
                 }
                 __syncwarp();
             }

@@ -27,7 +27,11 @@ from .specs import resolve_linear_specs, resolve_specs
 
 
 class PrunedAttentionCore(nn.Module):
-    """q, k, v (B,H,N,hd) fp32 views -> x (B,N,H*hd), ready for the output projection."""
+    """q, k, v (B,H,N,hd) views -> x (B,N,H*hd), ready for the output projection, in q's dtype.
+
+    q, k, v: float32, or all bfloat16 or all float16 (the 16-bit scope of ops.pruned_attention: the exponent-sign
+    predictor, top-k or dense, head_dim a multiple of 8 in [32, 128]; other pred_modes, ELSA and an "exact" per-call
+    override raise ValueError rather than widen).  A 16-bit x is the fp32 result rounded to nearest even."""
 
     def __init__(self, mx_specs, k: int, scale: Optional[float] = None, pred_mode: str = "ex_pred",
                  orthogonal_matrix: Optional[torch.Tensor] = None):
@@ -50,7 +54,7 @@ class PrunedAttentionCore(nn.Module):
                 pred_mode: Optional[str] = None) -> torch.Tensor:
         """dense / pred_mode: per-call overrides for the reference's exclude_timesteps steps."""
         B, H, N, hd = q.shape
-        buf = torch.empty((B, N, H, hd), dtype=torch.float32, device=q.device)
+        buf = torch.empty((B, N, H, hd), dtype=q.dtype, device=q.device)
         # write straight into (B,N,H,hd): the reference's x.transpose(1,2).reshape(B,N,C) is free
         # k <= 0: dense MXINT8 attention (the reference's top_k=False blocks) = every key kept
         top_k = self.k if (self.k > 0 and not dense) else k.shape[2]
@@ -271,7 +275,8 @@ class MxLinear(nn.Linear):
     """Drop-in for the reference's mx.Linear (microxscaling/mx/linear.py:227-320) on the MXINT8
     configuration of the workloads: same constructor (in_features, out_features, bias, mx_specs),
     forward = ops.mx_linear.  The MX-quantized weight operand is cached and rebuilt when the weight
-    tensor changes (inference: once)."""
+    tensor changes (inference: once; also after ``.to(dtype)``).  The output has the input's dtype (float32, bfloat16
+    or float16), whatever the parameters' dtype."""
 
     def __init__(self, in_features, out_features, bias=True, mx_specs=None, name=None):
         super().__init__(in_features, out_features, bias)
@@ -292,7 +297,7 @@ class MxLinear(nn.Linear):
         if torch.is_grad_enabled() and (self.weight.requires_grad or inputs.requires_grad):
             raise RuntimeError("MxLinear is the inference forward of mx.Linear (the reference's backward is out of scope): "
                                "call it under torch.no_grad() / inference_mode, or freeze the parameters")
-        key = (self.weight.data_ptr(), self.weight._version, str(self.weight.device))
+        key = (self.weight.data_ptr(), self.weight._version, str(self.weight.device), self.weight.dtype)
         if self._w_op is None or self._w_key != key:
             self._w_op = ops.mx_linear_prepare_weight(self.weight.detach(), self.mx_specs)
             self._w_key = key

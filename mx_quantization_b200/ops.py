@@ -433,35 +433,61 @@ def pruned_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, mx_specs
 
 # ---- MX Linear (SURVEY.md 8 f2) -------------------------------------------------------------------
 def mx_linear_prepare_weight(weight: torch.Tensor, mx_specs) -> torch.Tensor:
-    """MX-quantize an (out_features, in_features) fp32 weight once into the GEMM's operand order."""
+    """MX-quantize an (out_features, in_features) weight once into the GEMM's operand order.  ``weight``: float32,
+    bfloat16 or float16; a 16-bit weight gives the bytes of ``weight.float()``'s operand."""
     sp = resolve_linear_specs(mx_specs)
     lib = _lib.load()
-    if weight.dim() != 2 or weight.dtype != torch.float32 or not weight.is_cuda:
-        raise ValueError("weight must be a CUDA fp32 (out_features, in_features) tensor")
+    if not isinstance(weight, torch.Tensor) or weight.dim() != 2 or weight.dtype not in DTYPE_CODES or not weight.is_cuda:
+        raise ValueError("weight must be a CUDA float32, bfloat16 or float16 (out_features, in_features) tensor")
     w = weight if weight.stride(1) == 1 else weight.contiguous()
     N, K = w.shape
     with torch.cuda.device(w.device):
         w_op = torch.empty((lib.mxp_mx_linear_weight_bytes(N, K),), dtype=torch.uint8, device=w.device)
-        rc = lib.mxp_mx_linear_prepare_weight(_ptr(w), w.stride(0), N, K, sp.bfloat_bits, int(sp.flush),
-                                              _ptr(w_op), _stream())
+        rc = lib.mxp_mx_linear_prepare_weight_dt(_ptr(w), DTYPE_CODES[w.dtype], w.stride(0), N, K, sp.bfloat_bits,
+                                                 int(sp.flush), _ptr(w_op), _stream())
     _lib.check(rc, "mxp_mx_linear_prepare_weight")
     return w_op
+
+
+def _linear_rows(x: torch.Tensor) -> torch.Tensor:
+    """x (..., K) as (M, K) rows.  fp32: copied when the rows are not one strided 2-D view.  bf16 / fp16 (read
+    natively): a view with innermost stride 1, a 16-byte aligned base and a row stride that is a multiple of 8 elements,
+    else this raises - a copy would be the conversion-sized pass the native path avoids."""
+    if not isinstance(x, torch.Tensor):
+        raise TypeError("x: expected a torch.Tensor")
+    if x.dtype not in DTYPE_CODES:
+        raise ValueError(f"x: expected float32, bfloat16 or float16, got {x.dtype}")
+    K = x.shape[-1]
+    if x.dtype == torch.float32:
+        x2 = x.reshape(-1, K)
+        return x2 if x2.stride(1) == 1 else x2.contiguous()
+    try:
+        x2 = x.view(-1, K)
+    except RuntimeError:
+        x2 = None
+    if x2 is None or x2.stride(1) != 1 or x2.stride(0) % 8 or x2.data_ptr() % 16:
+        raise ValueError(f"x: a {x.dtype} input needs rows that form one 2-D view with innermost stride 1, a 16-byte "
+                         f"aligned base and a row stride that is a multiple of 8 elements, got shape {tuple(x.shape)} "
+                         f"strides {tuple(x.stride())}")
+    return x2
 
 
 def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
               out_features: Optional[int] = None) -> torch.Tensor:
     """Forward of the reference's mx.Linear (microxscaling/mx/linear.py:20-103) for MXINT8:
-    y = A1(A1(MXq(A1(x)) @ MXq(A1(W))^T) + A1(bias)).  ``weight`` is either the fp32 (N,K) tensor or
-    the operand returned by mx_linear_prepare_weight (then pass out_features)."""
+    y = A1(A1(MXq(A1(x)) @ MXq(A1(W))^T) + A1(bias)).  ``weight`` is either the (N,K) tensor or
+    the operand returned by mx_linear_prepare_weight (then pass out_features).
+
+    ``x``: float32, bfloat16 or float16; the result has x's dtype.  The weight and the bias may each be any of the
+    three types, independently of x.  A 16-bit call is the fp32 call on the widened x, weight and bias, its result
+    rounded to nearest even (lossless under bfloat 16 for a bf16 x: the fp32 result is a bf16 value), with the same
+    kernel launches (no conversion pass)."""
     sp = resolve_linear_specs(mx_specs)
     lib = _lib.load()
-    if x.dtype != torch.float32 or not x.is_cuda:
-        raise ValueError("x must be a CUDA fp32 tensor")
-    K = x.shape[-1]
-    x2 = x.reshape(-1, K)
-    if x2.stride(1) != 1:
-        x2 = x2.contiguous()
-    M = x2.shape[0]
+    x2 = _linear_rows(x)
+    if not x.is_cuda:
+        raise ValueError("x must be a CUDA tensor; there is no CPU fallback")
+    K, M = x2.shape[1], x2.shape[0]
     if weight.dtype == torch.uint8:
         if out_features is None:
             raise ValueError("out_features is required with a prepared weight operand")
@@ -472,14 +498,15 @@ def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
     else:
         N = weight.shape[0]
         w_op = mx_linear_prepare_weight(weight, mx_specs)
-    if bias is not None and (bias.dtype != torch.float32 or bias.numel() != N or not bias.is_contiguous()):
-        raise ValueError("bias must be a contiguous fp32 tensor with out_features elements")
+    if bias is not None and (bias.dtype not in DTYPE_CODES or bias.numel() != N or not bias.is_contiguous()):
+        raise ValueError("bias must be a contiguous float32, bfloat16 or float16 tensor with out_features elements")
     _same_device(x, w_op, bias)
     with torch.cuda.device(x.device):
-        out = torch.empty((M, N), dtype=torch.float32, device=x.device)
+        out = torch.empty((M, N), dtype=x.dtype, device=x.device)
         ws_bytes = lib.mxp_mx_linear_workspace_bytes(M, N, K)
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=x.device)
-        rc = lib.mxp_mx_linear(_ptr(x2), x2.stride(0), M, K, _ptr(w_op), N, _ptr(bias), sp.bfloat_bits,
-                               int(sp.flush), _ptr(out), out.stride(0), _ptr(ws), ws_bytes, _stream())
+        rc = lib.mxp_mx_linear_dt(_ptr(x2), DTYPE_CODES[x.dtype], x2.stride(0), M, K, _ptr(w_op), N, _ptr(bias),
+                                  DTYPE_CODES[bias.dtype] if bias is not None else _lib.MXP_DT_F32, sp.bfloat_bits,
+                                  int(sp.flush), _ptr(out), out.stride(0), _ptr(ws), ws_bytes, _stream())
     _lib.check(rc, "mxp_mx_linear")
     return out.reshape(*x.shape[:-1], N)
