@@ -15,8 +15,9 @@
 //                              warp 1   MMA issuer     (4 tcgen05.mma of K = 16 per stage, commit -> empty)
 //                              warps 2-5 epilogue      (TMEM lane = output row: A1, + bias, A1, then the store in
 //                                                       the output type: 128-bit fp32 or 64-bit bf16 / fp16, RNE)
-//                            Two CTAs per SM (2 x 256 TMEM columns): one CTA's epilogue overlaps the
-//                            other's main loop.
+//                            Persistent, one CTA per SM walking the output tiles; the accumulator is
+//                            double-buffered in TMEM (2 x 256 columns), so the epilogue of one tile overlaps
+//                            the main loop of the next.
 #pragma once
 #include "mxprune_predict_tc.cuh"
 
