@@ -47,7 +47,7 @@
 extern "C" {
 #endif
 
-#define MXP_ABI_VERSION 5
+#define MXP_ABI_VERSION 6
 
 /*
  * Element types of q/k/v/x and out for the *_dt entry points.  The fp32 entry points are the *_dt ones with
@@ -311,6 +311,37 @@ int mxp_mx_linear_prepare_weight_dt(const void* w, int w_dtype, int64_t ldw, int
 int mxp_mx_linear_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N,
                      const void* bias, int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo,
                      void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * Fused MX MLP (a transformer block's fc1 -> activation -> fc2, timm Mlp):
+ *     out = mx_linear(act(mx_linear(x, W1, b1)), W2, b2)
+ * as the library computes the composition, bit for bit: fc1's output is rounded to x's type (as mxp_mx_linear_dt
+ * stores it), the activation is torch.nn.functional.gelu on CUDA in fp32 opmath (bit-identical for every input)
+ * rounded to x's type again, and fc2 quantizes that along N1.  The fp32 rounding steps are identities.  The hidden
+ * activation is never written in a float type: fc1's epilogue applies the activation, quantizes each 32-element MX
+ * block in registers and writes fc2's bf16 operand into the workspace.
+ *   act      MXP_ACT_GELU (approximate='none', DeiT) or MXP_ACT_GELU_TANH (approximate='tanh', DiT, PixArt)
+ *   x        (M, K) rows of x_dtype with stride ldx (the rules of mxp_mx_linear_dt)
+ *   w1_op    fc1's prepared weight (N1, K);  w2_op  fc2's prepared weight (N2, N1)  (mxp_mx_linear_prepare_weight_dt)
+ *   b1, b2   N1 / N2 biases of any MXP_DT_* type each, or NULL
+ *   out      (M, N2) of x_dtype, row stride ldo (the rules of mxp_mx_linear_dt's out)
+ * K and N1 multiples of 64, N2 a multiple of 4.  Launches, in order: x's quantizer, the rounding of b1 and of b2 (each
+ * only when present), fc1 with the activation epilogue, fc2: 3 to 5 kernels.  workspace: mxp_mx_mlp_workspace_bytes
+ * bytes, 256-byte aligned (x's operand, the hidden operand ceil(M/128)*128 x N1 bf16, the rounded biases).
+ */
+#define MXP_ACT_GELU      0
+#define MXP_ACT_GELU_TANH 1
+size_t mxp_mx_mlp_workspace_bytes(int M, int K, int N1, int N2);
+int mxp_mx_mlp_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1,
+                  const void* b1, int b1_dtype, int act, const void* w2_op, int N2, const void* b2, int b2_dtype,
+                  int bfloat_bits, int flush, void* out, int64_t ldo,
+                  void* workspace, size_t workspace_bytes, void* stream);
+/*
+ * Parity aid: the fused MLP's activation applied elementwise to n contiguous elements of type dtype (MXP_DT_*), the
+ * result in the same type (rounded to nearest even from fp32 for 16-bit types).  Equals torch.nn.functional.gelu on
+ * CUDA bit for bit for every non-NaN input (NaN in, NaN out).
+ */
+int mxp_activation_dt(const void* x, int dtype, int64_t n, int act, void* out, void* stream);
 
 /*
  * Measurement aid: same as mxp_pruned_attention (tcgen05 path), but brackets the three kernels

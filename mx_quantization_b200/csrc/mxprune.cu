@@ -1335,6 +1335,40 @@ static int check_linear_rows(const char* name, const void* p, int dt, int64_t ld
     return MXP_OK;
 }
 
+// bias of element type dt -> A1(bias), N floats
+static int launch_round_bias(const void* bias, int dt, float* rbias, int N, int bf16, cudaStream_t st) {
+    const float* b = (const float*)bias;
+    const unsigned nblk = (unsigned)((N + 255) / 256);
+    if (dt == DT_BF16) k_round_bias<DT_BF16><<<nblk, 256, 0, st>>>(b, rbias, N, bf16);
+    else if (dt == DT_F16) k_round_bias<DT_F16><<<nblk, 256, 0, st>>>(b, rbias, N, bf16);
+    else k_round_bias<DT_F32><<<nblk, 256, 0, st>>>(b, rbias, N, bf16);
+    return check_launch("k_round_bias");
+}
+
+// k_mx_linear_umma<out_dt, EPI>: persistent, one CTA per SM (4 stages of 48 KiB, 512 TMEM columns for the
+// double-buffered accumulator); the same grid and shared memory for every output type and epilogue
+extern "C++" {
+template <int EPI>
+static int launch_linear_gemm(const LinearParams& lp, int out_dt, cudaStream_t st) {
+    const GemmOpLayout L = gemm_op_layout(lp.K);
+    const size_t dyn = lp.stages * (L.a_stage + L.b_stage) + 2048 + 4 * 32 * 36 * 4 + 1024;
+    const int ntiles = ((lp.M + GL_BM - 1) / GL_BM) * ((lp.N + GL_BN - 1) / GL_BN);
+    const int sms = sm_count();
+    const unsigned grid = (unsigned)(ntiles < sms ? ntiles : sms);
+    if (out_dt == DT_BF16) {
+        MXP_ENSURE_DYN_SMEM((k_mx_linear_umma<DT_BF16, EPI>), 227 * 1024);
+        k_mx_linear_umma<DT_BF16, EPI><<<grid, GL_T, dyn, st>>>(lp);
+    } else if (out_dt == DT_F16) {
+        MXP_ENSURE_DYN_SMEM((k_mx_linear_umma<DT_F16, EPI>), 227 * 1024);
+        k_mx_linear_umma<DT_F16, EPI><<<grid, GL_T, dyn, st>>>(lp);
+    } else {
+        MXP_ENSURE_DYN_SMEM((k_mx_linear_umma<DT_F32, EPI>), 227 * 1024);
+        k_mx_linear_umma<DT_F32, EPI><<<grid, GL_T, dyn, st>>>(lp);
+    }
+    return check_launch("k_mx_linear_umma");
+}
+}  // extern "C++"
+
 size_t mxp_mx_linear_weight_bytes(int N, int K) {
     return (size_t)((N + GL_BN - 1) / GL_BN) * GL_BN * (size_t)K * 2;
 }
@@ -1380,41 +1414,82 @@ int mxp_mx_linear_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, cons
     float* rbias = (float*)(a_op + align256((size_t)((M + GL_BM - 1) / GL_BM) * GL_BM * (size_t)K * 2));
     if ((rc = launch_quantize_gemm_operand(x, x_dtype, ldx, M, K, GL_BM, bfloat_bits == 16, flush != 0, a_op, st)))
         return rc;
-    if (bias) {
-        const float* b = (const float*)bias;
-        const unsigned nblk = (unsigned)((N + 255) / 256);
-        if (bias_dtype == DT_BF16) k_round_bias<DT_BF16><<<nblk, 256, 0, st>>>(b, rbias, N, bfloat_bits == 16);
-        else if (bias_dtype == DT_F16) k_round_bias<DT_F16><<<nblk, 256, 0, st>>>(b, rbias, N, bfloat_bits == 16);
-        else k_round_bias<DT_F32><<<nblk, 256, 0, st>>>(b, rbias, N, bfloat_bits == 16);
-        if ((rc = check_launch("k_round_bias"))) return rc;
-    }
+    if (bias && (rc = launch_round_bias(bias, bias_dtype, rbias, N, bfloat_bits == 16, st))) return rc;
     LinearParams lp{};
     lp.a_op = a_op; lp.w_op = (const unsigned char*)w_op; lp.bias = bias ? rbias : nullptr;
     lp.out = (float*)out; lp.ldo = ldo; lp.M = M; lp.N = N; lp.K = K; lp.bf16 = bfloat_bits == 16; lp.stages = 4;
-    const GemmOpLayout L = gemm_op_layout(K);
-    // persistent: one CTA per SM (4 stages of 48 KiB, 512 TMEM columns for the double-buffered accumulator); the
-    // same grid and shared memory for every output type
-    const size_t dyn = lp.stages * (L.a_stage + L.b_stage) + 2048 + 4 * 32 * 36 * 4 + 1024;
-    const int ntiles = ((M + GL_BM - 1) / GL_BM) * ((N + GL_BN - 1) / GL_BN);
-    int sms = 148;
-    {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess &&
-            cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0)
-            sms = n;
-    }
-    const unsigned grid = (unsigned)(ntiles < sms ? ntiles : sms);
-    if (x_dtype == DT_BF16) {
-        MXP_ENSURE_DYN_SMEM(k_mx_linear_umma<DT_BF16>, 227 * 1024);
-        k_mx_linear_umma<DT_BF16><<<grid, GL_T, dyn, st>>>(lp);
-    } else if (x_dtype == DT_F16) {
-        MXP_ENSURE_DYN_SMEM(k_mx_linear_umma<DT_F16>, 227 * 1024);
-        k_mx_linear_umma<DT_F16><<<grid, GL_T, dyn, st>>>(lp);
-    } else {
-        MXP_ENSURE_DYN_SMEM(k_mx_linear_umma<DT_F32>, 227 * 1024);
-        k_mx_linear_umma<DT_F32><<<grid, GL_T, dyn, st>>>(lp);
-    }
-    return check_launch("k_mx_linear_umma");
+    return launch_linear_gemm<EPI_STORE>(lp, x_dtype, st);
+}
+
+// ---- fused MX MLP: mx_linear(act(mx_linear(x, W1, b1)), W2, b2) with fc1's epilogue writing fc2's operand --------
+// workspace: x's operand | the hidden operand (fc2's A, K = N1) | A1(b1) | A1(b2)
+size_t mxp_mx_mlp_workspace_bytes(int M, int K, int N1, int N2) {
+    const size_t rows = (size_t)((M + GL_BM - 1) / GL_BM) * GL_BM;
+    return align256(rows * (size_t)K * 2) + align256(rows * (size_t)N1 * 2) + align256((size_t)N1 * 4) +
+           align256((size_t)N2 * 4);
+}
+
+int mxp_mx_mlp_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1, const void* b1,
+                  int b1_dtype, int act, const void* w2_op, int N2, const void* b2, int b2_dtype, int bfloat_bits,
+                  int flush, void* out, int64_t ldo, void* workspace, size_t workspace_bytes, void* stream) {
+    g_launches = 0;
+    int rc = check_linear(M, N1, K, bfloat_bits);
+    if (rc || (rc = check_linear(M, N2, N1, bfloat_bits))) return rc;         // fc2: K = N1, a multiple of 64
+    if (act != MXP_ACT_GELU && act != MXP_ACT_GELU_TANH)
+        return fail(MXP_E_BADARG, "act %d: MXP_ACT_GELU (0) or MXP_ACT_GELU_TANH (1)", act);
+    if ((rc = check_dtype("x", x_dtype)) || (rc = check_dtype("b1", b1_dtype)) || (rc = check_dtype("b2", b2_dtype)))
+        return rc;
+    if ((rc = check_linear_rows("x", x, x_dtype, ldx, K))) return rc;
+    const uintptr_t out_align = x_dtype == DT_F32 ? 15 : 7;
+    if (!w1_op || !w2_op || !out || ((uintptr_t)w1_op & 15) || ((uintptr_t)w2_op & 15) || ((uintptr_t)out & out_align) ||
+        (ldo & 3) || ldo < N2)
+        return fail(MXP_E_BADARG, "w1_op / w2_op / out: null or misaligned pointer, or out row stride %lld not >= %d and "
+                    "a multiple of 4", (long long)ldo, N2);
+    const size_t need = mxp_mx_mlp_workspace_bytes(M, K, N1, N2);
+    if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255))
+        return fail(MXP_E_BADARG, "workspace: need %zu bytes, 256-byte aligned", need);
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t rows = (size_t)((M + GL_BM - 1) / GL_BM) * GL_BM;
+    unsigned char* a_op = (unsigned char*)workspace;
+    unsigned char* h_op = a_op + align256(rows * (size_t)K * 2);
+    float* rb1 = (float*)(h_op + align256(rows * (size_t)N1 * 2));
+    float* rb2 = (float*)((unsigned char*)rb1 + align256((size_t)N1 * 4));
+    const int bf16 = bfloat_bits == 16;
+    if ((rc = launch_quantize_gemm_operand(x, x_dtype, ldx, M, K, GL_BM, bf16, flush != 0, a_op, st))) return rc;
+    if (b1 && (rc = launch_round_bias(b1, b1_dtype, rb1, N1, bf16, st))) return rc;
+    if (b2 && (rc = launch_round_bias(b2, b2_dtype, rb2, N2, bf16, st))) return rc;
+    LinearParams l1{};
+    l1.a_op = a_op; l1.w_op = (const unsigned char*)w1_op; l1.bias = b1 ? rb1 : nullptr;
+    l1.M = M; l1.N = N1; l1.K = K; l1.bf16 = bf16; l1.stages = 4; l1.flush = flush != 0; l1.h_op = h_op;
+    rc = act == MXP_ACT_GELU_TANH ? launch_linear_gemm<EPI_GELU_TANH>(l1, x_dtype, st)
+                                  : launch_linear_gemm<EPI_GELU>(l1, x_dtype, st);
+    if (rc) return rc;
+    LinearParams l2{};
+    l2.a_op = h_op; l2.w_op = (const unsigned char*)w2_op; l2.bias = b2 ? rb2 : nullptr;
+    l2.out = (float*)out; l2.ldo = ldo; l2.M = M; l2.N = N2; l2.K = N1; l2.bf16 = bf16; l2.stages = 4;
+    return launch_linear_gemm<EPI_STORE>(l2, x_dtype, st);
+}
+
+int mxp_activation_dt(const void* x, int dtype, int64_t n, int act, void* out, void* stream) {
+    g_launches = 0;
+    int rc = check_dtype("x", dtype);
+    if (rc) return rc;
+    if (act != MXP_ACT_GELU && act != MXP_ACT_GELU_TANH)
+        return fail(MXP_E_BADARG, "act %d: MXP_ACT_GELU (0) or MXP_ACT_GELU_TANH (1)", act);
+    if (n < 0 || (n > 0 && (!x || !out))) return fail(MXP_E_BADARG, "x / out: null pointer, or n = %lld < 0", (long long)n);
+    if (n == 0) return MXP_OK;
+    int64_t blocks = (n + 255) / 256;
+    if (blocks > (int64_t)sm_count() * 32) blocks = (int64_t)sm_count() * 32;
+    cudaStream_t st = (cudaStream_t)stream;
+    const float* xp = (const float*)x;
+    float* o = (float*)out;
+#define MXP_ACT(DT_) (act == MXP_ACT_GELU_TANH ? k_activation<DT_, EPI_GELU_TANH><<<(unsigned)blocks, 256, 0, st>>>(xp, n, o) \
+                                               : k_activation<DT_, EPI_GELU><<<(unsigned)blocks, 256, 0, st>>>(xp, n, o))
+    if (dtype == DT_BF16) MXP_ACT(DT_BF16);
+    else if (dtype == DT_F16) MXP_ACT(DT_F16);
+    else MXP_ACT(DT_F32);
+#undef MXP_ACT
+    return check_launch("k_activation");
 }
 
 int mxp_mx_linear(const float* x, int64_t ldx, int M, int K, const void* w_op, int N, const float* bias,

@@ -18,6 +18,9 @@
 //                            Persistent, one CTA per SM walking the output tiles; the accumulator is
 //                            double-buffered in TMEM (2 x 256 columns), so the epilogue of one tile overlaps
 //                            the main loop of the next.
+//                            EPI = EPI_GELU / EPI_GELU_TANH (the fused MLP's fc1): the epilogue applies the
+//                            activation and writes the NEXT GEMM's A operand instead of the output; each 32-column
+//                            pass over a TMEM row is one MX block of fc2's input, held by one thread.
 #pragma once
 #include "mxprune_predict_tc.cuh"
 
@@ -63,12 +66,53 @@ k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int r
     }
 }
 
+// Epilogues of k_mx_linear_umma: store the output, or apply an activation (MXP_ACT_* + 1) and write the next GEMM's
+// A operand.
+constexpr int EPI_STORE = 0, EPI_GELU = 1, EPI_GELU_TANH = 2;
+
+// torch.nn.functional.gelu on CUDA, bit for bit: ATen's GeluCUDAKernelImpl (ActivationGeluKernel.cu) in fp32 opmath,
+//     approximate='none'  x * 0.5 * (1 + erf(x * M_SQRT1_2))
+//     approximate='tanh'  0.5 * x * (1 + tanh(sqrt(2/pi) * (x + 0.044715 * x^3)))
+// with the operation order and the one contraction (kappa * x^3 + x -> FFMA) of torch's sm_100 SASS, and the same
+// CUDA libdevice erff / tanhf.  Explicit _rn intrinsics keep the compiler from contracting anything else.
+__device__ __forceinline__ float gelu_erf(float x) {
+    return __fmul_rn(__fmul_rn(x, 0.5f), __fadd_rn(1.0f, erff(__fmul_rn(x, 0.70710678118654752440f))));
+}
+__device__ __forceinline__ float gelu_tanh(float x) {
+    const float inner = __fmul_rn(0.7978845608028654f, __fmaf_rn(0.044715f, __fmul_rn(__fmul_rn(x, x), x), x));
+    return __fmul_rn(__fmul_rn(x, 0.5f), __fadd_rn(1.0f, tanhf(inner)));
+}
+template <int EPI>
+__device__ __forceinline__ float activation(float x) {
+    return EPI == EPI_GELU_TANH ? gelu_tanh(x) : gelu_erf(x);
+}
+// an fp32 value rounded to nearest even in DT and widened back (identity for fp32)
+template <int DT>
+__device__ __forceinline__ float round_to_dt(float x) {
+    if constexpr (DT == DT_BF16) return __bfloat162float(__float2bfloat16_rn(x));
+    else if constexpr (DT == DT_F16) return __half2float(__float2half_rn(x));
+    else return x;
+}
+
+// elementwise activation of n elements of type DT (the fused epilogue's function; parity aid)
+template <int DT, int EPI>
+__global__ void k_activation(const float* __restrict__ x, int64_t n, float* __restrict__ out) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const float y = activation<EPI>(__uint_as_float(load_elem_bits<DT>(x, i)));
+        if constexpr (DT == DT_F32) out[i] = y;
+        else if constexpr (DT == DT_BF16) reinterpret_cast<__nv_bfloat16*>(out)[i] = __float2bfloat16_rn(y);
+        else reinterpret_cast<__half*>(out)[i] = __float2half_rn(y);
+    }
+}
+
 struct LinearParams {
     const unsigned char *a_op, *w_op;
     const float* bias;                // already A1-rounded by the host wrapper kernel, or null
     float* out;                       // elements of the kernel's OUT_DT
     int64_t ldo;
     int M, N, K, bf16, stages;
+    int flush;                        // EPI != EPI_STORE: the next GEMM's quantizer setting
+    unsigned char* h_op;              // EPI != EPI_STORE: the next GEMM's A operand (K = N), written instead of out
 };
 
 // bias of element type DT -> A1(bias), N floats (tiny)
@@ -91,8 +135,10 @@ __device__ __forceinline__ void epilogue_barrier() {               // the 128 ep
 // Persistent: one CTA per SM walks the output tiles (feature tile fastest, so the CTAs that share an
 // activation tile run together and the weight operand stays L2-resident).  The accumulator is
 // double-buffered in TMEM (2 x 256 columns): the epilogue of tile i overlaps the main loop of tile i+1.
-// OUT_DT (DT_*) is the element type of p.out; only the final store depends on it.
-template <int OUT_DT>
+// OUT_DT (DT_*) is the element type of p.out; only the final store depends on it.  With EPI != EPI_STORE it is the
+// type the output and the activation are rounded to before fc2's quantizer reads them (what mx_linear stores and
+// what torch's GELU returns on a tensor of that type).
+template <int OUT_DT, int EPI = EPI_STORE>
 __global__ void __launch_bounds__(GL_T, 1)
 k_mx_linear_umma(const LinearParams p) {
     extern __shared__ __align__(1024) unsigned char smem_gl[];
@@ -176,11 +222,56 @@ k_mx_linear_umma(const LinearParams p) {
             const int tile_m = t / tiles_n, tile_n = t - tile_m * tiles_n;
             const int n0 = tile_n * GL_BN, buf = i & 1;
             float* sb = s_bias + buf * GL_BN;
-            for (int j = et; j < GL_BN; j += 128) sb[j] = (p.bias && n0 + j < p.N) ? __ldg(p.bias + n0 + j) : 0.f;
+            const float no_bias = EPI == EPI_STORE ? 0.f : -0.f;            // -0: the identity of the GELU epilogue's add
+            for (int j = et; j < GL_BN; j += 128) sb[j] = (p.bias && n0 + j < p.N) ? __ldg(p.bias + n0 + j) : no_bias;
             epilogue_barrier();
             mbar_wait(&bar_acc_full[buf], (uint32_t)((i >> 1) & 1));
             tcgen05_fence_after_sync();
             const uint32_t t0 = tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * GL_BN);
+            if constexpr (EPI != EPI_STORE) {
+                // thread = row; 32 TMEM columns = one MX block of fc2's input (n0 + c0 is a multiple of 32).  The
+                // block is quantized in registers and its four 16-byte chunks go straight to fc2's A operand
+                // [row tile][k step of 64][8 chunks][128 rows][16 B]: a warp writes 512 contiguous bytes per chunk.
+                const int row = tile_m * GL_BM + q * 32 + lane;
+                const int cend = p.N - n0 < GL_BN ? p.N - n0 : GL_BN;          // N is a multiple of 64
+                const size_t stage_bytes = (size_t)8 * GL_BM * 16;
+                unsigned char* h_tile = p.h_op + (size_t)tile_m * (p.N / GL_BK) * stage_bytes + (size_t)(q * 32 + lane) * 16;
+#pragma unroll 1
+                for (int c0 = 0; c0 < cend; c0 += 32) {
+                    uint32_t xv[32];
+                    tmem_ld_32x32b_x32(t0 + c0, xv);
+                    tmem_ld_wait();
+                    // branch-free, so that the 32 independent activations interleave: without a bias sb holds -0,
+                    // and A1(A1(y) + -0) == A1(y) for every y (A1 is idempotent), which is the store epilogue's value
+#pragma unroll
+                    for (int j4 = 0; j4 < 32; j4 += 4) {
+                        const float4 b4 = *reinterpret_cast<const float4*>(sb + c0 + j4);
+                        const float bj[4] = {b4.x, b4.y, b4.z, b4.w};
+#pragma unroll
+                        for (int j = 0; j < 4; ++j) {
+                            float y = __uint_as_float(xv[j4 + j]);
+                            if (bf16) y = bf16_half_away(y);                    // A1, linear.py:85-87
+                            y = __fadd_rn(y, bj[j]);
+                            if (bf16) y = bf16_half_away(y);                    // :89-93
+                            xv[j4 + j] = __float_as_uint(round_to_dt<OUT_DT>(y));
+                        }
+                    }
+                    const uint32_t row_mask = row < p.M ? ~0u : 0u;             // padding rows: zero operand rows
+#pragma unroll
+                    for (int j = 0; j < 32; ++j)
+                        xv[j] = __float_as_uint(round_to_dt<OUT_DT>(activation<EPI>(__uint_as_float(xv[j])))) & row_mask;
+                    BlockQ r;
+                    quantize_block_thread<false, false>(xv, 32, bf16, p.flush != 0, r);
+                    const int b = (n0 + c0) >> 5;
+                    unsigned char* dst = h_tile + (size_t)(b >> 1) * stage_bytes + (size_t)((b & 1) * 4) * GL_BM * 16;
+#pragma unroll
+                    for (int ch = 0; ch < 4; ++ch) *reinterpret_cast<uint4*>(dst + (size_t)ch * GL_BM * 16) = r.op[ch];
+                }
+                tcgen05_fence_before_sync();
+                epilogue_barrier();
+                if (et == 0) mbar_arrive(&bar_acc_empty[buf]);
+                continue;
+            }
             // Coalesced stores: each warp transposes its 32 rows x 32 columns through shared memory
             // (row pitch 36 words: conflict-free 128-bit writes and reads), so that 8 lanes write 128
             // contiguous bytes of one fp32 output row (64 bytes of a 16-bit one) instead of 32 lanes

@@ -129,7 +129,12 @@ class QuantizedAttention(nn.Module):
 
 class QuantizedMlp(nn.Module):
     """DeiT MLP with MX Linear layers - mirrors workloads/deit/scripts/main.py:159-196 (fc1 -> act -> fc2 -> drop;
-    the activation stays the host model's own module, as in the reference)."""
+    the activation stays the host model's own module, as in the reference).
+
+    When the activation is exactly ``torch.nn.GELU`` (either approximation) and fc1 / fc2 share one MX configuration, the
+    forward is one ops.mx_mlp call on the layers' cached weight operands: bit for bit the layer-by-layer composition, with
+    the hidden activation never written in a float type.  Any other activation (a subclass or another GELU class too)
+    runs the composition."""
 
     def __init__(self, orig_mlp, mx_specs=None):
         super().__init__()
@@ -139,6 +144,15 @@ class QuantizedMlp(nn.Module):
         self.fc1, self.fc2 = to_mx_linear(orig_mlp.fc1, mx_specs), to_mx_linear(orig_mlp.fc2, mx_specs)
 
     def forward(self, x):
+        if type(self.act) is nn.GELU and resolve_linear_specs(self.fc1.mx_specs) == resolve_linear_specs(self.fc2.mx_specs):
+            self.fc1._check_inference(x.requires_grad)
+            self.fc2._check_inference(False)
+            b1 = None if self.fc1.bias is None else self.fc1.bias.detach()
+            b2 = None if self.fc2.bias is None else self.fc2.bias.detach()
+            y = ops.mx_mlp(x, self.fc1._operand(), b1, self.fc2._operand(), b2, self.fc1.mx_specs,
+                           act="gelu_tanh" if self.act.approximate == "tanh" else "gelu",
+                           hidden_features=self.fc1.out_features, out_features=self.fc2.out_features)
+            return self.drop(y)
         return self.drop(self.fc2(self.act(self.fc1(x))))
 
 
@@ -293,13 +307,21 @@ class MxLinear(nn.Linear):
         self._w_op = None
         self._w_key = None
 
-    def forward(self, inputs):
-        if torch.is_grad_enabled() and (self.weight.requires_grad or inputs.requires_grad):
+    def _check_inference(self, inputs_require_grad: bool):
+        if torch.is_grad_enabled() and (self.weight.requires_grad or inputs_require_grad):
             raise RuntimeError("MxLinear is the inference forward of mx.Linear (the reference's backward is out of scope): "
                                "call it under torch.no_grad() / inference_mode, or freeze the parameters")
+
+    def _operand(self) -> torch.Tensor:
+        """The cached MX-quantized weight operand, rebuilt when the weight tensor has changed."""
         key = (self.weight.data_ptr(), self.weight._version, str(self.weight.device), self.weight.dtype)
         if self._w_op is None or self._w_key != key:
             self._w_op = ops.mx_linear_prepare_weight(self.weight.detach(), self.mx_specs)
             self._w_key = key
+        return self._w_op
+
+    def forward(self, inputs):
+        self._check_inference(inputs.requires_grad)
+        w_op = self._operand()
         b = None if self.bias is None else self.bias.detach()
-        return ops.mx_linear(inputs, self._w_op, b, self.mx_specs, out_features=self.out_features)
+        return ops.mx_linear(inputs, w_op, b, self.mx_specs, out_features=self.out_features)

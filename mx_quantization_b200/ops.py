@@ -472,6 +472,26 @@ def _linear_rows(x: torch.Tensor) -> torch.Tensor:
     return x2
 
 
+def _weight_operand(weight: torch.Tensor, K: int, out_features: Optional[int], mx_specs,
+                    what: str = "out_features") -> Tuple[torch.Tensor, int]:
+    """(w_op, N): a prepared operand checked against (out_features, K), or a raw (N, K) weight quantized now."""
+    lib = _lib.load()
+    if weight.dtype == torch.uint8:
+        if out_features is None:
+            raise ValueError(f"{what} is required with a prepared weight operand")
+        N = int(out_features)
+        if not weight.is_contiguous() or weight.numel() != lib.mxp_mx_linear_weight_bytes(N, K):
+            raise ValueError(f"prepared weight operand: expected {lib.mxp_mx_linear_weight_bytes(N, K)} contiguous bytes for "
+                             f"out_features={N}, in_features={K}, got {weight.numel()}")
+        return weight, N
+    return mx_linear_prepare_weight(weight, mx_specs), weight.shape[0]
+
+
+def _check_bias(bias: Optional[torch.Tensor], N: int) -> None:
+    if bias is not None and (bias.dtype not in DTYPE_CODES or bias.numel() != N or not bias.is_contiguous()):
+        raise ValueError("bias must be a contiguous float32, bfloat16 or float16 tensor with out_features elements")
+
+
 def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
               out_features: Optional[int] = None) -> torch.Tensor:
     """Forward of the reference's mx.Linear (microxscaling/mx/linear.py:20-103) for MXINT8:
@@ -488,18 +508,8 @@ def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
     if not x.is_cuda:
         raise ValueError("x must be a CUDA tensor; there is no CPU fallback")
     K, M = x2.shape[1], x2.shape[0]
-    if weight.dtype == torch.uint8:
-        if out_features is None:
-            raise ValueError("out_features is required with a prepared weight operand")
-        w_op, N = weight, int(out_features)
-        if not w_op.is_contiguous() or w_op.numel() != lib.mxp_mx_linear_weight_bytes(N, K):
-            raise ValueError(f"prepared weight operand: expected {lib.mxp_mx_linear_weight_bytes(N, K)} contiguous bytes for "
-                             f"out_features={N}, in_features={K}, got {w_op.numel()}")
-    else:
-        N = weight.shape[0]
-        w_op = mx_linear_prepare_weight(weight, mx_specs)
-    if bias is not None and (bias.dtype not in DTYPE_CODES or bias.numel() != N or not bias.is_contiguous()):
-        raise ValueError("bias must be a contiguous float32, bfloat16 or float16 tensor with out_features elements")
+    w_op, N = _weight_operand(weight, K, out_features, mx_specs)
+    _check_bias(bias, N)
     _same_device(x, w_op, bias)
     with torch.cuda.device(x.device):
         out = torch.empty((M, N), dtype=x.dtype, device=x.device)
@@ -510,3 +520,68 @@ def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
                                   int(sp.flush), _ptr(out), out.stride(0), _ptr(ws), ws_bytes, _stream())
     _lib.check(rc, "mxp_mx_linear")
     return out.reshape(*x.shape[:-1], N)
+
+
+# ---- fused MX MLP -----------------------------------------------------------------------------------------------------
+ACTIVATIONS = {"gelu": _lib.MXP_ACT_GELU, "gelu_tanh": _lib.MXP_ACT_GELU_TANH}
+
+
+def _act_code(act: str) -> int:
+    if act not in ACTIVATIONS:
+        raise ValueError(f"act must be one of {sorted(ACTIVATIONS)}, got {act!r}")
+    return ACTIVATIONS[act]
+
+
+def mx_mlp(x: torch.Tensor, w1, b1: Optional[torch.Tensor], w2, b2: Optional[torch.Tensor], mx_specs,
+           act: str = "gelu", hidden_features: Optional[int] = None, out_features: Optional[int] = None) -> torch.Tensor:
+    """A transformer MLP (fc1 -> GELU -> fc2) on MX Linear layers, fused:
+    ``mx_linear(F.gelu(mx_linear(x, w1, b1), approximate=...), w2, b2)`` bit for bit, with the hidden activation never
+    written in a float type (fc1's epilogue applies the GELU and writes fc2's MXINT8 operand).
+
+    ``act``: "gelu" (``approximate='none'``, DeiT) or "gelu_tanh" (``approximate='tanh'``, DiT, PixArt).  ``w1`` / ``w2``:
+    the (N1, K) / (N2, N1) weights, or operands from mx_linear_prepare_weight (then pass ``hidden_features`` /
+    ``out_features``).  ``x``, weights and biases: the dtype and stride rules of mx_linear; the result has x's dtype.
+    K and N1 must be multiples of 64, N2 a multiple of 4."""
+    sp = resolve_linear_specs(mx_specs)
+    code = _act_code(act)
+    lib = _lib.load()
+    x2 = _linear_rows(x)
+    if not x.is_cuda:
+        raise ValueError("x must be a CUDA tensor; there is no CPU fallback")
+    K, M = x2.shape[1], x2.shape[0]
+    for name, w, k_in in (("w1", w1, K), ("w2", w2, None)):
+        if not isinstance(w, torch.Tensor):
+            raise TypeError(f"{name}: expected a torch.Tensor")
+        if w.dtype != torch.uint8 and (w.dim() != 2 or (k_in is not None and w.shape[1] != k_in)):
+            raise ValueError(f"{name}: expected an (out_features, {k_in or 'in_features'}) weight, got {tuple(w.shape)}")
+    w1_op, N1 = _weight_operand(w1, K, hidden_features, mx_specs, "hidden_features")
+    if w2.dtype != torch.uint8 and w2.shape[1] != N1:
+        raise ValueError(f"w2: expected ({w2.shape[0]}, {N1}) for {N1} hidden features, got {tuple(w2.shape)}")
+    w2_op, N2 = _weight_operand(w2, N1, out_features, mx_specs)
+    _check_bias(b1, N1)
+    _check_bias(b2, N2)
+    _same_device(x, w1_op, b1, w2_op, b2)
+    with torch.cuda.device(x.device):
+        out = torch.empty((M, N2), dtype=x.dtype, device=x.device)
+        ws_bytes = lib.mxp_mx_mlp_workspace_bytes(M, K, N1, N2)
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=x.device)
+        f32 = _lib.MXP_DT_F32
+        rc = lib.mxp_mx_mlp_dt(_ptr(x2), DTYPE_CODES[x.dtype], x2.stride(0), M, K, _ptr(w1_op), N1, _ptr(b1),
+                               DTYPE_CODES[b1.dtype] if b1 is not None else f32, code, _ptr(w2_op), N2, _ptr(b2),
+                               DTYPE_CODES[b2.dtype] if b2 is not None else f32, sp.bfloat_bits, int(sp.flush),
+                               _ptr(out), out.stride(0), _ptr(ws), ws_bytes, _stream())
+    _lib.check(rc, "mxp_mx_mlp")
+    return out.reshape(*x.shape[:-1], N2)
+
+
+def activation(x: torch.Tensor, act: str = "gelu") -> torch.Tensor:
+    """The fused MLP's activation applied elementwise (parity aid): equals ``torch.nn.functional.gelu(x, approximate=...)``
+    on CUDA bit for bit.  ``x``: a contiguous CUDA float32, bfloat16 or float16 tensor; the result has its dtype."""
+    code = _act_code(act)
+    if not isinstance(x, torch.Tensor) or not x.is_cuda or x.dtype not in DTYPE_CODES or not x.is_contiguous():
+        raise ValueError("x must be a contiguous CUDA float32, bfloat16 or float16 tensor")
+    with torch.cuda.device(x.device):
+        out = torch.empty_like(x)
+        rc = _lib.load().mxp_activation_dt(_ptr(x), DTYPE_CODES[x.dtype], x.numel(), code, _ptr(out), _stream())
+    _lib.check(rc, "mxp_activation_dt")
+    return out
