@@ -47,7 +47,7 @@
 extern "C" {
 #endif
 
-#define MXP_ABI_VERSION 6
+#define MXP_ABI_VERSION 7
 
 /*
  * Element types of q/k/v/x and out for the *_dt entry points.  The fp32 entry points are the *_dt ones with
@@ -342,6 +342,35 @@ int mxp_mx_mlp_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const v
  * CUDA bit for bit for every non-NaN input (NaN in, NaN out).
  */
 int mxp_activation_dt(const void* x, int dtype, int64_t n, int act, void* out, void* stream);
+
+/*
+ * adaLN-modulated MX Linear / MLP (DiT's DiTBlock, PixArt's adaLN-single block):
+ *     out = residual + gate * mx_linear(x * (1 + scale) + shift, W, bias)
+ * mxp_mx_linear_adaln_dt takes the arguments of mxp_mx_linear_dt; mxp_mx_mlp_adaln_dt those of mxp_mx_mlp_dt, with the
+ * modulation applied to x (fc1's operand) and the gated residual to fc2's output.  The M rows are B = M / tokens batch
+ * entries of `tokens` rows each; row r belongs to entry b = r / tokens.  Every added tensor has x_dtype.
+ *   shift, scale      (B, K) rows with strides ld_shift / ld_scale (the rules of x); both NULL, or both given.  The GEMM
+ *                     operand is quantized from v = rd(rd(x * rd(1 + scale[b])) + shift[b]) instead of x.
+ *   residual          (M, N) rows with stride ld_residual;  gate  (B, N) rows with stride ld_gate (both the rules of
+ *                     out); both NULL, or both given.  The stored value is rd(residual + rd(gate[b] * y)), where y is
+ *                     the value mxp_mx_linear_dt stores (already rounded to x_dtype).
+ * Each operation is one fp32 add or multiply (no contraction), rd rounds to nearest even in x_dtype (the identity for
+ * fp32): the expressions as eager torch evaluates them on tensors of x_dtype, so the result equals the torch
+ * composition with the plain entry point bit for bit.  shift / scale / gate may be column slices of one (B, 6C) row
+ * (DiT's adaLN_modulation(c).chunk(6, dim=1)), read in place.  Padding rows of a partial 128-row tile read none of
+ * them.  tokens must divide M.  The launches and the workspace are those of the plain call.
+ */
+int mxp_mx_linear_adaln_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N,
+                           const void* bias, int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo,
+                           int tokens, const void* shift, int64_t ld_shift, const void* scale, int64_t ld_scale,
+                           const void* residual, int64_t ld_residual, const void* gate, int64_t ld_gate,
+                           void* workspace, size_t workspace_bytes, void* stream);
+int mxp_mx_mlp_adaln_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1,
+                        const void* b1, int b1_dtype, int act, const void* w2_op, int N2, const void* b2, int b2_dtype,
+                        int bfloat_bits, int flush, void* out, int64_t ldo, int tokens, const void* shift,
+                        int64_t ld_shift, const void* scale, int64_t ld_scale, const void* residual,
+                        int64_t ld_residual, const void* gate, int64_t ld_gate, void* workspace,
+                        size_t workspace_bytes, void* stream);
 
 /*
  * Measurement aid: same as mxp_pruned_attention (tcgen05 path), but brackets the three kernels

@@ -9,13 +9,14 @@ from ctypes import c_float, c_int, c_int64, c_size_t, c_void_p
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # MXPRUNE_LIB: developer override (e.g. the phase-accounting build csrc/libmxprune_timing.so, `make timing`)
 LIB_PATH = os.environ.get("MXPRUNE_LIB") or os.path.join(_HERE, "csrc", "libmxprune.so")
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 MXP_OK, MXP_E_BADARG, MXP_E_UNSUPPORTED, MXP_E_CUDA = 0, -1, -2, -3
 MXP_DT_F32, MXP_DT_BF16, MXP_DT_F16 = 0, 1, 2
 MXP_ACT_GELU, MXP_ACT_GELU_TANH = 0, 1
 
 _VIEW = [c_void_p, c_int64, c_int64, c_int64]          # ptr, sB, sH, sN
+_ADALN = [c_int] + [c_void_p, c_int64] * 4              # tokens, shift, scale, residual, gate (each with its row stride)
 
 _SIGNATURES = {
     "mxp_abi_version": (c_int, []),
@@ -67,6 +68,11 @@ _SIGNATURES = {
     "mxp_mx_mlp_dt": (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p,
                               c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
     "mxp_activation_dt": (c_int, [c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p]),
+    "mxp_mx_linear_adaln_dt": (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_int,
+                                       c_int, c_void_p, c_int64] + _ADALN + [c_void_p, c_size_t, c_void_p]),
+    "mxp_mx_mlp_adaln_dt": (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_int,
+                                    c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_int64] + _ADALN
+                            + [c_void_p, c_size_t, c_void_p]),
     "mxp_pruned_attention_profile": (c_int, _VIEW * 3 + [c_int] * 6 + [c_float, c_int, c_int] + _VIEW
                                      + [c_void_p, c_void_p, c_size_t, c_void_p, ctypes.POINTER(c_float)]),
 }

@@ -1310,14 +1310,17 @@ static int check_linear(int M, int N, int K, int bfloat_bits) {
     if (bfloat_bits != 16 && bfloat_bits != 32) return fail(MXP_E_UNSUPPORTED, "bfloat=%d: only 16 or 32 are on the path", bfloat_bits);
     return MXP_OK;
 }
+// mod: the adaLN modulation of x (ModParams), or null
 static int launch_quantize_gemm_operand(const void* x, int dt, int64_t ld, int rows, int K, int rows_tile, int bf16,
-                                        int flush, void* op, cudaStream_t st) {
+                                        int flush, void* op, cudaStream_t st, const ModParams* mod = nullptr) {
     const int rows_pad = (rows + rows_tile - 1) / rows_tile * rows_tile;
     const int64_t ntask = (int64_t)rows_pad * (K / 32);
     int64_t blocks = (ntask + 255) / 256;
     if (blocks > 148 * 32) blocks = 148 * 32;
-#define MXP_QG(DT_) k_quantize_gemm_operand<DT_><<<(unsigned)blocks, 256, 0, st>>>((const float*)x, ld, rows, rows_pad, K, \
-                                                                                rows_tile, bf16, flush, (unsigned char*)op)
+#define MXP_QG(DT_) (mod ? k_quantize_gemm_operand<DT_, true><<<(unsigned)blocks, 256, 0, st>>>( \
+                               (const float*)x, ld, rows, rows_pad, K, rows_tile, bf16, flush, (unsigned char*)op, *mod) \
+                         : k_quantize_gemm_operand<DT_><<<(unsigned)blocks, 256, 0, st>>>( \
+                               (const float*)x, ld, rows, rows_pad, K, rows_tile, bf16, flush, (unsigned char*)op, ModParams{}))
     if (dt == DT_BF16) MXP_QG(DT_BF16);
     else if (dt == DT_F16) MXP_QG(DT_F16);
     else MXP_QG(DT_F32);
@@ -1393,9 +1396,50 @@ int mxp_mx_linear_prepare_weight(const float* w, int64_t ldw, int N, int K, int 
     return mxp_mx_linear_prepare_weight_dt(w, MXP_DT_F32, ldw, N, K, bfloat_bits, flush, w_op, stream);
 }
 
-int mxp_mx_linear_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N, const void* bias,
-                     int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo, void* workspace,
-                     size_t workspace_bytes, void* stream) {
+// ---- adaLN additions of mxp_mx_linear_adaln_dt / mxp_mx_mlp_adaln_dt: the modulation of x (mod, K wide) and the
+// gated residual of the output (N wide), each optional
+struct Adaln {
+    int tokens;
+    const void *shift, *scale, *residual, *gate;
+    int64_t ld_shift, ld_scale, ld_residual, ld_gate;
+};
+
+// an (M / tokens, N) gate or (M, N) residual of x's type: the alignment and row-stride rules of out
+static int check_out_like(const char* name, const void* p, int dt, int64_t ld, int N) {
+    const uintptr_t align = dt == DT_F32 ? 15 : 7;
+    if (!p || ((uintptr_t)p & align) || (ld & 3) || ld < N)
+        return fail(MXP_E_BADARG, "%s: null or misaligned pointer, or row stride %lld not >= %d and a multiple of 4",
+                    name, (long long)ld, N);
+    return MXP_OK;
+}
+
+static int check_adaln(const Adaln& a, int dt, int M, int K, int N) {
+    if (a.tokens <= 0 || M % a.tokens)
+        return fail(MXP_E_BADARG, "tokens %d: need a positive divisor of the row count M=%d", a.tokens, M);
+    if (!a.shift != !a.scale) return fail(MXP_E_BADARG, "shift and scale: give both or neither");
+    if (!a.residual != !a.gate) return fail(MXP_E_BADARG, "residual and gate: give both or neither");
+    int rc = MXP_OK;
+    // shift / scale are read in 32-element blocks, 16 bytes at a time: the rules of x
+    if (a.shift && ((rc = check_linear_rows("shift", a.shift, dt, a.ld_shift, K)) ||
+                    (rc = check_linear_rows("scale", a.scale, dt, a.ld_scale, K))))
+        return rc;
+    if (a.residual && ((rc = check_out_like("residual", a.residual, dt, a.ld_residual, N)) ||
+                       (rc = check_out_like("gate", a.gate, dt, a.ld_gate, N))))
+        return rc;
+    return MXP_OK;
+}
+
+static ModParams make_mod(const Adaln& a) {
+    return ModParams{(const float*)a.shift, (const float*)a.scale, a.ld_shift, a.ld_scale, a.tokens};
+}
+static void set_gated_residual(LinearParams& lp, const Adaln& a) {
+    lp.residual = (const float*)a.residual; lp.ldr = a.ld_residual;
+    lp.gate = (const float*)a.gate; lp.ldg = a.ld_gate; lp.tokens = a.tokens;
+}
+
+static int mx_linear_impl(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N,
+                          const void* bias, int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo,
+                          const Adaln* ad, void* workspace, size_t workspace_bytes, void* stream) {
     g_launches = 0;
     int rc = check_linear(M, N, K, bfloat_bits);
     if (rc) return rc;
@@ -1406,19 +1450,44 @@ int mxp_mx_linear_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, cons
     if (!w_op || !out || ((uintptr_t)w_op & 15) || ((uintptr_t)out & out_align) || (ldo & 3) || ldo < N)
         return fail(MXP_E_BADARG, "w_op / out: null or misaligned pointer, or out row stride %lld not >= %d and a multiple "
                     "of 4", (long long)ldo, N);
+    if (ad && (rc = check_adaln(*ad, x_dtype, M, K, N))) return rc;
     const size_t need = mxp_mx_linear_workspace_bytes(M, N, K);
     if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255))
         return fail(MXP_E_BADARG, "workspace: need %zu bytes, 256-byte aligned", need);
     cudaStream_t st = (cudaStream_t)stream;
     unsigned char* a_op = (unsigned char*)workspace;
     float* rbias = (float*)(a_op + align256((size_t)((M + GL_BM - 1) / GL_BM) * GL_BM * (size_t)K * 2));
-    if ((rc = launch_quantize_gemm_operand(x, x_dtype, ldx, M, K, GL_BM, bfloat_bits == 16, flush != 0, a_op, st)))
+    ModParams mod{};
+    if (ad && ad->shift) mod = make_mod(*ad);
+    if ((rc = launch_quantize_gemm_operand(x, x_dtype, ldx, M, K, GL_BM, bfloat_bits == 16, flush != 0, a_op, st,
+                                           ad && ad->shift ? &mod : nullptr)))
         return rc;
     if (bias && (rc = launch_round_bias(bias, bias_dtype, rbias, N, bfloat_bits == 16, st))) return rc;
     LinearParams lp{};
     lp.a_op = a_op; lp.w_op = (const unsigned char*)w_op; lp.bias = bias ? rbias : nullptr;
     lp.out = (float*)out; lp.ldo = ldo; lp.M = M; lp.N = N; lp.K = K; lp.bf16 = bfloat_bits == 16; lp.stages = 4;
+    if (ad && ad->residual) {
+        set_gated_residual(lp, *ad);
+        return launch_linear_gemm<EPI_GATED_RESIDUAL>(lp, x_dtype, st);
+    }
     return launch_linear_gemm<EPI_STORE>(lp, x_dtype, st);
+}
+
+int mxp_mx_linear_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N, const void* bias,
+                     int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+    return mx_linear_impl(x, x_dtype, ldx, M, K, w_op, N, bias, bias_dtype, bfloat_bits, flush, out, ldo, nullptr,
+                          workspace, workspace_bytes, stream);
+}
+
+int mxp_mx_linear_adaln_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N,
+                           const void* bias, int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo,
+                           int tokens, const void* shift, int64_t ld_shift, const void* scale, int64_t ld_scale,
+                           const void* residual, int64_t ld_residual, const void* gate, int64_t ld_gate,
+                           void* workspace, size_t workspace_bytes, void* stream) {
+    const Adaln ad{tokens, shift, scale, residual, gate, ld_shift, ld_scale, ld_residual, ld_gate};
+    return mx_linear_impl(x, x_dtype, ldx, M, K, w_op, N, bias, bias_dtype, bfloat_bits, flush, out, ldo, &ad,
+                          workspace, workspace_bytes, stream);
 }
 
 // ---- fused MX MLP: mx_linear(act(mx_linear(x, W1, b1)), W2, b2) with fc1's epilogue writing fc2's operand --------
@@ -1429,9 +1498,10 @@ size_t mxp_mx_mlp_workspace_bytes(int M, int K, int N1, int N2) {
            align256((size_t)N2 * 4);
 }
 
-int mxp_mx_mlp_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1, const void* b1,
-                  int b1_dtype, int act, const void* w2_op, int N2, const void* b2, int b2_dtype, int bfloat_bits,
-                  int flush, void* out, int64_t ldo, void* workspace, size_t workspace_bytes, void* stream) {
+static int mx_mlp_impl(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1, const void* b1,
+                       int b1_dtype, int act, const void* w2_op, int N2, const void* b2, int b2_dtype, int bfloat_bits,
+                       int flush, void* out, int64_t ldo, const Adaln* ad, void* workspace, size_t workspace_bytes,
+                       void* stream) {
     g_launches = 0;
     int rc = check_linear(M, N1, K, bfloat_bits);
     if (rc || (rc = check_linear(M, N2, N1, bfloat_bits))) return rc;         // fc2: K = N1, a multiple of 64
@@ -1445,6 +1515,7 @@ int mxp_mx_mlp_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const v
         (ldo & 3) || ldo < N2)
         return fail(MXP_E_BADARG, "w1_op / w2_op / out: null or misaligned pointer, or out row stride %lld not >= %d and "
                     "a multiple of 4", (long long)ldo, N2);
+    if (ad && (rc = check_adaln(*ad, x_dtype, M, K, N2))) return rc;
     const size_t need = mxp_mx_mlp_workspace_bytes(M, K, N1, N2);
     if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255))
         return fail(MXP_E_BADARG, "workspace: need %zu bytes, 256-byte aligned", need);
@@ -1455,7 +1526,11 @@ int mxp_mx_mlp_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const v
     float* rb1 = (float*)(h_op + align256(rows * (size_t)N1 * 2));
     float* rb2 = (float*)((unsigned char*)rb1 + align256((size_t)N1 * 4));
     const int bf16 = bfloat_bits == 16;
-    if ((rc = launch_quantize_gemm_operand(x, x_dtype, ldx, M, K, GL_BM, bf16, flush != 0, a_op, st))) return rc;
+    ModParams mod{};
+    if (ad && ad->shift) mod = make_mod(*ad);
+    if ((rc = launch_quantize_gemm_operand(x, x_dtype, ldx, M, K, GL_BM, bf16, flush != 0, a_op, st,
+                                           ad && ad->shift ? &mod : nullptr)))
+        return rc;
     if (b1 && (rc = launch_round_bias(b1, b1_dtype, rb1, N1, bf16, st))) return rc;
     if (b2 && (rc = launch_round_bias(b2, b2_dtype, rb2, N2, bf16, st))) return rc;
     LinearParams l1{};
@@ -1467,7 +1542,29 @@ int mxp_mx_mlp_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const v
     LinearParams l2{};
     l2.a_op = h_op; l2.w_op = (const unsigned char*)w2_op; l2.bias = b2 ? rb2 : nullptr;
     l2.out = (float*)out; l2.ldo = ldo; l2.M = M; l2.N = N2; l2.K = N1; l2.bf16 = bf16; l2.stages = 4;
+    if (ad && ad->residual) {
+        set_gated_residual(l2, *ad);
+        return launch_linear_gemm<EPI_GATED_RESIDUAL>(l2, x_dtype, st);
+    }
     return launch_linear_gemm<EPI_STORE>(l2, x_dtype, st);
+}
+
+int mxp_mx_mlp_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1, const void* b1,
+                  int b1_dtype, int act, const void* w2_op, int N2, const void* b2, int b2_dtype, int bfloat_bits,
+                  int flush, void* out, int64_t ldo, void* workspace, size_t workspace_bytes, void* stream) {
+    return mx_mlp_impl(x, x_dtype, ldx, M, K, w1_op, N1, b1, b1_dtype, act, w2_op, N2, b2, b2_dtype, bfloat_bits, flush,
+                       out, ldo, nullptr, workspace, workspace_bytes, stream);
+}
+
+int mxp_mx_mlp_adaln_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1,
+                        const void* b1, int b1_dtype, int act, const void* w2_op, int N2, const void* b2, int b2_dtype,
+                        int bfloat_bits, int flush, void* out, int64_t ldo, int tokens, const void* shift,
+                        int64_t ld_shift, const void* scale, int64_t ld_scale, const void* residual,
+                        int64_t ld_residual, const void* gate, int64_t ld_gate, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+    const Adaln ad{tokens, shift, scale, residual, gate, ld_shift, ld_scale, ld_residual, ld_gate};
+    return mx_mlp_impl(x, x_dtype, ldx, M, K, w1_op, N1, b1, b1_dtype, act, w2_op, N2, b2, b2_dtype, bfloat_bits, flush,
+                       out, ldo, &ad, workspace, workspace_bytes, stream);
 }
 
 int mxp_activation_dt(const void* x, int dtype, int64_t n, int act, void* out, void* stream) {

@@ -21,6 +21,9 @@
 //                            EPI = EPI_GELU / EPI_GELU_TANH (the fused MLP's fc1): the epilogue applies the
 //                            activation and writes the NEXT GEMM's A operand instead of the output; each 32-column
 //                            pass over a TMEM row is one MX block of fc2's input, held by one thread.
+//                            EPI = EPI_GATED_RESIDUAL (an adaLN block's proj / fc2): the coalesced store path stores
+//                            residual + gate * y, with the residual read in the store's width and pattern.
+//   With MOD, k_quantize_gemm_operand applies the adaLN modulation x * (1 + scale) + shift to the elements it loads.
 #pragma once
 #include "mxprune_predict_tc.cuh"
 
@@ -43,12 +46,59 @@ __host__ __device__ inline GemmOpLayout gemm_op_layout(int K) {
     return L;
 }
 
-// rows_tile = 128 (activations) or 256 (weights); rows_pad = multiple of rows_tile (zero rows past `rows`).
-// x holds elements of type DT (DT_*); ld in elements.
+// an fp32 value rounded to nearest even in DT and widened back (identity for fp32)
 template <int DT>
+__device__ __forceinline__ float round_to_dt(float x) {
+    if constexpr (DT == DT_BF16) return __bfloat162float(__float2bfloat16_rn(x));
+    else if constexpr (DT == DT_F16) return __half2float(__float2half_rn(x));
+    else return x;
+}
+
+// four consecutive elements of type DT at element offset off as fp32 bit patterns: one 16-byte (fp32) or 8-byte load
+template <int DT>
+__device__ __forceinline__ uint4 load_elem4_bits(const float* p, int64_t off) {
+    if constexpr (DT == DT_F32) {
+        return *reinterpret_cast<const uint4*>(p + off);
+    } else {
+        const uint2 w = *reinterpret_cast<const uint2*>(reinterpret_cast<const uint16_t*>(p) + off);
+        return make_uint4(widen1<DT>((uint16_t)(w.x & 0xffffu)), widen1<DT>((uint16_t)(w.x >> 16)),
+                          widen1<DT>((uint16_t)(w.y & 0xffffu)), widen1<DT>((uint16_t)(w.y >> 16)));
+    }
+}
+
+// adaLN modulation of the activation operand (DiT / PixArt blocks: modulate(x, shift, scale)): row r of x belongs to
+// batch entry r / tokens, whose shift and scale rows (K elements of x's type each, row strides ld_shift / ld_scale)
+// turn x into x * (1 + scale) + shift, each operation rounded to x's type as eager torch evaluates it.
+struct ModParams {
+    const float *shift, *scale;
+    int64_t ld_shift, ld_scale;
+    int tokens;
+};
+// the 32 elements of one MX block (fp32 bit patterns of x's values, columns col..col+31 of batch entry bi), modulated
+template <int DT>
+__device__ __forceinline__ void modulate_block(uint32_t (&xv)[32], const ModParams& m, int bi, int col) {
+    const float* sc = view_elem<DT>(m.scale, (int64_t)bi * m.ld_scale + col);
+    const float* sh = view_elem<DT>(m.shift, (int64_t)bi * m.ld_shift + col);
+#pragma unroll
+    for (int j4 = 0; j4 < 32; j4 += 4) {
+        const uint4 s4 = load_elem4_bits<DT>(sc, j4), h4 = load_elem4_bits<DT>(sh, j4);
+        const uint32_t s[4] = {s4.x, s4.y, s4.z, s4.w}, h[4] = {h4.x, h4.y, h4.z, h4.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const float t = round_to_dt<DT>(__fadd_rn(1.0f, __uint_as_float(s[j])));                 // 1 + scale
+            const float u = round_to_dt<DT>(__fmul_rn(__uint_as_float(xv[j4 + j]), t));              // x * (1 + scale)
+            xv[j4 + j] = __float_as_uint(round_to_dt<DT>(__fadd_rn(u, __uint_as_float(h[j]))));      // + shift
+        }
+    }
+}
+
+// rows_tile = 128 (activations) or 256 (weights); rows_pad = multiple of rows_tile (zero rows past `rows`).
+// x holds elements of type DT (DT_*); ld in elements.  MOD: the operand is quantized from x modulated by `mod` (rows
+// past `rows` stay zero rows and read no modulation).
+template <int DT, bool MOD = false>
 __global__ void __launch_bounds__(256)
 k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int rows_pad, int K, int rows_tile,
-                        int bf16, int flush, unsigned char* __restrict__ op) {
+                        int bf16, int flush, unsigned char* __restrict__ op, const ModParams mod) {
     const int nb = K >> 5, ksteps = K / GL_BK;
     const int64_t ntask = (int64_t)rows_pad * nb;
     const size_t stage_bytes = (size_t)8 * rows_tile * 16;
@@ -56,6 +106,9 @@ k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int r
         const int b = (int)(t / rows_pad), row = (int)(t - (int64_t)b * rows_pad);      // block-major: coalesced stores
         uint32_t xv[32];
         load_block_bits<DT>(view_elem<DT>(x, (int64_t)row * ld + 32 * b), 32, row < rows, xv);
+        if constexpr (MOD) {
+            if (row < rows) modulate_block<DT>(xv, mod, row / mod.tokens, 32 * b);
+        }
         BlockQ r;
         quantize_block_thread<false, false>(xv, 32, bf16, flush, r);
         const int tile = row / rows_tile, rt = row - tile * rows_tile;
@@ -66,9 +119,9 @@ k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int r
     }
 }
 
-// Epilogues of k_mx_linear_umma: store the output, or apply an activation (MXP_ACT_* + 1) and write the next GEMM's
-// A operand.
-constexpr int EPI_STORE = 0, EPI_GELU = 1, EPI_GELU_TANH = 2;
+// Epilogues of k_mx_linear_umma: store the output, apply an activation (MXP_ACT_* + 1) and write the next GEMM's
+// A operand, or store residual + gate * output (the adaLN block's gated residual).
+constexpr int EPI_STORE = 0, EPI_GELU = 1, EPI_GELU_TANH = 2, EPI_GATED_RESIDUAL = 3;
 
 // torch.nn.functional.gelu on CUDA, bit for bit: ATen's GeluCUDAKernelImpl (ActivationGeluKernel.cu) in fp32 opmath,
 //     approximate='none'  x * 0.5 * (1 + erf(x * M_SQRT1_2))
@@ -85,13 +138,6 @@ __device__ __forceinline__ float gelu_tanh(float x) {
 template <int EPI>
 __device__ __forceinline__ float activation(float x) {
     return EPI == EPI_GELU_TANH ? gelu_tanh(x) : gelu_erf(x);
-}
-// an fp32 value rounded to nearest even in DT and widened back (identity for fp32)
-template <int DT>
-__device__ __forceinline__ float round_to_dt(float x) {
-    if constexpr (DT == DT_BF16) return __bfloat162float(__float2bfloat16_rn(x));
-    else if constexpr (DT == DT_F16) return __half2float(__float2half_rn(x));
-    else return x;
 }
 
 // elementwise activation of n elements of type DT (the fused epilogue's function; parity aid)
@@ -111,9 +157,26 @@ struct LinearParams {
     float* out;                       // elements of the kernel's OUT_DT
     int64_t ldo;
     int M, N, K, bf16, stages;
-    int flush;                        // EPI != EPI_STORE: the next GEMM's quantizer setting
-    unsigned char* h_op;              // EPI != EPI_STORE: the next GEMM's A operand (K = N), written instead of out
+    int flush;                        // EPI_GELU*: the next GEMM's quantizer setting
+    unsigned char* h_op;              // EPI_GELU*: the next GEMM's A operand (K = N), written instead of out
+    const float* residual;            // EPI_GATED_RESIDUAL: (M, N) of OUT_DT, row stride ldr
+    const float* gate;                // EPI_GATED_RESIDUAL: (M / tokens, N) of OUT_DT, row stride ldg; row r uses r / tokens
+    int64_t ldr, ldg;
+    int tokens;
 };
+
+// the gated residual of four outputs y (columns col..col+3 of row `row`, fp32 values before the store's rounding):
+// residual + gate * y, each operation rounded to DT as eager torch evaluates it on tensors of that type
+template <int DT>
+__device__ __forceinline__ float4 gated_residual4(float4 y, const LinearParams& p, int row, int col) {
+    const uint4 r = load_elem4_bits<DT>(p.residual, (int64_t)row * p.ldr + col);
+    const uint4 g = load_elem4_bits<DT>(p.gate, (int64_t)(row / p.tokens) * p.ldg + col);
+    auto f = [](float yv, uint32_t gv, uint32_t rv) {
+        const float gy = round_to_dt<DT>(__fmul_rn(__uint_as_float(gv), round_to_dt<DT>(yv)));
+        return round_to_dt<DT>(__fadd_rn(__uint_as_float(rv), gy));
+    };
+    return make_float4(f(y.x, g.x, r.x), f(y.y, g.y, r.y), f(y.z, g.z, r.z), f(y.w, g.w, r.w));
+}
 
 // bias of element type DT -> A1(bias), N floats (tiny)
 template <int DT>
@@ -135,9 +198,9 @@ __device__ __forceinline__ void epilogue_barrier() {               // the 128 ep
 // Persistent: one CTA per SM walks the output tiles (feature tile fastest, so the CTAs that share an
 // activation tile run together and the weight operand stays L2-resident).  The accumulator is
 // double-buffered in TMEM (2 x 256 columns): the epilogue of tile i overlaps the main loop of tile i+1.
-// OUT_DT (DT_*) is the element type of p.out; only the final store depends on it.  With EPI != EPI_STORE it is the
-// type the output and the activation are rounded to before fc2's quantizer reads them (what mx_linear stores and
-// what torch's GELU returns on a tensor of that type).
+// OUT_DT (DT_*) is the element type of p.out; only the final store depends on it.  With EPI_GELU* it is the type the
+// output and the activation are rounded to before fc2's quantizer reads them (what mx_linear stores and what torch's
+// GELU returns on a tensor of that type); with EPI_GATED_RESIDUAL also the type of the residual and the gate.
 template <int OUT_DT, int EPI = EPI_STORE>
 __global__ void __launch_bounds__(GL_T, 1)
 k_mx_linear_umma(const LinearParams p) {
@@ -153,6 +216,7 @@ k_mx_linear_umma(const LinearParams p) {
     uint64_t* bar_acc_empty = bar_acc_full + 2;                                                // [2]
     uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bar_acc_empty + 2);
 
+    constexpr bool ACT_EPI = EPI == EPI_GELU || EPI == EPI_GELU_TANH;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int tiles_n = (p.N + GL_BN - 1) / GL_BN, tiles_m = (p.M + GL_BM - 1) / GL_BM;
     const int ntiles = tiles_n * tiles_m;
@@ -222,13 +286,13 @@ k_mx_linear_umma(const LinearParams p) {
             const int tile_m = t / tiles_n, tile_n = t - tile_m * tiles_n;
             const int n0 = tile_n * GL_BN, buf = i & 1;
             float* sb = s_bias + buf * GL_BN;
-            const float no_bias = EPI == EPI_STORE ? 0.f : -0.f;            // -0: the identity of the GELU epilogue's add
+            const float no_bias = ACT_EPI ? -0.f : 0.f;                     // -0: the identity of the GELU epilogue's add
             for (int j = et; j < GL_BN; j += 128) sb[j] = (p.bias && n0 + j < p.N) ? __ldg(p.bias + n0 + j) : no_bias;
             epilogue_barrier();
             mbar_wait(&bar_acc_full[buf], (uint32_t)((i >> 1) & 1));
             tcgen05_fence_after_sync();
             const uint32_t t0 = tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * GL_BN);
-            if constexpr (EPI != EPI_STORE) {
+            if constexpr (ACT_EPI) {
                 // thread = row; 32 TMEM columns = one MX block of fc2's input (n0 + c0 is a multiple of 32).  The
                 // block is quantized in registers and its four 16-byte chunks go straight to fc2's A operand
                 // [row tile][k step of 64][8 chunks][128 rows][16 B]: a warp writes 512 contiguous bytes per chunk.
@@ -299,9 +363,11 @@ k_mx_linear_umma(const LinearParams p) {
                         y.x = __fadd_rn(y.x, b4.x); y.y = __fadd_rn(y.y, b4.y); y.z = __fadd_rn(y.z, b4.z); y.w = __fadd_rn(y.w, b4.w);
                         if (bf16) { y.x = bf16_half_away(y.x); y.y = bf16_half_away(y.y); y.z = bf16_half_away(y.z); y.w = bf16_half_away(y.w); }   // :89-93
                     }
-                    if (row < p.M && col_ok)
+                    if (row < p.M && col_ok) {                          // padding rows read no residual or gate
+                        if constexpr (EPI == EPI_GATED_RESIDUAL) y = gated_residual4<OUT_DT>(y, p, row, n0 + c0 + lc);
                         store_out4<OUT_DT>(p.out, (int64_t)row * p.ldo + n0 + c0 + lc,
                                            make_uint4(__float_as_uint(y.x), __float_as_uint(y.y), __float_as_uint(y.z), __float_as_uint(y.w)));
+                    }
                 }
                 __syncwarp();
             }

@@ -16,6 +16,9 @@ Implemented: mx_quant && top_k && approx/ex_pred with pred_mode "ex_pred" (the p
 mx_quant && top_k && !approx (top-k of the true scores); and mx_quant && !top_k (dense MXINT8 attention, what the
 reference runs in the last block of each model - same kernels with every key kept).  mx_quant=False (the reference's
 unquantized torch path) raises - no silent fallback.
+
+``QuantizedDiTBlock`` wraps a whole DiT block (workloads/DiT/models.py:271-297): its adaLN modulations and gated residuals
+run inside the MX Linear kernels of the Attention shim and of QuantizedMlp.
 """
 from typing import Optional
 
@@ -143,17 +146,32 @@ class QuantizedMlp(nn.Module):
         self.drop = nn.Dropout(getattr(getattr(orig_mlp, "drop", None), "p", 0.0))
         self.fc1, self.fc2 = to_mx_linear(orig_mlp.fc1, mx_specs), to_mx_linear(orig_mlp.fc2, mx_specs)
 
+    def _fused(self) -> bool:
+        return type(self.act) is nn.GELU and resolve_linear_specs(self.fc1.mx_specs) == resolve_linear_specs(self.fc2.mx_specs)
+
+    def _mx_mlp(self, x, **adaln):
+        self.fc1._check_inference(x.requires_grad)
+        self.fc2._check_inference(False)
+        b1 = None if self.fc1.bias is None else self.fc1.bias.detach()
+        b2 = None if self.fc2.bias is None else self.fc2.bias.detach()
+        return ops.mx_mlp(x, self.fc1._operand(), b1, self.fc2._operand(), b2, self.fc1.mx_specs,
+                          act="gelu_tanh" if self.act.approximate == "tanh" else "gelu",
+                          hidden_features=self.fc1.out_features, out_features=self.fc2.out_features, **adaln)
+
     def forward(self, x):
-        if type(self.act) is nn.GELU and resolve_linear_specs(self.fc1.mx_specs) == resolve_linear_specs(self.fc2.mx_specs):
-            self.fc1._check_inference(x.requires_grad)
-            self.fc2._check_inference(False)
-            b1 = None if self.fc1.bias is None else self.fc1.bias.detach()
-            b2 = None if self.fc2.bias is None else self.fc2.bias.detach()
-            y = ops.mx_mlp(x, self.fc1._operand(), b1, self.fc2._operand(), b2, self.fc1.mx_specs,
-                           act="gelu_tanh" if self.act.approximate == "tanh" else "gelu",
-                           hidden_features=self.fc1.out_features, out_features=self.fc2.out_features)
-            return self.drop(y)
+        if self._fused():
+            return self.drop(self._mx_mlp(x))
         return self.drop(self.fc2(self.act(self.fc1(x))))
+
+    def forward_adaln(self, x, shift, scale, residual, gate):
+        """The MLP half of DiT's DiTBlock.forward (workloads/DiT/models.py:297) on an already-normalized x (B, T, C):
+        ``residual + gate.unsqueeze(1) * self(modulate(x, shift, scale))``, modulate(x, shift, scale) =
+        ``x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1)`` (models.py:101-102).  On the fused route (that of forward,
+        while no dropout is active) it is one ops.mx_mlp call whose quantizer applies the modulation and whose fc2 store
+        applies the gated residual, bit for bit the expression; otherwise the expression runs as written."""
+        if self._fused() and not (self.training and self.drop.p > 0):
+            return self._mx_mlp(x, shift=shift, scale=scale, residual=residual, gate=gate)
+        return residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1))
 
 
 def apply_quantization_to_deit(model, config, mx_quant=True, top_k=True, k=20, approx_flag=True, pred_mode="ex_pred",
@@ -218,6 +236,52 @@ class Attention(nn.Module):
         x = self.proj_drop(self.proj(x))
         self.current_timestep += 1
         return x
+
+    def forward_adaln(self, x, shift, scale, residual, gate):
+        """The attention half of DiT's DiTBlock.forward (workloads/DiT/models.py:296) on an already-normalized x (B, N, C):
+        ``residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1))``, bit for bit.  The
+        qkv projection's quantizer applies the modulation as it loads x, and the output projection's store applies the
+        gated residual; the core call between them is forward's (dense on exclude_timesteps steps), and
+        current_timestep advances as in forward.  While proj_drop is active (training, p > 0) the expression runs as
+        written."""
+        if self.training and self.proj_drop.p > 0:
+            return residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1))
+        B, N, C = x.shape
+        qkv = self.qkv.forward_adaln(x, shift=shift, scale=scale)
+        q, k, v = qkv.reshape(B, N, 3, self.num_heads, self.head_dim).permute(2, 0, 3, 1, 4).unbind(0)
+        q, k = self.q_norm(q), self.k_norm(k)
+        x = self.core(q, k, v, dense=self.current_timestep in self.exclude_timesteps)
+        x = self.proj.forward_adaln(x, residual=residual, gate=gate)
+        self.current_timestep += 1
+        return x
+
+
+class QuantizedDiTBlock(nn.Module):
+    """DiT block with adaLN-Zero conditioning - mirrors workloads/DiT/models.py:271-297 (DiTBlock.forward, SURVEY.md 3c):
+        shift_msa, scale_msa, gate_msa, shift_mlp, scale_mlp, gate_mlp = adaLN_modulation(c).chunk(6, dim=1)
+        x = x + gate_msa.unsqueeze(1) * attn(modulate(norm1(x), shift_msa, scale_msa))
+        x = x + gate_mlp.unsqueeze(1) * mlp(modulate(norm2(x), shift_mlp, scale_mlp))
+    with the modulations and gated residuals inside the MX Linear kernels (Attention.forward_adaln,
+    QuantizedMlp.forward_adaln): bit for bit that expression on the same modules, without its elementwise passes.
+
+    ``orig_block``: a DiT-style block with ``norm1``, ``attn``, ``norm2``, ``mlp`` and ``adaLN_modulation``.  ``attn`` must
+    be the ``Attention`` shim; ``mlp`` (timm Mlp, models.py:287) is wrapped in QuantizedMlp unless it already is one.  The
+    norms (torch LayerNorm) and adaLN_modulation stay the host model's modules."""
+
+    def __init__(self, orig_block, mx_specs=None):
+        super().__init__()
+        if not isinstance(orig_block.attn, Attention):
+            raise TypeError(f"QuantizedDiTBlock: attn must be modules.Attention (the DiT shim), got "
+                            f"{type(orig_block.attn).__name__}")
+        self.norm1, self.attn, self.norm2 = orig_block.norm1, orig_block.attn, orig_block.norm2
+        mlp = orig_block.mlp
+        self.mlp = mlp if isinstance(mlp, QuantizedMlp) else QuantizedMlp(mlp, mx_specs=mx_specs)
+        self.adaLN_modulation = orig_block.adaLN_modulation
+
+    def forward(self, x, c):
+        shift_msa, scale_msa, gate_msa, shift_mlp, scale_mlp, gate_mlp = self.adaLN_modulation(c).chunk(6, dim=1)
+        x = self.attn.forward_adaln(self.norm1(x), shift_msa, scale_msa, x, gate_msa)
+        return self.mlp.forward_adaln(self.norm2(x), shift_mlp, scale_mlp, x, gate_mlp)
 
 
 class MXSelfAttention(nn.Module):
@@ -321,7 +385,11 @@ class MxLinear(nn.Linear):
         return self._w_op
 
     def forward(self, inputs):
+        return self.forward_adaln(inputs)
+
+    def forward_adaln(self, inputs, **adaln):
+        """forward with ops.mx_linear's adaLN arguments (shift=, scale=, residual=, gate=)."""
         self._check_inference(inputs.requires_grad)
         w_op = self._operand()
         b = None if self.bias is None else self.bias.detach()
-        return ops.mx_linear(inputs, w_op, b, self.mx_specs, out_features=self.out_features)
+        return ops.mx_linear(inputs, w_op, b, self.mx_specs, out_features=self.out_features, **adaln)

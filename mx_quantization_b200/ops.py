@@ -492,8 +492,48 @@ def _check_bias(bias: Optional[torch.Tensor], N: int) -> None:
         raise ValueError("bias must be a contiguous float32, bfloat16 or float16 tensor with out_features elements")
 
 
+def _adaln_args(x: torch.Tensor, K: int, N: int, shift, scale, residual, gate) -> tuple:
+    """The adaLN arguments of mxp_mx_*_adaln_dt (tokens, then each tensor's pointer and row stride) for a (B, T, K) x:
+    shift / scale (B, K) and gate (B, N) rows with innermost stride 1 (e.g. ``.chunk(6, dim=1)`` views, read in
+    place), a residual (B, T, N) whose rows form one (B*T, N) view with innermost stride 1; all of x's dtype."""
+    if (shift is None) != (scale is None):
+        raise ValueError("shift and scale: pass both or neither")
+    if (residual is None) != (gate is None):
+        raise ValueError("residual and gate: pass both or neither")
+    if x.dim() != 3:
+        raise ValueError(f"shift / scale / residual / gate need x of shape (B, T, in_features), got {tuple(x.shape)}")
+    B, T = x.shape[0], x.shape[1]
+    args = [T]
+    for name, t, shape in (("shift", shift, (B, K)), ("scale", scale, (B, K)), ("residual", residual, (B, T, N)),
+                           ("gate", gate, (B, N))):
+        if t is None:
+            args += [_ptr(None), 0]
+            continue
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"{name}: expected a torch.Tensor")
+        if t.dtype != x.dtype:
+            raise ValueError(f"{name} is {t.dtype} but x is {x.dtype}: shift, scale, residual and gate take x's dtype")
+        if tuple(t.shape) != shape:
+            raise ValueError(f"{name}: expected shape {shape}, got {tuple(t.shape)}")
+        rows = t
+        if t.dim() == 3:
+            try:
+                rows = t.view(-1, N)
+            except RuntimeError:
+                rows = None
+        if rows is None or rows.stride(1) != 1:
+            raise ValueError(f"{name}: needs rows with innermost stride 1{' forming one 2-D view' if t.dim() == 3 else ''}, "
+                             f"got strides {tuple(t.stride())}")
+        # a single row's stride is never used: pass the row width, which meets the library's rules
+        args += [_ptr(t), rows.stride(0) if rows.shape[0] > 1 else shape[-1]]
+    _same_device(x, shift, scale, residual, gate)
+    return tuple(args)
+
+
 def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
-              out_features: Optional[int] = None) -> torch.Tensor:
+              out_features: Optional[int] = None, *, shift: Optional[torch.Tensor] = None,
+              scale: Optional[torch.Tensor] = None, residual: Optional[torch.Tensor] = None,
+              gate: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Forward of the reference's mx.Linear (microxscaling/mx/linear.py:20-103) for MXINT8:
     y = A1(A1(MXq(A1(x)) @ MXq(A1(W))^T) + A1(bias)).  ``weight`` is either the (N,K) tensor or
     the operand returned by mx_linear_prepare_weight (then pass out_features).
@@ -501,7 +541,14 @@ def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
     ``x``: float32, bfloat16 or float16; the result has x's dtype.  The weight and the bias may each be any of the
     three types, independently of x.  A 16-bit call is the fp32 call on the widened x, weight and bias, its result
     rounded to nearest even (lossless under bfloat 16 for a bf16 x: the fp32 result is a bf16 value), with the same
-    kernel launches (no conversion pass)."""
+    kernel launches (no conversion pass).
+
+    adaLN (DiT's DiTBlock, models.py:293-297), for x of shape (B, T, K), each pair optional:
+      ``shift``, ``scale`` (B, K): the layer runs on ``x * (1 + scale[:, None]) + shift[:, None]`` (the quantizer
+          modulates the elements it loads; nothing is written);
+      ``residual`` (B, T, N), ``gate`` (B, N): the result is ``residual + gate[:, None] * y`` (the GEMM's store does it).
+    Bit for bit the eager torch composition on tensors of x's dtype, with the launches of the plain call.  The four
+    tensors have x's dtype; shift / scale / gate may be column slices of one (B, 6C) tensor (``.chunk(6, dim=1)``)."""
     sp = resolve_linear_specs(mx_specs)
     lib = _lib.load()
     x2 = _linear_rows(x)
@@ -511,13 +558,19 @@ def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
     w_op, N = _weight_operand(weight, K, out_features, mx_specs)
     _check_bias(bias, N)
     _same_device(x, w_op, bias)
+    adaln = any(t is not None for t in (shift, scale, residual, gate))
+    ad = _adaln_args(x, K, N, shift, scale, residual, gate) if adaln else ()
     with torch.cuda.device(x.device):
         out = torch.empty((M, N), dtype=x.dtype, device=x.device)
         ws_bytes = lib.mxp_mx_linear_workspace_bytes(M, N, K)
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=x.device)
-        rc = lib.mxp_mx_linear_dt(_ptr(x2), DTYPE_CODES[x.dtype], x2.stride(0), M, K, _ptr(w_op), N, _ptr(bias),
-                                  DTYPE_CODES[bias.dtype] if bias is not None else _lib.MXP_DT_F32, sp.bfloat_bits,
-                                  int(sp.flush), _ptr(out), out.stride(0), _ptr(ws), ws_bytes, _stream())
+        args = (_ptr(x2), DTYPE_CODES[x.dtype], x2.stride(0), M, K, _ptr(w_op), N, _ptr(bias),
+                DTYPE_CODES[bias.dtype] if bias is not None else _lib.MXP_DT_F32, sp.bfloat_bits,
+                int(sp.flush), _ptr(out), out.stride(0))
+        if adaln:
+            rc = lib.mxp_mx_linear_adaln_dt(*args, *ad, _ptr(ws), ws_bytes, _stream())
+        else:
+            rc = lib.mxp_mx_linear_dt(*args, _ptr(ws), ws_bytes, _stream())
     _lib.check(rc, "mxp_mx_linear")
     return out.reshape(*x.shape[:-1], N)
 
@@ -533,7 +586,9 @@ def _act_code(act: str) -> int:
 
 
 def mx_mlp(x: torch.Tensor, w1, b1: Optional[torch.Tensor], w2, b2: Optional[torch.Tensor], mx_specs,
-           act: str = "gelu", hidden_features: Optional[int] = None, out_features: Optional[int] = None) -> torch.Tensor:
+           act: str = "gelu", hidden_features: Optional[int] = None, out_features: Optional[int] = None, *,
+           shift: Optional[torch.Tensor] = None, scale: Optional[torch.Tensor] = None,
+           residual: Optional[torch.Tensor] = None, gate: Optional[torch.Tensor] = None) -> torch.Tensor:
     """A transformer MLP (fc1 -> GELU -> fc2) on MX Linear layers, fused:
     ``mx_linear(F.gelu(mx_linear(x, w1, b1), approximate=...), w2, b2)`` bit for bit, with the hidden activation never
     written in a float type (fc1's epilogue applies the GELU and writes fc2's MXINT8 operand).
@@ -541,7 +596,11 @@ def mx_mlp(x: torch.Tensor, w1, b1: Optional[torch.Tensor], w2, b2: Optional[tor
     ``act``: "gelu" (``approximate='none'``, DeiT) or "gelu_tanh" (``approximate='tanh'``, DiT, PixArt).  ``w1`` / ``w2``:
     the (N1, K) / (N2, N1) weights, or operands from mx_linear_prepare_weight (then pass ``hidden_features`` /
     ``out_features``).  ``x``, weights and biases: the dtype and stride rules of mx_linear; the result has x's dtype.
-    K and N1 must be multiples of 64, N2 a multiple of 4."""
+    K and N1 must be multiples of 64, N2 a multiple of 4.
+
+    ``shift``, ``scale`` (B, K), ``residual`` (B, T, N2), ``gate`` (B, N2): the adaLN arguments of mx_linear for a
+    (B, T, K) x, the modulation applied to fc1's input and the gated residual to fc2's output:
+    ``residual + gate[:, None] * mlp(x * (1 + scale[:, None]) + shift[:, None])`` bit for bit, same launches."""
     sp = resolve_linear_specs(mx_specs)
     code = _act_code(act)
     lib = _lib.load()
@@ -561,15 +620,21 @@ def mx_mlp(x: torch.Tensor, w1, b1: Optional[torch.Tensor], w2, b2: Optional[tor
     _check_bias(b1, N1)
     _check_bias(b2, N2)
     _same_device(x, w1_op, b1, w2_op, b2)
+    adaln = any(t is not None for t in (shift, scale, residual, gate))
+    ad = _adaln_args(x, K, N2, shift, scale, residual, gate) if adaln else ()
     with torch.cuda.device(x.device):
         out = torch.empty((M, N2), dtype=x.dtype, device=x.device)
         ws_bytes = lib.mxp_mx_mlp_workspace_bytes(M, K, N1, N2)
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=x.device)
         f32 = _lib.MXP_DT_F32
-        rc = lib.mxp_mx_mlp_dt(_ptr(x2), DTYPE_CODES[x.dtype], x2.stride(0), M, K, _ptr(w1_op), N1, _ptr(b1),
-                               DTYPE_CODES[b1.dtype] if b1 is not None else f32, code, _ptr(w2_op), N2, _ptr(b2),
-                               DTYPE_CODES[b2.dtype] if b2 is not None else f32, sp.bfloat_bits, int(sp.flush),
-                               _ptr(out), out.stride(0), _ptr(ws), ws_bytes, _stream())
+        args = (_ptr(x2), DTYPE_CODES[x.dtype], x2.stride(0), M, K, _ptr(w1_op), N1, _ptr(b1),
+                DTYPE_CODES[b1.dtype] if b1 is not None else f32, code, _ptr(w2_op), N2, _ptr(b2),
+                DTYPE_CODES[b2.dtype] if b2 is not None else f32, sp.bfloat_bits, int(sp.flush),
+                _ptr(out), out.stride(0))
+        if adaln:
+            rc = lib.mxp_mx_mlp_adaln_dt(*args, *ad, _ptr(ws), ws_bytes, _stream())
+        else:
+            rc = lib.mxp_mx_mlp_dt(*args, _ptr(ws), ws_bytes, _stream())
     _lib.check(rc, "mxp_mx_mlp")
     return out.reshape(*x.shape[:-1], N2)
 
