@@ -17,6 +17,11 @@
 //            same arithmetic, on the same inputs, as the entry that attains the maximum
 //   pass C   p = e * inv -> A1 -> MXINT8 code with the window's exponent -> one bf16 element scattered
 //            into the (zero-filled) P operand of its 4-window group;  O += P_g . V_g on the tensor core.
+// KMAX != 0 (rows of at most 2 KMAX kept keys): once the list is complete each lane copies its share - score and
+// key index - into registers.  Pass B then keeps e in registers, and pass C converts every entry in one sweep
+// before the group barrier (only the window record is still a shared-memory load, addressed from a register);
+// per 4-window group only the scatter of the finished elements remains.  Same operations in the same order as
+// the list path, so the same bits.
 // The list overlays the K operand (dead once S is complete; K is re-fetched per query tile, from L2).
 // Masks must hold at most top_k kept keys per row (guaranteed for masks produced by the selection kernels).
 //
@@ -29,6 +34,7 @@
 namespace mxp {
 
 constexpr int K2S_LSTR = 144;          // list stride in entries: 128 rows + 16 (odd / even ranks hit disjoint banks)
+constexpr int K2S_KMAX = 16;           // entries per lane of the register path: rows of up to 2 * K2S_KMAX kept keys
 
 struct K2sSmem {
     int cap;                            // list entries per row
@@ -53,8 +59,9 @@ __device__ __forceinline__ float exp_sub(float x, float m) { return exp_nonpos(_
 
 // One head (all its query tiles) through the sparse exact-attention epilogue.  q_op / k_op / v_op: this head's
 // MMA-ready operands (global memory); mask_head: this head's [Nq][NW] mask words (global or shared memory);
-// out_head: the head's output rows (row stride o_sN); OT / out16: output type (store_o_tile).
-template <bool BF16, int OT = DT_F32>
+// out_head: the head's output rows (row stride o_sN); OT / out16: output type (store_o_tile); KMAX: 0 = list path,
+// else the register path, which needs L.cap <= 2 * KMAX.
+template <bool BF16, int OT = DT_F32, int KMAX = 0>
 __device__ __forceinline__ void attend_sparse_head(GroupCtx& g, const OpsLayout& O, const K2sSmem& L, int Nq, int Nk,
                                                    int hd, float scale, bool flush, const unsigned char* q_op,
                                                    const unsigned char* k_op, const unsigned char* v_op,
@@ -193,7 +200,30 @@ __device__ __forceinline__ void attend_sparse_head(GroupCtx& g, const OpsLayout&
         // ---- pass B: e = exp(t - max) over the row's list, the two lanes alternating; row sum
         const int nmine = (ntot - part + 1) >> 1;                   // entries part, part + 2, ...
         float sum0 = 0.f, sum1 = 0.f;
-        {
+        float ev[KMAX ? KMAX : 1];                                  // register path: this lane's e values ...
+        uint32_t jv[KMAX ? KMAX : 1];                               // ... and key indices
+        if constexpr (KMAX != 0) {
+            // all loads first (predicated, back to back), then the arithmetic without branches: slots past nmine
+            // hold e = 0, and adding +0 leaves the (non-negative) partial sums bit for bit as they were
+            const float* pl = s_list + part * K2S_LSTR + rr;
+            const unsigned char* pj = s_lj + part * K2S_LSTR + rr;
+#pragma unroll
+            for (int it = 0; it < KMAX; ++it) {
+                ev[it] = 0.f;
+                jv[it] = 0u;
+                if (it < nmine) {
+                    ev[it] = pl[2 * it * K2S_LSTR];
+                    jv[it] = pj[2 * it * K2S_LSTR];
+                }
+            }
+#pragma unroll
+            for (int it = 0; it < KMAX; ++it) {
+                const float e = exp_sub(ev[it], m_use);
+                ev[it] = it < nmine ? e : 0.f;
+                if (it & 1) sum1 += ev[it];
+                else sum0 += ev[it];
+            }
+        } else {
             float* pl = s_list + part * K2S_LSTR + rr;
             int it = 0;
             for (; it + 2 <= nmine; it += 2) {
@@ -216,6 +246,7 @@ __device__ __forceinline__ void attend_sparse_head(GroupCtx& g, const OpsLayout&
         const float inv = sum > 0.f ? 1.0f / sum : 0.f;
 
         // ---- window exponents (A8: P blocks are 32 consecutive ORIGINAL key positions)
+        bool slow = false;                                          // a window of this lane takes the slow exponent path
 #pragma unroll
         for (int t = 0; t < 4; ++t) {
             const int w = 4 * (t >> 1) + 2 * part + (t & 1);
@@ -232,19 +263,64 @@ __device__ __forceinline__ void attend_sparse_head(GroupCtx& g, const OpsLayout&
                     wb = bf16_pow2_bits(ec - 6) | ((bf16_pow2_bits(ec + 1) | 0x8000u) << 16);
                 } else {
                     s1 = (float)e;                                  // negative: the slow path, exponent itself
+                    slow = true;
                 }
             }
             s_ew[w * K2T + rr] = make_uint2(__float_as_uint(s1), wb);
         }
 
         // ---- pass C: P = e * inv -> A1 -> MXINT8 with the window's exponent -> bf16 element of the A operand
+        unsigned char* const prow = sP + rr * 16;
+        const unsigned char* const erow = reinterpret_cast<const unsigned char*>(s_ew + rr);
+        auto window_rec = [&](int j) { return *reinterpret_cast<const uint2*>(erow + ((j & 0xe0) << 5)); };   // (j >> 5) * 128 * 8
+        auto p_bits = [&](float ev) {
+            uint32_t pbits = __float_as_uint(ev * inv);
+            if (bf16) pbits = bf16_half_away(pbits);
+            return pbits;
+        };
+        auto fast_val = [&](uint32_t pbits, const uint2& ew) {
+            // code = min(127, floor(p * 2^(6-e) + 0.5)) without F2I / I2F (see K1)
+            const float v = fminf(fmaf(__uint_as_float(pbits), __uint_as_float(ew.x), 0.5f), 127.0f);
+            const uint32_t cb = __float_as_uint(__fadd_rd(v, 8405760.0f)) & 0xffffu;         // bf16 pattern of 128 + code
+            return bf2_as_u32(__hfma2(u32_as_bf2(cb), u32_as_bf2(ew.y), u32_as_bf2(ew.y >> 16)));
+        };
+        auto any_val = [&](uint32_t pbits, const uint2& ew) {
+            const float s1 = __uint_as_float(ew.x);
+            if (s1 >= 0.f) return fast_val(pbits, ew);
+            const int e = (int)s1;
+            const float rq = __uint_as_float(pbits) * exp2i(-e) * 64.0f + 0.5f;
+            return __float_as_uint((float)min(__float2int_rz(rq), 127) * exp2i(e - 6)) >> 16;
+        };
+        // element (window j >> 5 & 3, key j & 31) of a group: chunk (j & 127) >> 3, 2-byte slot j & 7
+        auto p_off = [](uint32_t j) { return ((j & 127u) * 0x102u) & 0x780eu; };
+        auto put = [&](int j, uint32_t val) {
+            *reinterpret_cast<unsigned short*>(prow + p_off((uint32_t)j)) = (unsigned short)val;
+        };
+        if constexpr (KMAX != 0) {
+            // Every entry converted ahead of the group loop (the row's window records come from the two lanes of this warp).
+            // jv[it] becomes: element in bits 0..15, its P-group offset in bits 16..31 with bit 20 + group set (offsets
+            // have bits 4..10 clear); entries past nmine stay 0, in no group.  One branch per warp for the slow path.
+            __syncwarp();
+            auto pack = [&](uint32_t j, uint32_t val) {
+                return (val & 0xffffu) | ((p_off(j) | (16u << (j >> 7))) << 16);
+            };
+            if (__any_sync(FULL, slow)) {
+#pragma unroll
+                for (int it = 0; it < KMAX; ++it)
+                    if (it < nmine) jv[it] = pack(jv[it], any_val(p_bits(ev[it]), window_rec((int)jv[it])));
+            } else {                                                // branch-free; slots past nmine read window 0's record
+#pragma unroll
+                for (int it = 0; it < KMAX; ++it) {
+                    const uint32_t v = pack(jv[it], fast_val(p_bits(ev[it]), window_rec((int)jv[it])));
+                    jv[it] = it < nmine ? v : 0u;
+                }
+            }
+        }
         // (the P operand overlays the staging areas of ALL threads: every warp must have finished its walk)
         MXP_PROF(g, 14);
         group_sync(g);
         MXP_PROF(g, 15);
         bool first_mma = true;
-        unsigned char* const prow = sP + rr * 16;
-        const unsigned char* const erow = reinterpret_cast<const unsigned char*>(s_ew + rr);
         for (int gi = 0; gi < NG; ++gi) {
             if (gi > 0) {                                           // previous group's MMAs have finished reading sP
                 mbar_wait(g.bar_o, g.ph_o);
@@ -257,63 +333,47 @@ __device__ __forceinline__ void attend_sparse_head(GroupCtx& g, const OpsLayout&
                 for (int q = 0; q < 4; ++q)
                     *reinterpret_cast<uint4*>(prow + (size_t)((2 * part + j) * 4 + q) * K2T * 16) = make_uint4(0u, 0u, 0u, 0u);
             __syncwarp();
-            const int tbeg = gi ? n0 : 0, tend = gi ? ntot : min(n0, ntot);
-            // One list entry -> one bf16 element of the P operand.  The window's exponent record is a dependent shared-memory
-            // load (entry -> key index -> window -> record), so two entries are processed together with ONE branch for the
-            // rare slow exponent path (both chains in flight), and the next pair's entry is fetched before the current pair
-            // is converted.
-            auto window_rec = [&](int j) { return *reinterpret_cast<const uint2*>(erow + ((j & 0xe0) << 5)); };   // (j >> 5) * 128 * 8
-            auto p_bits = [&](float ev) {
-                uint32_t pbits = __float_as_uint(ev * inv);
-                if (bf16) pbits = bf16_half_away(pbits);
-                return pbits;
-            };
-            auto fast_val = [&](uint32_t pbits, const uint2& ew) {
-                // code = min(127, floor(p * 2^(6-e) + 0.5)) without F2I / I2F (see K1)
-                const float v = fminf(fmaf(__uint_as_float(pbits), __uint_as_float(ew.x), 0.5f), 127.0f);
-                const uint32_t cb = __float_as_uint(__fadd_rd(v, 8405760.0f)) & 0xffffu;         // bf16 pattern of 128 + code
-                return bf2_as_u32(__hfma2(u32_as_bf2(cb), u32_as_bf2(ew.y), u32_as_bf2(ew.y >> 16)));
-            };
-            auto any_val = [&](uint32_t pbits, const uint2& ew) {
-                const float s1 = __uint_as_float(ew.x);
-                if (s1 >= 0.f) return fast_val(pbits, ew);
-                const int e = (int)s1;
-                const float rq = __uint_as_float(pbits) * exp2i(-e) * 64.0f + 0.5f;
-                return __float_as_uint((float)min(__float2int_rz(rq), 127) * exp2i(e - 6)) >> 16;
-            };
-            auto put = [&](int j, uint32_t val) {
-                // element (window j >> 5 & 3, key j & 31): chunk (j & 127) >> 3 of the group, 2-byte slot j & 7
-                *reinterpret_cast<unsigned short*>(prow + ((((uint32_t)j & 127u) * 0x102u) & 0x780eu)) = (unsigned short)val;
-            };
-            const int first = tbeg + ((part ^ tbeg) & 1);           // this lane's parity class: t = part (mod 2)
-            const int nmy = (tend - first + 1) >> 1;
-            const float* pl = s_list + first * K2S_LSTR + rr;
-            const unsigned char* pj = s_lj + first * K2S_LSTR + rr;
-            int it = 0;
-            int j0 = 0, j1 = 0;
-            float e0 = 0.f, e1 = 0.f;
-            if (nmy >= 2) { j0 = pj[0]; j1 = pj[2 * K2S_LSTR]; e0 = pl[0]; e1 = pl[2 * K2S_LSTR]; }
-            for (; it + 2 <= nmy; it += 2) {
-                const uint2 w0 = window_rec(j0), w1 = window_rec(j1);
-                const int cj0 = j0, cj1 = j1;
-                const uint32_t pb0 = p_bits(e0), pb1 = p_bits(e1);
-                pl += 4 * K2S_LSTR;
-                pj += 4 * K2S_LSTR;
-                if (it + 4 <= nmy) { j0 = pj[0]; j1 = pj[2 * K2S_LSTR]; e0 = pl[0]; e1 = pl[2 * K2S_LSTR]; }
-                uint32_t v0, v1;
-                if (__uint_as_float(w0.x) >= 0.f && __uint_as_float(w1.x) >= 0.f) {
-                    v0 = fast_val(pb0, w0);
-                    v1 = fast_val(pb1, w1);
-                } else {
-                    v0 = any_val(pb0, w0);
-                    v1 = any_val(pb1, w1);
+            if constexpr (KMAX != 0) {
+                const uint32_t gbit = 16u << (16 + gi);
+#pragma unroll
+                for (int it = 0; it < KMAX; ++it)
+                    if (jv[it] & gbit) *reinterpret_cast<unsigned short*>(prow + ((jv[it] >> 16) & 0x780eu)) = (unsigned short)jv[it];
+            } else {
+                const int tbeg = gi ? n0 : 0, tend = gi ? ntot : min(n0, ntot);
+                // One list entry -> one bf16 element of the P operand.  The window's exponent record is a dependent shared-memory
+                // load (entry -> key index -> window -> record), so two entries are processed together with ONE branch for the
+                // rare slow exponent path (both chains in flight), and the next pair's entry is fetched before the current pair
+                // is converted.
+                const int first = tbeg + ((part ^ tbeg) & 1);           // this lane's parity class: t = part (mod 2)
+                const int nmy = (tend - first + 1) >> 1;
+                const float* pl = s_list + first * K2S_LSTR + rr;
+                const unsigned char* pj = s_lj + first * K2S_LSTR + rr;
+                int it = 0;
+                int j0 = 0, j1 = 0;
+                float e0 = 0.f, e1 = 0.f;
+                if (nmy >= 2) { j0 = pj[0]; j1 = pj[2 * K2S_LSTR]; e0 = pl[0]; e1 = pl[2 * K2S_LSTR]; }
+                for (; it + 2 <= nmy; it += 2) {
+                    const uint2 w0 = window_rec(j0), w1 = window_rec(j1);
+                    const int cj0 = j0, cj1 = j1;
+                    const uint32_t pb0 = p_bits(e0), pb1 = p_bits(e1);
+                    pl += 4 * K2S_LSTR;
+                    pj += 4 * K2S_LSTR;
+                    if (it + 4 <= nmy) { j0 = pj[0]; j1 = pj[2 * K2S_LSTR]; e0 = pl[0]; e1 = pl[2 * K2S_LSTR]; }
+                    uint32_t v0, v1;
+                    if (__uint_as_float(w0.x) >= 0.f && __uint_as_float(w1.x) >= 0.f) {
+                        v0 = fast_val(pb0, w0);
+                        v1 = fast_val(pb1, w1);
+                    } else {
+                        v0 = any_val(pb0, w0);
+                        v1 = any_val(pb1, w1);
+                    }
+                    put(cj0, v0);
+                    put(cj1, v1);
                 }
-                put(cj0, v0);
-                put(cj1, v1);
-            }
-            if (it < nmy) {
-                const int j = pj[0];
-                put(j, any_val(p_bits(pl[0]), window_rec(j)));
+                if (it < nmy) {
+                    const int j = pj[0];
+                    put(j, any_val(p_bits(pl[0]), window_rec(j)));
+                }
             }
             MXP_PROF(g, 16);
             fence_proxy_async_smem();
@@ -352,7 +412,8 @@ __device__ __forceinline__ void attend_sparse_head(GroupCtx& g, const OpsLayout&
     }
 }
 
-template <bool BF16, int OT = DT_F32>
+// KMAX: as attend_sparse_head (the launcher takes the register path for top_k <= 2 * K2S_KMAX)
+template <bool BF16, int OT = DT_F32, int KMAX = 0>
 __global__ void __launch_bounds__(K2P_T, 2)
 k_attend_sparse(const AttnParams p, const int top_k) {
     extern __shared__ __align__(128) unsigned char smem_k2s[];
@@ -369,11 +430,11 @@ k_attend_sparse(const AttnParams p, const int top_k) {
     __syncthreads();
     tcgen05_fence_after_sync();
     GroupCtx g{tid, 0, smem_k2s, &bars[0], &bars[1], &bars[2], tmem_base_s, 0u, 0u, 0u, nullptr, 0};
-    attend_sparse_head<BF16, OT>(g, O, L, p.Nq, p.Nk, p.hd, p.scale, p.flush != 0,
-                                 p.q_op + (size_t)head * O.q_head_bytes, p.k_op + (size_t)head * O.k_head_bytes,
-                                 p.v_op + (size_t)head * O.v_head_bytes, p.mask + (size_t)head * p.Nq * O.nw,
-                                 out_elem(p.out, bb * p.o_sB + hh * p.o_sH, OT != DT_F32), p.o_sN, (int)blockIdx.y,
-                                 (int)gridDim.y, OT != DT_F32);
+    attend_sparse_head<BF16, OT, KMAX>(g, O, L, p.Nq, p.Nk, p.hd, p.scale, p.flush != 0,
+                                       p.q_op + (size_t)head * O.q_head_bytes, p.k_op + (size_t)head * O.k_head_bytes,
+                                       p.v_op + (size_t)head * O.v_head_bytes, p.mask + (size_t)head * p.Nq * O.nw,
+                                       out_elem(p.out, bb * p.o_sB + hh * p.o_sH, OT != DT_F32), p.o_sN, (int)blockIdx.y,
+                                       (int)gridDim.y, OT != DT_F32);
     if ((tid >> 5) == 0) tmem_dealloc(g.tmem, tcols);
 }
 

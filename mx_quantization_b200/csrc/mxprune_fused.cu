@@ -13,14 +13,21 @@
 
 namespace mxp {
 
-// k_attend_sparse with output element type OT (== p.out_dt); grid and dyn from attend_sparse_try
+// k_attend_sparse with output element type OT (== p.out_dt) and register bound KMAX; grid and dyn from attend_sparse_try
+template <int OT, int KMAX>
+static int launch_attend_sparse_ok(const AttnParams& p, int top_k, dim3 grid, size_t dyn, cudaStream_t st) {
+    MXP_ENSURE_DYN_SMEM((k_attend_sparse<true, OT, KMAX>), 160 * 1024);
+    MXP_ENSURE_DYN_SMEM((k_attend_sparse<false, OT, KMAX>), 160 * 1024);
+    if (p.bf16) k_attend_sparse<true, OT, KMAX><<<grid, K2P_T, dyn, st>>>(p, top_k);
+    else k_attend_sparse<false, OT, KMAX><<<grid, K2P_T, dyn, st>>>(p, top_k);
+    return check_launch("k_attend_sparse");
+}
+
+// rows of up to 2 * K2S_KMAX kept keys take the register path, longer ones the list path
 template <int OT>
 static int launch_attend_sparse_ot(const AttnParams& p, int top_k, dim3 grid, size_t dyn, cudaStream_t st) {
-    MXP_ENSURE_DYN_SMEM((k_attend_sparse<true, OT>), 160 * 1024);
-    MXP_ENSURE_DYN_SMEM((k_attend_sparse<false, OT>), 160 * 1024);
-    if (p.bf16) k_attend_sparse<true, OT><<<grid, K2P_T, dyn, st>>>(p, top_k);
-    else k_attend_sparse<false, OT><<<grid, K2P_T, dyn, st>>>(p, top_k);
-    return check_launch("k_attend_sparse");
+    if (top_k <= 2 * K2S_KMAX) return launch_attend_sparse_ok<OT, K2S_KMAX>(p, top_k, grid, dyn, st);
+    return launch_attend_sparse_ok<OT, 0>(p, top_k, grid, dyn, st);
 }
 
 int attend_sparse_try(const AttnParams& p, int top_k, cudaStream_t st, int* rc_out) {

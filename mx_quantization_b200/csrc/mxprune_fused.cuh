@@ -488,8 +488,8 @@ __device__ __forceinline__ void fused_phase1(GroupCtx& gc, K1State& st, uint64_t
                               mask_head, tile_begin, tile_step);
 }
 // HD != 0: head_dim at compile time; such instantiations carry the cost-follows-k epilogue only (the launcher sends
-// dense-epilogue calls to the HD = 0 kernels)
-template <bool BF16, int HD, int DT>
+// dense-epilogue calls to the HD = 0 kernels); so do the KMAX != 0 ones (launched for sparse calls only)
+template <bool BF16, int HD, int DT, int KMAX>
 __device__ __forceinline__ void fused_phase2(GroupCtx& gc, const FusedParams& p, int head, const unsigned char* slot,
                                           const uint32_t* mask_head, int tile_begin, int tile_step) {
     const int hd = HD ? HD : p.hd, Nq = p.Nq, Nk = p.Nk;
@@ -497,10 +497,10 @@ __device__ __forceinline__ void fused_phase2(GroupCtx& gc, const FusedParams& p,
     const int bb = head / p.H, hh = head - bb * p.H;
     const bool out16 = DT != DT_F32 && p.out16 != 0;
     float* out_head = out16 ? out_elem(p.out, bb * p.o_sB + hh * p.o_sH, true) : p.out + bb * p.o_sB + hh * p.o_sH;
-    if (HD != 0 || p.sparse) {
+    if (HD != 0 || KMAX != 0 || p.sparse) {
         const K2sSmem L2 = k2s_smem_layout(O, p.top_k);
-        attend_sparse_head<BF16, DT>(gc, O, L2, Nq, Nk, hd, p.scale, p.flush != 0, slot, slot + p.slot_k, slot + p.slot_v,
-                                     mask_head, out_head, p.o_sN, tile_begin, tile_step, out16);
+        attend_sparse_head<BF16, DT, KMAX>(gc, O, L2, Nq, Nk, hd, p.scale, p.flush != 0, slot, slot + p.slot_k, slot + p.slot_v,
+                                           mask_head, out_head, p.o_sN, tile_begin, tile_step, out16);
     } else {
         attend_pair_head<BF16, false, DT>(gc, O, Nq, Nk, hd, p.scale, p.flush != 0, slot, slot + p.slot_k, slot + p.slot_v,
                                           mask_head, out_head, p.o_sN, nullptr, nullptr, tile_begin, tile_step, out16);
@@ -508,8 +508,9 @@ __device__ __forceinline__ void fused_phase2(GroupCtx& gc, const FusedParams& p,
 }
 
 // NC, HG: key-column geometry of phase 1 (see k_predict_topk_tc); BF16: A1 rounding on (bfloat 16); HD: head_dim at
-// compile time (0 = any); DT: element type of q / k / v (DT_*) - the output is fp32 or, with p.out16, that type
-template <int NC, int HG, bool BF16, int HD, int DT = DT_F32>
+// compile time (0 = any); DT: element type of q / k / v (DT_*) - the output is fp32 or, with p.out16, that type;
+// KMAX: register bound of the cost-follows-k epilogue (0: list path; != 0: register path, sparse epilogue only)
+template <int NC, int HG, bool BF16, int HD, int DT = DT_F32, int KMAX = 0>
 __global__ void __launch_bounds__(FUSED_T, 1)
 k_fused_pruned_attention(const __grid_constant__ FusedParams p, const __grid_constant__ FusedMaps maps) {
     extern __shared__ __align__(1024) unsigned char smem_fused[];
@@ -588,7 +589,7 @@ k_fused_pruned_attention(const __grid_constant__ FusedParams p, const __grid_con
         tcgen05_fence_after_sync();
         if (lock && tid == 0) atomicExch(&s_lock, 0);               // every thread of the group has left phase 1
         MXP_PROF(gc, 21);
-        fused_phase2<BF16, HD, DT>(gc, p, head, slot, mask_head, tile_begin, tile_step);
+        fused_phase2<BF16, HD, DT, KMAX>(gc, p, head, slot, mask_head, tile_begin, tile_step);
         // phase 2 ends with fence.proxy.async + group barrier: its shared memory and TMEM may be reused, and its TMA
         // reads of the slot have completed (every copy was waited for), so the next head may overwrite the slot
     }
