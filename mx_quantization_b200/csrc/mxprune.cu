@@ -114,7 +114,9 @@ k_quantize_blocks(View x, int rows_per_bh, int H, int64_t total_rows, int hd, in
         quantize_block_thread<true, false>(xv, nd, bf16 != 0, flush != 0, r);
         exps[row * nb + b] = (int8_t)r.e;
         uint32_t* dst = reinterpret_cast<uint32_t*>(codes + row * hd + 32 * b);
-        if ((hd & 15) == 0) {
+        // two 16-byte stores only for a full block with 16-byte aligned rows: a partial last block (hd % 32 == 16)
+        // writes its own nd bytes, not the first codes of the next row
+        if ((hd & 15) == 0 && nd == 32) {
             reinterpret_cast<uint4*>(dst)[0] = make_uint4(r.cw[0], r.cw[1], r.cw[2], r.cw[3]);
             reinterpret_cast<uint4*>(dst)[1] = make_uint4(r.cw[4], r.cw[5], r.cw[6], r.cw[7]);
         } else {
