@@ -6,7 +6,8 @@ Public API (mirrors the reference's operator interface for this path):
     pruned_attention(q, k, v, mx_specs, top_k, scale=None, return_mask=False)
     predict_topk / sparse_attention / quantize_mxint8 / predict_scores / exp_sign_approx
     mx_linear / mx_mlp (MX Linear, and the fused fc1 -> GELU -> fc2 MLP; both take adaLN's shift / scale / residual / gate)
-    modules.QuantizedAttentionCore / DeiT, DiT, PixArt attention shims / QuantizedMlp / QuantizedDiTBlock (a DiT block)
+    modules.QuantizedAttentionCore / DeiT, DiT, PixArt attention shims / QuantizedMlp (timm Mlp or diffusers FeedForward)
+    / QuantizedDiTBlock (a DiT block) / QuantizedPixArtBlock (a PixArt-alpha adaLN-single block)
 """
 from .ops import (exp_sign_approx, last_launch_count, limits, mx_linear, mx_linear_prepare_weight,  # noqa: F401
                   mx_mlp, predict_scores, predict_topk,

@@ -18,7 +18,8 @@ reference runs in the last block of each model - same kernels with every key kep
 unquantized torch path) raises - no silent fallback.
 
 ``QuantizedDiTBlock`` wraps a whole DiT block (workloads/DiT/models.py:271-297): its adaLN modulations and gated residuals
-run inside the MX Linear kernels of the Attention shim and of QuantizedMlp.
+run inside the MX Linear kernels of the Attention shim and of QuantizedMlp.  ``QuantizedPixArtBlock`` does the same for
+PixArt-alpha's adaLN-single block, with q, k and v from one projection GEMM.
 """
 from typing import Optional
 
@@ -130,24 +131,51 @@ class QuantizedAttention(nn.Module):
         return x
 
 
+def _feed_forward_layers(net):
+    """diffusers' FeedForward.net (PixArt's feed-forward) -> (fc1, act, hidden dropout p, fc2, output dropout p):
+    net[0] a GELU module that owns fc1 as ``.proj`` and applies ``F.gelu(approximate=.approximate)``, net[1] the Dropout
+    between the activation and fc2, net[2] fc2, and an optional trailing Dropout.  Recognised by structure (diffusers is
+    not a dependency); anything else raises TypeError."""
+    act = net[0] if len(net) else None
+    if not isinstance(getattr(act, "proj", None), nn.Linear) or getattr(act, "approximate", None) not in ("none", "tanh"):
+        raise TypeError(f"QuantizedMlp: net[0] must be a GELU module with a Linear .proj and .approximate 'none' or "
+                        f"'tanh' (diffusers' FeedForward), got {type(act).__name__}")
+    if (len(net) not in (3, 4) or not isinstance(net[1], nn.Dropout) or not isinstance(net[2], nn.Linear)
+            or (len(net) == 4 and not isinstance(net[3], nn.Dropout))):
+        raise TypeError("QuantizedMlp: a FeedForward's net must be [GELU, Dropout, Linear] with an optional trailing "
+                        f"Dropout, got [{', '.join(type(m).__name__ for m in net)}]")
+    return act.proj, nn.GELU(approximate=act.approximate), net[1].p, net[2], net[3].p if len(net) == 4 else 0.0
+
+
 class QuantizedMlp(nn.Module):
     """DeiT MLP with MX Linear layers - mirrors workloads/deit/scripts/main.py:159-196 (fc1 -> act -> fc2 -> drop;
     the activation stays the host model's own module, as in the reference).
 
+    ``orig_mlp`` may also be diffusers' ``FeedForward`` (PixArt: ``net = [GELU(proj=fc1), Dropout, fc2, (Dropout)]``,
+    recognised by structure): fc1 is ``net[0].proj``, the activation ``nn.GELU(approximate=net[0].approximate)`` and fc2
+    ``net[2]``; its dropout between the activation and fc2 is ``drop_hidden``.
+
     When the activation is exactly ``torch.nn.GELU`` (either approximation) and fc1 / fc2 share one MX configuration, the
     forward is one ops.mx_mlp call on the layers' cached weight operands: bit for bit the layer-by-layer composition, with
-    the hidden activation never written in a float type.  Any other activation (a subclass or another GELU class too)
-    runs the composition."""
+    the hidden activation never written in a float type.  Any other activation (a subclass or another GELU class too),
+    and an active ``drop_hidden`` while training, runs the composition."""
 
     def __init__(self, orig_mlp, mx_specs=None):
         super().__init__()
         self.mx_specs = mx_specs
-        self.act = orig_mlp.act
-        self.drop = nn.Dropout(getattr(getattr(orig_mlp, "drop", None), "p", 0.0))
-        self.fc1, self.fc2 = to_mx_linear(orig_mlp.fc1, mx_specs), to_mx_linear(orig_mlp.fc2, mx_specs)
+        net = getattr(orig_mlp, "net", None)
+        if net is not None:
+            fc1, self.act, p_hidden, fc2, p = _feed_forward_layers(net)
+        else:
+            fc1, self.act, fc2 = orig_mlp.fc1, orig_mlp.act, orig_mlp.fc2
+            p_hidden, p = 0.0, getattr(getattr(orig_mlp, "drop", None), "p", 0.0)
+        self.drop_hidden = nn.Dropout(p_hidden)
+        self.drop = nn.Dropout(p)
+        self.fc1, self.fc2 = to_mx_linear(fc1, mx_specs), to_mx_linear(fc2, mx_specs)
 
     def _fused(self) -> bool:
-        return type(self.act) is nn.GELU and resolve_linear_specs(self.fc1.mx_specs) == resolve_linear_specs(self.fc2.mx_specs)
+        return (type(self.act) is nn.GELU and not (self.training and self.drop_hidden.p > 0)
+                and resolve_linear_specs(self.fc1.mx_specs) == resolve_linear_specs(self.fc2.mx_specs))
 
     def _mx_mlp(self, x, **adaln):
         self.fc1._check_inference(x.requires_grad)
@@ -161,7 +189,7 @@ class QuantizedMlp(nn.Module):
     def forward(self, x):
         if self._fused():
             return self.drop(self._mx_mlp(x))
-        return self.drop(self.fc2(self.act(self.fc1(x))))
+        return self.drop(self.fc2(self.drop_hidden(self.act(self.fc1(x)))))
 
     def forward_adaln(self, x, shift, scale, residual, gate):
         """The MLP half of DiT's DiTBlock.forward (workloads/DiT/models.py:297) on an already-normalized x (B, T, C):
@@ -296,6 +324,7 @@ class MXSelfAttention(nn.Module):
         self.to_out = nn.Sequential(nn.Linear(dim, dim, bias=has_bias), nn.Dropout(p=0.0))
         self.core = None
         self.current_timestep = 0
+        self._qkv_op = self._qkv_bias = self._qkv_key = None
 
     def set_config(self, mx_quant=False, mx_specs=None, top_k=False, k=20, ex_pred=False, exclude_timesteps=None,
                    pred_mode="ex_pred", block_idx=None, anal=False, file_name_dict=None, orthogonal_matrix=None):
@@ -324,6 +353,48 @@ class MXSelfAttention(nn.Module):
         self.current_timestep += 1
         return x
 
+    def _qkv_operand(self):
+        """(operand, bias) of to_q, to_k and to_v as one (3C, C) layer: ``mx_linear_prepare_weight(cat([Wq, Wk, Wv]))``
+        and ``cat([bq, bk, bv])``.  Cached; rebuilt when any of the six tensors changes (data_ptr, version, device, dtype,
+        as MxLinear._operand keys its own) or after any of the three layers' invalidate(), which load_state_dict calls."""
+        layers = (self.to_q, self.to_k, self.to_v)
+        key = tuple((m._w_gen,) + tuple((t.data_ptr(), t._version, str(t.device), t.dtype)
+                                        for t in (m.weight, m.bias) if t is not None) for m in layers)
+        if self._qkv_key != key:
+            self._qkv_op = ops.mx_linear_prepare_weight(torch.cat([m.weight.detach() for m in layers]), self.to_q.mx_specs)
+            self._qkv_bias = None if self.to_q.bias is None else torch.cat([m.bias.detach() for m in layers])
+            self._qkv_key = key
+        return self._qkv_op, self._qkv_bias
+
+    def forward_adaln(self, x, shift, scale, residual, gate):
+        """The self-attention half of PixArt's adaLN-single block (diffusers' BasicTransformerBlock) on the normalized
+        hidden states x (B, N, C): ``residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) +
+        shift.unsqueeze(1))``, bit for bit.  shift / scale / gate: (B, C) rows, e.g. ``.squeeze(1)`` of the block's
+        (B, 1, C) chunks, read in place.
+
+        q, k and v come from ONE mx_linear call on the concatenated (3C, C) weight, whose quantizer applies the
+        modulation: the GEMM has no split-K, so every output column is reduced in the same order whichever 256-column
+        tile holds it, and its bits are those of the separate projection.  The core reads q, k, v as strided views of
+        the (B, N, 3C) result (dense on exclude_timesteps steps, as forward), to_out[0]'s store applies the gated
+        residual, and current_timestep advances.  While to_out's dropout is active (training, p > 0), or when the three
+        projections have different MX configurations, the expression runs as written."""
+        if self.core is None:
+            raise RuntimeError("MXSelfAttention.set_config(...) must be called first")
+        layers = (self.to_q, self.to_k, self.to_v)
+        if ((self.training and self.to_out[1].p > 0)
+                or len({resolve_linear_specs(m.mx_specs) for m in layers}) != 1):
+            return residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1))
+        for m in layers:
+            m._check_inference(x.requires_grad)
+        B, N, C = x.shape
+        w_op, b = self._qkv_operand()
+        qkv = ops.mx_linear(x, w_op, b, self.to_q.mx_specs, out_features=3 * C, shift=shift, scale=scale)
+        q, k, v = qkv.view(B, N, 3, self.num_heads, self.head_dim).permute(2, 0, 3, 1, 4).unbind(0)
+        x = self.core(q, k, v, dense=self.current_timestep in self.exclude_timesteps)
+        x = self.to_out[0].forward_adaln(x, residual=residual, gate=gate)
+        self.current_timestep += 1
+        return x
+
 
 class MXCrossAttention(MXSelfAttention):
     """PixArt-alpha cross-attention shim - mirrors workloads/PixArt/models/MX_transformer_block.py:720-859:
@@ -348,6 +419,63 @@ class MXCrossAttention(MXSelfAttention):
         self.current_timestep += 1
         return x
 
+    def forward_adaln(self, *args, **kwargs):
+        raise TypeError("MXCrossAttention has no adaLN form (PixArt's block adds its output without a gate); "
+                        "forward_adaln is the self-attention half's")
+
+
+class QuantizedPixArtBlock(nn.Module):
+    """PixArt-alpha transformer block: diffusers' BasicTransformerBlock with norm_type="ada_norm_single", which the
+    reference's MXBasicTransformerBlock keeps.  forward computes, bit for bit on the same modules:
+        shift_msa, scale_msa, gate_msa, shift_mlp, scale_mlp, gate_mlp = (
+            scale_shift_table[None] + timestep.reshape(B, 6, -1)).chunk(6, dim=1)
+        h = gate_msa * attn1(norm1(h) * (1 + scale_msa) + shift_msa) + h
+        h = attn2(h, encoder_hidden_states, attention_mask=encoder_attention_mask) + h
+        h = gate_mlp * ff(norm2(h) * (1 + scale_mlp) + shift_mlp) + h
+    The self-attention and feed-forward halves run with their modulations and gated residuals inside the MX Linear
+    kernels (MXSelfAttention.forward_adaln, with q, k and v from one GEMM, and QuantizedMlp.forward_adaln); IEEE add and
+    multiply commute, so the kernels' ``h + gate * y`` is ``gate * y + h``.  attn2 runs its own forward and its residual
+    is a torch add.
+
+    ``orig_block``: ``attn1`` an MXSelfAttention and ``attn2`` an MXCrossAttention (or None), both after set_config;
+    ``ff`` a QuantizedMlp or diffusers' FeedForward (wrapped in QuantizedMlp); ``norm1`` / ``norm2`` (torch LayerNorm)
+    and the (6, C) ``scale_shift_table`` stay the host model's."""
+
+    def __init__(self, orig_block, mx_specs=None):
+        super().__init__()
+        attn1, attn2, ff = orig_block.attn1, orig_block.attn2, orig_block.ff
+        if not isinstance(attn1, MXSelfAttention) or isinstance(attn1, MXCrossAttention):
+            raise TypeError(f"QuantizedPixArtBlock: attn1 must be modules.MXSelfAttention, got {type(attn1).__name__}")
+        if attn2 is not None and not isinstance(attn2, MXCrossAttention):
+            raise TypeError(f"QuantizedPixArtBlock: attn2 must be modules.MXCrossAttention or None, got "
+                            f"{type(attn2).__name__}")
+        for name, a in (("attn1", attn1), ("attn2", attn2)):
+            if a is not None and a.core is None:
+                raise RuntimeError(f"QuantizedPixArtBlock: {name}.set_config(...) must be called first")
+        if not isinstance(ff, QuantizedMlp) and not hasattr(ff, "net"):
+            raise TypeError(f"QuantizedPixArtBlock: ff must be QuantizedMlp or diffusers' FeedForward, got "
+                            f"{type(ff).__name__}")
+        self.norm1, self.attn1, self.attn2, self.norm2 = orig_block.norm1, attn1, attn2, orig_block.norm2
+        self.ff = ff if isinstance(ff, QuantizedMlp) else QuantizedMlp(ff, mx_specs=mx_specs)
+        self.scale_shift_table = orig_block.scale_shift_table
+
+    def forward(self, hidden_states, attention_mask=None, encoder_hidden_states=None, encoder_attention_mask=None,
+                timestep=None, **kwargs):
+        """BasicTransformerBlock.forward's arguments; ``encoder_attention_mask`` is the additive (B, 1, S) text bias the
+        diffusers transformer builds.  The other keyword arguments are ignored, as the attention shims ignore theirs."""
+        if attention_mask is not None:
+            raise ValueError("QuantizedPixArtBlock: a self-attention attention_mask cannot be applied on the fused path "
+                             "(PixArt passes none)")
+        if timestep is None:
+            raise ValueError("QuantizedPixArtBlock: timestep (the adaLN-single embedding, (B, 6 * C)) is required")
+        h = hidden_states
+        shift_msa, scale_msa, gate_msa, shift_mlp, scale_mlp, gate_mlp = (
+            t.squeeze(1) for t in (self.scale_shift_table[None] + timestep.reshape(h.shape[0], 6, -1)).chunk(6, dim=1))
+        h = self.attn1.forward_adaln(self.norm1(h), shift_msa, scale_msa, h, gate_msa)
+        if self.attn2 is not None:
+            h = self.attn2(h, encoder_hidden_states, attention_mask=encoder_attention_mask) + h
+        return self.ff.forward_adaln(self.norm2(h), shift_mlp, scale_mlp, h, gate_mlp)
+
 
 class MxLinear(nn.Linear):
     """Drop-in for the reference's mx.Linear (microxscaling/mx/linear.py:227-320) on the MXINT8
@@ -363,6 +491,7 @@ class MxLinear(nn.Linear):
         self.name = name
         self._w_op = None
         self._w_key = None
+        self._w_gen = 0             # counts invalidate() calls: keys operands cached outside the layer (MXSelfAttention's)
         # a loaded checkpoint writes the weight through .data (no version bump): drop the cached operand
         self.register_load_state_dict_post_hook(lambda module, incompatible_keys: module.invalidate())
 
@@ -370,6 +499,7 @@ class MxLinear(nn.Linear):
         """Drop the cached MX-quantized weight operand (call after writing the weight through ``.data``)."""
         self._w_op = None
         self._w_key = None
+        self._w_gen += 1
 
     def _check_inference(self, inputs_require_grad: bool):
         if torch.is_grad_enabled() and (self.weight.requires_grad or inputs_require_grad):
