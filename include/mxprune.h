@@ -47,7 +47,7 @@
 extern "C" {
 #endif
 
-#define MXP_ABI_VERSION 7
+#define MXP_ABI_VERSION 8
 
 /*
  * Element types of q/k/v/x and out for the *_dt entry points.  The fp32 entry points are the *_dt ones with
@@ -371,6 +371,48 @@ int mxp_mx_mlp_adaln_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, c
                         int64_t ld_shift, const void* scale, int64_t ld_scale, const void* residual,
                         int64_t ld_residual, const void* gate, int64_t ld_gate, void* workspace,
                         size_t workspace_bytes, void* stream);
+
+/*
+ * Pre-norm MX Linear / MLP with every block addition optional (DeiT's timm Block, DiT, PixArt-alpha):
+ *     out = add(f(modulate(layer_norm(x))))
+ * mxp_mx_linear_ex_dt takes the arguments of mxp_mx_linear_adaln_dt, mxp_mx_mlp_ex_dt those of mxp_mx_mlp_adaln_dt,
+ * with three differences:
+ *   layer_norm        1: the operand is quantized from torch.nn.functional.layer_norm(x, (K,), ln_weight, ln_bias,
+ *                     ln_eps) on CUDA, bit for bit (mxp_layer_norm_dt's y, rounded to x_dtype), before the
+ *                     modulation; 0: no norm (ln_weight / ln_bias must be NULL).
+ *   ln_weight, ln_bias  K elements of x_dtype each, 16-byte (fp32) or 8-byte (16-bit) aligned; both or neither.
+ *   residual without gate  a plain add: the stored value is rd(residual + y) (DeiT's x + attn(norm1(x))).  With the
+ *                     gate it is the gated residual of the adaLN entry points.  gate without residual is an error.
+ * Without shift / scale / gate, tokens only has to divide M (pass M).  Launches, in order: with the norm, the row
+ * statistics kernel (k_layer_norm: one warp per row of x, writing each row's fp32 mean and rstd to the
+ * workspace); then exactly the launches of the plain call (x's quantizer applies the norm and the modulation as it
+ * loads x; the last GEMM's store applies the residual).  workspace: mxp_mx_linear_ex_workspace_bytes /
+ * mxp_mx_mlp_ex_workspace_bytes bytes, 256-byte aligned: the plain call's workspace followed by the statistics,
+ * 2 * align256(4 * M) bytes (without the norm the plain call's size suffices).
+ */
+size_t mxp_mx_linear_ex_workspace_bytes(int M, int N, int K);
+size_t mxp_mx_mlp_ex_workspace_bytes(int M, int K, int N1, int N2);
+int mxp_mx_linear_ex_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N,
+                        const void* bias, int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo,
+                        int layer_norm, const void* ln_weight, const void* ln_bias, float ln_eps, int tokens,
+                        const void* shift, int64_t ld_shift, const void* scale, int64_t ld_scale, const void* residual,
+                        int64_t ld_residual, const void* gate, int64_t ld_gate, void* workspace,
+                        size_t workspace_bytes, void* stream);
+int mxp_mx_mlp_ex_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1, const void* b1,
+                     int b1_dtype, int act, const void* w2_op, int N2, const void* b2, int b2_dtype, int bfloat_bits,
+                     int flush, void* out, int64_t ldo, int layer_norm, const void* ln_weight, const void* ln_bias,
+                     float ln_eps, int tokens, const void* shift, int64_t ld_shift, const void* scale, int64_t ld_scale,
+                     const void* residual, int64_t ld_residual, const void* gate, int64_t ld_gate, void* workspace,
+                     size_t workspace_bytes, void* stream);
+/*
+ * Parity aid: the LayerNorm the _ex entry points apply, on (M, K) rows of x (dtype MXP_DT_*, row stride ldx):
+ * torch.native_layer_norm(x, (K,), weight, bias, eps) on CUDA bit for bit - y (contiguous (M, K) of dtype), and the
+ * fp32 mean and rstd of each row.  weight and bias: K elements of dtype each, or both NULL.  K a multiple of 4 up to
+ * 2^24 (the rows torch's vectorized kernel takes); x, y, weight and bias 16-byte (fp32) or 8-byte (16-bit) aligned,
+ * ldx a multiple of 4.  One launch (k_layer_norm), no workspace.
+ */
+int mxp_layer_norm_dt(const void* x, int dtype, int64_t ldx, int M, int K, const void* weight, const void* bias,
+                      float eps, void* y, float* mean, float* rstd, void* stream);
 
 /*
  * Measurement aid: same as mxp_pruned_attention (tcgen05 path), but brackets the three kernels

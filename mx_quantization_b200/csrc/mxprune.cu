@@ -1312,22 +1312,44 @@ static int check_linear(int M, int N, int K, int bfloat_bits) {
     if (bfloat_bits != 16 && bfloat_bits != 32) return fail(MXP_E_UNSUPPORTED, "bfloat=%d: only 16 or 32 are on the path", bfloat_bits);
     return MXP_OK;
 }
-// mod: the adaLN modulation of x (ModParams), or null
+// mod: the adaLN modulation of x (ModParams), or null; norm_kind / norm: the LayerNorm of x (LN_PLAIN / LN_AFFINE,
+// with the row statistics k_layer_norm wrote to norm->mean / rstd), or LN_NONE
 static int launch_quantize_gemm_operand(const void* x, int dt, int64_t ld, int rows, int K, int rows_tile, int bf16,
-                                        int flush, void* op, cudaStream_t st, const ModParams* mod = nullptr) {
+                                        int flush, void* op, cudaStream_t st, const ModParams* mod = nullptr,
+                                        int norm_kind = LN_NONE, const NormParams* norm = nullptr) {
     const int rows_pad = (rows + rows_tile - 1) / rows_tile * rows_tile;
     const int64_t ntask = (int64_t)rows_pad * (K / 32);
     int64_t blocks = (ntask + 255) / 256;
     if (blocks > 148 * 32) blocks = 148 * 32;
-#define MXP_QG(DT_) (mod ? k_quantize_gemm_operand<DT_, true><<<(unsigned)blocks, 256, 0, st>>>( \
-                               (const float*)x, ld, rows, rows_pad, K, rows_tile, bf16, flush, (unsigned char*)op, *mod) \
-                         : k_quantize_gemm_operand<DT_><<<(unsigned)blocks, 256, 0, st>>>( \
-                               (const float*)x, ld, rows, rows_pad, K, rows_tile, bf16, flush, (unsigned char*)op, ModParams{}))
+    const NormParams np = norm ? *norm : NormParams{};
+#define MXP_QG2(DT_, MOD_, NORM_) k_quantize_gemm_operand<DT_, MOD_, NORM_><<<(unsigned)blocks, 256, 0, st>>>( \
+        (const float*)x, ld, rows, rows_pad, K, rows_tile, bf16, flush, (unsigned char*)op, mod ? *mod : ModParams{}, np)
+#define MXP_QG1(DT_, NORM_) (mod ? MXP_QG2(DT_, true, NORM_) : MXP_QG2(DT_, false, NORM_))
+#define MXP_QG(DT_) (norm_kind == LN_AFFINE ? MXP_QG1(DT_, LN_AFFINE) \
+                     : norm_kind == LN_PLAIN ? MXP_QG1(DT_, LN_PLAIN) : MXP_QG1(DT_, LN_NONE))
     if (dt == DT_BF16) MXP_QG(DT_BF16);
     else if (dt == DT_F16) MXP_QG(DT_F16);
     else MXP_QG(DT_F32);
 #undef MXP_QG
+#undef MXP_QG1
+#undef MXP_QG2
     return check_launch("k_quantize_gemm_operand");
+}
+
+// k_layer_norm<dt, norm_kind>: one warp per row; y (the normalized rows) may be null (statistics only)
+static int launch_layer_norm(const void* x, int dt, int64_t ld, int rows, int K, float eps, int norm_kind,
+                             const void* w, const void* b, float* mean, float* rstd, void* y, cudaStream_t st) {
+    const unsigned grid = (unsigned)((rows + LN_ROWS - 1) / LN_ROWS);
+    const float *xp = (const float*)x, *wp = (const float*)w, *bp = (const float*)b;
+#define MXP_LN(DT_) (norm_kind == LN_AFFINE ? k_layer_norm<DT_, LN_AFFINE><<<grid, LN_ROWS * 32, 0, st>>>( \
+                         xp, ld, rows, K, eps, wp, bp, mean, rstd, (float*)y) \
+                     : k_layer_norm<DT_, LN_PLAIN><<<grid, LN_ROWS * 32, 0, st>>>(xp, ld, rows, K, eps, wp, bp, mean, \
+                                                                                  rstd, (float*)y))
+    if (dt == DT_BF16) MXP_LN(DT_BF16);
+    else if (dt == DT_F16) MXP_LN(DT_F16);
+    else MXP_LN(DT_F32);
+#undef MXP_LN
+    return check_launch("k_layer_norm");
 }
 
 // rows of a GEMM input (x or W): a 16-byte aligned base, a row stride >= K whose rows stay 16-byte aligned
@@ -1398,12 +1420,17 @@ int mxp_mx_linear_prepare_weight(const float* w, int64_t ldw, int N, int K, int 
     return mxp_mx_linear_prepare_weight_dt(w, MXP_DT_F32, ldw, N, K, bfloat_bits, flush, w_op, stream);
 }
 
-// ---- adaLN additions of mxp_mx_linear_adaln_dt / mxp_mx_mlp_adaln_dt: the modulation of x (mod, K wide) and the
-// gated residual of the output (N wide), each optional
+// ---- additions of the adaLN and the _ex entry points: the LayerNorm of x (K wide), the modulation of x (mod, K wide)
+// and the residual (gated, or with plain_add a plain add) of the output (N wide), each optional
 struct Adaln {
     int tokens;
     const void *shift, *scale, *residual, *gate;
     int64_t ld_shift, ld_scale, ld_residual, ld_gate;
+    bool plain_add;                   // a residual without a gate is a plain add (the _ex entry points)
+    int layer_norm;                   // 0 or 1
+    const void *ln_weight, *ln_bias;
+    float ln_eps;
+    int norm_kind() const { return !layer_norm ? LN_NONE : ln_weight ? LN_AFFINE : LN_PLAIN; }
 };
 
 // an (M / tokens, N) gate or (M, N) residual of x's type: the alignment and row-stride rules of out
@@ -1419,25 +1446,55 @@ static int check_adaln(const Adaln& a, int dt, int M, int K, int N) {
     if (a.tokens <= 0 || M % a.tokens)
         return fail(MXP_E_BADARG, "tokens %d: need a positive divisor of the row count M=%d", a.tokens, M);
     if (!a.shift != !a.scale) return fail(MXP_E_BADARG, "shift and scale: give both or neither");
-    if (!a.residual != !a.gate) return fail(MXP_E_BADARG, "residual and gate: give both or neither");
+    if (a.gate && !a.residual) return fail(MXP_E_BADARG, "gate without residual");
+    if (a.residual && !a.gate && !a.plain_add) return fail(MXP_E_BADARG, "residual and gate: give both or neither");
+    if (a.layer_norm != 0 && a.layer_norm != 1) return fail(MXP_E_BADARG, "layer_norm %d: 0 or 1", a.layer_norm);
+    if (!a.ln_weight != !a.ln_bias) return fail(MXP_E_BADARG, "ln_weight and ln_bias: give both or neither");
+    if (a.ln_weight && !a.layer_norm) return fail(MXP_E_BADARG, "ln_weight / ln_bias without layer_norm");
+    // the norm's weight and bias are read 4 elements (16 or 8 bytes) at a time
+    const uintptr_t ln_align = dt == DT_F32 ? 15 : 7;
+    if (a.ln_weight && (((uintptr_t)a.ln_weight & ln_align) || ((uintptr_t)a.ln_bias & ln_align)))
+        return fail(MXP_E_BADARG, "ln_weight / ln_bias: misaligned pointer");
+    if (a.layer_norm && !(a.ln_eps >= 0.f)) return fail(MXP_E_BADARG, "ln_eps: need a number >= 0");
     int rc = MXP_OK;
     // shift / scale are read in 32-element blocks, 16 bytes at a time: the rules of x
     if (a.shift && ((rc = check_linear_rows("shift", a.shift, dt, a.ld_shift, K)) ||
                     (rc = check_linear_rows("scale", a.scale, dt, a.ld_scale, K))))
         return rc;
-    if (a.residual && ((rc = check_out_like("residual", a.residual, dt, a.ld_residual, N)) ||
-                       (rc = check_out_like("gate", a.gate, dt, a.ld_gate, N))))
-        return rc;
+    if (a.residual && (rc = check_out_like("residual", a.residual, dt, a.ld_residual, N))) return rc;
+    if (a.gate && (rc = check_out_like("gate", a.gate, dt, a.ld_gate, N))) return rc;
     return MXP_OK;
 }
 
 static ModParams make_mod(const Adaln& a) {
     return ModParams{(const float*)a.shift, (const float*)a.scale, a.ld_shift, a.ld_scale, a.tokens};
 }
-static void set_gated_residual(LinearParams& lp, const Adaln& a) {
-    lp.residual = (const float*)a.residual; lp.ldr = a.ld_residual;
-    lp.gate = (const float*)a.gate; lp.ldg = a.ld_gate; lp.tokens = a.tokens;
+// the store of the GEMM's output: plain, or with the residual (gated or plain add)
+static int launch_output_gemm(LinearParams& lp, const Adaln* a, int out_dt, cudaStream_t st) {
+    if (!a || !a->residual) return launch_linear_gemm<EPI_STORE>(lp, out_dt, st);
+    lp.residual = (const float*)a->residual; lp.ldr = a->ld_residual;
+    if (!a->gate) return launch_linear_gemm<EPI_RESIDUAL>(lp, out_dt, st);
+    lp.gate = (const float*)a->gate; lp.ldg = a->ld_gate; lp.tokens = a->tokens;
+    return launch_linear_gemm<EPI_GATED_RESIDUAL>(lp, out_dt, st);
 }
+
+// x's operand: the per-row LayerNorm statistics into `stats` (when the norm is on), then the quantizer
+static int launch_activation_operand(const void* x, int dt, int64_t ldx, int M, int K, int bf16, int flush,
+                                     unsigned char* a_op, float* stats, const Adaln* ad, cudaStream_t st) {
+    ModParams mod{};
+    if (ad && ad->shift) mod = make_mod(*ad);
+    const int nk = ad ? ad->norm_kind() : LN_NONE;
+    float *mean = stats, *rstd = stats + align256((size_t)M * 4) / 4;
+    const NormParams np{mean, rstd, (const float*)(ad ? ad->ln_weight : nullptr), (const float*)(ad ? ad->ln_bias : nullptr)};
+    int rc;
+    if (nk != LN_NONE && (rc = launch_layer_norm(x, dt, ldx, M, K, ad->ln_eps, nk, np.w, np.b, mean, rstd, nullptr, st)))
+        return rc;
+    return launch_quantize_gemm_operand(x, dt, ldx, M, K, GL_BM, bf16, flush, a_op, st, ad && ad->shift ? &mod : nullptr,
+                                        nk, &np);
+}
+
+// the per-row mean and rstd (fp32 each) of the _ex entry points: after the plain call's workspace
+static size_t ln_stats_bytes(int M) { return 2 * align256((size_t)M * 4); }
 
 static int mx_linear_impl(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N,
                           const void* bias, int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo,
@@ -1453,26 +1510,21 @@ static int mx_linear_impl(const void* x, int x_dtype, int64_t ldx, int M, int K,
         return fail(MXP_E_BADARG, "w_op / out: null or misaligned pointer, or out row stride %lld not >= %d and a multiple "
                     "of 4", (long long)ldo, N);
     if (ad && (rc = check_adaln(*ad, x_dtype, M, K, N))) return rc;
-    const size_t need = mxp_mx_linear_workspace_bytes(M, N, K);
+    const size_t plain = mxp_mx_linear_workspace_bytes(M, N, K);
+    const size_t need = plain + (ad && ad->layer_norm ? ln_stats_bytes(M) : 0);
     if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255))
         return fail(MXP_E_BADARG, "workspace: need %zu bytes, 256-byte aligned", need);
     cudaStream_t st = (cudaStream_t)stream;
     unsigned char* a_op = (unsigned char*)workspace;
     float* rbias = (float*)(a_op + align256((size_t)((M + GL_BM - 1) / GL_BM) * GL_BM * (size_t)K * 2));
-    ModParams mod{};
-    if (ad && ad->shift) mod = make_mod(*ad);
-    if ((rc = launch_quantize_gemm_operand(x, x_dtype, ldx, M, K, GL_BM, bfloat_bits == 16, flush != 0, a_op, st,
-                                           ad && ad->shift ? &mod : nullptr)))
+    float* stats = (float*)((unsigned char*)workspace + plain);
+    if ((rc = launch_activation_operand(x, x_dtype, ldx, M, K, bfloat_bits == 16, flush != 0, a_op, stats, ad, st)))
         return rc;
     if (bias && (rc = launch_round_bias(bias, bias_dtype, rbias, N, bfloat_bits == 16, st))) return rc;
     LinearParams lp{};
     lp.a_op = a_op; lp.w_op = (const unsigned char*)w_op; lp.bias = bias ? rbias : nullptr;
     lp.out = (float*)out; lp.ldo = ldo; lp.M = M; lp.N = N; lp.K = K; lp.bf16 = bfloat_bits == 16; lp.stages = 4;
-    if (ad && ad->residual) {
-        set_gated_residual(lp, *ad);
-        return launch_linear_gemm<EPI_GATED_RESIDUAL>(lp, x_dtype, st);
-    }
-    return launch_linear_gemm<EPI_STORE>(lp, x_dtype, st);
+    return launch_output_gemm(lp, ad, x_dtype, st);
 }
 
 int mxp_mx_linear_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N, const void* bias,
@@ -1487,7 +1539,8 @@ int mxp_mx_linear_adaln_dt(const void* x, int x_dtype, int64_t ldx, int M, int K
                            int tokens, const void* shift, int64_t ld_shift, const void* scale, int64_t ld_scale,
                            const void* residual, int64_t ld_residual, const void* gate, int64_t ld_gate,
                            void* workspace, size_t workspace_bytes, void* stream) {
-    const Adaln ad{tokens, shift, scale, residual, gate, ld_shift, ld_scale, ld_residual, ld_gate};
+    const Adaln ad{tokens, shift, scale, residual, gate, ld_shift, ld_scale, ld_residual, ld_gate, false, 0, nullptr,
+                   nullptr, 0.f};
     return mx_linear_impl(x, x_dtype, ldx, M, K, w_op, N, bias, bias_dtype, bfloat_bits, flush, out, ldo, &ad,
                           workspace, workspace_bytes, stream);
 }
@@ -1518,7 +1571,8 @@ static int mx_mlp_impl(const void* x, int x_dtype, int64_t ldx, int M, int K, co
         return fail(MXP_E_BADARG, "w1_op / w2_op / out: null or misaligned pointer, or out row stride %lld not >= %d and "
                     "a multiple of 4", (long long)ldo, N2);
     if (ad && (rc = check_adaln(*ad, x_dtype, M, K, N2))) return rc;
-    const size_t need = mxp_mx_mlp_workspace_bytes(M, K, N1, N2);
+    const size_t plain = mxp_mx_mlp_workspace_bytes(M, K, N1, N2);
+    const size_t need = plain + (ad && ad->layer_norm ? ln_stats_bytes(M) : 0);
     if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255))
         return fail(MXP_E_BADARG, "workspace: need %zu bytes, 256-byte aligned", need);
     cudaStream_t st = (cudaStream_t)stream;
@@ -1528,11 +1582,8 @@ static int mx_mlp_impl(const void* x, int x_dtype, int64_t ldx, int M, int K, co
     float* rb1 = (float*)(h_op + align256(rows * (size_t)N1 * 2));
     float* rb2 = (float*)((unsigned char*)rb1 + align256((size_t)N1 * 4));
     const int bf16 = bfloat_bits == 16;
-    ModParams mod{};
-    if (ad && ad->shift) mod = make_mod(*ad);
-    if ((rc = launch_quantize_gemm_operand(x, x_dtype, ldx, M, K, GL_BM, bf16, flush != 0, a_op, st,
-                                           ad && ad->shift ? &mod : nullptr)))
-        return rc;
+    float* stats = (float*)((unsigned char*)workspace + plain);
+    if ((rc = launch_activation_operand(x, x_dtype, ldx, M, K, bf16, flush != 0, a_op, stats, ad, st))) return rc;
     if (b1 && (rc = launch_round_bias(b1, b1_dtype, rb1, N1, bf16, st))) return rc;
     if (b2 && (rc = launch_round_bias(b2, b2_dtype, rb2, N2, bf16, st))) return rc;
     LinearParams l1{};
@@ -1544,11 +1595,7 @@ static int mx_mlp_impl(const void* x, int x_dtype, int64_t ldx, int M, int K, co
     LinearParams l2{};
     l2.a_op = h_op; l2.w_op = (const unsigned char*)w2_op; l2.bias = b2 ? rb2 : nullptr;
     l2.out = (float*)out; l2.ldo = ldo; l2.M = M; l2.N = N2; l2.K = N1; l2.bf16 = bf16; l2.stages = 4;
-    if (ad && ad->residual) {
-        set_gated_residual(l2, *ad);
-        return launch_linear_gemm<EPI_GATED_RESIDUAL>(l2, x_dtype, st);
-    }
-    return launch_linear_gemm<EPI_STORE>(l2, x_dtype, st);
+    return launch_output_gemm(l2, ad, x_dtype, st);
 }
 
 int mxp_mx_mlp_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1, const void* b1,
@@ -1564,9 +1611,61 @@ int mxp_mx_mlp_adaln_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, c
                         int64_t ld_shift, const void* scale, int64_t ld_scale, const void* residual,
                         int64_t ld_residual, const void* gate, int64_t ld_gate, void* workspace,
                         size_t workspace_bytes, void* stream) {
-    const Adaln ad{tokens, shift, scale, residual, gate, ld_shift, ld_scale, ld_residual, ld_gate};
+    const Adaln ad{tokens, shift, scale, residual, gate, ld_shift, ld_scale, ld_residual, ld_gate, false, 0, nullptr,
+                   nullptr, 0.f};
     return mx_mlp_impl(x, x_dtype, ldx, M, K, w1_op, N1, b1, b1_dtype, act, w2_op, N2, b2, b2_dtype, bfloat_bits, flush,
                        out, ldo, &ad, workspace, workspace_bytes, stream);
+}
+
+size_t mxp_mx_linear_ex_workspace_bytes(int M, int N, int K) {
+    return mxp_mx_linear_workspace_bytes(M, N, K) + ln_stats_bytes(M);
+}
+size_t mxp_mx_mlp_ex_workspace_bytes(int M, int K, int N1, int N2) {
+    return mxp_mx_mlp_workspace_bytes(M, K, N1, N2) + ln_stats_bytes(M);
+}
+
+int mxp_mx_linear_ex_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w_op, int N,
+                        const void* bias, int bias_dtype, int bfloat_bits, int flush, void* out, int64_t ldo,
+                        int layer_norm, const void* ln_weight, const void* ln_bias, float ln_eps, int tokens,
+                        const void* shift, int64_t ld_shift, const void* scale, int64_t ld_scale, const void* residual,
+                        int64_t ld_residual, const void* gate, int64_t ld_gate, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+    const Adaln ad{tokens, shift, scale, residual, gate, ld_shift, ld_scale, ld_residual, ld_gate, true, layer_norm,
+                   ln_weight, ln_bias, ln_eps};
+    return mx_linear_impl(x, x_dtype, ldx, M, K, w_op, N, bias, bias_dtype, bfloat_bits, flush, out, ldo, &ad,
+                          workspace, workspace_bytes, stream);
+}
+
+int mxp_mx_mlp_ex_dt(const void* x, int x_dtype, int64_t ldx, int M, int K, const void* w1_op, int N1, const void* b1,
+                     int b1_dtype, int act, const void* w2_op, int N2, const void* b2, int b2_dtype, int bfloat_bits,
+                     int flush, void* out, int64_t ldo, int layer_norm, const void* ln_weight, const void* ln_bias,
+                     float ln_eps, int tokens, const void* shift, int64_t ld_shift, const void* scale, int64_t ld_scale,
+                     const void* residual, int64_t ld_residual, const void* gate, int64_t ld_gate, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+    const Adaln ad{tokens, shift, scale, residual, gate, ld_shift, ld_scale, ld_residual, ld_gate, true, layer_norm,
+                   ln_weight, ln_bias, ln_eps};
+    return mx_mlp_impl(x, x_dtype, ldx, M, K, w1_op, N1, b1, b1_dtype, act, w2_op, N2, b2, b2_dtype, bfloat_bits, flush,
+                       out, ldo, &ad, workspace, workspace_bytes, stream);
+}
+
+int mxp_layer_norm_dt(const void* x, int dtype, int64_t ldx, int M, int K, const void* weight, const void* bias,
+                      float eps, void* y, float* mean, float* rstd, void* stream) {
+    g_launches = 0;
+    int rc = check_dtype("x", dtype);
+    if (rc) return rc;
+    if (M <= 0 || K <= 0 || (K & 3) || K > (1 << 24))
+        return fail(MXP_E_UNSUPPORTED, "shape M=%d K=%d: need M > 0 and K a positive multiple of 4 up to 2^24", M, K);
+    const uintptr_t al = dtype == DT_F32 ? 15 : 7;
+    if (!x || ((uintptr_t)x & al) || (ldx & 3) || ldx < K || !y || ((uintptr_t)y & al))
+        return fail(MXP_E_BADARG, "x / y: null or misaligned pointer, or x row stride %lld not >= %d and a multiple of 4",
+                    (long long)ldx, K);
+    if (!weight != !bias) return fail(MXP_E_BADARG, "weight and bias: give both or neither");
+    if (weight && (((uintptr_t)weight & al) || ((uintptr_t)bias & al)))
+        return fail(MXP_E_BADARG, "weight / bias: misaligned pointer");
+    if (!(eps >= 0.f)) return fail(MXP_E_BADARG, "eps: need a number >= 0");
+    if (!mean || !rstd) return fail(MXP_E_BADARG, "mean / rstd: null pointer");
+    return launch_layer_norm(x, dtype, ldx, M, K, eps, weight ? LN_AFFINE : LN_PLAIN, weight, bias, mean, rstd, y,
+                             (cudaStream_t)stream);
 }
 
 int mxp_activation_dt(const void* x, int dtype, int64_t n, int act, void* out, void* stream) {

@@ -21,10 +21,14 @@
 //                            EPI = EPI_GELU / EPI_GELU_TANH (the fused MLP's fc1): the epilogue applies the
 //                            activation and writes the NEXT GEMM's A operand instead of the output; each 32-column
 //                            pass over a TMEM row is one MX block of fc2's input, held by one thread.
-//                            EPI = EPI_GATED_RESIDUAL (an adaLN block's proj / fc2): the coalesced store path stores
-//                            residual + gate * y, with the residual read in the store's width and pattern.
-//   With MOD, k_quantize_gemm_operand applies the adaLN modulation x * (1 + scale) + shift to the elements it loads.
+//                            EPI = EPI_GATED_RESIDUAL (an adaLN block's proj / fc2) / EPI_RESIDUAL (a pre-norm block's):
+//                            the coalesced store path stores residual + gate * y / residual + y, with the residual read
+//                            in the store's width and pattern, its loads issued before the pass's TMEM read.
+//   k_layer_norm             torch's LayerNorm row statistics (and, as a parity aid, its output), bit for bit.
+//   With NORM, k_quantize_gemm_operand normalizes the elements it loads with those statistics; with MOD it then applies
+//   the adaLN modulation x * (1 + scale) + shift.
 #pragma once
+#include <type_traits>
 #include "mxprune_predict_tc.cuh"
 
 namespace mxp {
@@ -54,16 +58,24 @@ __device__ __forceinline__ float round_to_dt(float x) {
     else return x;
 }
 
+// four consecutive elements of type DT as loaded (16 bytes of fp32 or 8 bytes of 16-bit), and as fp32 bit patterns
+template <int DT>
+using elem4_raw_t = std::conditional_t<DT == DT_F32, uint4, uint2>;
+template <int DT>
+__device__ __forceinline__ elem4_raw_t<DT> load_elem4_raw(const float* p, int64_t off) {
+    if constexpr (DT == DT_F32) return *reinterpret_cast<const uint4*>(p + off);
+    else return *reinterpret_cast<const uint2*>(reinterpret_cast<const uint16_t*>(p) + off);
+}
+template <int DT>
+__device__ __forceinline__ uint4 widen_elem4(elem4_raw_t<DT> w) {
+    if constexpr (DT == DT_F32) return w;
+    else return make_uint4(widen1<DT>((uint16_t)(w.x & 0xffffu)), widen1<DT>((uint16_t)(w.x >> 16)),
+                           widen1<DT>((uint16_t)(w.y & 0xffffu)), widen1<DT>((uint16_t)(w.y >> 16)));
+}
 // four consecutive elements of type DT at element offset off as fp32 bit patterns: one 16-byte (fp32) or 8-byte load
 template <int DT>
 __device__ __forceinline__ uint4 load_elem4_bits(const float* p, int64_t off) {
-    if constexpr (DT == DT_F32) {
-        return *reinterpret_cast<const uint4*>(p + off);
-    } else {
-        const uint2 w = *reinterpret_cast<const uint2*>(reinterpret_cast<const uint16_t*>(p) + off);
-        return make_uint4(widen1<DT>((uint16_t)(w.x & 0xffffu)), widen1<DT>((uint16_t)(w.x >> 16)),
-                          widen1<DT>((uint16_t)(w.y & 0xffffu)), widen1<DT>((uint16_t)(w.y >> 16)));
-    }
+    return widen_elem4<DT>(load_elem4_raw<DT>(p, off));
 }
 
 // adaLN modulation of the activation operand (DiT / PixArt blocks: modulate(x, shift, scale)): row r of x belongs to
@@ -92,13 +104,121 @@ __device__ __forceinline__ void modulate_block(uint32_t (&xv)[32], const ModPara
     }
 }
 
+// ---- LayerNorm: torch.nn.functional.layer_norm on CUDA, bit for bit.  For rows whose width is a multiple of 4 torch
+// runs ATen's vectorized_layer_norm_kernel<T, float, false> (layer_norm_kernel.cu) with one (32, 4) block per row (the
+// grid and block of its launches in a torch.profiler trace on a B200, for fp32, bf16 and fp16 and K from 64 to 4096):
+// thread t = x + 32 y folds the elements 4t + 512 j .. +3 in order into a Welford triple (mean, sigma2, count), with
+// the division of the update as a reciprocal multiply; a SHFL.DOWN tree (16, 8, 4, 2, 1) combines each warp and a
+// shared-memory tree (2, 1) the warps.  var = sigma2 / K, rstd = rsqrtf(var + eps), and each element is
+// rstd * (x - mean), then weight * that + bias (one FFMA) with an affine norm, rounded to x's type.  The operations,
+// their order and the contractions below are those of torch's sm_100 SASS.
+constexpr int LN_TX = 32, LN_TY = 4, LN_THREADS = LN_TX * LN_TY;
+constexpr int LN_NONE = 0, LN_PLAIN = 1, LN_AFFINE = 2;
+
+struct WelfordLN { float mean, sigma2, count; };
+__device__ __forceinline__ WelfordLN welford_add(float v, WelfordLN c) {
+    const float delta = __fsub_rn(v, c.mean);
+    const float n = __fadd_rn(c.count, 1.0f);
+    const float mean = __fmaf_rn(delta, __frcp_rn(n), c.mean);
+    return {mean, __fmaf_rn(delta, __fsub_rn(v, mean), c.sigma2), n};
+}
+// ATen's cuWelfordCombine(b, a)
+__device__ __forceinline__ WelfordLN welford_combine(WelfordLN b, WelfordLN a) {
+    const float count = __fadd_rn(a.count, b.count);
+    if (!(count > 0.f)) return {0.f, 0.f, count};
+    const float delta = __fsub_rn(b.mean, a.mean), coef = __frcp_rn(count);
+    const float na = __fmul_rn(a.count, coef), nb = __fmul_rn(b.count, coef);
+    return {__fmaf_rn(na, a.mean, __fmul_rn(nb, b.mean)),
+            __fmaf_rn(nb, __fmul_rn(__fmul_rn(delta, delta), a.count), __fadd_rn(a.sigma2, b.sigma2)), count};
+}
+// one normalized element, rounded to DT as torch stores it
+template <int DT, int NORM>
+__device__ __forceinline__ float ln_elem(float x, float mean, float rstd, float w, float b) {
+    const float n = __fmul_rn(rstd, __fsub_rn(x, mean));
+    return round_to_dt<DT>(NORM == LN_AFFINE ? __fmaf_rn(w, n, b) : n);
+}
+
+// One warp per row of x (row stride ld, K % 4 == 0), LN_ROWS rows per block: writes mean_out[row] and rstd_out[row].
+// Lane l carries the Welford triples of torch's LN_TY threads (l, y) of that row, so each triple folds the same elements
+// in the same order and meets the same partners in the same trees as in torch's (32, 4) block: the SHFL.DOWN tree runs
+// once per y, and the shared-memory tree becomes combine(y0, y2), combine(y1, y3), then combine of the two.  Only the
+// scheduling differs: four independent chains per lane and no block barrier, instead of one chain per thread.  With y
+// (contiguous (rows, K) of DT) it also writes the normalized row, with weight / bias (K elements of DT each) when
+// NORM == LN_AFFINE.
+constexpr int LN_ROWS = 8;
+template <int DT, int NORM>
+__global__ void __launch_bounds__(LN_ROWS * 32)
+k_layer_norm(const float* __restrict__ x, int64_t ld, int rows, int K, float eps, const float* __restrict__ w,
+             const float* __restrict__ b, float* __restrict__ mean_out, float* __restrict__ rstd_out,
+             float* __restrict__ y) {
+    const int lane = threadIdx.x & 31, row = blockIdx.x * LN_ROWS + (threadIdx.x >> 5);
+    if (row >= rows) return;                                        // warp-uniform
+    const float* xr = view_elem<DT>(x, (int64_t)row * ld);
+    const int nv = K / 4;
+    WelfordLN wd[LN_TY];
+#pragma unroll
+    for (int ty = 0; ty < LN_TY; ++ty) wd[ty] = WelfordLN{0.f, 0.f, 0.f};
+    for (int base = 0; base < nv; base += LN_THREADS) {            // torch's thread t = lane + 32 ty reads i = t + 128 j
+#pragma unroll
+        for (int ty = 0; ty < LN_TY; ++ty) {
+            const int i = base + lane + LN_TX * ty;
+            if (i < nv) {
+                const uint4 v = load_elem4_bits<DT>(xr, 4 * i);
+                wd[ty] = welford_add(__uint_as_float(v.x), wd[ty]);
+                wd[ty] = welford_add(__uint_as_float(v.y), wd[ty]);
+                wd[ty] = welford_add(__uint_as_float(v.z), wd[ty]);
+                wd[ty] = welford_add(__uint_as_float(v.w), wd[ty]);
+            }
+        }
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+#pragma unroll
+        for (int ty = 0; ty < LN_TY; ++ty) {
+            const WelfordLN o{__shfl_down_sync(0xffffffffu, wd[ty].mean, off),
+                              __shfl_down_sync(0xffffffffu, wd[ty].sigma2, off),
+                              __shfl_down_sync(0xffffffffu, wd[ty].count, off)};
+            wd[ty] = welford_combine(wd[ty], o);
+        }
+    }
+    static_assert(LN_TY == 4, "the cross-warp tree below is torch's for 4 warps");
+    wd[0] = welford_combine(wd[0], wd[2]);
+    wd[1] = welford_combine(wd[1], wd[3]);
+    wd[0] = welford_combine(wd[0], wd[1]);
+    const float mean = __shfl_sync(0xffffffffu, wd[0].mean, 0);
+    const float var = __shfl_sync(0xffffffffu, __fdiv_rn(wd[0].sigma2, (float)K), 0);
+    const float rstd = rsqrtf(__fadd_rn(var, eps));
+    if (lane == 0) { mean_out[row] = mean; rstd_out[row] = rstd; }
+    if (!y) return;
+#pragma unroll 1                                                    // (unrolled, the fp32 affine instance takes a stack frame)
+    for (int i = lane; i < nv; i += LN_TX) {
+        const uint4 v = load_elem4_bits<DT>(xr, 4 * i);
+        uint4 wv = make_uint4(0, 0, 0, 0), bv = wv;
+        if constexpr (NORM == LN_AFFINE) { wv = load_elem4_bits<DT>(w, 4 * i); bv = load_elem4_bits<DT>(b, 4 * i); }
+        const uint4 o = make_uint4(
+            __float_as_uint(ln_elem<DT, NORM>(__uint_as_float(v.x), mean, rstd, __uint_as_float(wv.x), __uint_as_float(bv.x))),
+            __float_as_uint(ln_elem<DT, NORM>(__uint_as_float(v.y), mean, rstd, __uint_as_float(wv.y), __uint_as_float(bv.y))),
+            __float_as_uint(ln_elem<DT, NORM>(__uint_as_float(v.z), mean, rstd, __uint_as_float(wv.z), __uint_as_float(bv.z))),
+            __float_as_uint(ln_elem<DT, NORM>(__uint_as_float(v.w), mean, rstd, __uint_as_float(wv.w), __uint_as_float(bv.w))));
+        store_out4<DT>(y, (int64_t)row * K + 4 * i, o);
+    }
+}
+
+// LayerNorm of the activation operand: the per-row (mean, rstd) written by k_layer_norm, and with NORM == LN_AFFINE
+// the weight and bias (K elements of x's type each)
+struct NormParams {
+    const float *mean, *rstd;
+    const float *w, *b;
+};
+
 // rows_tile = 128 (activations) or 256 (weights); rows_pad = multiple of rows_tile (zero rows past `rows`).
-// x holds elements of type DT (DT_*); ld in elements.  MOD: the operand is quantized from x modulated by `mod` (rows
-// past `rows` stay zero rows and read no modulation).
-template <int DT, bool MOD = false>
+// x holds elements of type DT (DT_*); ld in elements.  NORM: the elements are first normalized as torch's LayerNorm
+// stores them (ln_elem); MOD: then modulated by `mod`.  Rows past `rows` stay zero rows and read neither.
+template <int DT, bool MOD = false, int NORM = LN_NONE>
 __global__ void __launch_bounds__(256)
 k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int rows_pad, int K, int rows_tile,
-                        int bf16, int flush, unsigned char* __restrict__ op, const ModParams mod) {
+                        int bf16, int flush, unsigned char* __restrict__ op, const ModParams mod,
+                        const NormParams norm) {
     const int nb = K >> 5, ksteps = K / GL_BK;
     const int64_t ntask = (int64_t)rows_pad * nb;
     const size_t stage_bytes = (size_t)8 * rows_tile * 16;
@@ -106,6 +226,24 @@ k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int r
         const int b = (int)(t / rows_pad), row = (int)(t - (int64_t)b * rows_pad);      // block-major: coalesced stores
         uint32_t xv[32];
         load_block_bits<DT>(view_elem<DT>(x, (int64_t)row * ld + 32 * b), 32, row < rows, xv);
+        if constexpr (NORM != LN_NONE) {
+            if (row < rows) {
+                const float mean = norm.mean[row], rstd = norm.rstd[row];
+#pragma unroll
+                for (int j4 = 0; j4 < 32; j4 += 4) {
+                    uint4 w4 = make_uint4(0, 0, 0, 0), b4 = w4;
+                    if constexpr (NORM == LN_AFFINE) {
+                        w4 = load_elem4_bits<DT>(norm.w, 32 * b + j4);
+                        b4 = load_elem4_bits<DT>(norm.b, 32 * b + j4);
+                    }
+                    const uint32_t wj[4] = {w4.x, w4.y, w4.z, w4.w}, bj[4] = {b4.x, b4.y, b4.z, b4.w};
+#pragma unroll
+                    for (int j = 0; j < 4; ++j)
+                        xv[j4 + j] = __float_as_uint(ln_elem<DT, NORM>(__uint_as_float(xv[j4 + j]), mean, rstd,
+                                                                       __uint_as_float(wj[j]), __uint_as_float(bj[j])));
+                }
+            }
+        }
         if constexpr (MOD) {
             if (row < rows) modulate_block<DT>(xv, mod, row / mod.tokens, 32 * b);
         }
@@ -120,8 +258,9 @@ k_quantize_gemm_operand(const float* __restrict__ x, int64_t ld, int rows, int r
 }
 
 // Epilogues of k_mx_linear_umma: store the output, apply an activation (MXP_ACT_* + 1) and write the next GEMM's
-// A operand, or store residual + gate * output (the adaLN block's gated residual).
-constexpr int EPI_STORE = 0, EPI_GELU = 1, EPI_GELU_TANH = 2, EPI_GATED_RESIDUAL = 3;
+// A operand, store residual + gate * output (the adaLN block's gated residual) or residual + output (a pre-norm
+// block's residual add).
+constexpr int EPI_STORE = 0, EPI_GELU = 1, EPI_GELU_TANH = 2, EPI_GATED_RESIDUAL = 3, EPI_RESIDUAL = 4;
 
 // torch.nn.functional.gelu on CUDA, bit for bit: ATen's GeluCUDAKernelImpl (ActivationGeluKernel.cu) in fp32 opmath,
 //     approximate='none'  x * 0.5 * (1 + erf(x * M_SQRT1_2))
@@ -159,23 +298,20 @@ struct LinearParams {
     int M, N, K, bf16, stages;
     int flush;                        // EPI_GELU*: the next GEMM's quantizer setting
     unsigned char* h_op;              // EPI_GELU*: the next GEMM's A operand (K = N), written instead of out
-    const float* residual;            // EPI_GATED_RESIDUAL: (M, N) of OUT_DT, row stride ldr
+    const float* residual;            // EPI_GATED_RESIDUAL / EPI_RESIDUAL: (M, N) of OUT_DT, row stride ldr
     const float* gate;                // EPI_GATED_RESIDUAL: (M / tokens, N) of OUT_DT, row stride ldg; row r uses r / tokens
     int64_t ldr, ldg;
     int tokens;
 };
 
-// the gated residual of four outputs y (columns col..col+3 of row `row`, fp32 values before the store's rounding):
-// residual + gate * y, each operation rounded to DT as eager torch evaluates it on tensors of that type
-template <int DT>
-__device__ __forceinline__ float4 gated_residual4(float4 y, const LinearParams& p, int row, int col) {
-    const uint4 r = load_elem4_bits<DT>(p.residual, (int64_t)row * p.ldr + col);
-    const uint4 g = load_elem4_bits<DT>(p.gate, (int64_t)(row / p.tokens) * p.ldg + col);
-    auto f = [](float yv, uint32_t gv, uint32_t rv) {
-        const float gy = round_to_dt<DT>(__fmul_rn(__uint_as_float(gv), round_to_dt<DT>(yv)));
-        return round_to_dt<DT>(__fadd_rn(__uint_as_float(rv), gy));
-    };
-    return make_float4(f(y.x, g.x, r.x), f(y.y, g.y, r.y), f(y.z, g.z, r.z), f(y.w, g.w, r.w));
+// the residual store of one output y (fp32 value before the store's rounding) with the residual r and, when GATED, the
+// gate g (bit patterns of DT values): rd(r + rd(g * rd(y))), or rd(r + rd(y)) without the gate, each operation rounded
+// to DT as eager torch evaluates it on tensors of that type
+template <int DT, bool GATED>
+__device__ __forceinline__ float residual1(float y, uint32_t r, uint32_t g) {
+    float v = round_to_dt<DT>(y);
+    if constexpr (GATED) v = round_to_dt<DT>(__fmul_rn(__uint_as_float(g), v));
+    return round_to_dt<DT>(__fadd_rn(__uint_as_float(r), v));
 }
 
 // bias of element type DT -> A1(bias), N floats (tiny)
@@ -343,8 +479,25 @@ k_mx_linear_umma(const LinearParams p) {
             float* tr = s_tr + (warp - 2) * (32 * 36);
             const int lr = lane >> 3, lc = (lane & 7) * 4;          // this lane's row (mod 4) and column group
             const int row_base = tile_m * GL_BM + q * 32;
+            constexpr bool RES_EPI = EPI == EPI_GATED_RESIDUAL || EPI == EPI_RESIDUAL, GATED = EPI == EPI_GATED_RESIDUAL;
 #pragma unroll 1
             for (int c0 = 0; c0 < GL_BN; c0 += 32) {
+                // residual stores: the pass's residual (and gate) loads are issued before its TMEM read, so that their
+                // latency overlaps the read and the transpose instead of stalling each store; they are widened at use
+                elem4_raw_t<OUT_DT> res[RES_EPI ? 8 : 1], gat[GATED ? 8 : 1];
+                if constexpr (RES_EPI) {
+#pragma unroll
+                    for (int i8 = 0; i8 < 8; ++i8) {
+                        const int row = row_base + lr + 4 * i8;
+                        res[i8] = {};
+                        if constexpr (GATED) gat[i8] = {};
+                        if (row < p.M && n0 + c0 + lc < p.N) {          // padding rows read no residual or gate
+                            res[i8] = load_elem4_raw<OUT_DT>(p.residual, (int64_t)row * p.ldr + n0 + c0 + lc);
+                            if constexpr (GATED)
+                                gat[i8] = load_elem4_raw<OUT_DT>(p.gate, (int64_t)(row / p.tokens) * p.ldg + n0 + c0 + lc);
+                        }
+                    }
+                }
                 uint32_t r[32];
                 tmem_ld_32x32b_x32(t0 + c0, r);
                 tmem_ld_wait();
@@ -363,8 +516,14 @@ k_mx_linear_umma(const LinearParams p) {
                         y.x = __fadd_rn(y.x, b4.x); y.y = __fadd_rn(y.y, b4.y); y.z = __fadd_rn(y.z, b4.z); y.w = __fadd_rn(y.w, b4.w);
                         if (bf16) { y.x = bf16_half_away(y.x); y.y = bf16_half_away(y.y); y.z = bf16_half_away(y.z); y.w = bf16_half_away(y.w); }   // :89-93
                     }
-                    if (row < p.M && col_ok) {                          // padding rows read no residual or gate
-                        if constexpr (EPI == EPI_GATED_RESIDUAL) y = gated_residual4<OUT_DT>(y, p, row, n0 + c0 + lc);
+                    if (row < p.M && col_ok) {
+                        if constexpr (RES_EPI) {
+                            const uint4 rv = widen_elem4<OUT_DT>(res[i8]);
+                            uint4 gv = rv;
+                            if constexpr (GATED) gv = widen_elem4<OUT_DT>(gat[i8]);
+                            y = make_float4(residual1<OUT_DT, GATED>(y.x, rv.x, gv.x), residual1<OUT_DT, GATED>(y.y, rv.y, gv.y),
+                                            residual1<OUT_DT, GATED>(y.z, rv.z, gv.z), residual1<OUT_DT, GATED>(y.w, rv.w, gv.w));
+                        }
                         store_out4<OUT_DT>(p.out, (int64_t)row * p.ldo + n0 + c0 + lc,
                                            make_uint4(__float_as_uint(y.x), __float_as_uint(y.y), __float_as_uint(y.z), __float_as_uint(y.w)));
                     }

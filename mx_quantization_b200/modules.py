@@ -18,7 +18,8 @@ reference runs in the last block of each model - same kernels with every key kep
 unquantized torch path) raises - no silent fallback.
 
 ``QuantizedDiTBlock`` wraps a whole DiT block (workloads/DiT/models.py:271-297): its adaLN modulations and gated residuals
-run inside the MX Linear kernels of the Attention shim and of QuantizedMlp.  ``QuantizedPixArtBlock`` does the same for
+run inside the MX Linear kernels of the Attention shim and of QuantizedMlp.  ``QuantizedDeiTBlock`` does the same for
+DeiT's pre-norm block: its LayerNorms run in the quantizers and its residual adds in the output stores.  ``QuantizedPixArtBlock`` does the same for
 PixArt-alpha's adaLN-single block, with q, k and v from one projection GEMM.
 """
 from typing import Optional
@@ -91,6 +92,28 @@ def _require_hot_path(mx_quant, top_k, approx, pred_mode, where) -> str:
     return pred_mode
 
 
+def _fused_norm(norm, x):
+    """The ops.mx_linear / mx_mlp arguments that make x's quantizer apply ``norm`` (ln_eps, ln_weight, ln_bias), {} for
+    no norm, or None when the norm must run in torch: it qualifies when it is exactly ``nn.LayerNorm`` over x's last
+    dimension with both affine parameters in x's dtype, or with neither."""
+    if norm is None:
+        return {}
+    if type(norm) is not nn.LayerNorm or tuple(norm.normalized_shape) != (x.shape[-1],):
+        return None
+    w, b = norm.weight, norm.bias
+    if w is None and b is None:
+        return dict(ln_eps=norm.eps)
+    if w is None or b is None or w.dtype != x.dtype or b.dtype != x.dtype:
+        return None
+    return dict(ln_eps=norm.eps, ln_weight=w.detach(), ln_bias=b.detach())
+
+
+def _norm_route(norm, x):
+    """(x for the projection, its quantizer's norm arguments): x itself with the fused norm, else ``norm(x)``."""
+    kw = _fused_norm(norm, x)
+    return (x, kw) if kw is not None else (norm(x), {})
+
+
 def to_mx_linear(lin: nn.Linear, mx_specs) -> "MxLinear":
     """nn.Linear -> MxLinear sharing the parameters (what apply_quantization_to_deit /
     MXBasicTransformerBlock.set_config do with mx.Linear: deit main.py:231-318,
@@ -129,6 +152,21 @@ class QuantizedAttention(nn.Module):
         x = self.proj_drop(self.proj(x))
         self.current_timestep += 1
         return x
+
+    def forward_prenorm(self, x, norm):
+        """The attention half of a pre-norm block (timm's Block): ``x + self(norm(x))``, bit for bit.  The qkv
+        projection's quantizer applies the norm when it qualifies (exactly nn.LayerNorm over C, both or no affine
+        parameters in x's dtype; otherwise torch's norm runs first), and the output projection's store adds x.  The core
+        call is forward's.  While proj_drop is active (training, p > 0) the expression runs as written."""
+        if self.training and self.proj_drop.p > 0:
+            return x + self(norm(x))
+        B, N, C = x.shape
+        h, kw = _norm_route(norm, x)
+        qkv = self.qkv.forward_adaln(h, **kw).reshape(B, N, 3, self.num_heads, C // self.num_heads).permute(2, 0, 3, 1, 4)
+        y = self.core(qkv[0], qkv[1], qkv[2])
+        y = self.proj.forward_adaln(y, add=x)
+        self.current_timestep += 1
+        return y
 
 
 def _feed_forward_layers(net):
@@ -191,15 +229,29 @@ class QuantizedMlp(nn.Module):
             return self.drop(self._mx_mlp(x))
         return self.drop(self.fc2(self.drop_hidden(self.act(self.fc1(x)))))
 
-    def forward_adaln(self, x, shift, scale, residual, gate):
+    def forward_adaln(self, x, shift, scale, residual, gate, norm=None):
         """The MLP half of DiT's DiTBlock.forward (workloads/DiT/models.py:297) on an already-normalized x (B, T, C):
         ``residual + gate.unsqueeze(1) * self(modulate(x, shift, scale))``, modulate(x, shift, scale) =
         ``x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1)`` (models.py:101-102).  On the fused route (that of forward,
         while no dropout is active) it is one ops.mx_mlp call whose quantizer applies the modulation and whose fc2 store
-        applies the gated residual, bit for bit the expression; otherwise the expression runs as written."""
+        applies the gated residual, bit for bit the expression; otherwise the expression runs as written.  With ``norm``,
+        x is the un-normalized input and the expression runs on ``norm(x)``; the quantizer applies a qualifying norm
+        (see QuantizedAttention.forward_prenorm)."""
         if self._fused() and not (self.training and self.drop.p > 0):
-            return self._mx_mlp(x, shift=shift, scale=scale, residual=residual, gate=gate)
+            x, kw = _norm_route(norm, x)
+            return self._mx_mlp(x, shift=shift, scale=scale, residual=residual, gate=gate, **kw)
+        if norm is not None:
+            x = norm(x)
         return residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1))
+
+    def forward_prenorm(self, x, norm):
+        """The MLP half of a pre-norm block (timm's Block): ``x + self(norm(x))``, bit for bit.  On the fused route it is
+        one ops.mx_mlp call whose quantizer applies a qualifying norm and whose fc2 store adds x; otherwise the
+        expression runs as written."""
+        if self._fused() and not (self.training and self.drop.p > 0):
+            h, kw = _norm_route(norm, x)
+            return self._mx_mlp(h, add=x, **kw)
+        return x + self(norm(x))
 
 
 def apply_quantization_to_deit(model, config, mx_quant=True, top_k=True, k=20, approx_flag=True, pred_mode="ex_pred",
@@ -265,17 +317,21 @@ class Attention(nn.Module):
         self.current_timestep += 1
         return x
 
-    def forward_adaln(self, x, shift, scale, residual, gate):
+    def forward_adaln(self, x, shift, scale, residual, gate, norm=None):
         """The attention half of DiT's DiTBlock.forward (workloads/DiT/models.py:296) on an already-normalized x (B, N, C):
         ``residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1))``, bit for bit.  The
         qkv projection's quantizer applies the modulation as it loads x, and the output projection's store applies the
         gated residual; the core call between them is forward's (dense on exclude_timesteps steps), and
         current_timestep advances as in forward.  While proj_drop is active (training, p > 0) the expression runs as
-        written."""
+        written.  With ``norm``, x is the un-normalized input and the expression runs on ``norm(x)``; the quantizer
+        applies a qualifying norm (exactly nn.LayerNorm over C, both or no affine parameters in x's dtype)."""
         if self.training and self.proj_drop.p > 0:
+            if norm is not None:
+                x = norm(x)
             return residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1))
         B, N, C = x.shape
-        qkv = self.qkv.forward_adaln(x, shift=shift, scale=scale)
+        x, kw = _norm_route(norm, x)
+        qkv = self.qkv.forward_adaln(x, shift=shift, scale=scale, **kw)
         q, k, v = qkv.reshape(B, N, 3, self.num_heads, self.head_dim).permute(2, 0, 3, 1, 4).unbind(0)
         q, k = self.q_norm(q), self.k_norm(k)
         x = self.core(q, k, v, dense=self.current_timestep in self.exclude_timesteps)
@@ -290,7 +346,9 @@ class QuantizedDiTBlock(nn.Module):
         x = x + gate_msa.unsqueeze(1) * attn(modulate(norm1(x), shift_msa, scale_msa))
         x = x + gate_mlp.unsqueeze(1) * mlp(modulate(norm2(x), shift_mlp, scale_mlp))
     with the modulations and gated residuals inside the MX Linear kernels (Attention.forward_adaln,
-    QuantizedMlp.forward_adaln): bit for bit that expression on the same modules, without its elementwise passes.
+    QuantizedMlp.forward_adaln): bit for bit that expression on the same modules, without its elementwise passes.  The
+    quantizers of qkv and fc1 also apply norm1 / norm2 when they qualify (DiT's nn.LayerNorm(C, elementwise_affine=False,
+    eps=1e-6) does); any other norm runs in torch.
 
     ``orig_block``: a DiT-style block with ``norm1``, ``attn``, ``norm2``, ``mlp`` and ``adaLN_modulation``.  ``attn`` must
     be the ``Attention`` shim; ``mlp`` (timm Mlp, models.py:287) is wrapped in QuantizedMlp unless it already is one.  The
@@ -308,8 +366,48 @@ class QuantizedDiTBlock(nn.Module):
 
     def forward(self, x, c):
         shift_msa, scale_msa, gate_msa, shift_mlp, scale_mlp, gate_mlp = self.adaLN_modulation(c).chunk(6, dim=1)
-        x = self.attn.forward_adaln(self.norm1(x), shift_msa, scale_msa, x, gate_msa)
-        return self.mlp.forward_adaln(self.norm2(x), shift_mlp, scale_mlp, x, gate_mlp)
+        x = self.attn.forward_adaln(x, shift_msa, scale_msa, x, gate_msa, norm=self.norm1)
+        return self.mlp.forward_adaln(x, shift_mlp, scale_mlp, x, gate_mlp, norm=self.norm2)
+
+
+class QuantizedDeiTBlock(nn.Module):
+    """DeiT's transformer block (timm 0.4.12 ``Block``: norm1, attn, drop_path, norm2, mlp) - forward computes, bit for
+    bit on the same modules:
+        x = x + drop_path(attn(norm1(x)))
+        x = x + drop_path(mlp(norm2(x)))
+    with each norm applied by the quantizer of the GEMM that reads it (qkv, fc1) and each residual add done by the store
+    of the GEMM that ends its half (proj, fc2): QuantizedAttention.forward_prenorm and QuantizedMlp.forward_prenorm.  A
+    norm that is not exactly nn.LayerNorm over C with both or no affine parameters in x's dtype runs in torch.  While
+    drop_path is active (training, drop_prob > 0) the block runs the expression as written.
+
+    ``orig_block``: ``attn`` must already be a QuantizedAttention (apply_quantization_to_deit makes it one); ``mlp`` is
+    wrapped in QuantizedMlp unless it already is one.  A LayerScale (``ls1`` / ``ls2`` other than nn.Identity) is not
+    on the path and raises TypeError.  The state_dict keys are the wrapped block's."""
+
+    def __init__(self, orig_block, mx_specs=None):
+        super().__init__()
+        if not isinstance(orig_block.attn, QuantizedAttention):
+            raise TypeError(f"QuantizedDeiTBlock: attn must be modules.QuantizedAttention (the DeiT shim), got "
+                            f"{type(orig_block.attn).__name__}")
+        for name in ("ls1", "ls2"):
+            ls = getattr(orig_block, name, None)
+            if ls is not None and not isinstance(ls, nn.Identity):
+                raise TypeError(f"QuantizedDeiTBlock: {name} ({type(ls).__name__}) is not on the path; only nn.Identity")
+        self.norm1, self.attn, self.drop_path, self.norm2 = (orig_block.norm1, orig_block.attn, orig_block.drop_path,
+                                                             orig_block.norm2)
+        mlp = orig_block.mlp
+        self.mlp = mlp if isinstance(mlp, QuantizedMlp) else QuantizedMlp(mlp, mx_specs=mx_specs)
+
+    def _drop_path_active(self) -> bool:
+        return (self.training and not isinstance(self.drop_path, nn.Identity)
+                and getattr(self.drop_path, "drop_prob", 1.0) != 0)
+
+    def forward(self, x):
+        if self._drop_path_active():
+            x = x + self.drop_path(self.attn(self.norm1(x)))
+            return x + self.drop_path(self.mlp(self.norm2(x)))
+        x = self.attn.forward_prenorm(x, self.norm1)
+        return self.mlp.forward_prenorm(x, self.norm2)
 
 
 class MXSelfAttention(nn.Module):
@@ -366,7 +464,7 @@ class MXSelfAttention(nn.Module):
             self._qkv_key = key
         return self._qkv_op, self._qkv_bias
 
-    def forward_adaln(self, x, shift, scale, residual, gate):
+    def forward_adaln(self, x, shift, scale, residual, gate, norm=None):
         """The self-attention half of PixArt's adaLN-single block (diffusers' BasicTransformerBlock) on the normalized
         hidden states x (B, N, C): ``residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) +
         shift.unsqueeze(1))``, bit for bit.  shift / scale / gate: (B, C) rows, e.g. ``.squeeze(1)`` of the block's
@@ -377,18 +475,23 @@ class MXSelfAttention(nn.Module):
         tile holds it, and its bits are those of the separate projection.  The core reads q, k, v as strided views of
         the (B, N, 3C) result (dense on exclude_timesteps steps, as forward), to_out[0]'s store applies the gated
         residual, and current_timestep advances.  While to_out's dropout is active (training, p > 0), or when the three
-        projections have different MX configurations, the expression runs as written."""
+        projections have different MX configurations, the expression runs as written.  With ``norm``, x is the
+        un-normalized input and the expression runs on ``norm(x)``; the quantizer applies a qualifying norm (exactly
+        nn.LayerNorm over C, both or no affine parameters in x's dtype)."""
         if self.core is None:
             raise RuntimeError("MXSelfAttention.set_config(...) must be called first")
         layers = (self.to_q, self.to_k, self.to_v)
         if ((self.training and self.to_out[1].p > 0)
                 or len({resolve_linear_specs(m.mx_specs) for m in layers}) != 1):
+            if norm is not None:
+                x = norm(x)
             return residual + gate.unsqueeze(1) * self(x * (1 + scale.unsqueeze(1)) + shift.unsqueeze(1))
         for m in layers:
             m._check_inference(x.requires_grad)
         B, N, C = x.shape
         w_op, b = self._qkv_operand()
-        qkv = ops.mx_linear(x, w_op, b, self.to_q.mx_specs, out_features=3 * C, shift=shift, scale=scale)
+        x, kw = _norm_route(norm, x)
+        qkv = ops.mx_linear(x, w_op, b, self.to_q.mx_specs, out_features=3 * C, shift=shift, scale=scale, **kw)
         q, k, v = qkv.view(B, N, 3, self.num_heads, self.head_dim).permute(2, 0, 3, 1, 4).unbind(0)
         x = self.core(q, k, v, dense=self.current_timestep in self.exclude_timesteps)
         x = self.to_out[0].forward_adaln(x, residual=residual, gate=gate)
@@ -402,6 +505,10 @@ class MXCrossAttention(MXSelfAttention):
     (B,1,S) is applied to the true and the predicted scores (:794-803, :821-822)."""
 
     def forward(self, hidden_states, encoder_hidden_states=None, attention_mask=None, **kwargs):
+        return self.to_out(self._attend(hidden_states, encoder_hidden_states, attention_mask))
+
+    def _attend(self, hidden_states, encoder_hidden_states, attention_mask):
+        """The core's output (B, N, C) for to_out; current_timestep advances."""
         if self.core is None:
             raise RuntimeError("MXCrossAttention.set_config(...) must be called first")
         if encoder_hidden_states is None:
@@ -415,9 +522,18 @@ class MXCrossAttention(MXSelfAttention):
             raise NotImplementedError("boolean masks (-inf bias) are not on the path; pass the additive fp32 mask")
         bias = None if attention_mask is None else attention_mask.to(torch.float32).reshape(B, S)
         excluded = self.current_timestep in self.exclude_timesteps
-        x = self.to_out(self.core(q, k, v, key_bias=bias, pred_mode="exact" if excluded else None))
+        x = self.core(q, k, v, key_bias=bias, pred_mode="exact" if excluded else None)
         self.current_timestep += 1
         return x
+
+    def forward_residual(self, hidden_states, encoder_hidden_states=None, attention_mask=None):
+        """``self(hidden_states, encoder_hidden_states, attention_mask) + hidden_states`` (PixArt's cross-attention
+        residual), bit for bit, with the add in to_out[0]'s store.  While to_out's dropout is active (training, p > 0)
+        the expression runs as written."""
+        if self.training and self.to_out[1].p > 0:
+            return self(hidden_states, encoder_hidden_states, attention_mask=attention_mask) + hidden_states
+        x = self._attend(hidden_states, encoder_hidden_states, attention_mask)
+        return self.to_out[0].forward_adaln(x, add=hidden_states)
 
     def forward_adaln(self, *args, **kwargs):
         raise TypeError("MXCrossAttention has no adaLN form (PixArt's block adds its output without a gate); "
@@ -434,8 +550,9 @@ class QuantizedPixArtBlock(nn.Module):
         h = gate_mlp * ff(norm2(h) * (1 + scale_mlp) + shift_mlp) + h
     The self-attention and feed-forward halves run with their modulations and gated residuals inside the MX Linear
     kernels (MXSelfAttention.forward_adaln, with q, k and v from one GEMM, and QuantizedMlp.forward_adaln); IEEE add and
-    multiply commute, so the kernels' ``h + gate * y`` is ``gate * y + h``.  attn2 runs its own forward and its residual
-    is a torch add.
+    multiply commute, so the kernels' ``h + gate * y`` is ``gate * y + h``.  The quantizers of the q/k/v GEMM and of fc1
+    apply norm1 / norm2 when they qualify (PixArt's nn.LayerNorm(C, elementwise_affine=False, eps=1e-6) does; any other
+    norm runs in torch).  attn2 runs its own forward with ``+ h`` in to_out's store (MXCrossAttention.forward_residual).
 
     ``orig_block``: ``attn1`` an MXSelfAttention and ``attn2`` an MXCrossAttention (or None), both after set_config;
     ``ff`` a QuantizedMlp or diffusers' FeedForward (wrapped in QuantizedMlp); ``norm1`` / ``norm2`` (torch LayerNorm)
@@ -471,10 +588,10 @@ class QuantizedPixArtBlock(nn.Module):
         h = hidden_states
         shift_msa, scale_msa, gate_msa, shift_mlp, scale_mlp, gate_mlp = (
             t.squeeze(1) for t in (self.scale_shift_table[None] + timestep.reshape(h.shape[0], 6, -1)).chunk(6, dim=1))
-        h = self.attn1.forward_adaln(self.norm1(h), shift_msa, scale_msa, h, gate_msa)
+        h = self.attn1.forward_adaln(h, shift_msa, scale_msa, h, gate_msa, norm=self.norm1)
         if self.attn2 is not None:
-            h = self.attn2(h, encoder_hidden_states, attention_mask=encoder_attention_mask) + h
-        return self.ff.forward_adaln(self.norm2(h), shift_mlp, scale_mlp, h, gate_mlp)
+            h = self.attn2.forward_residual(h, encoder_hidden_states, attention_mask=encoder_attention_mask)
+        return self.ff.forward_adaln(h, shift_mlp, scale_mlp, h, gate_mlp, norm=self.norm2)
 
 
 class MxLinear(nn.Linear):

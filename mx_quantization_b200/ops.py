@@ -530,10 +530,95 @@ def _adaln_args(x: torch.Tensor, K: int, N: int, shift, scale, residual, gate) -
     return tuple(args)
 
 
+def _norm_args(x: torch.Tensor, K: int, ln_eps, ln_weight, ln_bias) -> tuple:
+    """The LayerNorm arguments of mxp_mx_*_ex_dt (layer_norm, ln_weight, ln_bias, ln_eps): the norm is on when ``ln_eps``
+    is given; ``ln_weight`` / ``ln_bias`` are (K,) contiguous tensors of x's dtype, both or neither."""
+    if (ln_weight is None) != (ln_bias is None):
+        raise ValueError("ln_weight and ln_bias: pass both or neither")
+    if ln_eps is None:
+        if ln_weight is not None:
+            raise ValueError("ln_weight / ln_bias need ln_eps (the LayerNorm's eps)")
+        return (0, None, None, 0.0)
+    eps = float(ln_eps)
+    if not eps >= 0.0:
+        raise ValueError(f"ln_eps: need a number >= 0, got {ln_eps!r}")
+    for name, t in (("ln_weight", ln_weight), ("ln_bias", ln_bias)):
+        if t is None:
+            continue
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"{name}: expected a torch.Tensor")
+        if t.dtype != x.dtype or tuple(t.shape) != (K,) or not t.is_contiguous() or t.data_ptr() % 16:
+            raise ValueError(f"{name}: expected a contiguous, 16-byte aligned ({K},) tensor of x's dtype {x.dtype}, got "
+                             f"{t.dtype} {tuple(t.shape)} strides {tuple(t.stride())}")
+    _same_device(x, ln_weight, ln_bias)
+    return (1, _ptr(ln_weight), _ptr(ln_bias), eps)
+
+
+def _ex_args(x: torch.Tensor, M: int, K: int, N: int, ln_eps, ln_weight, ln_bias, add, shift, scale, residual,
+             gate) -> tuple:
+    """The norm and block arguments of mxp_mx_*_ex_dt.  ``add`` (x.shape[:-1] + (N,), x's dtype, rows with innermost
+    stride 1 forming one 2-D view) takes the residual slot without a gate; the adaLN tensors need a (B, T, K) x."""
+    norm = _norm_args(x, K, ln_eps, ln_weight, ln_bias)
+    if add is not None and (residual is not None or gate is not None):
+        raise ValueError("add is the plain residual add: pass it without residual / gate")
+    if any(t is not None for t in (shift, scale, residual, gate)):
+        ad = list(_adaln_args(x, K, N, shift, scale, residual, gate))
+    else:
+        ad = [M] + [_ptr(None), 0] * 4
+    if add is not None:
+        if not isinstance(add, torch.Tensor):
+            raise TypeError("add: expected a torch.Tensor")
+        shape = tuple(x.shape[:-1]) + (N,)
+        if add.dtype != x.dtype or tuple(add.shape) != shape:
+            raise ValueError(f"add: expected shape {shape} of x's dtype {x.dtype}, got {add.dtype} {tuple(add.shape)}")
+        try:
+            rows = add.view(-1, N)
+        except RuntimeError:
+            rows = None
+        if rows is None or rows.stride(1) != 1 or rows.data_ptr() % (16 if x.dtype == torch.float32 else 8) \
+                or (rows.shape[0] > 1 and rows.stride(0) % 4):
+            raise ValueError(f"add: needs rows with innermost stride 1 forming one 2-D view, an aligned base and a row "
+                             f"stride that is a multiple of 4, got strides {tuple(add.stride())}")
+        _same_device(x, add)
+        ad[5:7] = [_ptr(add), rows.stride(0) if rows.shape[0] > 1 else N]
+    return norm + tuple(ad)
+
+
+def layer_norm(x: torch.Tensor, weight: Optional[torch.Tensor] = None, bias: Optional[torch.Tensor] = None,
+               eps: float = 1e-5) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The LayerNorm mx_linear / mx_mlp apply with ``ln_eps`` (parity aid): ``torch.native_layer_norm(x, (K,), weight,
+    bias, eps)`` on CUDA bit for bit - (y, mean, rstd), mean and rstd fp32 of shape x.shape[:-1] + (1,).  ``x``: a CUDA
+    float32, bfloat16 or float16 tensor whose rows form one 2-D view with innermost stride 1 (K a multiple of 4);
+    ``weight`` / ``bias``: (K,) tensors of x's dtype, both or neither."""
+    if not isinstance(x, torch.Tensor) or not x.is_cuda or x.dtype not in DTYPE_CODES or x.dim() < 1:
+        raise ValueError("x must be a CUDA float32, bfloat16 or float16 tensor")
+    K = x.shape[-1]
+    try:
+        x2 = x.view(-1, K)
+    except RuntimeError:
+        x2 = None
+    if x2 is None or x2.stride(1) != 1 or (x2.shape[0] > 1 and x2.stride(0) % 4) or \
+            x2.data_ptr() % (16 if x.dtype == torch.float32 else 8):
+        raise ValueError(f"x: needs rows with innermost stride 1 forming one 2-D view, an aligned base and a row stride "
+                         f"that is a multiple of 4, got strides {tuple(x.stride())}")
+    _, w, b, e = _norm_args(x, K, eps, weight, bias)
+    M = x2.shape[0]
+    with torch.cuda.device(x.device):
+        y = torch.empty(x.shape, dtype=x.dtype, device=x.device)
+        stats = torch.empty((2, M), dtype=torch.float32, device=x.device)
+        rc = _lib.load().mxp_layer_norm_dt(_ptr(x2), DTYPE_CODES[x.dtype], x2.stride(0) if M > 1 else K, M, K, w, b, e,
+                                           _ptr(y), _ptr(stats[0]), _ptr(stats[1]), _stream())
+    _lib.check(rc, "mxp_layer_norm_dt")
+    shape = tuple(x.shape[:-1]) + (1,)
+    return y, stats[0].view(shape), stats[1].view(shape)
+
+
 def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
               out_features: Optional[int] = None, *, shift: Optional[torch.Tensor] = None,
               scale: Optional[torch.Tensor] = None, residual: Optional[torch.Tensor] = None,
-              gate: Optional[torch.Tensor] = None) -> torch.Tensor:
+              gate: Optional[torch.Tensor] = None, ln_eps: Optional[float] = None,
+              ln_weight: Optional[torch.Tensor] = None, ln_bias: Optional[torch.Tensor] = None,
+              add: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Forward of the reference's mx.Linear (microxscaling/mx/linear.py:20-103) for MXINT8:
     y = A1(A1(MXq(A1(x)) @ MXq(A1(W))^T) + A1(bias)).  ``weight`` is either the (N,K) tensor or
     the operand returned by mx_linear_prepare_weight (then pass out_features).
@@ -548,7 +633,14 @@ def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
           modulates the elements it loads; nothing is written);
       ``residual`` (B, T, N), ``gate`` (B, N): the result is ``residual + gate[:, None] * y`` (the GEMM's store does it).
     Bit for bit the eager torch composition on tensors of x's dtype, with the launches of the plain call.  The four
-    tensors have x's dtype; shift / scale / gate may be column slices of one (B, 6C) tensor (``.chunk(6, dim=1)``)."""
+    tensors have x's dtype; shift / scale / gate may be column slices of one (B, 6C) tensor (``.chunk(6, dim=1)``).
+
+    Pre-norm block (DeiT's timm Block), for any x, each optional:
+      ``ln_eps`` (with ``ln_weight``, ``ln_bias`` (K,) of x's dtype, both or neither): the layer runs on
+          ``F.layer_norm(x, (K,), ln_weight, ln_bias, ln_eps)`` (a row statistics kernel, then the quantizer normalizes
+          the elements it loads), before any modulation;
+      ``add`` (x.shape[:-1] + (N,)): the result is ``add + y`` (the GEMM's store does it); not with residual / gate.
+    The result is ``add + f(modulate(F.layer_norm(x)))`` bit for bit, f the plain call; the norm adds one launch."""
     sp = resolve_linear_specs(mx_specs)
     lib = _lib.load()
     x2 = _linear_rows(x)
@@ -558,16 +650,22 @@ def mx_linear(x: torch.Tensor, weight, bias: Optional[torch.Tensor], mx_specs,
     w_op, N = _weight_operand(weight, K, out_features, mx_specs)
     _check_bias(bias, N)
     _same_device(x, w_op, bias)
+    ex = ln_eps is not None or ln_weight is not None or ln_bias is not None or add is not None
     adaln = any(t is not None for t in (shift, scale, residual, gate))
-    ad = _adaln_args(x, K, N, shift, scale, residual, gate) if adaln else ()
+    if ex:
+        ad = _ex_args(x, M, K, N, ln_eps, ln_weight, ln_bias, add, shift, scale, residual, gate)
+    else:
+        ad = _adaln_args(x, K, N, shift, scale, residual, gate) if adaln else ()
     with torch.cuda.device(x.device):
         out = torch.empty((M, N), dtype=x.dtype, device=x.device)
-        ws_bytes = lib.mxp_mx_linear_workspace_bytes(M, N, K)
+        ws_bytes = (lib.mxp_mx_linear_ex_workspace_bytes if ex else lib.mxp_mx_linear_workspace_bytes)(M, N, K)
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=x.device)
         args = (_ptr(x2), DTYPE_CODES[x.dtype], x2.stride(0), M, K, _ptr(w_op), N, _ptr(bias),
                 DTYPE_CODES[bias.dtype] if bias is not None else _lib.MXP_DT_F32, sp.bfloat_bits,
                 int(sp.flush), _ptr(out), out.stride(0))
-        if adaln:
+        if ex:
+            rc = lib.mxp_mx_linear_ex_dt(*args, *ad, _ptr(ws), ws_bytes, _stream())
+        elif adaln:
             rc = lib.mxp_mx_linear_adaln_dt(*args, *ad, _ptr(ws), ws_bytes, _stream())
         else:
             rc = lib.mxp_mx_linear_dt(*args, _ptr(ws), ws_bytes, _stream())
@@ -588,7 +686,9 @@ def _act_code(act: str) -> int:
 def mx_mlp(x: torch.Tensor, w1, b1: Optional[torch.Tensor], w2, b2: Optional[torch.Tensor], mx_specs,
            act: str = "gelu", hidden_features: Optional[int] = None, out_features: Optional[int] = None, *,
            shift: Optional[torch.Tensor] = None, scale: Optional[torch.Tensor] = None,
-           residual: Optional[torch.Tensor] = None, gate: Optional[torch.Tensor] = None) -> torch.Tensor:
+           residual: Optional[torch.Tensor] = None, gate: Optional[torch.Tensor] = None,
+           ln_eps: Optional[float] = None, ln_weight: Optional[torch.Tensor] = None,
+           ln_bias: Optional[torch.Tensor] = None, add: Optional[torch.Tensor] = None) -> torch.Tensor:
     """A transformer MLP (fc1 -> GELU -> fc2) on MX Linear layers, fused:
     ``mx_linear(F.gelu(mx_linear(x, w1, b1), approximate=...), w2, b2)`` bit for bit, with the hidden activation never
     written in a float type (fc1's epilogue applies the GELU and writes fc2's MXINT8 operand).
@@ -600,7 +700,11 @@ def mx_mlp(x: torch.Tensor, w1, b1: Optional[torch.Tensor], w2, b2: Optional[tor
 
     ``shift``, ``scale`` (B, K), ``residual`` (B, T, N2), ``gate`` (B, N2): the adaLN arguments of mx_linear for a
     (B, T, K) x, the modulation applied to fc1's input and the gated residual to fc2's output:
-    ``residual + gate[:, None] * mlp(x * (1 + scale[:, None]) + shift[:, None])`` bit for bit, same launches."""
+    ``residual + gate[:, None] * mlp(x * (1 + scale[:, None]) + shift[:, None])`` bit for bit, same launches.
+
+    ``ln_eps``, ``ln_weight``, ``ln_bias``, ``add``: mx_linear's pre-norm arguments, the norm applied to fc1's input
+    and ``add`` (x.shape[:-1] + (N2,)) to fc2's output: ``add + mlp(F.layer_norm(x, (K,), ln_weight, ln_bias, ln_eps))``
+    bit for bit."""
     sp = resolve_linear_specs(mx_specs)
     code = _act_code(act)
     lib = _lib.load()
@@ -620,18 +724,24 @@ def mx_mlp(x: torch.Tensor, w1, b1: Optional[torch.Tensor], w2, b2: Optional[tor
     _check_bias(b1, N1)
     _check_bias(b2, N2)
     _same_device(x, w1_op, b1, w2_op, b2)
+    ex = ln_eps is not None or ln_weight is not None or ln_bias is not None or add is not None
     adaln = any(t is not None for t in (shift, scale, residual, gate))
-    ad = _adaln_args(x, K, N2, shift, scale, residual, gate) if adaln else ()
+    if ex:
+        ad = _ex_args(x, M, K, N2, ln_eps, ln_weight, ln_bias, add, shift, scale, residual, gate)
+    else:
+        ad = _adaln_args(x, K, N2, shift, scale, residual, gate) if adaln else ()
     with torch.cuda.device(x.device):
         out = torch.empty((M, N2), dtype=x.dtype, device=x.device)
-        ws_bytes = lib.mxp_mx_mlp_workspace_bytes(M, K, N1, N2)
+        ws_bytes = (lib.mxp_mx_mlp_ex_workspace_bytes if ex else lib.mxp_mx_mlp_workspace_bytes)(M, K, N1, N2)
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=x.device)
         f32 = _lib.MXP_DT_F32
         args = (_ptr(x2), DTYPE_CODES[x.dtype], x2.stride(0), M, K, _ptr(w1_op), N1, _ptr(b1),
                 DTYPE_CODES[b1.dtype] if b1 is not None else f32, code, _ptr(w2_op), N2, _ptr(b2),
                 DTYPE_CODES[b2.dtype] if b2 is not None else f32, sp.bfloat_bits, int(sp.flush),
                 _ptr(out), out.stride(0))
-        if adaln:
+        if ex:
+            rc = lib.mxp_mx_mlp_ex_dt(*args, *ad, _ptr(ws), ws_bytes, _stream())
+        elif adaln:
             rc = lib.mxp_mx_mlp_adaln_dt(*args, *ad, _ptr(ws), ws_bytes, _stream())
         else:
             rc = lib.mxp_mx_mlp_dt(*args, _ptr(ws), ws_bytes, _stream())
