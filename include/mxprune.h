@@ -65,7 +65,9 @@ extern "C" {
 int mxp_abi_version(void);
 const char* mxp_last_error(void);           /* thread-local, never NULL */
 
-/* Largest key count and head_dim the kernels accept. */
+/* Largest key count and head_dim the kernels accept.  Every entry point that takes keys (predict_scores, predict_topk*,
+ * sparse_attention*, pruned_attention*) returns MXP_E_UNSUPPORTED for more keys before it launches anything; the
+ * quantizer takes any number of rows. */
 void mxp_limits(int* max_keys, int* max_head_dim);
 
 /*

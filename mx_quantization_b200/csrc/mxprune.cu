@@ -21,6 +21,7 @@ using namespace mxp;
 namespace {
 
 constexpr int MAX_HD = 128;
+constexpr int MAX_KEYS = 8192;        // mxp_limits(): the most keys the attention entry points accept
 constexpr int MAX_KEYS_FUSED = 256;   // keys held in registers, 8 per lane
 
 int check_view(const char* name, const void* p, int64_t sB, int64_t sH, int64_t sN, int hd, int dt = DT_F32) {
@@ -38,6 +39,12 @@ int check_shape(int B, int H, int Nq, int Nk, int hd, int bfloat_bits) {
     if (hd < 4 || hd > MAX_HD || (hd & 3)) return fail(MXP_E_UNSUPPORTED, "head_dim %d: need a multiple of 4 in [4,%d]", hd, MAX_HD);
     if (bfloat_bits != 16 && bfloat_bits != 32) return fail(MXP_E_UNSUPPORTED, "bfloat=%d: only 16 or 32 are on the path", bfloat_bits);
     if ((int64_t)B * H > 0x7fffffffLL) return fail(MXP_E_UNSUPPORTED, "B*H too large");
+    return MXP_OK;
+}
+
+// the entry points that take keys check their count up front, before any launch; the quantizer takes any row count
+int check_keys(int Nk) {
+    if (Nk > MAX_KEYS) return fail(MXP_E_UNSUPPORTED, "Nk=%d: at most %d keys (mxp_limits)", Nk, MAX_KEYS);
     return MXP_OK;
 }
 
@@ -841,7 +848,7 @@ int mxp_debug_fused_timing(void* device_buffer) {
 const char* mxp_last_error(void) { return g_err; }
 int mxp_last_launch_count(void) { return g_launches; }
 void mxp_limits(int* max_keys, int* max_head_dim) {
-    if (max_keys) *max_keys = 8192;
+    if (max_keys) *max_keys = MAX_KEYS;
     if (max_head_dim) *max_head_dim = MAX_HD;
 }
 
@@ -905,7 +912,7 @@ int mxp_predict_scores(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
                        float* scores, void* stream) {
     g_launches = 0;
     int rc = check_shape(B, H, Nq, Nk, hd, bfloat_bits);
-    if (rc) return rc;
+    if (rc || (rc = check_keys(Nk))) return rc;
     if ((rc = check_view("q", q, q_sB, q_sH, q_sN, hd))) return rc;
     if ((rc = check_view("k", k, k_sB, k_sH, k_sN, hd))) return rc;
     if (!scores) return fail(MXP_E_BADARG, "scores: null pointer");
@@ -965,7 +972,7 @@ int mxp_predict_topk_dt(const void* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
                         int8_t* k_codes, int8_t* k_exps, void* workspace, size_t workspace_bytes, void* stream) {
     g_launches = 0;
     int rc = check_shape(B, H, Nq, Nk, hd, bfloat_bits);
-    if (rc) return rc;
+    if (rc || (rc = check_keys(Nk))) return rc;
     if ((rc = check_dtype("q/k", in_dtype)) || (rc = check_half_scope(in_dtype, hd))) return rc;
     if ((rc = check_view("q", q, q_sB, q_sH, q_sN, hd, in_dtype))) return rc;
     if ((rc = check_view("k", k, k_sB, k_sH, k_sN, hd, in_dtype))) return rc;
@@ -1019,7 +1026,7 @@ int mxp_sparse_attention_dt(const int8_t* q_codes, const int8_t* q_exps, const i
                             void* stream) {
     g_launches = 0;
     int rc = check_shape(B, H, Nq, Nk, hd, bfloat_bits);
-    if (rc) return rc;
+    if (rc || (rc = check_keys(Nk))) return rc;
     if ((rc = check_dtype("v", v_dtype)) || (rc = check_dtype("out", out_dtype))) return rc;
     if (out_dtype != DT_F32 && out_dtype != v_dtype)
         return fail(MXP_E_BADARG, "out: element type %d must be fp32 or v's (%d)", out_dtype, v_dtype);
@@ -1106,7 +1113,7 @@ static int pruned_attention_impl(const float* q, int64_t q_sB, int64_t q_sH, int
     if (key_bias && (g_attn_path != 0 || ((uintptr_t)key_bias & 3)))
         return fail(MXP_E_UNSUPPORTED, "key_bias needs the tcgen05 attention path and a 4-byte aligned pointer");
     int rc = check_shape(B, H, Nq, Nk, hd, bfloat_bits);
-    if (rc) return rc;
+    if (rc || (rc = check_keys(Nk))) return rc;
     if ((rc = check_half_scope(dt, hd))) return rc;
     if ((rc = check_view("q", q, q_sB, q_sH, q_sN, hd, dt))) return rc;
     if ((rc = check_view("k", k, k_sB, k_sH, k_sN, hd, dt))) return rc;
@@ -1252,7 +1259,7 @@ int mxp_predict_topk_mode(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_
                           uint32_t* mask, int32_t* idx, void* workspace, size_t workspace_bytes, void* stream) {
     g_launches = 0;
     int rc = check_shape(B, H, Nq, Nk, hd, bfloat_bits);
-    if (rc) return rc;
+    if (rc || (rc = check_keys(Nk))) return rc;
     if ((rc = check_view("q", q, q_sB, q_sH, q_sN, hd))) return rc;
     if ((rc = check_view("k", k, k_sB, k_sH, k_sN, hd))) return rc;
     if (!mask) return fail(MXP_E_BADARG, "mask: null pointer");
@@ -1289,7 +1296,7 @@ int mxp_predict_topk_elsa(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_
                           int bfloat_bits, int flush, uint32_t* mask, int32_t* idx, void* stream) {
     g_launches = 0;
     int rc = check_shape(B, H, N, N, hd, bfloat_bits);
-    if (rc) return rc;
+    if (rc || (rc = check_keys(N))) return rc;
     if ((rc = check_view("q", q, q_sB, q_sH, q_sN, hd))) return rc;
     if ((rc = check_view("k", k, k_sB, k_sH, k_sN, hd))) return rc;
     if (!mask) return fail(MXP_E_BADARG, "mask: null pointer");

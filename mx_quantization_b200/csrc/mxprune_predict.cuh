@@ -497,7 +497,7 @@ k_predict_topk_rows(const PredParams p) {
 //   emit           keys > T kept, keys == T kept in ascending index until top_k
 // Keys are the exact 15-bit integers of the short kernel when the exponent window allows
 // (L = 3 levels) and order-preserving fp32 keys otherwise (L = 6) - chosen per row.
-// K record per key: NB sign words + one word of per-block shifts (ek_b - kmin_b), 16 bytes.
+// K record per key: NB sign words + one word of per-block shifts (ek_b - kmin_b), 16 bytes (20 at NB = 4).
 // ==========================================================================================
 constexpr int K1L_BINS = 64;
 
@@ -507,7 +507,8 @@ struct K1LSmem {
 };
 __host__ __device__ inline K1LSmem k1l_smem_layout(int nb, int Nk) {
     K1LSmem L;
-    L.rw = nb <= 3 ? 4 : 8;
+    // records are read one word at a time: no padding at NB = 4, so 8192 keys fit the launcher's 200 KiB (196 672 bytes)
+    L.rw = nb <= 3 ? 4 : nb + 1;
     size_t o = (size_t)Nk * L.rw * 4;
     o = (o + 15) & ~(size_t)15;
     L.off_hist = o; o += (size_t)K1L_BINS * K1T * 4;

@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests."""
+import math
 import os
 
 import numpy as np
@@ -49,6 +50,30 @@ def make_qkv(B, H, N, hd, seed=0, kind="randn", Nk=None):
         q[0, 0, 1 % N, 0] = float(np.nextafter(np.float32(8.0), np.float32(0)))
         k[0, 0, 1 % Nk, 1] = -float(np.nextafter(np.float32(16.0), np.float32(0)))
     return q, k, v
+
+
+def long_inputs(kind, H, N, hd, seed):
+    """q, k (1, H, N, hd) for the long-sequence selection: kinds that stress its sampled window and its key windows."""
+    g = torch.Generator().manual_seed(seed)
+    q, k = torch.randn(1, H, N, hd, generator=g), torch.randn(1, H, N, hd, generator=g)
+    if kind.startswith("lognormal"):
+        s = float(kind[len("lognormal"):])
+        q = q * torch.exp(s * torch.randn(1, H, N, 1, generator=g))
+        k = k * torch.exp(s * torch.randn(1, H, N, 1, generator=g))
+    elif kind == "ties":                # few distinct key rows: long runs of equal scores
+        k = k[:, :, :7].repeat(1, 1, (N + 6) // 7, 1)[:, :, :N].contiguous()
+    elif kind == "constant":            # every key row the same: all scores of a row tie
+        k = k[:, :, :1].expand(1, H, N, hd).contiguous()
+    elif kind == "zeros":               # zero keys in the second half, zero query rows here and there
+        k[:, :, N // 2:] = 0.0
+        q[:, :, ::17] = 0.0
+    elif kind == "skewed":              # the sampled first keys misrepresent the rest of the row
+        k[:, :, :256] *= 0.05
+        k[:, :, 256:] += 0.5
+    elif kind == "outliers":            # a few huge keys widen the static key window
+        k[:, :, 5::511] *= 40.0
+        q[:, :, 3::97, :32] *= 0.01
+    return q, k
 
 
 def fused_qkv_views(q, k, v):
@@ -138,7 +163,6 @@ def mode_window_ok(qc, qe, kc, ke, hd, mode, bits=20):
     BLAS agree in any order (DESIGN.md 2, footnote 1), so the selected sets are pinned.  Operand widths: an MXINT8 side
     adds 7 bits below its block exponent, MXINT4 3, the exponent-sign / leading-one sides none; a block sum adds
     ceil(log2(width)) + 1."""
-    import math
     side = {"partial_Q": (7, 0), "partial_K": (0, 7), "MXINT4": (3, 3), "two_step_leading_ones": (7, 7), "true_ex": (7, 7),
             "exact": (7, 7), "ex_pred": (0, 0)}[mode]
     eq = O.predictor_exponents(qc, qe).to(torch.int64)
@@ -147,3 +171,65 @@ def mode_window_ok(qc, qe, kc, ke, hd, mode, bits=20):
     widths = torch.tensor([math.ceil(math.log2(w)) + 1 for w in O.block_widths(hd)])
     spread = (s + widths).amax(-1) - s.amin(-1) + side[0] + side[1]
     return (spread <= bits).all(-1)
+
+
+# ---- guard bands -----------------------------------------------------------------------------------------------------
+GUARD_BYTES = 256
+CANARY_INT = 0x80       # int8 -128: never a code or an exponent; 0x80808080 is no key index
+CANARY_FLOAT = 0xFF     # NaN in fp32, bf16 and fp16: an output element left unwritten fails any comparison
+
+
+class Guarded:
+    """A ``shape`` output of ``dtype`` inside a buffer of canary bytes: GUARD_BYTES before and after it, and
+    ``row_pad`` elements after each row (a padded row stride, as an ``out=`` view of a larger buffer has)."""
+
+    def __init__(self, shape, dtype, row_pad=0):
+        es = torch.empty((), dtype=dtype).element_size()
+        g = GUARD_BYTES // es
+        inner = shape[-1] + row_pad
+        rows = math.prod(shape[:-1])
+        total = 2 * g + rows * inner
+        strides, s = [], 1
+        for n in reversed((*shape[:-1], inner)):
+            strides.insert(0, s)
+            s *= n
+        self.canary = CANARY_FLOAT if dtype.is_floating_point else CANARY_INT
+        self.buf = torch.full((total * es,), self.canary, dtype=torch.uint8, device="cuda")
+        self.t = self.buf.view(dtype).as_strided(shape, strides, g)
+        covered = torch.zeros(total, dtype=torch.bool, device="cuda")
+        covered.as_strided(shape, strides, g).fill_(True)
+        self.outside = ~covered.repeat_interleave(es)
+
+    def assert_intact(self, what):
+        hit = ((self.buf != self.canary) & self.outside).nonzero().flatten()
+        assert hit.numel() == 0, (f"{what}: {hit.numel()} bytes outside the output were written, the first at byte "
+                                  f"{int(hit[0]) - GUARD_BYTES} from the output's start")
+
+    def assert_untouched(self, what):
+        """Nothing at all was written: every byte, inside the output too, still holds the canary."""
+        hit = (self.buf != self.canary).nonzero().flatten()
+        assert hit.numel() == 0, f"{what}: {hit.numel()} bytes were written by a call that failed"
+
+
+def select_guarded(q, k, top_k, bfloat=32):
+    """mxp_predict_topk_dt with mask, idx and both code / exponent outputs in guarded buffers.  The guards are checked
+    before the return code: a call that fails must not have written past its outputs either.  Returns the outputs on
+    the CPU."""
+    from mx_quantization_b200 import _lib, ops
+    lib = _lib.load()
+    B, H, Nq, hd = q.shape
+    Nk = k.shape[2]
+    nb, nw = (hd + 31) // 32, (Nk + 31) // 32
+    g = {"mask": Guarded((B, H, Nq, nw), torch.int32), "idx": Guarded((B, H, Nq, top_k), torch.int32),
+         "q_codes": Guarded((B, H, Nq, hd), torch.int8), "q_exps": Guarded((B, H, Nq, nb), torch.int8),
+         "k_codes": Guarded((B, H, Nk, hd), torch.int8), "k_exps": Guarded((B, H, Nk, nb), torch.int8)}
+    ws_bytes = lib.mxp_predict_topk_workspace_bytes(B, H, Nq, Nk, hd)
+    ws = torch.empty((max(ws_bytes, 1),), dtype=torch.uint8, device="cuda")
+    p = ops._ptr
+    rc = lib.mxp_predict_topk_dt(p(q), *q.stride()[:3], p(k), *k.stride()[:3], ops.DTYPE_CODES[q.dtype], B, H, Nq, Nk,
+                                 hd, top_k, bfloat, 0, p(g["mask"].t), p(g["idx"].t), p(g["q_codes"].t),
+                                 p(g["q_exps"].t), p(g["k_codes"].t), p(g["k_exps"].t), p(ws), ws_bytes, ops._stream())
+    for name, b in g.items():
+        b.assert_intact(name)
+    _lib.check(rc, "mxp_predict_topk_dt")
+    return {name: b.t.cpu() for name, b in g.items()}

@@ -10,13 +10,12 @@ Each output lives inside a larger buffer of canary bytes; after the call every b
 the canary, so a store that strays past a row or past the end of the output fails the test even where it changes no
 value the test reads back.
 """
-import math
-
 import pytest
 import torch
 
 from oracle import mxint8_oracle as O
-from tests.helpers import assert_out_close, canonical_idx_from_mask, make_qkv, mx_specs, unpack_mask
+from tests.helpers import (Guarded, assert_out_close, canonical_idx_from_mask, make_qkv, mx_specs, select_guarded,
+                           unpack_mask)
 
 pytestmark = pytest.mark.gpu
 
@@ -32,39 +31,6 @@ def mxq():
     import mx_quantization_b200 as m
     assert torch.cuda.is_available(), "GPU tests need a CUDA device"
     return m
-
-
-# ---- guard bands -----------------------------------------------------------------------------------------------------
-GUARD_BYTES = 256
-CANARY_INT = 0x80       # int8 -128: never a code or an exponent; 0x80808080 is no key index
-CANARY_FLOAT = 0xFF     # NaN in fp32, bf16 and fp16: an output element left unwritten fails any comparison
-
-
-class Guarded:
-    """A ``shape`` output of ``dtype`` inside a buffer of canary bytes: GUARD_BYTES before and after it, and
-    ``row_pad`` elements after each row (a padded row stride, as an ``out=`` view of a larger buffer has)."""
-
-    def __init__(self, shape, dtype, row_pad=0):
-        es = torch.empty((), dtype=dtype).element_size()
-        g = GUARD_BYTES // es
-        inner = shape[-1] + row_pad
-        rows = math.prod(shape[:-1])
-        total = 2 * g + rows * inner
-        strides, s = [], 1
-        for n in reversed((*shape[:-1], inner)):
-            strides.insert(0, s)
-            s *= n
-        self.canary = CANARY_FLOAT if dtype.is_floating_point else CANARY_INT
-        self.buf = torch.full((total * es,), self.canary, dtype=torch.uint8, device="cuda")
-        self.t = self.buf.view(dtype).as_strided(shape, strides, g)
-        covered = torch.zeros(total, dtype=torch.bool, device="cuda")
-        covered.as_strided(shape, strides, g).fill_(True)
-        self.outside = ~covered.repeat_interleave(es)
-
-    def assert_intact(self, what):
-        hit = ((self.buf != self.canary) & self.outside).nonzero().flatten()
-        assert hit.numel() == 0, (f"{what}: {hit.numel()} bytes outside the output were written, the first at byte "
-                                  f"{int(hit[0]) - GUARD_BYTES} from the output's start")
 
 
 def _out_view(shape, dtype):
@@ -165,28 +131,6 @@ def test_predict_scores(mxq, hd):
 
 
 # ---- 3. selection ----------------------------------------------------------------------------------------------------
-def _select_guarded(q, k, top_k, bfloat=32):
-    """mxp_predict_topk_dt with mask, idx and both code / exponent outputs in guarded buffers."""
-    from mx_quantization_b200 import _lib, ops
-    lib = _lib.load()
-    B, H, Nq, hd = q.shape
-    Nk = k.shape[2]
-    nb, nw = (hd + 31) // 32, (Nk + 31) // 32
-    g = {"mask": Guarded((B, H, Nq, nw), torch.int32), "idx": Guarded((B, H, Nq, top_k), torch.int32),
-         "q_codes": Guarded((B, H, Nq, hd), torch.int8), "q_exps": Guarded((B, H, Nq, nb), torch.int8),
-         "k_codes": Guarded((B, H, Nk, hd), torch.int8), "k_exps": Guarded((B, H, Nk, nb), torch.int8)}
-    ws_bytes = lib.mxp_predict_topk_workspace_bytes(B, H, Nq, Nk, hd)
-    ws = torch.empty((max(ws_bytes, 1),), dtype=torch.uint8, device="cuda")
-    p = ops._ptr
-    rc = lib.mxp_predict_topk_dt(p(q), *q.stride()[:3], p(k), *k.stride()[:3], ops.DTYPE_CODES[q.dtype], B, H, Nq, Nk,
-                                 hd, top_k, bfloat, 0, p(g["mask"].t), p(g["idx"].t), p(g["q_codes"].t),
-                                 p(g["q_exps"].t), p(g["k_codes"].t), p(g["k_exps"].t), p(ws), ws_bytes, ops._stream())
-    _lib.check(rc, "mxp_predict_topk_dt")
-    for name, b in g.items():
-        b.assert_intact(name)
-    return {name: b.t.cpu() for name, b in g.items()}
-
-
 def _check_selection(r, q, k, top_k, bfloat=32):
     Nk = k.shape[2]
     qc, qe = O.quantize_mxint8(q, 32, bfloat)
@@ -206,7 +150,7 @@ def test_selection_tensor_core(mxq, hd, Nk):
     q, k, _ = make_qkv(1, 2, 70, hd, seed=300 + hd, kind="edges", Nk=Nk)
     top_k = max(1, int(0.3 * Nk))
     for bfloat in (32, 16):
-        _check_selection(_select_guarded(q.cuda(), k.cuda(), top_k, bfloat), q, k, top_k, bfloat)
+        _check_selection(select_guarded(q.cuda(), k.cuda(), top_k, bfloat), q, k, top_k, bfloat)
 
 
 @pytest.mark.parametrize("hd", H4)
@@ -216,7 +160,7 @@ def test_selection_cuda_core(mxq, hd):
         for Nk in (77, 256):
             q, k, _ = make_qkv(1, 2, 70, hd, seed=400 + hd, kind="edges", Nk=Nk)
             top_k = max(1, int(0.3 * Nk))
-            _check_selection(_select_guarded(q.cuda(), k.cuda(), top_k), q, k, top_k)
+            _check_selection(select_guarded(q.cuda(), k.cuda(), top_k), q, k, top_k)
     finally:
         restore()
 

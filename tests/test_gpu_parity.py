@@ -7,8 +7,8 @@ import pytest
 import torch
 
 from oracle import mxint8_oracle as O
-from tests.helpers import (assert_out_close, canonical_idx_from_mask, fused_qkv_views, load_golden, make_qkv,
-                           mode_window_ok, mx_specs, unpack_mask)
+from tests.helpers import (assert_out_close, canonical_idx_from_mask, fused_qkv_views, load_golden, long_inputs,
+                           make_qkv, mode_window_ok, mx_specs, unpack_mask)
 
 pytestmark = pytest.mark.gpu
 
@@ -493,29 +493,6 @@ def test_long_sequence_end_to_end(mxq, B, H, N, hd, kind, bfloat, kfrac, pred_pa
         mxq.set_predict_path("tcgen05")
 
 
-def _long_inputs(kind, H, N, hd, seed):
-    g = torch.Generator().manual_seed(seed)
-    q, k = torch.randn(1, H, N, hd, generator=g), torch.randn(1, H, N, hd, generator=g)
-    if kind.startswith("lognormal"):
-        s = float(kind[len("lognormal"):])
-        q = q * torch.exp(s * torch.randn(1, H, N, 1, generator=g))
-        k = k * torch.exp(s * torch.randn(1, H, N, 1, generator=g))
-    elif kind == "ties":                # few distinct key rows: long runs of equal scores
-        k = k[:, :, :7].repeat(1, 1, (N + 6) // 7, 1)[:, :, :N].contiguous()
-    elif kind == "constant":            # every key row the same: all scores of a row tie
-        k = k[:, :, :1].expand(1, H, N, hd).contiguous()
-    elif kind == "zeros":               # zero keys in the second half, zero query rows here and there
-        k[:, :, N // 2:] = 0.0
-        q[:, :, ::17] = 0.0
-    elif kind == "skewed":              # the sampled first keys misrepresent the rest of the row
-        k[:, :, :256] *= 0.05
-        k[:, :, 256:] += 0.5
-    elif kind == "outliers":            # a few huge keys widen the static key window
-        k[:, :, 5::511] *= 40.0
-        q[:, :, 3::97, :32] *= 0.01
-    return q, k
-
-
 @pytest.mark.parametrize("kind", ["randn", "lognormal0.25", "lognormal0.5", "lognormal1.5", "ties", "constant", "zeros",
                                   "skewed", "outliers"])
 @pytest.mark.parametrize("N,hd,kfrac", [(640, 72, 0.25), (1100, 64, 0.1), (2048, 72, 0.5)])
@@ -524,7 +501,7 @@ def test_long_selection_paths_agree(mxq, kind, N, hd, kfrac):
     or of 2^fs key values), the radix levels alone (fused path 0), and, outside the tensor-core window, the CUDA-core integer
     kernel: masks AND index lists must be identical, whatever the input does to the sample (funcs: main.py:118-123 top-k of
     the predicted scores; the canonical tie rule of SURVEY 8a)."""
-    q, k = _long_inputs(kind, 2, N, hd, seed=N + hd)
+    q, k = long_inputs(kind, 2, N, hd, seed=N + hd)
     specs = mx_specs(32, False)
     top_k = max(1, int(kfrac * N))
     res = {}
