@@ -192,7 +192,10 @@ int mxp_pruned_attention(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_s
  *     true_scores += attn_bias ;  pred_scores = ex_q @ ex_k^T + attn_bias
  * key_bias[b * kb_sB + j] is that bias for key j of batch element b (the reference's (B,1,1,S) mask,
  * the same for every head and query row; finite values, e.g. (1 - mask) * -10000).  Nq and Nk may
- * differ (Nk <= 256).  Everything else as mxp_pruned_attention.
+ * differ; every Nk of mxp_pruned_attention (up to mxp_limits' max_keys).  Beyond 256 keys the tensor-core
+ * selection adds the bias to its integer keys; rows it cannot rank exactly (a bias no integer key carries, a threshold
+ * among keys below its window) are ranked by the CUDA-core kernel on fp32 keys fl32(pred + bias_j), exact for any
+ * finite bias, and the streamed attention kernel adds bias_j after score * scale.  Everything else as mxp_pruned_attention.
  */
 int mxp_pruned_attention_biased(const float* q, int64_t q_sB, int64_t q_sH, int64_t q_sN,
                                 const float* k, int64_t k_sB, int64_t k_sH, int64_t k_sN,
@@ -230,7 +233,8 @@ int mxp_pruned_attention_dt(const void* q, int64_t q_sB, int64_t q_sH, int64_t q
  * (callers: main.py:107-123, DiT models.py:178-194, MX_transformer_block.py:659-673).  Modes 1-6 need Nk <= 256 and head_dim a multiple
  * of 8, >= 32 (MXP_E_UNSUPPORTED otherwise); `scale` ranks the exact mode and scales the attention in
  * every mode.  key_bias (may be NULL) is the additive cross-attention bias of mxp_pruned_attention_biased, added
- * in fp32 to the ranked value of every mode (MX_transformer_block.py:803,822).  mxp_predict_topk_mode is the
+ * in fp32 to the ranked value of every mode (MX_transformer_block.py:803,822); modes 1-6 keep their Nk <= 256 limit
+ * with a bias too (mode 0 takes it up to max_keys).  mxp_predict_topk_mode is the
  * selection alone (mask / idx as mxp_predict_topk).
  */
 #define MXP_PRED_EXP_SIGN  0

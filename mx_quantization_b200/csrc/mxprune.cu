@@ -466,14 +466,18 @@ inline int pick_kpl(int Nk) {
     return 8;
 }
 
-template <int NB, int DT = DT_F32>
+template <int NB, int DT = DT_F32, bool BIAS = false>
 int launch_predict_topk_long(const PredParams& p, cudaStream_t st) {
-    if (DT == DT_F32 && p.dt == DT_BF16) return launch_predict_topk_long<NB, DT_BF16>(p, st);
-    if (DT == DT_F32 && p.dt == DT_F16) return launch_predict_topk_long<NB, DT_F16>(p, st);
-    const K1LSmem L = k1l_smem_layout(NB, p.Nk);
-    if (L.total > 200 * 1024)
-        return fail(MXP_E_UNSUPPORTED, "Nk=%d: key records need %zu bytes of shared memory (limit 200 KiB)", p.Nk, L.total);
-    cudaError_t e = cudaFuncSetAttribute(k_predict_topk_long<NB, DT>,
+    if (DT == DT_F32 && p.dt == DT_BF16) return launch_predict_topk_long<NB, DT_BF16, BIAS>(p, st);
+    if (DT == DT_F32 && p.dt == DT_F16) return launch_predict_topk_long<NB, DT_F16, BIAS>(p, st);
+    if (!BIAS && p.key_bias) return launch_predict_topk_long<NB, DT, true>(p, st);
+    const K1LSmem L = k1l_smem_layout(NB, p.Nk, BIAS);
+    // the staged bias (4 bytes per key) takes the layout past 200 KiB at 8192 keys and NB = 4; 227 KiB still hold it
+    const size_t limit = BIAS ? SMEM_PER_SM : 200 * 1024;
+    if (L.total > limit)
+        return fail(MXP_E_UNSUPPORTED, "Nk=%d: key records need %zu bytes of shared memory (limit %zu bytes)", p.Nk,
+                    L.total, limit);
+    cudaError_t e = cudaFuncSetAttribute(k_predict_topk_long<NB, DT, BIAS>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
     if (e != cudaSuccess) return fail(MXP_E_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     const int heads = p.B * p.H;
@@ -482,7 +486,7 @@ int launch_predict_topk_long(const PredParams& p, cudaStream_t st) {
     if (splits > tiles) splits = tiles;
     if (splits < 1) splits = 1;
     dim3 grid((unsigned)heads, (unsigned)splits);
-    k_predict_topk_long<NB, DT><<<grid, K1T, L.total, st>>>(p);
+    k_predict_topk_long<NB, DT, BIAS><<<grid, K1T, L.total, st>>>(p);
     return check_launch("k_predict_topk_long");
 }
 
@@ -554,8 +558,6 @@ int launch_attend_pair_ot(const AttnParams& p, dim3 grid, size_t dyn, cudaStream
 // mxprune_attend_long.cuh), one key block runs k_attend_pair (two lanes per query row, 256 threads).
 int launch_attend(const AttnParams& p, cudaStream_t st) {
     const OpsLayout O = ops_layout(p.Nq, p.Nk, p.hd);
-    if (p.key_bias && !O.single)
-        return fail(MXP_E_UNSUPPORTED, "key_bias: the additive key bias is implemented for Nk <= 256 (cross-attention)");
     if (!O.single) return launch_attend_long_pair(p, st);
     const K2Smem L = k2_smem_layout(O);
     if (L.total > 160 * 1024) return fail(MXP_E_UNSUPPORTED, "attention operands need %zu bytes of shared memory", L.total);
@@ -728,13 +730,16 @@ inline LongWsLayout long_ws_layout(int B, int H, int Nq, int Nk, int hd) {
     return W;
 }
 
-// returns 1 if the shape is outside this path's domain or no workspace was supplied
+// returns 1 if the shape is outside this path's domain or no workspace was supplied.  With an additive key bias the
+// selection adds it to every score (k_select_long_tc<true>) and the flagged rows' kernel adds it to its fp32 keys
+// (k_predict_topk_long<.., BIAS>)
 static int try_predict_topk_long_tc(const PredParams& p, cudaStream_t st, int* rc_out) {
     if (g_predict_path != 0) return 1;
     const LongWsLayout W = long_ws_layout(p.B, p.H, p.Nq, p.Nk, p.hd);
     if (W.total == 0 || !p.long_ws || p.long_ws_bytes < W.total || ((uintptr_t)p.long_ws & 255)) return 1;
     const OpsLayout O = ops_layout(p.Nq, p.Nk, p.hd);
-    const KLSmem L = kl_smem_layout(O);
+    const bool biased = p.key_bias != nullptr;
+    const KLSmem L = kl_smem_layout(O, biased);
     if (L.total > 227 * 1024) return 1;
     unsigned char* w = (unsigned char*)p.long_ws;
     const int heads = p.B * p.H, nb = (p.hd + 31) / 32;
@@ -777,8 +782,9 @@ static int try_predict_topk_long_tc(const PredParams& p, cudaStream_t st, int* r
     }
     {
         {
-            static std::atomic<uint64_t> done_{0};
-            if ((*rc_out = ensure_dyn_smem(k_select_long_tc, 227 * 1024, done_))) return 0;
+            static std::atomic<uint64_t> done_{0}, done_b{0};
+            if ((*rc_out = biased ? ensure_dyn_smem(k_select_long_tc<true>, 227 * 1024, done_b)
+                                  : ensure_dyn_smem(k_select_long_tc<false>, 227 * 1024, done_))) return 0;
         }
         LongSelParams sp{};
         sp.q_pp = w + W.q_pp; sp.k_pp = w + W.k_pp; sp.q_ep = (const int8_t*)(w + W.q_ep);
@@ -796,7 +802,9 @@ static int try_predict_topk_long_tc(const PredParams& p, cudaStream_t st, int* r
             if (n_pairs % d == 0) { splits = d; break; }
         const size_t dyn = L.total;
         sp.splits = splits;
-        k_select_long_tc<<<dim3((unsigned)((size_t)heads * splits)), KL_T, dyn, st>>>(sp);
+        sp.key_bias = p.key_bias; sp.kb_sB = p.kb_sB;
+        if (biased) k_select_long_tc<true><<<dim3((unsigned)((size_t)heads * splits)), KL_T, dyn, st>>>(sp);
+        else k_select_long_tc<false><<<dim3((unsigned)((size_t)heads * splits)), KL_T, dyn, st>>>(sp);
         if ((*rc_out = check_launch("k_select_long_tc"))) return 0;
     }
     // rows outside the integer-key window: the CUDA-core kernel, restricted to the flagged rows
@@ -951,8 +959,6 @@ size_t mxp_predict_topk_workspace_bytes(int B, int H, int Nq, int Nk, int hd) {
 
 static int predict_topk_impl(const PredParams& p, cudaStream_t st) {
     int rc = MXP_OK;
-    if (p.key_bias && p.Nk > K1_MAX_KEYS)
-        return fail(MXP_E_UNSUPPORTED, "key_bias: the additive key bias is implemented for Nk <= 256 (cross-attention)");
     if (p.pred_mode < 0 || p.pred_mode > 7) return fail(MXP_E_BADARG, "pred_mode=%d outside [0, 7]", p.pred_mode);
     if (p.pred_mode != 0) return predict_topk_wide(p, st);
     if (try_predict_topk_tc(p, st, &rc) == 0) return rc;

@@ -32,8 +32,10 @@ __host__ __device__ inline KLPSmem klp_smem_layout(const OpsLayout& O) {
     return L;
 }
 
-// OT: output element type (DT_*)
-template <bool BF16, int OT = DT_F32>
+// OT: output element type (DT_*).  BIAS: p.key_bias is set - t = fl32(fl32(s * scale) + bias_j) as in k_attend_pair.
+// The bias is read through the read-only cache (a lane's 32 keys of a window are consecutive), not staged: shared
+// memory for it would cost the second CTA per SM at head_dim 72 / 80
+template <bool BF16, int OT = DT_F32, bool BIAS = false>
 __global__ void __launch_bounds__(K2P_T, 2)
 k_attend_long_pair(const AttnParams p) {
     extern __shared__ __align__(128) unsigned char smem_klp[];
@@ -65,6 +67,9 @@ k_attend_long_pair(const AttnParams p) {
     const unsigned char* v_op = p.v_op + (size_t)head * O.v_head_bytes;
     float* out_head = out_elem(p.out, bb * p.o_sB + hh * p.o_sH, OT != DT_F32);
     const uint32_t kbytes = (uint32_t)O.k_blk_bytes, vbytes = (uint32_t)O.v_blk_bytes;
+    const float* const bias_b = BIAS ? p.key_bias + bb * p.kb_sB : nullptr;
+    // BIAS: bias of key j (keys past Nk read the last key's; they are never kept)
+    auto bias_at = [&](int j) { return __ldg(bias_b + min(j, Nk - 1)); };
 
     if (tid == 0) {
         mbar_init(&bar_k[0], 1); mbar_init(&bar_k[1], 1);
@@ -115,6 +120,7 @@ k_attend_long_pair(const AttnParams p) {
         float m = -INFINITY, l = 0.f;
         for (int blk = 0; blk < nblk; ++blk) {
             const int s = blk & 1;
+            const int kb = blk * 128 + 64 * part;                   // key of this lane's column 0
             // S(blk + 1) into the other TMEM buffer (its last reader, the epilogue of blk - 1, ended with a barrier)
             if (blk + 1 < nblk) {
                 if (tid == 0) {
@@ -150,7 +156,9 @@ k_attend_long_pair(const AttnParams p) {
                 for (int c = 0; c < 32; ++c) {                      // dropped keys become -inf: no part in the maximum, exp = 0
                     float sv = __uint_as_float(r[c]);
                     if (bf16) sv = bf16_half_away(sv);
-                    const float tv = ((mwj >> c) & 1u) ? __fmul_rn(sv, scale) : -INFINITY;
+                    float ts = __fmul_rn(sv, scale);
+                    if (BIAS) ts = __fadd_rn(ts, bias_at(kb + 32 * j + c));
+                    const float tv = ((mwj >> c) & 1u) ? ts : -INFINITY;
                     r[c] = __float_as_uint(tv);
                     mb4[c & 3] = fmaxf(mb4[c & 3], tv);
                 }
@@ -195,6 +203,7 @@ k_attend_long_pair(const AttnParams p) {
         bool first_mma = true;
         for (int blk = 0; blk < nblk; ++blk) {
             const int vb = blk & 1;
+            const int kb = blk * 128 + 64 * part;                   // key of this lane's column 0
             uint32_t mw[2];
 #pragma unroll
             for (int j = 0; j < 2; ++j) {
@@ -228,7 +237,9 @@ k_attend_long_pair(const AttnParams p) {
                 for (int c = 0; c < 32; ++c) {
                     float sv = __uint_as_float(r[c]);
                     if (bf16) sv = bf16_half_away(sv);
-                    const float ex = exp_fast_nonpos(__fsub_rn(__fmul_rn(sv, scale), m_fin));      // as in pass 1: sum(p) stays 1
+                    float ts = __fmul_rn(sv, scale);
+                    if (BIAS) ts = __fadd_rn(ts, bias_at(kb + 32 * j + c));
+                    const float ex = exp_fast_nonpos(__fsub_rn(ts, m_fin));     // as in pass 1: sum(p) stays 1
                     const float ev = ((mwj >> c) & 1u) ? ex : 0.f;
                     uint32_t pb = __float_as_uint(ev * inv);
                     if (bf16) pb = bf16_half_away(pb);

@@ -16,8 +16,16 @@ template <int OT>
 static int launch_attend_long_pair_ot(const AttnParams& p, dim3 grid, size_t dyn, cudaStream_t st) {
     MXP_ENSURE_DYN_SMEM((k_attend_long_pair<true, OT>), (int)(SMEM_PER_SM - 2048));
     MXP_ENSURE_DYN_SMEM((k_attend_long_pair<false, OT>), (int)(SMEM_PER_SM - 2048));
-    if (p.bf16) k_attend_long_pair<true, OT><<<grid, K2P_T, dyn, st>>>(p);
-    else k_attend_long_pair<false, OT><<<grid, K2P_T, dyn, st>>>(p);
+    if (p.key_bias) {
+        MXP_ENSURE_DYN_SMEM((k_attend_long_pair<true, OT, true>), (int)(SMEM_PER_SM - 2048));
+        MXP_ENSURE_DYN_SMEM((k_attend_long_pair<false, OT, true>), (int)(SMEM_PER_SM - 2048));
+        if (p.bf16) k_attend_long_pair<true, OT, true><<<grid, K2P_T, dyn, st>>>(p);
+        else k_attend_long_pair<false, OT, true><<<grid, K2P_T, dyn, st>>>(p);
+    } else if (p.bf16) {
+        k_attend_long_pair<true, OT><<<grid, K2P_T, dyn, st>>>(p);
+    } else {
+        k_attend_long_pair<false, OT><<<grid, K2P_T, dyn, st>>>(p);
+    }
     return check_launch("k_attend_long_pair");
 }
 

@@ -498,19 +498,23 @@ k_predict_topk_rows(const PredParams p) {
 // Keys are the exact 15-bit integers of the short kernel when the exponent window allows
 // (L = 3 levels) and order-preserving fp32 keys otherwise (L = 6) - chosen per row.
 // K record per key: NB sign words + one word of per-block shifts (ek_b - kmin_b), 16 bytes (20 at NB = 4).
+// With an additive key bias (BIAS) every row ranks fl32(pred + bias_j) on the fp32 keys; the batch's Nk bias values
+// are staged once next to the records.
 // ==========================================================================================
 constexpr int K1L_BINS = 64;
 
 struct K1LSmem {
     int rw;                         // 32-bit words per key record
-    size_t off_hist, off_misc, total;
+    size_t off_bias, off_hist, off_misc, total;
 };
-__host__ __device__ inline K1LSmem k1l_smem_layout(int nb, int Nk) {
+__host__ __device__ inline K1LSmem k1l_smem_layout(int nb, int Nk, bool bias = false) {
     K1LSmem L;
     // records are read one word at a time: no padding at NB = 4, so 8192 keys fit the launcher's 200 KiB (196 672 bytes)
+    // without a bias, and 227 KiB (229 440 bytes) with one
     L.rw = nb <= 3 ? 4 : nb + 1;
     size_t o = (size_t)Nk * L.rw * 4;
     o = (o + 15) & ~(size_t)15;
+    L.off_bias = o; if (bias) o += ((size_t)Nk * 4 + 15) & ~(size_t)15;
     L.off_hist = o; o += (size_t)K1L_BINS * K1T * 4;
     L.off_misc = o; o += 64;
     L.total = o;
@@ -526,10 +530,12 @@ struct LongRow {
     bool fast;
 };
 
-template <int NB>
-__device__ __forceinline__ uint32_t long_key(const LongRow<NB>& R, const uint32_t* rec, const int (&kmin)[NB], int hd) {
+// BIAS: bias_j (the key's staged bias) is added in fp32 to the predicted score (rows are never fast then)
+template <int NB, bool BIAS = false>
+__device__ __forceinline__ uint32_t long_key(const LongRow<NB>& R, const uint32_t* rec, const int (&kmin)[NB], int hd,
+                                             float bias_j = 0.f) {
     const uint32_t shw = rec[NB];
-    if (R.fast) {
+    if (!BIAS && R.fast) {
         int S = R.moff;
 #pragma unroll
         for (int b = 0; b < NB; ++b) {
@@ -547,18 +553,20 @@ __device__ __forceinline__ uint32_t long_key(const LongRow<NB>& R, const uint32_
         const float t = exp2i(kmin[b] + (int)((shw >> (8 * b)) & 0xffu)) * cnt;
         s = (b == 0) ? t * R.wq[0] : fmaf(t, R.wq[b], s);
     }
+    if (BIAS) s = __fadd_rn(s, bias_j);                         // pred_scores + attn_bias, fp32
     return ordered_key(s);
 }
 
-// DT: element type of the q / k views (DT_*)
-template <int NB, int DT = DT_F32>
+// DT: element type of the q / k views (DT_*); BIAS: p.key_bias is set (see long_key)
+template <int NB, int DT = DT_F32, bool BIAS = false>
 __global__ void __launch_bounds__(K1T)
 k_predict_topk_long(const PredParams p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int Nk = p.Nk, Nq = p.Nq, hd = p.hd, kk = p.top_k;
-    const K1LSmem L = k1l_smem_layout(NB, Nk);
+    const K1LSmem L = k1l_smem_layout(NB, Nk, BIAS);
     const int RW = L.rw;
     uint32_t* s_rec = reinterpret_cast<uint32_t*>(smem_raw);
+    float* s_bias = reinterpret_cast<float*>(smem_raw + L.off_bias);      // BIAS only
     uint32_t* s_hist = reinterpret_cast<uint32_t*>(smem_raw + L.off_hist);
     int* s_kmin = reinterpret_cast<int*>(smem_raw + L.off_misc);
     int* s_kmax = s_kmin + 4;
@@ -596,6 +604,7 @@ k_predict_topk_long(const PredParams p) {
                 if (write_k) p.k_exps[krow * NB + b] = (int8_t)kq.e[b];
             }
             s_rec[j * RW + NB] = epw;
+            if (BIAS) s_bias[j] = __ldg(p.key_bias + bb * p.kb_sB + j);
         }
         if (write_kop) {
             const int kch = OL.hdp >> 3, rows_pad = OL.nblk * OL.kb_rows;
@@ -654,7 +663,7 @@ k_predict_topk_long(const PredParams p) {
         int g = 0x7fffffff;
 #pragma unroll
         for (int b = 0; b < NB; ++b) g = min(g, rq.ep[b] + kmin[b]);
-        R.fast = !wide;
+        R.fast = !BIAS && !wide;
         long long M = 0;
 #pragma unroll
         for (int b = 0; b < NB; ++b) {
@@ -681,7 +690,7 @@ k_predict_topk_long(const PredParams p) {
             for (int b = 0; b < K1L_BINS; ++b) my_hist[b * K1T] = 0u;
             if (lo >= 0) {
                 for (int j = 0; j < Nk; ++j) {
-                    const uint32_t u = long_key<NB>(R, s_rec + j * RW, kmin, hd);
+                    const uint32_t u = long_key<NB, BIAS>(R, s_rec + j * RW, kmin, hd, BIAS ? s_bias[j] : 0.f);
                     const uint32_t hi = (lo + 6 >= 32) ? 0u : (u >> (lo + 6));
                     if (hi == prefix) my_hist[((u >> lo) & 63u) * K1T] += 1u;
                 }
@@ -702,7 +711,7 @@ k_predict_topk_long(const PredParams p) {
             int rem = krem, pos = 0;
             uint32_t word = 0u;
             for (int j = 0; j < Nk; ++j) {
-                const uint32_t u = long_key<NB>(R, s_rec + j * RW, kmin, hd);
+                const uint32_t u = long_key<NB, BIAS>(R, s_rec + j * RW, kmin, hd, BIAS ? s_bias[j] : 0.f);
                 bool keep = u > T;
                 if (u == T && rem > 0) { keep = true; --rem; }
                 word |= (keep ? 1u : 0u) << (j & 31);

@@ -121,16 +121,19 @@ struct LongSelParams {
     int H, Nq, Nk, hd, top_k;
     int adaptive;                   // 1: sampled fine window in front of the radix levels (see below)
     int splits;                     // CTAs per head (linear grid, a head's CTAs adjacent: its Kp operand stays in L2)
+    const float* key_bias;          // BIAS: additive key bias key_bias[b * kb_sB + j] (see k_select_long_tc)
+    int64_t kb_sB;
 };
 
 struct KLSmem {
-    size_t off_k, off_hist, off_misc, total;
+    size_t off_k, off_bias, off_hist, off_misc, total;
     int bins;
 };
-__host__ __device__ inline KLSmem kl_smem_layout(const OpsLayout& O) {
+__host__ __device__ inline KLSmem kl_smem_layout(const OpsLayout& O, bool bias = false) {
     KLSmem L;
     size_t o = 2 * O.q_tile_bytes;
     L.off_k = o;    o += 2 * O.k_blk_bytes;
+    L.off_bias = o; if (bias) o += 2 * 128 * 4;     // BIAS: bias_j - bmax of two key blocks
     // the fine window wants 128 counters per lane; head dims whose operand tiles leave no room keep 64
     L.bins = (o + (size_t)KL_FBINS * KL_T * 2 + 128 <= (size_t)227 * 1024) ? KL_FBINS : KL_BINS;
     L.off_hist = o; o += (size_t)L.bins * KL_T * 2;
@@ -163,6 +166,27 @@ __device__ __forceinline__ void kl_compare_window(const uint32_t (&r)[32], float
     eq_out = eq;
 }
 
+// BIAS: the 32 scores of one TMEM read (this lane's keys sd[0..31]) -> score + (bias_j - bmax), clamped below at xfloor
+// (the value of key 0): keys below the row's window all land on key 0
+__device__ __forceinline__ void kl_add_bias(uint32_t (&r)[32], const float* sd, float xfloor) {
+#pragma unroll
+    for (int c = 0; c < 32; c += 4) {
+        const float4 d = *reinterpret_cast<const float4*>(sd + c);
+        r[c] = __float_as_uint(fmaxf(__fadd_rn(__uint_as_float(r[c]), d.x), xfloor));
+        r[c + 1] = __float_as_uint(fmaxf(__fadd_rn(__uint_as_float(r[c + 1]), d.y), xfloor));
+        r[c + 2] = __float_as_uint(fmaxf(__fadd_rn(__uint_as_float(r[c + 2]), d.z), xfloor));
+        r[c + 3] = __float_as_uint(fmaxf(__fadd_rn(__uint_as_float(r[c + 3]), d.w), xfloor));
+    }
+}
+
+// lowest power of two of which the fp32 value x != 0 is a multiple
+__device__ __forceinline__ int kl_unit_exp(float x) {
+    const uint32_t b = __float_as_uint(x) & 0x7fffffffu;
+    const int e = (int)(b >> 23);
+    const uint32_t m = e ? ((b & 0x7fffffu) | 0x800000u) : b;
+    return (e ? e - 150 : -149) + __ffs((int)m) - 1;
+}
+
 // One CTA = one PAIR of 128-row query tiles of one head (16 warps: warps 0-7 the even tile, 8-15 the odd
 // one; 512 TMEM columns = two score buffers per tile) sharing every K block it streams.
 //
@@ -174,13 +198,25 @@ __device__ __forceinline__ void kl_compare_window(const uint32_t (&r)[32], float
 // passes instead of three or four.  A row whose sample spreads over more than KL_MAX_RANGE values takes bins of 2^fs keys
 // (fs <= 6) and ONE radix level for the fs bits inside the bin (three passes for its pair).  A row whose threshold lands in a
 // clamp bin, or whose sample is wider still, sends its tile pair through the radix levels - same result, the old cost.
+//
+// BIAS (additive key bias, ranked value fl32(pred + bias_j)): the bias is added on the CUDA cores to every score read
+// from TMEM, as x = score + d_j with d_j = fl32(bias_j - bmax) (bmax: the batch's largest bias), so the keys stay
+// integers of the row's unit 2^(g+1) below the unbiased window's top.  With 2^u the unit of every bias, 2^du that of
+// every d_j and m = min(g, u), a row keeps the fast path when du >= g + 1 (integer keys), g <= u + 1 or every d_j is 0
+// (the d_j of keys inside the window are exact), and |bmax| and the window's span (2^(g+1) times key 0's offset) are
+// <= 2^(23+m) (the reference's pred + bias_j is exact inside the window).  Then every key inside the window equals the
+// reference's value up to the constant bmax, and every key below it (x below the value of key 0, e.g. PixArt's -10000
+// mask) is also below every key inside it in the reference.  Those keys are clamped to key 0.  A row whose threshold lands on key 0 (fewer than
+// top_k keys inside the window) is flagged in the emit pass and re-ranked by the CUDA-core kernel, as rows outside the
+// window are.
+template <bool BIAS = false>
 __global__ void __launch_bounds__(KL_T, 1)
 k_select_long_tc(const LongSelParams p) {
     extern __shared__ __align__(1024) unsigned char smem_kl[];
     unsigned char* const smem = smem_kl;
     const int Nk = p.Nk, Nq = p.Nq, hd = p.hd, kk = p.top_k;
     const OpsLayout O = ops_layout(Nq, Nk, hd);
-    const KLSmem L = kl_smem_layout(O);
+    const KLSmem L = kl_smem_layout(O, BIAS);
     const int nb = (hd + 31) >> 5, nblk = O.nblk;
     unsigned char* sQ = smem;
     unsigned char* sK = smem + L.off_k;
@@ -193,6 +229,10 @@ k_select_long_tc(const LongSelParams p) {
     int* s_gen = s_nlev + 1;                            // 1: this tile pair takes the radix levels
     int* s_wide = s_nlev + 2;                           // 1: some row of the pair has keys wider than 15 bits
     int* s_l2 = s_nlev + 3;                             // 1: some row's fine bins hold more than one key value
+    uint32_t* s_bmax = reinterpret_cast<uint32_t*>(s_nlev + 4);    // BIAS: order-preserving bits of the largest bias
+    int* s_bunit = s_nlev + 5;                          // BIAS: exponent of the coarsest unit every bias is a multiple of
+    int* s_dunit = s_nlev + 6;                          // BIAS: the same for every bias_j - bmax
+    float* s_d = reinterpret_cast<float*>(smem + L.off_bias);      // BIAS: [2][128] bias_j - bmax of key blocks
 
     const int head = blockIdx.x / p.splits;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -209,12 +249,49 @@ k_select_long_tc(const LongSelParams p) {
         mbar_init(&bar_k[0], 1); mbar_init(&bar_k[1], 1);
         mbar_init(&bar_mma[0], 1); mbar_init(&bar_mma[1], 1);
         mbar_init(bar_q, 1);
+        if (BIAS) { *s_bmax = 0u; *s_bunit = 0x7fffffff; *s_dunit = 0x7fffffff; }
     }
     if (warp == 0) tmem_alloc(s_tmem, 512u);
     tcgen05_fence_before_sync();
     __syncthreads();
     tcgen05_fence_after_sync();
     const uint32_t tmem = *s_tmem;
+    const float* const bias_b = BIAS ? p.key_bias + (head / p.H) * p.kb_sB : nullptr;
+    float bmax = 0.f;
+    int bunit = 0x7fffffff, dunit = 0x7fffffff;
+    if (BIAS) {                                          // the batch's largest bias and the units of the biases / d_j
+        uint32_t mx = 0u;
+        int un = 0x7fffffff;
+        for (int j = tid; j < Nk; j += KL_T) {
+            const float b = __ldg(bias_b + j);
+            const uint32_t u = __float_as_uint(b);
+            mx = max(mx, (u & 0x80000000u) ? ~u : u | 0x80000000u);
+            if (b != 0.f) un = min(un, kl_unit_exp(b));
+        }
+        mx = __reduce_max_sync(FULL, mx);
+        un = __reduce_min_sync(FULL, un);
+        if (lane == 0) { atomicMax(s_bmax, mx); atomicMin(s_bunit, un); }
+        __syncthreads();
+        const uint32_t m = *s_bmax;
+        bmax = __uint_as_float((m & 0x80000000u) ? m & 0x7fffffffu : ~m);
+        bunit = *s_bunit;
+        int du = 0x7fffffff;
+        for (int j = tid; j < Nk; j += KL_T) {
+            const float d = __fsub_rn(__ldg(bias_b + j), bmax);
+            if (d != 0.f) du = min(du, kl_unit_exp(d));
+        }
+        du = __reduce_min_sync(FULL, du);
+        if (lane == 0) atomicMin(s_dunit, du);
+        __syncthreads();
+        dunit = *s_dunit;
+    }
+    // BIAS: bias_j - bmax of key block blk -> s_d[(blk & 1) * 128 ..] (keys past Nk: 0, the score of Kp's zero rows)
+    auto stage_bias = [&](int blk) {
+        if (tid < 128) {
+            const int j = blk * 128 + tid;
+            s_d[(blk & 1) * 128 + tid] = j < Nk ? __fsub_rn(__ldg(bias_b + j), bmax) : 0.f;
+        }
+    };
     const uint32_t my_lane = (uint32_t)lane_base << 16;
     const uint32_t my_col = (uint32_t)(half * 256);     // this tile's two 128-column score buffers
     const uint32_t idesc = umma_idesc_bf16_f32(128, 128);
@@ -291,11 +368,20 @@ k_select_long_tc(const LongSelParams p) {
             }
         }
         if (M > KL_WIDE_M) fast = false;
+        if (BIAS && fast) {
+            const int mu = min(g, bunit);
+            const float span = (float)((((int)M + 1) >> 1) + 1) * exp2i(g + 1);      // key 0's offset x 2^(g+1)
+            const float lim = 23 + mu < -126 ? 0.f : exp2i(min(23 + mu, 127));
+            if (dunit < g + 1 || (dunit != 0x7fffffff && g > bunit + 1) || !(fabsf(bmax) <= lim) || !(span <= lim))
+                fast = false;
+        }
         const bool narrow = M <= K1_MAX_M;                          // keys fit the 15-bit fp16 patterns of the short kernels
         if (valid && part == 0) p.flags[row] = fast ? 0 : 1;
         if (!fast) M = 0;
         const int moff = ((int)M + 1) & ~1;
         const float scl = fast ? exp2i(-g - 1) : 0.f;
+        // BIAS: the score value of key 0 (scores clamp there); any value for other rows (scl = 0)
+        const float xfloor = fast ? -(float)((moff >> 1) + 1) * exp2i(g + 1) : 0.f;
         // histogram passes rank on the plain key u = S/2 + moff/2 + 1 (fewest digits); the emit pass adds
         // the fp16 bias of the short kernel so that two keys per word compare with one HSET2
         const uint32_t key0 = (uint32_t)((moff >> 1) + 1);          // key of a score of exactly 0
@@ -325,6 +411,10 @@ k_select_long_tc(const LongSelParams p) {
         bool adapt = nlev > 0 && *s_gen == 0 && 5 * nsamp + 4 * nblk < 2 * (nlev + 1) * nblk;
         int lo_key = 0, fs = 0;                                     // fine bin e <-> keys [lo_key + (e << fs), + 2^fs)
         if (adapt) {
+            if (BIAS) {
+                for (int b = 0; b < nsamp; ++b) stage_bias(b);
+                __syncthreads();
+            }
             if (tid == 0) {
                 for (int b = 0; b < nsamp; ++b) {
                     mbar_expect_tx(&bar_k[b], (uint32_t)O.k_blk_bytes);
@@ -350,6 +440,7 @@ k_select_long_tc(const LongSelParams p) {
                     uint32_t r[32];
                     tmem_ld_16x32bx2_s64_x32(tbase + (q4 >> 1) * 128 + (q4 & 1) * 32, r);
                     tmem_ld_wait();
+                    if (BIAS) kl_add_bias(r, s_d + (q4 >> 1) * 128 + 64 * part + 32 * (q4 & 1), xfloor);
 #pragma unroll
                     for (int c = 0; c < 32; ++c) {
                         const float f = fmaf(__uint_as_float(r[c]), scl, cadd);
@@ -370,6 +461,7 @@ k_select_long_tc(const LongSelParams p) {
                     uint32_t r[32];
                     tmem_ld_16x32bx2_s64_x32(tbase + (q4 >> 1) * 128 + (q4 & 1) * 32, r);
                     tmem_ld_wait();
+                    if (BIAS) kl_add_bias(r, s_d + (q4 >> 1) * 128 + 64 * part + 32 * (q4 & 1), xfloor);
                     if (fast) {
 #pragma unroll
                         for (int c = 0; c < 32; ++c) {
@@ -424,6 +516,8 @@ k_select_long_tc(const LongSelParams p) {
                 for (int b = 0; b < nbins; ++b) my_hist[b * KL_T] = 0;
             }
             int rem = krem, pos = 0;                                // emit state (identical in both lanes)
+            // BIAS: a threshold on key 0 lies among the clamped keys: the row goes to the CUDA-core kernel
+            if (BIAS && emit && valid && fast && part == 0 && prefix == 0u) p.flags[row] = 1;
             // emit compares fp16 patterns: the biased key against T + bias, or (wide pair) the key re-centred on T against 0x4000
             const uint32_t T = wide_pair ? 0x4000u : prefix + K1_KEY_BIAS;
             const int aw = 0x4000 - (0x4B000000 + (int)prefix);
@@ -435,6 +529,8 @@ k_select_long_tc(const LongSelParams p) {
                 }
             }
             for (int it = 0; it <= nblk; ++it) {
+                // BIAS: block it's buffer was last read in iteration it - 1, which ended with a barrier
+                if (BIAS && it < nblk) stage_bias(it);
                 if (it < nblk) {
                     const int s = it & 1;
                     mbar_wait(&bar_k[s], (ph_k >> s) & 1u);
@@ -459,6 +555,7 @@ k_select_long_tc(const LongSelParams p) {
                                 uint32_t r[32];
                                 tmem_ld_16x32bx2_s64_x32(tbase + q2 * 32, r);
                                 tmem_ld_wait();
+                                if (BIAS) kl_add_bias(r, s_d + s * 128 + 64 * part + 32 * q2, xfloor);
                                 if (counting) {
                                     // fine window: bin = clamp((key - lo_key) >> fs, 0, 127), one VIADDMNMX.  The counter
                                     // updates go in PAIRS - both loads issued before either store, the second store adding
@@ -509,6 +606,7 @@ k_select_long_tc(const LongSelParams p) {
                             uint32_t r[32];
                             tmem_ld_16x32bx2_s64_x32(tbase + q2 * 32, r);
                             tmem_ld_wait();
+                            if (BIAS) kl_add_bias(r, s_d + s * 128 + 64 * part + 32 * q2, xfloor);
                             uint32_t gt, eq;
                             if (wide_pair) kl_compare_window<true>(r, scl, cadd, aw, t2, gt, eq);
                             else kl_compare_window<false>(r, scl, cadd_e, 0, t2, gt, eq);

@@ -377,7 +377,7 @@ def pruned_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, mx_specs
     ``key_bias``: PixArt cross-attention's additive text mask (MX_transformer_block.py:794-803,
     821-822), any fp32 tensor (also with 16-bit q, k, v) with B * Nk elements laid out (B, ..., Nk) - e.g. the reference's
     (B,1,1,S) attention_mask; it is added to the true AND the predicted scores.  Nq may differ
-    from Nk (Nk <= 256 with a bias).
+    from Nk; with pred_mode "ex_pred" a bias takes every Nk up to 8192, the other modes keep Nk <= 256.
     """
     sp = resolve_specs(mx_specs)
     lib = _lib.load()
